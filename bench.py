@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — pivots/sec + tableau-update HBM GB/s on the BASELINE.json workload.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config.workload): cfg4 of BASELINE.json — the dense 16384 x 32768 fp64 LP
 D(16384, 32768, seed 0) of SURVEY.md §8d.  One *step* = PIVOTS_PER_STEP (1000) consecutive
@@ -50,6 +50,7 @@ if ROOT not in sys.path:
 
 N_ROWS, M_COLS, SEED = 16384, 32768, 0
 PIVOTS_PER_STEP = 1000
+DUMP_SAMPLE_CELLS = 1 << 20        # body cells --dump-outputs samples (the cfg4 body is 4.3 GB)
 METRIC = "pivots/sec (16k x 32k fp64 tableau)"
 UNIT = "pivots/s"
 GOLDEN = os.path.join(ROOT, "tests", "golden")
@@ -354,6 +355,28 @@ def cpu_baseline_sample(rows, c, gold, budget_s=20.0):
     return {"value": timed / t_used, "unit": UNIT, "cores": threads, "kind": "port",
             "sample": f"first {timed} pivots (after 1 untimed) of the same 16384x32768 tableau, "
                       f"oracle/spx_oracle.c with OpenMP on {threads} threads"}
+
+
+def dump_outputs(out_dir, tab, status, npiv, last_step):
+    """--dump-outputs: what a caller of the timed loop holds after its last step, one float64 .npy per array: the
+    step's pivots, the b column, the f row, x / objective / labels (DeviceTableau.solution()) and a fixed seeded sample
+    of the body cells with their row-major indices.  The inputs are seeded, so two builds run with the same arguments
+    can be compared file for file."""
+    import torch
+    n, m = tab.n, tab.m
+    cur = tab.cur(npiv)
+    sol = tab.solution(status, npiv)
+    index = np.unique(np.random.default_rng(SEED).integers(0, n * m, DUMP_SAMPLE_CELLS))
+    r, c = np.divmod(index, m)
+    sample = tab.A[cur].view(-1)[torch.from_numpy(r * tab.ld + c).to(tab.device)]
+    arrays = {"status": [status, npiv], "trace": sol.trace[max(0, npiv - last_step): npiv],
+              "b": tab.b[cur, :n], "f_row": tab.A[cur, n, :m], "x": sol.x, "objective": [sol.obj2, sol.objective],
+              "row_labels": sol.rowlab, "column_labels": sol.collab, "body_sample_index": index, "body_sample": sample}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if isinstance(a, torch.Tensor) else a
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+    return sorted(arrays)
 
 
 def batched_leg(dev, rank, world, dist=None, reps=20, B=65536, golden=True):
@@ -668,6 +691,9 @@ def run_ours(args):
             torch.cuda.synchronize()
         launches = int(N.load().spx_launch_count(0))
         total_ms = ev0.elapsed_time(ev1)
+        if args.dump_outputs:                             # before the checks, so a diverging build is dumped too
+            names = dump_outputs(args.dump_outputs, tab, st, npiv, P)
+            log(f"[rank {rank}] wrote {', '.join(names)} (.npy) to {args.dump_outputs}")
         assert npiv == need and st == N.PIVOT, (st, npiv)
         tr = tab.trace[:need].cpu().numpy()
 
@@ -1047,7 +1073,12 @@ def main():
     ap.add_argument("--max-connections", type=int, default=0,
                     help="CUDA_DEVICE_MAX_CONNECTIONS for this process (hardware work queues the streams share; the CUDA "
                          "default is 8); 0 = leave the environment alone.  Must be set before CUDA initialises.")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last step computed to DIR/<name>.npy (float64): its "
+                         "pivots, b, the f row, x, objective, labels and a seeded sample of the body cells")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1):
+        ap.error("--dump-outputs covers the single-GPU timed loop (--impl ours --gpus 1)")
     if args.max_connections > 0:
         os.environ["CUDA_DEVICE_MAX_CONNECTIONS"] = str(args.max_connections)
     if args.warmup < 3 and args.impl == "ours":

@@ -1,11 +1,11 @@
 #!/usr/bin/env python
 """Generate the golden fixtures in tests/golden/ by RUNNING THE REFERENCE.
 
-Run in the build container (where /root/reference exists):
+Run with $SIMPLEX_REF pointing at the original project's src/ directory:
 
-    python tests/golden/make_golden.py [small] [cfg2] [cfg3] [cfg5] [cfg4]
+    SIMPLEX_REF=<original project>/src python tests/golden/make_golden.py [small] [cfg2] [cfg3] [cfg5] [cfg4]
 
-The reference's solver (/root/reference/src/simplex.py) is stdlib-only, so it is
+The reference's solver (its src/simplex.py) is stdlib-only, so it is
 imported and driven with its own pick_element() / recalculate_matrix() /
 get_solution().  Every fixture records its provenance:
 
@@ -14,7 +14,8 @@ get_solution().  Every fixture records its provenance:
                 reference cannot reach), which tests/test_oracle.py checks
                 bit-for-bit against every "reference" fixture.
 
-The GPU box has no /root/reference; tests there read only these JSON files.
+The reference's sources are not part of this repository; the tests read only
+these JSON files (and the reference too where $SIMPLEX_REF is set).
 Floats are stored as float.hex() strings so fixtures are bit-exact.
 """
 from __future__ import annotations
@@ -31,7 +32,9 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF_SRC = os.environ.get("SIMPLEX_REF", "/root/reference/src")
+REF_SRC = os.environ.get("SIMPLEX_REF", "")
+if not REF_SRC:
+    raise SystemExit("set SIMPLEX_REF to the original project's src/ directory")
 sys.path.insert(0, REF_SRC)
 
 import simplex as ref  # noqa: E402  (the reference)

@@ -1,6 +1,7 @@
 """CPU (gloo, world 2) tests of bench.py's multi-GPU bookkeeping — the parts that deadlocked or crashed on real GPUs
 before they were covered here: the "late"-LP preflight (trace + b + f + body checksum against the oracle golden, with the
-same collectives on every rank whatever happens on one of them) and the int64 transport of unsigned checksums."""
+same collectives on every rank whatever happens on one of them) and the int64 transport of unsigned checksums; on a GPU,
+the arrays --dump-outputs writes."""
 import os
 import socket
 import sys
@@ -92,6 +93,38 @@ def test_late_lp_preflight_under_gloo(fail_rank):
     else:
         assert [g[1] for g in got] == [False, False]
         assert "injected failure" in got[fail_rank][3]
+
+
+@pytest.mark.gpu
+def test_dump_outputs_equal_the_oracle(tmp_path):
+    """bench.py --dump-outputs on a small tableau: every array it writes is float64 and equals, bit for bit, what the
+    oracle holds after the same pivots."""
+    if not torch.cuda.is_available():
+        pytest.skip("needs a CUDA device")
+    import bench
+    import oracle
+    from simplex_method_solver_b200 import workloads as W
+    from simplex_method_solver_b200.engine import DeviceTableau
+    n, m, k, step = 96, 700, 40, 16
+    rows, c = W.dense_lp(n, m, seed=3)
+    tab = DeviceTableau(n, m, device="cuda:0", trace_capacity=k + 64)
+    tab.load(rows, c, max_pivots=k + 64)
+    st, npiv = tab.solve(chunk=step, stop_after=k)
+    assert npiv == k
+    bench.dump_outputs(str(tmp_path / "out"), tab, st, npiv, step)
+    got = {p.stem: np.load(p) for p in (tmp_path / "out").glob("*.npy")}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert sum(a.nbytes for a in got.values()) < 64 << 20
+    o = oracle.solve(rows, c, max_pivots=k)
+    body = o.table[: n * (m + 1)].reshape(n, m + 1)
+    assert got["status"].tolist() == [st, k]
+    assert got["trace"].tolist() == o.trace[k - step:].tolist()
+    assert got["b"].tobytes() == body[:, m].tobytes() and got["f_row"].tobytes() == o.table[n * (m + 1):].tobytes()
+    idx = got["body_sample_index"].astype(np.int64)
+    assert (np.diff(idx) > 0).all() and idx[-1] < n * m
+    assert got["body_sample"].tobytes() == body[:, :m].reshape(-1)[idx].tobytes()
+    assert got["x"].tobytes() == o.x.tobytes() and got["objective"].tobytes() == np.array([o.obj2, o.objm]).tobytes()
+    assert got["row_labels"].tolist() == o.rowlab.tolist() and got["column_labels"].tolist() == o.collab.tolist()
 
 
 def test_price_engine_choice():

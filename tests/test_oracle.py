@@ -1,16 +1,20 @@
 """CPU tests of the oracle (oracle/spx_oracle.c): it must reproduce every golden vector that
-tests/golden/make_golden.py recorded from the live reference (/root/reference/src/simplex.py)
-and, when the reference sources are present (build container only), the reference itself on
-fresh random LPs.  Bit-exact: pivot sequences, labels and every fp64 cell.
+tests/golden/make_golden.py recorded from the original project's src/simplex.py, the record of
+tests/golden/fresh_cases.json on further seeded LPs and, where $SIMPLEX_REF points at the
+original's sources, the original itself on those LPs.  Bit-exact: pivot sequences, labels and
+every fp64 cell.
 """
 import hashlib
+import json
+import os
 
 import numpy as np
 import pytest
 
 import oracle
 from simplex_method_solver_b200 import workloads as W
-from util import END_TO_STATUS, bits, case_inputs, flat_of, label_codes, table_sha, unhex
+from util import (END_TO_STATUS, FRESH_SHARDED_LPS, bits, case_inputs, drive_reference, flat_of, fresh_dantzig_lps,
+                  fresh_lps, label_codes, make_lp, table_sha, unhex)
 
 
 def test_oracle_builds_and_reports_threads():
@@ -117,88 +121,77 @@ def test_cfg4_generator_digest_small_sibling(cfg_digests):
     assert np.array_equal(rows, np.hstack([A, b[:, None]])) and np.array_equal(c, cc)
 
 
-# --------------------------------------------------------------------------- live reference
-def _drive_reference(ref, rows, c, cap):
-    """The driving pattern of simplex.py:261-269 (no Info accumulation)."""
-    sm = ref.SimplexMethod([list(map(float, r)) for r in rows], [float(v) for v in c])
-    trace = []
-    end = "cap"
-    while len(trace) < cap:
-        try:
-            ok, i, j, _e = sm.pick_element()
-        except ValueError as e:
-            end = str(e)
-            break
-        if not ok:
-            end = "optimal"
-            break
-        trace.append([i, j])
-        sm.recalculate_matrix()
-    else:
-        # cap reached: is the next pick terminal?  (the oracle reports CAP only on a real pivot)
-        try:
-            ok, *_ = sm.pick_element()
-            end = "cap" if ok else "optimal"
-        except ValueError as e:
-            end = str(e)
-    flat = np.asarray([v for row in sm.table for v in row], dtype=np.float64)
-    return end, trace, flat, sm.row, sm.column
+# --------------------------------------------------------------------------- fresh LPs: stored record + live reference
+@pytest.fixture(scope="module")
+def fresh_cases():
+    """tests/golden/fresh_cases.json (made by tests/golden/make_fresh_cases.py; its "provenance" says whether the
+    original's simplex.py or the oracle computed it)."""
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "fresh_cases.json")) as fh:
+        return json.load(fh)
+
+
+def _assert_recorded(o, rec, m, what):
+    assert o.status == END_TO_STATUS[rec["end"]], what
+    assert o.trace.tolist() == rec["trace"], what
+    assert table_sha(o.table) == rec["table_sha256"], what
+    if "row_labels" in rec:
+        assert oracle.label_strings(o.rowlab, o.collab, m) == (rec["row_labels"], rec["column_labels"]), what
+
+
+def _assert_live(o, ref, rows, c, cap, what):
+    end, trace, flat, rl, cl = drive_reference(ref, rows, c, cap)
+    assert o.status == END_TO_STATUS[end], what
+    assert o.trace.tolist() == trace, what
+    assert np.array_equal(bits(o.table), bits(flat)), what
+    assert oracle.label_strings(o.rowlab, o.collab, rows.shape[1] - 1) == (rl, cl), what
 
 
 @pytest.mark.parametrize("family", ["gui2dp", "smallint", "dense"])
-def test_oracle_equals_live_reference(reference_module, family):
-    """Fresh random LPs (not the committed goldens) through the reference itself."""
-    rng = np.random.default_rng({"gui2dp": 11, "smallint": 12, "dense": 13}[family])
-    for t in range(150):
-        n, m = int(rng.integers(1, 10)), int(rng.integers(2, 7))
-        if family == "gui2dp":
-            A = np.round(rng.uniform(-50, 50, (n, m)), 2)
-            b = np.round(rng.uniform(-500, 2000, n), 2)
-            c = np.round(rng.uniform(-3, 3, m), 2)
-        elif family == "smallint":
-            A = rng.integers(-3, 4, (n, m)).astype(float)
-            b = rng.integers(-2, 7, n).astype(float)
-            c = rng.integers(-3, 4, m).astype(float)
-        else:
-            A = -rng.uniform(0.1, 1.0, (n, m)); b = rng.uniform(1.0, 2.0, n); c = -rng.uniform(0.1, 1.0, m)
-        rows = np.hstack([A, b[:, None]])
-        end, trace, flat, rl, cl = _drive_reference(reference_module, rows, c, 60)
+def test_oracle_equals_live_reference(reference_module, fresh_cases, family):
+    """Fresh seeded LPs (not those of reference_cases.json): the oracle against the stored record and, where
+    $SIMPLEX_REF is set, against the original's simplex.py itself."""
+    recs = fresh_cases["families"][family]
+    assert len(recs) == 150
+    for t, (rows, c) in enumerate(fresh_lps(family)):
         o = oracle.solve(rows, c, max_pivots=60)
-        assert o.status == END_TO_STATUS[end], (family, t)
-        assert o.trace.tolist() == trace, (family, t)
-        assert np.array_equal(bits(o.table), bits(flat)), (family, t)
-        assert oracle.label_strings(o.rowlab, o.collab, m) == (rl, cl), (family, t)
+        _assert_recorded(o, recs[t], rows.shape[1] - 1, (family, t))
+        if reference_module is not None:
+            _assert_live(o, reference_module, rows, c, 60, (family, t))
 
 
-def test_oracle_pick_update_equal_live_reference_medium(reference_module):
-    """One 60 x 90 dense LP, 25 pivots, every cell after every pivot."""
-    rows, c = W.dense_lp(60, 90, 5)
-    sm = reference_module.SimplexMethod(rows.tolist(), c.tolist())
+def test_oracle_pick_update_equal_live_reference_medium(reference_module, fresh_cases):
+    """One 60 x 90 dense LP, 25 pivots: every pick (row, column, pivot element) and the whole table after every
+    pivot, against the stored record and, where $SIMPLEX_REF is set, against the original's every cell."""
+    g = fresh_cases["medium"]
+    rows, c = W.dense_lp(g["n"], g["m"], g["seed"])
+    assert len(g["pivots"]) == 25
+    sm = reference_module.SimplexMethod(rows.tolist(), c.tolist()) if reference_module is not None else None
     T = flat_of(rows, c)
-    for _ in range(25):
-        ok, i, j, e = sm.pick_element()
+    for k, (i, j, e_hex, sha) in enumerate(g["pivots"]):
         st, r, cc, ee = oracle.pick(T, 60, 90)
-        assert ok and st == oracle.PIVOT and (i, j, e) == (r, cc, ee)
-        sm.recalculate_matrix()
+        assert st == oracle.PIVOT and (r, cc, float(ee).hex()) == (i, j, e_hex), k
         T = oracle.update(T, 60, 90, r, cc)
-        got = np.asarray([v for row in sm.table for v in row])
-        assert np.array_equal(bits(got), bits(T))
+        assert table_sha(T) == sha, k
+        if sm is not None:
+            ok, i, j, e = sm.pick_element()
+            assert ok and (i, j, e) == (r, cc, ee)
+            sm.recalculate_matrix()
+            got = np.asarray([v for row in sm.table for v in row])
+            assert np.array_equal(bits(got), bits(T))
 
 
-@pytest.mark.parametrize("n,m,cap,kind", [(24, 200, 40, "late"), (40, 400, 64, "late"), (20, 160, 30, "late"),
-                                          (12, 300, 30, "smallint")])
-def test_oracle_equals_live_reference_on_the_sharded_test_lps(reference_module, n, m, cap, kind):
+@pytest.mark.parametrize("n,m,cap,kind", FRESH_SHARDED_LPS)
+def test_oracle_equals_live_reference_on_the_sharded_test_lps(reference_module, fresh_cases, n, m, cap, kind):
     """The LP families the sharded-flow tests use (util.make_lp: entering column on the LAST column block and
-    moving between blocks; degenerate small integers) through the reference itself, so the oracle those tests
-    compare against is pinned on exactly this kind of input too."""
-    from util import make_lp
+    moving between blocks; degenerate small integers), against the stored record and, where $SIMPLEX_REF is set, the
+    original's simplex.py, so the oracle those tests compare against is pinned on exactly this kind of input too."""
+    rec = next(r for r in fresh_cases["sharded"] if (r["n"], r["m"], r["cap"], r["kind"]) == (n, m, cap, kind))
     rows, c = make_lp(n, m, 7, kind)
-    end, trace, flat, rl, cl = _drive_reference(reference_module, rows, c, cap)
     o = oracle.solve(rows, c, max_pivots=cap)
-    assert o.status == END_TO_STATUS[end]
-    assert o.trace.tolist() == trace and len(trace) >= 10
-    assert np.array_equal(bits(o.table), bits(flat))
-    assert oracle.label_strings(o.rowlab, o.collab, m) == (rl, cl)
+    assert len(rec["trace"]) >= 10
+    _assert_recorded(o, rec, m, (n, m, kind))
+    if reference_module is not None:
+        _assert_live(o, reference_module, rows, c, cap, (n, m, kind))
 
 
 def test_golden_file_provenance(ref_cases):
@@ -279,30 +272,25 @@ def test_dantzig_rule_golden_cases(dantzig_cases):
     assert differs >= 30                      # the rule really is a different rule on these LPs
 
 
-def test_dantzig_rule_equals_reference_driven_by_column_swap(reference_module):
-    """Fresh LPs (not in the fixtures) through the live reference under the extension rule."""
-    import importlib.util
-    import os
-    spec = importlib.util.spec_from_file_location(
-        "make_golden", os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "make_golden.py"))
-    mg = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mg)
-    rng = np.random.default_rng(77)
-    for t in range(90):
-        n, m = int(rng.integers(1, 12)), int(rng.integers(2, 9))
-        if t % 3 == 0:
-            A, b, c = (np.round(rng.uniform(-50, 50, (n, m)), 2), np.round(rng.uniform(-500, 2000, n), 2),
-                       np.round(rng.uniform(-3, 3, m), 2))
-        elif t % 3 == 1:
-            A, b, c = (rng.integers(-3, 4, (n, m)).astype(float), rng.integers(-2, 7, n).astype(float),
-                       rng.integers(-3, 4, m).astype(float))
-        else:
-            A, b, c = -rng.uniform(0.1, 1, (n, m)), rng.uniform(1, 2, n), -rng.uniform(0.1, 1, m)
-        rows = np.hstack([A, b[:, None]])
-        sm, trace, end, _ = mg.drive_dantzig(rows.tolist(), c.tolist(), 150)
+def test_dantzig_rule_equals_reference_driven_by_column_swap(reference_module, fresh_cases):
+    """Fresh LPs (not in the fixtures) under the extension rule: the oracle against the stored record and, where
+    $SIMPLEX_REF is set, against the original driven by make_golden.py's column swap."""
+    recs = fresh_cases["dantzig"]
+    assert len(recs) == 90
+    mg = None
+    if reference_module is not None:
+        import importlib.util
+        spec = importlib.util.spec_from_file_location(
+            "make_golden", os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "make_golden.py"))
+        mg = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(mg)
+    for t, (rows, c) in enumerate(fresh_dantzig_lps()):
         o = oracle.solve(rows, c, max_pivots=150, rule="dantzig")
-        assert o.status == END_TO_STATUS[end] and o.trace.tolist() == trace, t
-        assert table_sha(o.table) == mg.table_sha(sm.table), t
+        _assert_recorded(o, recs[t], rows.shape[1] - 1, t)
+        if mg is not None:
+            sm, trace, end, _ = mg.drive_dantzig(rows.tolist(), c.tolist(), 150)
+            assert o.status == END_TO_STATUS[end] and o.trace.tolist() == trace, t
+            assert table_sha(o.table) == mg.table_sha(sm.table), t
 
 
 # --------------------------------------------------------------------------- fixtures bench.py asserts at run time
