@@ -44,7 +44,7 @@
 extern "C" {
 #endif
 
-#define SPX_ABI_VERSION 4
+#define SPX_ABI_VERSION 5
 
 /* status codes == the outcomes of pick_element(), simplex.py:70-141 */
 #define SPX_PIVOT       1   /* (True, r, c, e)                                   :91,:141 */
@@ -107,6 +107,7 @@ int64_t     spx_launch_count(int reset);
 #define SPX_OPT_SHARD_CTAS       14 /* sharded / look-ahead pricing kernel: at most this many CTAs (0 = one per SM) */
 #define SPX_OPT_RESIDENT_VARIANT 15 /* L2-resident persistent loop: 0 default (price, sweep, one grid barrier per pivot), 1 = look-ahead pricing inside the CTA with the sweep rows prefetched by cp.async (bit-identical; measured slower on cfg2, kept selectable) */
 #define SPX_OPT_FUSE_PAIRS       12 /* fused update kernel: column pairs per lane, i.e. strip width / 64 (0 = default 2; 1 or 2) */
+#define SPX_OPT_CLUSTER_SIZE     16 /* K7 (spx_solve_batched_cluster): CTAs per LP, 1, 2, 4, 8 or 16 (0 = default: spx_cluster_size(n, m)); a size whose footprint does not fit is rejected */
 int         spx_set_option(int32_t option, int64_t value);
 int64_t     spx_get_option(int32_t option);
 /* Device self-test of the hoisted-reciprocal division used by K3 against the
@@ -228,6 +229,31 @@ int spx_solve_batched(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule
                       int32_t *d_rowlab, int32_t *d_collab,
                       int32_t *d_trace, double *d_snap, void *stream);
 int64_t spx_batched_max_cells(void);
+
+/* ---- K7: batches of independent mid-size LPs, one thread-block cluster per LP -- */
+/* The whole loop of get_solution(), simplex.py:179-199 (pick_element :70-141 and
+ * recalculate_matrix :143-177 inlined), for tables above spx_batched_max_cells():
+ * a cluster of S CTAs solves one LP with its table in their shared memory, CTA k
+ * holding body rows [k*R, k*R+R), R = ceil(n/S), and a copy of the f row; the pivot
+ * row travels over distributed shared memory, two cluster barriers per pivot.
+ * Arguments, outputs and results are those of spx_solve_batched, bit for bit
+ * (labels start at x1..xm / y1..yn, :30-31; final tables in place in d_T; d_snap
+ * slot k = the table before pivot k, :181,198; d_obj as :49).
+ * Capacity: with Q = ceil(m/S), one CTA needs
+ *     8*(R*(m+2) + 2*m + 1) + 4*(R + Q)  <=  230400 bytes
+ * for some S in {1, 2, 4, 8, 16} (e.g. D(100,100): S = 1, D(128,256): 2,
+ * D(256,512): 8, D(512,800): 16; n <= 528 at m = 800; m <= 9499).  Shape, rule, B and the non-null
+ * outputs are checked before the device is touched; a device that cannot
+ * co-schedule one cluster of S CTAs is an error, not a fall-back. */
+int spx_solve_batched_cluster(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule,
+                              int32_t max_pivots, double *d_x, double *d_obj,
+                              int32_t *d_status, int32_t *d_npiv,
+                              int32_t *d_rowlab, int32_t *d_collab,
+                              int32_t *d_trace, double *d_snap, void *stream);
+/* Host only (no device): the smallest S in {1, 2, 4, 8, 16} whose footprint above
+ * fits, i.e. the cluster size K7 uses for an n x m LP unless SPX_OPT_CLUSTER_SIZE
+ * forces one; 0 when the LP does not fit one cluster. */
+int32_t spx_cluster_size(int32_t n, int32_t m);
 
 /* ---- column-sharded large tableau (one process per GPU) ------------------- */
 /* Rank g owns global columns [col0, col0+m_loc) of the body as a local split

@@ -47,6 +47,10 @@ cudaError_t lazy_guard_selftest(const double *, const double *, const double *, 
 cudaError_t init_state(spx_state *, int32_t *, int32_t *, int, int, int64_t, cudaStream_t);
 cudaError_t solve_batched(double *, int64_t, int, int, int, int, double *, double *, int32_t *,
                           int32_t *, int32_t *, int32_t *, int32_t *, double *, cudaStream_t);
+int cluster_size(int64_t, int64_t);
+int cluster_size_for_solve(int64_t, int64_t);
+cudaError_t solve_batched_cluster(double *, int64_t, int, int, int, int, int, double *, double *, int32_t *,
+                                  int32_t *, int32_t *, int32_t *, int32_t *, double *, cudaStream_t);
 } // namespace spx_launch
 
 namespace spx_host {
@@ -526,6 +530,35 @@ int spx_solve_batched(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule
     cudaError_t e = spx_launch::solve_batched(d_T, B, n, m, rule, max_pivots, d_x, d_obj, d_status, d_npiv,
                                               d_rowlab, d_collab, d_trace, d_snap, as_stream(stream));
     return check(e, "batched launch");
+}
+
+// ---- K7 -------------------------------------------------------------------------
+int32_t spx_cluster_size(int32_t n, int32_t m) { return spx_launch::cluster_size(n, m); }
+
+int spx_solve_batched_cluster(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule, int32_t max_pivots,
+                              double *d_x, double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab,
+                              int32_t *d_collab, int32_t *d_trace, double *d_snap, void *stream) {
+    SPX_REQUIRE(B >= 0 && n >= 1 && m >= 1 && max_pivots >= 0, "spx_solve_batched_cluster: bad arguments");
+    SPX_REQUIRE(B == 0 || (d_T && d_status && d_npiv), "spx_solve_batched_cluster: null T/status/npiv");
+    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_solve_batched_cluster: unknown rule %d",
+                rule);
+    SPX_REQUIRE(spx_launch::cluster_size(n, m) > 0,
+                "spx_solve_batched_cluster: a %d x %d LP exceeds one cluster (16 CTAs of 227 KB shared memory: "
+                "8*(R*(m+2)+2m+1) + 4*(R+Q) <= 230400 bytes with R = ceil(n/16), Q = ceil(m/16))", n, m);
+    const int S = spx_launch::cluster_size_for_solve(n, m);
+    SPX_REQUIRE(S > 0, "spx_solve_batched_cluster: a %d x %d LP does not fit a cluster of SPX_OPT_CLUSTER_SIZE = %d CTAs",
+                n, m, (int)spx_launch::get_option(SPX_OPT_CLUSTER_SIZE));
+    SPX_REQUIRE(B <= INT32_MAX / S, "spx_solve_batched_cluster: B = %lld LPs x S = %d CTAs exceed one grid",
+                (long long)B, S);
+    const cudaError_t e = spx_launch::solve_batched_cluster(d_T, B, n, m, S, rule, max_pivots, d_x, d_obj, d_status,
+                                                            d_npiv, d_rowlab, d_collab, d_trace, d_snap,
+                                                            as_stream(stream));
+    if (e == cudaErrorInvalidClusterSize) {
+        set_error("spx_solve_batched_cluster: the device cannot co-schedule one cluster of S = %d CTAs for a %d x %d "
+                  "LP (cudaOccupancyMaxActiveClusters = 0)", S, n, m);
+        return -1;
+    }
+    return check(e, "cluster launch");
 }
 
 // ---- column-sharded flow ----------------------------------------------------------

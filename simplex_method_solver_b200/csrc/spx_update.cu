@@ -416,7 +416,7 @@ int64_t colbuf_doubles(int n) {
     return ((int64_t)n + 1 + UPD_TR_MAX - 1) / UPD_TR_MAX * UPD_TR_MAX + UPD_TR_MAX;
 }
 
-int64_t g_opt[16] = {0, 0, 4, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+int64_t g_opt[17] = {0, 0, 4, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
 
 // Rows per tile.  Measured on B200 (tools/upd_lab.py, profiles/r1c_update_variants.md): the smallest
 // tile — 8 rows = exactly one 8-deep load batch per thread, 4 CTAs (64 registers) per SM — is the
@@ -430,7 +430,7 @@ static int pick_tr(int n, int m_loc) {
 
 // process-wide tuning knobs (spx_set_option); every setting computes the same bits
 
-int64_t get_option(int key) { return (key >= 0 && key < 16) ? g_opt[key] : -1; }
+int64_t get_option(int key) { return (key >= 0 && key < 17) ? g_opt[key] : -1; }
 int set_option(int key, int64_t value) {
     switch (key) {
     case SPX_OPT_UPDATE_KERNEL:    if (value < 0 || value > 2) return -1; break;
@@ -448,6 +448,7 @@ int set_option(int key, int64_t value) {
     case SPX_OPT_SHARD_THREADS:    if (value < 0 || value > 512 || value % 32 || value == 32) return -1; break;
     case SPX_OPT_SHARD_CTAS:       if (value < 0 || value > 4096) return -1; break;
     case SPX_OPT_RESIDENT_VARIANT: if (value < 0 || value > 1) return -1; break;
+    case SPX_OPT_CLUSTER_SIZE:     if (value < 0 || value > 16 || (value & (value - 1))) return -1; break;
     default: return -1;
     }
     g_opt[key] = value;

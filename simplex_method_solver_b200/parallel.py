@@ -644,11 +644,12 @@ class PeerShardedTableau(ShardedTableau):
 
 def solve_batched_sharded(tables: np.ndarray, n: int, m: int, max_pivots: int = 64, rule: str = "reference",
                           rank: Optional[int] = None, world: Optional[int] = None, device=None,
-                          solver=None):
+                          solver=None, engine: str = "auto"):
     """Each rank solves its contiguous share of the batch; no collective on the data path.
 
     Returns (start, count, BatchResult) for this rank.  `solver` defaults to the CUDA
-    ``solve_batched``; tests pass a stand-in.
+    ``solve_batched``; tests pass a stand-in.  `engine` is passed on to ``solve_batched``
+    (and to a stand-in only when it is not "auto").
     """
     if rank is None:
         rank = dist.get_rank() if dist.is_initialized() else 0
@@ -657,5 +658,6 @@ def solve_batched_sharded(tables: np.ndarray, n: int, m: int, max_pivots: int = 
     start, count = shard_range(tables.shape[0], rank, world)
     if solver is None:
         from .batched import solve_batched as solver
-    res = solver(tables[start:start + count], n, m, max_pivots=max_pivots, rule=rule, device=device)
+    kw = {} if engine == "auto" else {"engine": engine}
+    res = solver(tables[start:start + count], n, m, max_pivots=max_pivots, rule=rule, device=device, **kw)
     return start, count, res

@@ -19,6 +19,11 @@ Differences from the reference, all opt-in or unavoidable:
     large tableaus need no list-of-lists; inputs are never mutated.
   * ``solve()`` returns the trace / x / objective without per-pivot snapshots,
     which the reference cannot avoid (it deep-copies the table per pivot, :198).
+  * ``engine="cluster"``: ``get_solution()`` runs the whole loop in the batched
+    cluster kernel (K7, one thread-block cluster of up to 16 CTAs holds the
+    table in shared memory), which writes the per-pivot snapshots itself; for
+    LPs above the one-CTA limit of ``engine="warp"``.  ``solve()`` keeps the
+    streaming loop, as with ``"warp"``.
   * ``engine="sharded"``: one process per GPU (torchrun); every rank constructs
     the same ``SimplexMethod`` and calls ``solve()`` — the body is split into
     column blocks over the ranks of ``group`` (the default process group) and
@@ -35,7 +40,7 @@ import numpy as np
 import torch
 
 from . import _native as N
-from .batched import DeviceBatch
+from .batched import DeviceBatch, kernel_for
 from .engine import DeviceTableau, Solution, as_rows_function
 
 CAP_TEXT = "pivot limit reached"
@@ -86,7 +91,7 @@ class SimplexMethod:
         self.column = ['y' + str(k) for k in range(1, self.n + 1)] + ['f']    # :31,:33
         if rule not in N.RULES:
             raise ValueError(f"unknown rule {rule!r}")
-        if engine not in ("auto", "warp", "stream", "sharded"):
+        if engine not in ("auto", "warp", "stream", "sharded", "cluster"):
             raise ValueError(f"unknown engine {engine!r}")
         self._rule = N.RULES[rule]
         self._engine = engine
@@ -229,6 +234,9 @@ class SimplexMethod:
     def _use_warp(self):
         if self._engine == "stream":
             return False
+        if self._engine == "cluster":
+            kernel_for(self.n, self.m, "cluster")        # ValueError above the cluster capacity
+            return True
         cells = self.n * (self.m + 1) + self.m
         fits = cells <= N.load().spx_batched_max_cells()
         if self._engine == "warp" and not fits:
@@ -274,13 +282,15 @@ class SimplexMethod:
                            None, None, x1, x2, self.f(x1, x2)))   # :197-198
 
     def _solve_warp(self, result, budget, snapshots):
-        """Whole loop in one warp-resident kernel launch per round of `cap` pivots."""
+        """Whole loop in one shared-memory-resident kernel launch (K4, or K7 with engine="cluster")
+        per round of `cap` pivots."""
         n, m = self.n, self.m
+        engine = "cluster" if self._engine == "cluster" else "smem"
         cap = 64
         while True:
             cap = min(cap, max(budget, 0))
             db = DeviceBatch(1, n, m, max_pivots=cap, trace=True, snapshots=True,
-                             device=self._dev.device)
+                             device=self._dev.device, engine=engine)
             self._dev.export_device_flat(self._npiv, db.T[0])
             db.run(self._rule)
             res = db.result()

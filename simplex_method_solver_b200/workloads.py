@@ -31,6 +31,23 @@ def dense_lp(n: int, m: int, seed: int = 0):
     return rows, c
 
 
+def phase1_lp(n: int, m: int, seed: int = 0):
+    """D(n, m, seed) pushed into phase 1: a tenth of the rows (at least one) get a negated and
+    b = -b * U(0.05, 0.2) (origin infeasible, simplex.py:72-91), and 5 % of the a cells are exact zeros.
+    Ends OPTIMAL after a few hundred to a few thousand pivots at the sizes of tools/cluster_bench.py.
+
+    Returns (rows [n, m+1] fp64, c [m] fp64).
+    """
+    rows, c = dense_lp(n, m, seed)
+    g = np.random.default_rng([seed, 1])
+    idx = g.choice(n, max(1, n // 10), replace=False)
+    rows[idx, :m] = -rows[idx, :m]
+    rows[idx, m] = -rows[idx, m] * g.uniform(0.05, 0.2, idx.shape[0])
+    body = rows[:, :m]
+    body[g.random((n, m)) < 0.05] = 0.0
+    return rows, c
+
+
 def gui_batch(B: int, seed: int = 0):
     """P(B, seed): GUI-like 8-constraint / 2-variable LPs (cfg3: B=65536).
 
