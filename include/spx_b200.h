@@ -44,7 +44,7 @@
 extern "C" {
 #endif
 
-#define SPX_ABI_VERSION 5
+#define SPX_ABI_VERSION 6
 
 /* status codes == the outcomes of pick_element(), simplex.py:70-141 */
 #define SPX_PIVOT       1   /* (True, r, c, e)                                   :91,:141 */
@@ -254,6 +254,44 @@ int spx_solve_batched_cluster(double *d_T, int64_t B, int32_t n, int32_t m, int3
  * fits, i.e. the cluster size K7 uses for an n x m LP unless SPX_OPT_CLUSTER_SIZE
  * forces one; 0 when the LP does not fit one cluster. */
 int32_t spx_cluster_size(int32_t n, int32_t m);
+
+/* ---- ragged batches: LPs of any mix of shapes in one call (K4 and K7) ----------- */
+/* Each LP k has its own shape (n_k, m_k) and its own cap max_pivots_k.  Every buffer
+ * is packed in batch order: LP k's slice starts at the prefix sum over LPs 0..k-1 of
+ *     d_T, d_snap-table   cells          d_x, d_rowlab   m
+ *     d_collab            n              d_trace         max_pivots (pairs of int32)
+ *     d_snap              (max_pivots+1)*cells
+ * and d_obj, d_status, d_npiv hold one element per LP.  Each LP's results are those
+ * of spx_solve_batched / spx_solve_batched_cluster for that LP alone, bit for bit.
+ *
+ * Routing: SPX_ENGINE_AUTO sends an LP to K4 when cells <= spx_batched_max_cells(),
+ * else to K7 (at spx_cluster_size(n, m), or SPX_OPT_CLUSTER_SIZE when set); SMEM and
+ * CLUSTER send every LP to that engine.  One solve makes at most 7 launches, in
+ * sequence on `stream`: K4 warp mode (LPs of <= 96 cells) if any, K4 CTA mode if any,
+ * one K7 launch per distinct cluster size.  Within a launch the LPs run largest first
+ * (by cells, ties by batch index). */
+#define SPX_ENGINE_AUTO    0
+#define SPX_ENGINE_SMEM    1
+#define SPX_ENGINE_CLUSTER 2
+/* bytes of the plan of a batch of B LPs (-1 when B < 0) */
+int64_t spx_ragged_plan_bytes(int64_t B);
+/* Host only, no device.  h_shapes[B][3] = {n, m, max_pivots} in batch order.  Validates
+ * every LP (the error text names the first bad LP's index and the capacity it exceeds),
+ * reads SPX_OPT_CLUSTER_SIZE, and writes into h_plan (plan_bytes >= spx_ragged_plan_bytes(B))
+ * the per-LP descriptors (shape and offsets above) and the launch list (kernel, cluster
+ * size, block size, dynamic shared memory, the LP indices largest first).
+ * h_totals[5] = the packed lengths of T, x (= rowlab), collab, trace (pairs) and snap. */
+int spx_ragged_plan(const int32_t *h_shapes, int64_t B, int32_t engine, void *h_plan, int64_t plan_bytes,
+                    int64_t *h_totals);
+/* Solves the batch h_plan describes.  d_plan is a byte copy of h_plan in device memory,
+ * made by the caller (nothing allocates behind the caller's back and there is no hidden
+ * synchronising copy).  The launches are read from h_plan, the descriptors from d_plan.
+ * Plan header, rule and pointers are checked before the device is touched; a plan of
+ * B = 0 returns 0.  Outputs and NULL conventions as spx_solve_batched. */
+int spx_solve_batched_ragged(double *d_T, const void *h_plan, const void *d_plan, int32_t rule,
+                             double *d_x, double *d_obj, int32_t *d_status, int32_t *d_npiv,
+                             int32_t *d_rowlab, int32_t *d_collab, int32_t *d_trace, double *d_snap,
+                             void *stream);
 
 /* ---- column-sharded large tableau (one process per GPU) ------------------- */
 /* Rank g owns global columns [col0, col0+m_loc) of the body as a local split

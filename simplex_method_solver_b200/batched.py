@@ -1,4 +1,5 @@
-"""Batches of independent LPs of one shape, each solved whole inside one kernel.
+"""Batches of independent LPs, each solved whole inside one kernel: of one shape (``solve_batched``,
+``DeviceBatch``) or of any mix of shapes (``solve_ragged``, ``DeviceRaggedBatch``).
 
 Each LP is the reference's whole get_solution() loop
 (/root/reference/src/simplex.py:179-199) with its tableau in shared memory:
@@ -9,10 +10,14 @@ Each LP is the reference's whole get_solution() loop
 ``engine="auto"`` takes K4 for every shape K4 accepts and K7 above that.  Both
 compute the same bits.  LPs never communicate, so a batch splits over GPUs by
 contiguous ranges with no collective (see parallel.shard_range).
+
+A ragged batch is packed in batch order (LP k's table, x, labels, trace and snapshots
+start at prefix sums over LPs 0..k-1, see include/spx_b200.h) and solved by one plan of
+at most seven launches: K4 warp mode, K4 CTA mode, one K7 launch per cluster size.
 """
 from __future__ import annotations
 
-from typing import NamedTuple, Optional
+from typing import NamedTuple, Optional, Sequence, Union
 
 import numpy as np
 import torch
@@ -135,4 +140,197 @@ def solve_batched(tables, n: int, m: int, max_pivots: int = 64, rule: str = "ref
                            z((0, max_pivots + 1, db.cells)) if snapshots else None)
     db.upload(tables)
     db.run(N.RULES[rule])
+    return db.result()
+
+
+# ---------------------------------------------------------------------------- ragged batches
+ENGINE_CODES = {"auto": N.ENGINE_AUTO, "smem": N.ENGINE_SMEM, "cluster": N.ENGINE_CLUSTER}
+# the plan spx_ragged_plan writes (csrc/spx_common.cuh: RaggedPlan, RaggedLaunch, RaggedLp)
+_LAUNCH = np.dtype([("kernel", "<i4"), ("S", "<i4"), ("threads", "<i4"), ("per_cta", "<i4"), ("smem", "<i8"),
+                    ("first", "<i8"), ("count", "<i8"), ("slot_doubles", "<i8")])
+_HEADER = np.dtype([("magic", "<u4"), ("abi", "<i4"), ("B", "<i8"), ("engine", "<i4"), ("nlaunch", "<i4"),
+                    ("totals", "<i8", 5), ("lp_offset", "<i8"), ("order_offset", "<i8"), ("launch", _LAUNCH, 7)])
+_LP = np.dtype([("n", "<i4"), ("m", "<i4"), ("max_pivots", "<i4"), ("cells", "<i4"), ("t", "<i8"), ("xm", "<i8"),
+                ("xn", "<i8"), ("tr", "<i8"), ("sn", "<i8")])
+LAUNCH_KINDS = ("warp", "cta", "cluster")
+
+
+class RaggedPlan(NamedTuple):
+    plan: np.ndarray              # the plan bytes (uint8), as spx_ragged_plan wrote them
+    totals: np.ndarray            # [5] packed lengths: T, x (= rowlab), collab, trace pairs, snap
+    lps: np.ndarray               # [B] descriptors: n, m, max_pivots, cells and the offsets t, xm, xn, tr, sn
+    launches: list                # per launch: dict(kind, S, threads, smem, lps = LP indices in launch order)
+
+
+def ragged_plan(shapes, max_pivots, engine: str = "auto") -> RaggedPlan:
+    """Host only: the library's plan for LPs of `shapes` [B, 2] (n, m) with caps `max_pivots` [B]."""
+    if engine not in ENGINE_CODES:
+        raise ValueError(f"unknown engine {engine!r}; one of {ENGINES}")
+    L = N.load()
+    shapes = np.asarray(shapes, dtype=np.int64).reshape(-1, 2)
+    B = shapes.shape[0]
+    caps = np.broadcast_to(np.asarray(max_pivots, dtype=np.int64), (B,))
+    if not (np.all(np.abs(shapes) <= _INT32_MAX) and np.all(np.abs(caps) <= _INT32_MAX)):
+        raise ValueError("shapes and caps must fit int32")
+    h = np.ascontiguousarray(np.concatenate([shapes, caps[:, None]], axis=1), dtype=np.int32)
+    nbytes = int(L.spx_ragged_plan_bytes(B))
+    plan = np.zeros(max(nbytes, 16), dtype=np.uint8)
+    totals = np.zeros(5, dtype=np.int64)
+    rc = L.spx_ragged_plan(h.ctypes.data, B, ENGINE_CODES[engine], plan.ctypes.data, nbytes, totals.ctypes.data)
+    if rc != 0:
+        raise ValueError(L.spx_last_error().decode(errors="replace"))
+    hd = plan[: _HEADER.itemsize].view(_HEADER)[0]
+    lo, oo = int(hd["lp_offset"]), int(hd["order_offset"])
+    lps = plan[lo: lo + B * _LP.itemsize].view(_LP)
+    order = plan[oo: oo + 4 * B].view("<i4")
+    launches = []
+    for q in range(int(hd["nlaunch"])):
+        la = hd["launch"][q]
+        f, c = int(la["first"]), int(la["count"])
+        launches.append({"kind": LAUNCH_KINDS[int(la["kernel"])], "S": int(la["S"]), "threads": int(la["threads"]),
+                         "smem": int(la["smem"]), "lps": order[f: f + c].copy()})
+    return RaggedPlan(plan, totals, lps, launches)
+
+
+class RaggedResult(NamedTuple):
+    """Results of a ragged batch, packed in batch order at the plan's offsets."""
+    status: np.ndarray            # [B] int32
+    npiv: np.ndarray              # [B] int32
+    x: np.ndarray                 # [sum m]
+    obj: np.ndarray               # [B]
+    tables: np.ndarray            # [sum cells] final reference-flat tables
+    rowlab: np.ndarray            # [sum m] int32
+    collab: np.ndarray            # [sum n] int32
+    trace: Optional[np.ndarray]   # [sum max_pivots, 2] int32
+    snaps: Optional[np.ndarray]   # [sum (max_pivots+1)*cells]
+    shapes: np.ndarray            # [B, 3] int64: n, m, max_pivots
+    offsets: np.ndarray           # [B, 5] int64: first cell / x / collab / trace pair / snapshot cell of each LP
+
+    def lp(self, k: int) -> BatchResult:
+        """LP k alone, with the shapes and dtypes ``solve_batched(flat_k[None], n_k, m_k, max_pivots=cap_k)`` returns."""
+        n, m, cap = (int(v) for v in self.shapes[k])
+        t, xm, xn, tr, sn = (int(v) for v in self.offsets[k])
+        cells = n * (m + 1) + m
+        trace = None
+        if self.trace is not None:        # DeviceBatch keeps at least one (zeroed) pair per LP
+            trace = self.trace[tr: tr + cap][None] if cap > 0 else np.zeros((1, 1, 2), dtype=np.int32)
+        return BatchResult(self.status[k: k + 1], self.npiv[k: k + 1], self.x[xm: xm + m][None], self.obj[k: k + 1],
+                           self.tables[t: t + cells][None], self.rowlab[xm: xm + m][None],
+                           self.collab[xn: xn + n][None], trace,
+                           None if self.snaps is None else self.snaps[sn: sn + (cap + 1) * cells].reshape(1, cap + 1, cells))
+
+
+def _caps(max_pivots: Union[int, Sequence[int]], B: int) -> np.ndarray:
+    caps = np.asarray(max_pivots, dtype=np.int64)
+    if caps.ndim == 0:
+        caps = np.full(B, int(caps), dtype=np.int64)
+    if caps.shape != (B,):
+        raise ValueError(f"max_pivots must be an int or one int per LP ({B}), got shape {caps.shape}")
+    bad = np.flatnonzero(caps < 0)
+    if bad.size:
+        raise ValueError(f"LP {int(bad[0])}: max_pivots = {int(caps[bad[0]])} must be >= 0")
+    return caps
+
+
+def kernels_for(shapes, engine: str = "auto") -> list:
+    """``kernel_for`` of every LP; its ValueError is prefixed with the index of the first LP it rejects."""
+    shapes = np.asarray(shapes, dtype=np.int64).reshape(-1, 2)
+    if shapes.shape[0] == 0:
+        return []
+    uniq, first, inv = np.unique(shapes, axis=0, return_index=True, return_inverse=True)
+    kinds = [None] * len(uniq)
+    for u in np.argsort(first, kind="stable"):     # in batch order, so the first bad LP is named
+        n, m = (int(v) for v in uniq[u])
+        try:
+            kinds[u] = kernel_for(n, m, engine)
+        except ValueError as e:
+            raise ValueError(f"LP {int(first[u])}: {e}") from None
+    return [kinds[i] for i in inv.reshape(-1)]
+
+
+class DeviceRaggedBatch:
+    """Device buffers and the plan of one ragged batch; reusable across solves (as ``DeviceBatch``).
+
+    shapes: [B] (n, m) pairs; max_pivots: an int or one int per LP.  ``kernels`` is each LP's
+    "smem" (K4) or "cluster" (K7) and ``launches`` the number of kernel launches of one ``run``.
+    """
+
+    def __init__(self, shapes, max_pivots: Union[int, Sequence[int]] = 64, trace: bool = True,
+                 snapshots: bool = False, device=None, engine: str = "auto"):
+        N.lib()
+        self.device = torch.device(device if device is not None else "cuda")
+        self.shapes2 = np.asarray(shapes, dtype=np.int64).reshape(-1, 2)
+        self.B = int(self.shapes2.shape[0])
+        self.caps = _caps(max_pivots, self.B)
+        self.kernels = kernels_for(self.shapes2, engine)
+        self.plan = ragged_plan(self.shapes2, self.caps, engine)
+        self.launches = len(self.plan.launches)
+        self.shapes = np.concatenate([self.shapes2, self.caps[:, None]], axis=1)
+        lp = self.plan.lps
+        self.offsets = np.stack([lp["t"], lp["xm"], lp["xn"], lp["tr"], lp["sn"]], axis=1).astype(np.int64)
+        tot = [int(v) for v in self.plan.totals]
+        dev, f64, i32 = self.device, torch.float64, torch.int32
+        q = lambda k: max(k, 1)  # noqa: E731
+        self.d_plan = torch.from_numpy(self.plan.plan).to(dev)      # uploaded once
+        self.T = torch.empty(q(tot[0]), dtype=f64, device=dev)
+        self.x = torch.empty(q(tot[1]), dtype=f64, device=dev)
+        self.obj = torch.empty(q(self.B), dtype=f64, device=dev)
+        self.status = torch.empty(q(self.B), dtype=i32, device=dev)
+        self.npiv = torch.empty(q(self.B), dtype=i32, device=dev)
+        self.rowlab = torch.empty(q(tot[1]), dtype=i32, device=dev)
+        self.collab = torch.empty(q(tot[2]), dtype=i32, device=dev)
+        self.trace = torch.zeros((q(tot[3]), 2), dtype=i32, device=dev) if trace else None
+        self.snaps = torch.empty(q(tot[4]), dtype=f64, device=dev) if snapshots else None
+        self.totals = tot
+
+    def upload(self, packed, non_blocking: bool = False):
+        """packed: the B reference-flat tables back to back, [sum cells] fp64 (numpy or a (pinned) CPU tensor)."""
+        src = torch.from_numpy(packed) if isinstance(packed, np.ndarray) else packed
+        if tuple(src.shape) != (self.totals[0],):
+            raise ValueError(f"packed tables must be [{self.totals[0]}] (the sum of the LPs' cells)")
+        self.T[: self.totals[0]].copy_(src, non_blocking=non_blocking)
+
+    def run(self, rule: int = N.RULE_REFERENCE):
+        """Launch the plan on the resident batch (asynchronous on the current stream)."""
+        with torch.cuda.device(self.device):
+            N.call("spx_solve_batched_ragged", self.T.data_ptr(), self.plan.plan.ctypes.data, self.d_plan.data_ptr(),
+                   rule, self.x.data_ptr(), self.obj.data_ptr(), self.status.data_ptr(), self.npiv.data_ptr(),
+                   self.rowlab.data_ptr(), self.collab.data_ptr(), N.ptr(self.trace), N.ptr(self.snaps),
+                   torch.cuda.current_stream(self.device).cuda_stream)
+
+    def result(self) -> RaggedResult:
+        B, tot = self.B, self.totals
+        g = lambda t, k: None if t is None else t[:k].cpu().numpy()  # noqa: E731
+        return RaggedResult(g(self.status, B), g(self.npiv, B), g(self.x, tot[1]), g(self.obj, B), g(self.T, tot[0]),
+                            g(self.rowlab, tot[1]), g(self.collab, tot[2]), g(self.trace, tot[3]),
+                            g(self.snaps, tot[4]), self.shapes.copy(), self.offsets.copy())
+
+
+def pack_ragged(lps):
+    """(constraints, function) pairs -> ([B, 2] shapes, [sum cells] packed reference-flat tables)."""
+    from .engine import as_rows_function
+    parts, shapes = [], []
+    for constraints, function in lps:
+        rows, c = as_rows_function(constraints, function)
+        shapes.append((rows.shape[0], c.shape[0]))
+        parts += [rows.reshape(-1), c]
+    packed = np.concatenate(parts) if parts else np.zeros(0)
+    return np.asarray(shapes, dtype=np.int64).reshape(-1, 2), np.ascontiguousarray(packed, dtype=np.float64)
+
+
+def solve_ragged(lps, max_pivots: Union[int, Sequence[int]] = 64, rule: str = "reference", trace: bool = True,
+                 snapshots: bool = False, device=None, engine: str = "auto") -> RaggedResult:
+    """Solve independent LPs of any mix of shapes in one call.
+
+    lps: a sequence of ``(constraints, function)`` pairs as ``SimplexMethod`` takes them (e.g.
+    ``[problem_io.solver_inputs(p) for p in problems]``); max_pivots: an int or one int per LP.
+    Each LP's results are, bit for bit, those ``solve_batched`` returns for that LP alone
+    (``RaggedResult.lp(k)``).  engine: "auto" (per LP, K4 when it fits one CTA, else K7),
+    "smem" or "cluster" for every LP.
+    """
+    shapes, packed = pack_ragged(lps)
+    db = DeviceRaggedBatch(shapes, max_pivots, trace, snapshots, device, engine)
+    if db.B:
+        db.upload(packed)
+        db.run(N.RULES[rule])
     return db.result()

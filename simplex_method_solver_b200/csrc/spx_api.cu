@@ -2,10 +2,12 @@
 // Plain pointers and sizes only; no torch types.  Every entry validates its
 // arguments, launches on the caller's stream and reports failures through
 // spx_last_error().
+#include <algorithm>
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <vector>
 
 #include "spx_common.cuh"
 
@@ -51,6 +53,16 @@ int cluster_size(int64_t, int64_t);
 int cluster_size_for_solve(int64_t, int64_t);
 cudaError_t solve_batched_cluster(double *, int64_t, int, int, int, int, int, double *, double *, int32_t *,
                                   int32_t *, int32_t *, int32_t *, int32_t *, double *, cudaStream_t);
+int64_t ragged_batched_bytes(int, int, int *);
+int ragged_cta_threads(int64_t);
+int ragged_warps_per_cta(int64_t, int64_t);
+int64_t ragged_cluster_bytes(int, int, int);
+cudaError_t solve_ragged_batched(const spx::RaggedLaunch &, const spx::RaggedLp *, const int32_t *, double *, int,
+                                 double *, double *, int32_t *, int32_t *, int32_t *, int32_t *, int32_t *, double *,
+                                 cudaStream_t);
+cudaError_t solve_ragged_cluster(const spx::RaggedLaunch &, const spx::RaggedLp *, const int32_t *, double *, int,
+                                 double *, double *, int32_t *, int32_t *, int32_t *, int32_t *, int32_t *, double *,
+                                 cudaStream_t);
 } // namespace spx_launch
 
 namespace spx_host {
@@ -559,6 +571,156 @@ int spx_solve_batched_cluster(double *d_T, int64_t B, int32_t n, int32_t m, int3
         return -1;
     }
     return check(e, "cluster launch");
+}
+
+// ---- ragged batches (K4 + K7) --------------------------------------------------------
+static int64_t ragged_lp_offset() { return ((int64_t)sizeof(spx::RaggedPlan) + 15) / 16 * 16; }
+
+int64_t spx_ragged_plan_bytes(int64_t B) {
+    if (B < 0 || B > INT32_MAX) return -1;
+    return ragged_lp_offset() + B * (int64_t)sizeof(spx::RaggedLp) + (B * 4 + 15) / 16 * 16;
+}
+
+int spx_ragged_plan(const int32_t *h_shapes, int64_t B, int32_t engine, void *h_plan, int64_t plan_bytes,
+                    int64_t *h_totals) {
+    using namespace spx;
+    SPX_REQUIRE(B >= 0 && B <= INT32_MAX, "spx_ragged_plan: bad batch size B = %lld", (long long)B);
+    SPX_REQUIRE(engine >= SPX_ENGINE_AUTO && engine <= SPX_ENGINE_CLUSTER, "spx_ragged_plan: unknown engine %d", engine);
+    SPX_REQUIRE(h_plan && h_totals && (B == 0 || h_shapes), "spx_ragged_plan: null shapes/plan/totals");
+    SPX_REQUIRE(plan_bytes >= spx_ragged_plan_bytes(B), "spx_ragged_plan: plan_bytes = %lld < spx_ragged_plan_bytes(%lld) = %lld",
+                (long long)plan_bytes, (long long)B, (long long)spx_ragged_plan_bytes(B));
+    RaggedPlan *P = static_cast<RaggedPlan *>(h_plan);
+    RaggedLp *lps = reinterpret_cast<RaggedLp *>(static_cast<char *>(h_plan) + ragged_lp_offset());
+    int32_t *order = reinterpret_cast<int32_t *>(lps + B);
+    // class of every LP: 0 warp mode, 1 CTA mode, 2 + log2(S) cluster; and its shared-memory footprint
+    std::vector<int8_t> cls((size_t)B);
+    std::vector<int64_t> bytes((size_t)B);
+    int64_t tot[5] = {0, 0, 0, 0, 0};
+    for (int64_t k = 0; k < B; ++k) {
+        const int32_t n = h_shapes[3 * k], m = h_shapes[3 * k + 1], cap = h_shapes[3 * k + 2];
+        SPX_REQUIRE(n >= 1 && m >= 1 && cap >= 0, "spx_ragged_plan: LP %lld: bad shape n=%d m=%d max_pivots=%d",
+                    (long long)k, n, m, cap);
+        const int64_t cells = spx_cells(n, m);
+        const bool k4 = engine == SPX_ENGINE_SMEM || (engine == SPX_ENGINE_AUTO && cells <= spx_batched_max_cells());
+        if (k4) {
+            int kern = 0;
+            bytes[k] = spx_launch::ragged_batched_bytes(n, m, &kern);
+            SPX_REQUIRE(bytes[k] > 0 || cells > spx_batched_max_cells(),
+                        "spx_ragged_plan: LP %lld: a %d x %d LP (%lld cells) does not fit the shared memory of one CTA; "
+                        "use engine auto or cluster", (long long)k, n, m, (long long)cells);
+            SPX_REQUIRE(bytes[k] > 0, "spx_ragged_plan: LP %lld: %lld cells per LP exceed the shared-memory resident "
+                        "limit %lld; use spx_solve", (long long)k, (long long)cells, (long long)spx_batched_max_cells());
+            cls[k] = (int8_t)kern;
+        } else {
+            SPX_REQUIRE(spx_launch::cluster_size(n, m) > 0,
+                        "spx_ragged_plan: LP %lld: a %d x %d LP exceeds one cluster (16 CTAs of 227 KB shared memory: "
+                        "8*(R*(m+2)+2m+1) + 4*(R+Q) <= 230400 bytes with R = ceil(n/16), Q = ceil(m/16))",
+                        (long long)k, n, m);
+            const int S = spx_launch::cluster_size_for_solve(n, m);
+            SPX_REQUIRE(S > 0, "spx_ragged_plan: LP %lld: a %d x %d LP does not fit a cluster of SPX_OPT_CLUSTER_SIZE = %d CTAs",
+                        (long long)k, n, m, (int)spx_launch::get_option(SPX_OPT_CLUSTER_SIZE));
+            bytes[k] = spx_launch::ragged_cluster_bytes(n, m, S);
+            cls[k] = (int8_t)(2 + __builtin_ctz((unsigned)S));
+        }
+        lps[k] = RaggedLp{n, m, cap, (int32_t)cells, tot[0], tot[1], tot[2], tot[3], tot[4]};
+        tot[0] += cells;
+        tot[1] += m;
+        tot[2] += n;
+        tot[3] += cap;
+        tot[4] += ((int64_t)cap + 1) * cells;
+    }
+    // launches: warp mode, CTA mode, then K7 by cluster size; inside each, by cells descending, ties by index
+    std::vector<int32_t> idx((size_t)B);
+    for (int64_t k = 0; k < B; ++k) idx[k] = (int32_t)k;
+    std::stable_sort(idx.begin(), idx.end(), [&](int32_t u, int32_t v) {
+        return cls[u] != cls[v] ? cls[u] < cls[v] : lps[u].cells > lps[v].cells;
+    });
+    std::memset(P, 0, sizeof(RaggedPlan));
+    int nl = 0;
+    for (int64_t q = 0; q < B;) {
+        const int c = cls[idx[q]];
+        int64_t e = q, big = 0;
+        while (e < B && cls[idx[e]] == c) { big = std::max(big, bytes[idx[e]]); ++e; }
+        RaggedLaunch &l = P->launch[nl++];
+        l.first = q;
+        l.count = e - q;
+        l.S = 1;
+        l.per_cta = 1;
+        if (c == RAGGED_WARP) {
+            const int64_t slot = (big + 15) / 16 * 16;
+            l.kernel = RAGGED_WARP;
+            l.per_cta = spx_launch::ragged_warps_per_cta(slot, l.count);
+            l.threads = 32 * l.per_cta;
+            l.smem = slot * l.per_cta;
+            l.slot_doubles = slot / 8;
+        } else if (c == RAGGED_CTA) {
+            l.kernel = RAGGED_CTA;
+            l.threads = spx_launch::ragged_cta_threads(lps[idx[q]].cells);     // the largest LP comes first
+            l.smem = big;
+        } else {
+            l.kernel = RAGGED_CLUSTER;
+            l.S = 1 << (c - 2);
+            l.threads = 512;
+            l.smem = big;
+            SPX_REQUIRE(l.count <= INT32_MAX / l.S, "spx_ragged_plan: %lld LPs x S = %d CTAs exceed one grid",
+                        (long long)l.count, l.S);
+        }
+        q = e;
+    }
+    std::copy(idx.begin(), idx.end(), order);
+    P->magic = RAGGED_MAGIC;
+    P->abi = SPX_ABI_VERSION;
+    P->B = B;
+    P->engine = engine;
+    P->nlaunch = nl;
+    for (int i = 0; i < 5; ++i) P->totals[i] = h_totals[i] = tot[i];
+    P->lp_offset = ragged_lp_offset();
+    P->order_offset = ragged_lp_offset() + B * (int64_t)sizeof(RaggedLp);
+    return 0;
+}
+
+int spx_solve_batched_ragged(double *d_T, const void *h_plan, const void *d_plan, int32_t rule, double *d_x,
+                             double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab, int32_t *d_collab,
+                             int32_t *d_trace, double *d_snap, void *stream) {
+    using namespace spx;
+    SPX_REQUIRE(h_plan, "spx_solve_batched_ragged: null plan");
+    const RaggedPlan *P = static_cast<const RaggedPlan *>(h_plan);
+    SPX_REQUIRE(P->magic == RAGGED_MAGIC && P->abi == SPX_ABI_VERSION,
+                "spx_solve_batched_ragged: h_plan is not a plan of this library (magic / ABI version mismatch)");
+    int64_t counted = 0;
+    bool sane = P->B >= 0 && P->nlaunch >= 0 && P->nlaunch <= RAGGED_MAX_LAUNCHES &&
+                P->lp_offset == ragged_lp_offset() && P->order_offset == P->lp_offset + P->B * (int64_t)sizeof(RaggedLp);
+    for (int i = 0; sane && i < P->nlaunch; ++i) {
+        const RaggedLaunch &l = P->launch[i];
+        sane = l.first == counted && l.count >= 1 && l.kernel >= RAGGED_WARP && l.kernel <= RAGGED_CLUSTER &&
+               l.per_cta >= 1 && l.threads >= 32 && l.S >= 1 && l.S <= 16;
+        counted += l.count;
+    }
+    SPX_REQUIRE(sane && counted == P->B, "spx_solve_batched_ragged: inconsistent plan header (B = %lld)", (long long)P->B);
+    if (P->B == 0) return 0;
+    SPX_REQUIRE(d_plan && d_T && d_status && d_npiv, "spx_solve_batched_ragged: null d_plan/T/status/npiv");
+    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_solve_batched_ragged: unknown rule %d", rule);
+    const RaggedLp *lps = reinterpret_cast<const RaggedLp *>(static_cast<const char *>(d_plan) + P->lp_offset);
+    const int32_t *order = reinterpret_cast<const int32_t *>(static_cast<const char *>(d_plan) + P->order_offset);
+    cudaStream_t s = as_stream(stream);
+    for (int i = 0; i < P->nlaunch; ++i) {
+        const RaggedLaunch &l = P->launch[i];
+        if (l.kernel != RAGGED_CLUSTER) {
+            if (check(spx_launch::solve_ragged_batched(l, lps, order, d_T, rule, d_x, d_obj, d_status, d_npiv, d_rowlab,
+                                                       d_collab, d_trace, d_snap, s), "ragged batched launch"))
+                return -1;
+            continue;
+        }
+        const cudaError_t e = spx_launch::solve_ragged_cluster(l, lps, order, d_T, rule, d_x, d_obj, d_status, d_npiv,
+                                                               d_rowlab, d_collab, d_trace, d_snap, s);
+        if (e == cudaErrorInvalidClusterSize) {
+            set_error("spx_solve_batched_ragged: the device cannot co-schedule one cluster of S = %d CTAs with %lld bytes "
+                      "of shared memory each (cudaOccupancyMaxActiveClusters = 0)", l.S, (long long)l.smem);
+            return -1;
+        }
+        if (check(e, "ragged cluster launch")) return -1;
+    }
+    return 0;
 }
 
 // ---- column-sharded flow ----------------------------------------------------------

@@ -18,6 +18,12 @@ namespace {
 
 using namespace spx;
 
+constexpr size_t SMEM_LIMIT = 227 * 1024;
+constexpr int64_t CTA_MODE_MIN_CELLS = 96;    // above this one CTA (not one warp) solves an LP
+constexpr int     CTA_CELLS_PER_WARP = 32;    // CTA mode: cells per warp (2..8 warps)
+constexpr size_t  WARP_LUT_BYTES = CTA_MODE_MIN_CELLS * 4;   // ragged warp mode: per-warp lookup table (384 B)
+constexpr size_t  RAGGED_STATIC = 16;         // ragged kernels: static shared memory (s_ctl), checked at launch
+
 struct BatchedArgs {
     double  *T;          // [B][cells] in/out
     int64_t  B;
@@ -224,6 +230,158 @@ batched_kernel(BatchedArgs a, int warps_per_cta, int warp_doubles) {
     }
 }
 
+// One LP of a ragged batch, start to finish: batched_kernel's loop with the shape and the offsets taken from the LP's
+// descriptor `d`, by its group of nl threads (tl = index in the group): one warp (CTA == false) or the first nl
+// threads of the CTA (CTA == true).  base: its two tables, x, labels in shared memory.  In warp mode the warps of one
+// CTA have different shapes, so each warp has its own cell -> (row, col) lookup table (cell_i, cell_j) instead of a
+// CTA-wide one; in CTA mode the group synchronises with a named barrier of its own nl threads.
+// (batched_kernel keeps its own copy of the loop: it runs at the 40-register cap of its launch bounds in warp mode,
+// and any restructuring of its code moves its spills.)
+template <bool CTA>
+__device__ __forceinline__ void ragged_body(const BatchedArgs &a, const RaggedLp &d, int64_t lp, const uint16_t *cell_i,
+                                             const uint16_t *cell_j, double *base, int *s_ctl, int tl, int nl) {
+    const int n = d.n, m = d.m, w1 = m + 1;
+    const int cells = n * w1 + m;
+    const int max_pivots = d.max_pivots;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    auto group_sync = [&]() {
+        if (!CTA) __syncwarp();
+        else asm volatile("bar.sync 1, %0;" :: "r"(nl) : "memory");
+    };
+
+    double *cur = base;
+    double *nxt = base + cells;
+    double *xs  = base + 2 * cells;                       // [m]
+    int32_t *rl = reinterpret_cast<int32_t *>(xs + m);    // [m] header labels
+    int32_t *cl = rl + m;                                 // [n] row labels
+
+    double *Tg = a.T + d.t;
+    for (int k = tl; k < cells; k += nl) cur[k] = Tg[k];
+    for (int j = tl; j < m; j += nl) rl[j] = j;           // 'x1'..'xm'  :30
+    for (int i = tl; i < n; i += nl) cl[i] = m + i;       // 'y1'..'yn'  :31
+    group_sync();
+    const int fo = n * w1;                                // offset of the f row
+    const double f0 = (m >= 1) ? cur[fo] : 0.0;           // self.function is never mutated (:29,:49)
+    const double f1 = (m >= 2) ? cur[fo + 1] : 0.0;
+
+    int npiv = 0, status;
+    double *snap = a.snap ? a.snap + d.sn : nullptr;
+    int32_t *trace = a.trace ? a.trace + 2 * d.tr : nullptr;
+
+    for (;;) {
+        if (snap) {
+            double *sg = snap + (int64_t)npiv * cells;
+            for (int k = tl; k < cells; k += nl) sg[k] = cur[k];
+        }
+        int r = -1, c = -1;
+        if (!CTA) {
+            status = warp_pick(cur, n, m, a.rule, lane, r, c);
+        } else {
+            if (warp == 0) {
+                const int st = warp_pick(cur, n, m, a.rule, lane, r, c);
+                if (lane == 0) { s_ctl[0] = st; s_ctl[1] = r; s_ctl[2] = c; }
+            }
+            group_sync();
+            status = s_ctl[0]; r = s_ctl[1]; c = s_ctl[2];
+        }
+        if (status != SPX_PIVOT) break;
+        if (npiv >= max_pivots) { status = SPX_CAP; break; }
+        if (trace && tl == 0) { trace[2 * npiv] = r; trace[2 * npiv + 1] = c; }
+
+        // ---- K3: out-of-place pivot (:149-177), all reads from `cur`; the four cell kinds
+        // (:156 pivot row, :160 pivot column, :163 pivot cell, :173-175 the rest) differ only in
+        // the numerator, so one division by the pivot serves them all without divergence
+        const double p = cur[r * w1 + c];
+        const PivotDiv pd = pivot_div_prepare(p);
+        const double *prow = cur + r * w1;
+        for (int k = tl; k < cells; k += nl) {
+            const int i = cell_i[k], j = cell_j[k];
+            const double t = cur[k];
+            const double ci = cur[i * w1 + c];
+            const bool pr = (i == r), pc = (j == c);
+            double num = __dsub_rn(__dmul_rn(t, p), __dmul_rn(prow[j], ci));
+            num = pc ? ci : num;
+            num = pr ? -t : num;
+            num = (pr && pc) ? 1.0 : num;
+            nxt[k] = pivot_div(num, pd);
+        }
+        if (tl == 0) { const int32_t t = rl[c]; rl[c] = cl[r]; cl[r] = t; }      // :152
+        group_sync();                                      // (CTA: also orders s_ctl against the next pick)
+        double *sw = cur; cur = nxt; nxt = sw;
+        ++npiv;
+    }
+
+    // ---- epilogue: final table, labels, find_optimum()/f() (:48-68)
+    for (int k = tl; k < cells; k += nl) Tg[k] = cur[k];
+    for (int j = tl; j < m; j += nl) xs[j] = 0.0;
+    group_sync();
+    for (int i = tl; i < n; i += nl) {
+        const int lab = cl[i];
+        if (lab < m) xs[lab] = cur[i * w1 + m];
+    }
+    group_sync();
+    if (a.x) for (int j = tl; j < m; j += nl) a.x[d.xm + j] = xs[j];
+    if (a.rowlab) for (int j = tl; j < m; j += nl) a.rowlab[d.xm + j] = rl[j];
+    if (a.collab) for (int i = tl; i < n; i += nl) a.collab[d.xn + i] = cl[i];
+    if (tl == 0) {
+        a.status[lp] = status;
+        a.npiv[lp] = npiv;
+        if (a.obj) a.obj[lp] = (m >= 2) ? __dadd_rn(__dmul_rn(f0, xs[0]), __dmul_rn(f1, xs[1])) : 0.0;
+    }
+}
+
+// The ragged batch: LP order[slot] of each slot, shape and offsets from lps[].  Warp mode: slot = warp of the grid,
+// warp slots of warp_doubles doubles, each a 384-byte lookup table and then the LP's tables, x and labels; same launch
+// bounds as batched_kernel<false>.  CTA mode: slot = CTA; the CTA is launched at the warp count of
+// the largest LP of the launch, builds the lookup table of its own LP, and only the warps its LP needs stay (the
+// warp count the uniform entry gives that shape: 32 cells per warp, 2..16 warps).
+template <bool CTA>
+__global__ void __launch_bounds__(CTA ? 512 : 256, CTA ? 1 : 6)
+ragged_batched_kernel(BatchedArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
+                      int warps_per_cta, int warp_doubles) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ int s_ctl[4];
+    const int warp = threadIdx.x >> 5;
+    const int64_t slot = CTA ? (int64_t)blockIdx.x : (int64_t)blockIdx.x * warps_per_cta + warp;
+    if (!CTA) {
+        if (warp >= warps_per_cta || slot >= a.B) return;
+        const int64_t lp = order[slot];
+        const RaggedLp d = lps[lp];
+        const int lane = threadIdx.x & 31, w1 = d.m + 1;
+        // the warp's slot: its own lookup table (<= 96 cells), then its tables, x and labels
+        unsigned char *slot_raw = smem_raw + (size_t)warp * warp_doubles * sizeof(double);
+        uint16_t *cell_i = reinterpret_cast<uint16_t *>(slot_raw);
+        uint16_t *cell_j = cell_i + CTA_MODE_MIN_CELLS;
+        for (int k = lane; k < d.cells; k += 32) {
+            const int i = k / w1;
+            cell_i[k] = (uint16_t)i;
+            cell_j[k] = (uint16_t)(k - i * w1);
+        }
+        __syncwarp();
+        double *base = reinterpret_cast<double *>(slot_raw + WARP_LUT_BYTES);
+        ragged_body<false>(a, d, lp, cell_i, cell_j, base, s_ctl, lane, 32);
+        return;
+    }
+    const int64_t lp = order[slot];
+    const RaggedLp d = lps[lp];
+    const int w1 = d.m + 1, cells = d.cells;
+    uint16_t *cell_i = reinterpret_cast<uint16_t *>(smem_raw);
+    uint16_t *cell_j = cell_i + cells;
+    for (int k = threadIdx.x; k < cells; k += blockDim.x) {
+        const int i = k / w1;
+        cell_i[k] = (uint16_t)i;
+        cell_j[k] = (uint16_t)(k - i * w1);
+    }
+    __syncthreads();
+    int warps = (cells + CTA_CELLS_PER_WARP - 1) / CTA_CELLS_PER_WARP;
+    warps = warps < 2 ? 2 : (warps > 16 ? 16 : warps);
+    const int nl = warps * 32 < (int)blockDim.x ? warps * 32 : (int)blockDim.x;
+    if ((int)threadIdx.x >= nl) return;
+    const size_t lut_bytes = ((size_t)cells * 4 + 15) / 16 * 16;
+    double *base = reinterpret_cast<double *>(smem_raw + lut_bytes);
+    ragged_body<true>(a, d, lp, cell_i, cell_j, base, s_ctl, (int)threadIdx.x, nl);
+}
+
 size_t warp_bytes(int n, int m) {
     const size_t cells = (size_t)n * (m + 1) + m;
     size_t b = (2 * cells + m) * sizeof(double) + (size_t)(n + m) * sizeof(int32_t);
@@ -233,9 +391,6 @@ size_t lut_bytes(int n, int m) {
     const size_t cells = (size_t)n * (m + 1) + m;
     return (cells * 4 + 15) / 16 * 16;
 }
-constexpr size_t SMEM_LIMIT = 227 * 1024;
-constexpr int64_t CTA_MODE_MIN_CELLS = 96;    // above this one CTA (not one warp) solves an LP
-constexpr int64_t CTA_CELLS_PER_WARP = 32;    // CTA mode: cells per warp (2..8 warps)
 
 } // namespace
 
@@ -286,6 +441,60 @@ cudaError_t solve_batched(double *T, int64_t B, int n, int m, int rule, int max_
     }
     const int64_t ctas = (B + wpc - 1) / wpc;
     batched_kernel<false><<<(unsigned)ctas, wpc * 32, smem, stream>>>(a, wpc, (int)(wb / sizeof(double)));
+    spx_host::count_launch();
+    return cudaGetLastError();
+}
+
+// ---- ragged batches: the plan's numbers for K4 ----
+// shared memory of one LP: CTA mode lookup table + tables, or warp mode slot (no table); -1 when K4 cannot take it
+// (the uniform entry's limits)
+int64_t ragged_batched_bytes(int n, int m, int *kernel) {
+    if (n < 1 || m < 1 || n > 65535 || m > 65534) return -1;
+    const int64_t cells = (int64_t)n * (m + 1) + m;
+    // the dynamic and the static shared memory of a CTA share SMEM_LIMIT
+    if (cells > batched_max_cells() || lut_bytes(n, m) + warp_bytes(n, m) > SMEM_LIMIT - RAGGED_STATIC) return -1;
+    *kernel = cells > CTA_MODE_MIN_CELLS ? RAGGED_CTA : RAGGED_WARP;
+    return cells > CTA_MODE_MIN_CELLS ? (int64_t)(lut_bytes(n, m) + warp_bytes(n, m))
+                                      : (int64_t)(WARP_LUT_BYTES + warp_bytes(n, m));
+}
+// CTA mode: the uniform entry's warp count for this many cells (32 cells per warp, 2..16 warps)
+int ragged_cta_threads(int64_t cells) {
+    int warps = (int)((cells + CTA_CELLS_PER_WARP - 1) / CTA_CELLS_PER_WARP);
+    return 32 * (warps < 2 ? 2 : (warps > 16 ? 16 : warps));
+}
+// warp mode: LPs per CTA for warp slots of `slot` bytes (the lookup table included), as the uniform entry (at most 8, ~48 KB per CTA)
+int ragged_warps_per_cta(int64_t slot, int64_t count) {
+    int64_t wpc = (48 * 1024) / slot;
+    wpc = wpc > 8 ? 8 : (wpc < 1 ? 1 : wpc);
+    return (int)(wpc > count ? count : wpc);
+}
+
+cudaError_t solve_ragged_batched(const RaggedLaunch &l, const RaggedLp *lps, const int32_t *order, double *T, int rule,
+                                 double *x, double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab,
+                                 int32_t *collab, int32_t *trace, double *snap, cudaStream_t stream) {
+    if (l.count <= 0) return cudaSuccess;
+    BatchedArgs a{T, l.count, 0, 0, rule, 0, x, obj, status, npiv, rowlab, collab, trace, snap};
+    static size_t configured_dev[64][2] = {};
+    size_t *configured = configured_dev[spx_host::device_slot()];
+    const bool cta = (l.kernel == RAGGED_CTA);
+    if (l.smem > 48 * 1024 && (size_t)l.smem > configured[cta]) {
+        cudaFuncAttributes fa;
+        cudaError_t e = cta ? cudaFuncGetAttributes(&fa, ragged_batched_kernel<true>)
+                            : cudaFuncGetAttributes(&fa, ragged_batched_kernel<false>);
+        if (e != cudaSuccess) return e;
+        if (fa.sharedSizeBytes > RAGGED_STATIC) return cudaErrorInvalidValue;
+        const int dyn = (int)(SMEM_LIMIT - RAGGED_STATIC);
+        e = cta ? cudaFuncSetAttribute(ragged_batched_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn)
+                : cudaFuncSetAttribute(ragged_batched_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn);
+        if (e != cudaSuccess) return e;
+        configured[cta] = SMEM_LIMIT - RAGGED_STATIC;
+    }
+    const int64_t ctas = (l.count + l.per_cta - 1) / l.per_cta;
+    if (cta)
+        ragged_batched_kernel<true><<<(unsigned)ctas, l.threads, (size_t)l.smem, stream>>>(a, lps, order + l.first, 1, 0);
+    else
+        ragged_batched_kernel<false><<<(unsigned)ctas, l.threads, (size_t)l.smem, stream>>>(a, lps, order + l.first,
+                                                                                        l.per_cta, (int)l.slot_doubles);
     spx_host::count_launch();
     return cudaGetLastError();
 }

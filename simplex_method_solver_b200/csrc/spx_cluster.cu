@@ -72,7 +72,11 @@ struct EqKey {          // Dantzig: the f cell whose orderable image is the mini
     __device__ bool operator()(double v) const { return v < 0.0 && orderable(v) == key; }
 };
 
-__global__ void __launch_bounds__(CLUSTER_THREADS, 1) cluster_kernel(ClusterArgs a) {
+// The body of both kernels.  RAGGED == false: shape, R, Q and offsets from the arguments (one shape per launch).
+// RAGGED == true: LP order[blockIdx.x / S] of a ragged batch, its shape and offsets from lps[], R and Q from its shape.
+template <bool RAGGED>
+__device__ __forceinline__ void cluster_body(const ClusterArgs &a, const RaggedLp *__restrict__ lps,
+                                             const int32_t *__restrict__ order) {
     cg::cluster_group cluster = cg::this_cluster();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ Scratch sc;
@@ -80,9 +84,12 @@ __global__ void __launch_bounds__(CLUSTER_THREADS, 1) cluster_kernel(ClusterArgs
     __shared__ int s_ctl[3];                               // {status, r, c} of the merged decision
     __shared__ double s_x01[2];                            // rank 0: b of the rows labelled x1, x2 (:49)
 
-    const int n = a.n, m = a.m, w1 = m + 1, S = a.S, R = a.R, Q = a.Q;
+    RaggedLp d;
+    if (RAGGED) d = lps[order[blockIdx.x / (unsigned)a.S]];
+    const int n = RAGGED ? d.n : a.n, m = RAGGED ? d.m : a.m, w1 = m + 1, S = a.S;
+    const int R = RAGGED ? (n + S - 1) / S : a.R, Q = RAGGED ? (m + S - 1) / S : a.Q;
     const int rank = (int)cluster.block_rank();
-    const int64_t lp = (int64_t)(blockIdx.x / (unsigned)S);
+    const int64_t lp = RAGGED ? (int64_t)order[blockIdx.x / (unsigned)S] : (int64_t)(blockIdx.x / (unsigned)S);
     const int tid = (int)threadIdx.x, nt = (int)blockDim.x;
     const int r0 = rank * R;                               // first body row of this band
     const int rows = max(0, min(R, n - r0));
@@ -99,7 +106,7 @@ __global__ void __launch_bounds__(CLUSTER_THREADS, 1) cluster_kernel(ClusterArgs
 
     const int64_t cells = (int64_t)n * w1 + m;
     const int fo = n * w1;                                 // offset of the f row
-    double *Tg = a.T + lp * cells;
+    double *Tg = a.T + (RAGGED ? d.t : lp * cells);
     for (int k = tid; k < bandcells; k += nt) band[k] = Tg[(int64_t)r0 * w1 + k];
     for (int j = tid; j < m; j += nt) f[j] = Tg[fo + j];
     for (int i = tid; i < rows; i += nt) cl[i] = m + r0 + i;
@@ -111,8 +118,8 @@ __global__ void __launch_bounds__(CLUSTER_THREADS, 1) cluster_kernel(ClusterArgs
     const float inv_w1 = 1.0f / (float)w1;
 
     int npiv = 0, status;
-    double *snap = a.snap ? a.snap + lp * (int64_t)(a.max_pivots + 1) * cells : nullptr;
-    int32_t *trace = a.trace ? a.trace + lp * (int64_t)a.max_pivots * 2 : nullptr;
+    double *snap = a.snap ? a.snap + (RAGGED ? d.sn : lp * (int64_t)(a.max_pivots + 1) * cells) : nullptr;
+    int32_t *trace = a.trace ? a.trace + (RAGGED ? 2 * d.tr : lp * (int64_t)a.max_pivots * 2) : nullptr;
 
     for (;;) {
         if (snap) {
@@ -183,7 +190,7 @@ __global__ void __launch_bounds__(CLUSTER_THREADS, 1) cluster_kernel(ClusterArgs
         status = s_ctl[0];
         const int r = s_ctl[1], c = s_ctl[2];
         if (status != SPX_PIVOT) break;
-        if (npiv >= a.max_pivots) { status = SPX_CAP; break; }
+        if (npiv >= (RAGGED ? d.max_pivots : a.max_pivots)) { status = SPX_CAP; break; }
 
         // ---- stash the old pivot row (from its owner) and the band's old pivot-column entries
         const int owner = r / R, holder = c / Q;           // owners of row r and of the header label of column c
@@ -232,7 +239,7 @@ __global__ void __launch_bounds__(CLUSTER_THREADS, 1) cluster_kernel(ClusterArgs
     // ---- epilogue: final table, labels, find_optimum()/f() (:48-68)
     for (int k = tid; k < bandcells; k += nt) Tg[(int64_t)r0 * w1 + k] = band[k];
     if (rank == 0) for (int j = tid; j < m; j += nt) Tg[fo + j] = f[j];
-    double *xg = a.x ? a.x + lp * m : nullptr;
+    double *xg = a.x ? a.x + (RAGGED ? d.xm : lp * m) : nullptr;
     // labels are a permutation of 0..n+m-1: x_j is the b of the row labelled x_j, or 0 when a column carries it
     for (int i = tid; i < rows; i += nt) {
         const int lab = cl[i];
@@ -241,12 +248,12 @@ __global__ void __launch_bounds__(CLUSTER_THREADS, 1) cluster_kernel(ClusterArgs
             if (xg) xg[lab] = v;
             if (lab < 2) *cluster.map_shared_rank(&s_x01[lab], 0) = v;
         }
-        if (a.collab) a.collab[lp * n + r0 + i] = lab;
+        if (a.collab) a.collab[(RAGGED ? d.xn : lp * n) + r0 + i] = lab;
     }
     for (int j = tid; j < cols; j += nt) {
         const int lab = rl[j];
         if (xg && lab < m) xg[lab] = 0.0;
-        if (a.rowlab) a.rowlab[lp * m + j0 + j] = lab;
+        if (a.rowlab) a.rowlab[(RAGGED ? d.xm : lp * m) + j0 + j] = lab;
     }
     cluster.sync();                                        // s_x01 complete; no CTA leaves while a peer may read it
     if (rank == 0 && tid == 0) {
@@ -254,6 +261,16 @@ __global__ void __launch_bounds__(CLUSTER_THREADS, 1) cluster_kernel(ClusterArgs
         a.npiv[lp] = npiv;
         if (a.obj) a.obj[lp] = (m >= 2) ? __dadd_rn(__dmul_rn(f0, s_x01[0]), __dmul_rn(f1, s_x01[1])) : 0.0;
     }
+}
+
+__global__ void __launch_bounds__(CLUSTER_THREADS, 1) cluster_kernel(ClusterArgs a) {
+    cluster_body<false>(a, nullptr, nullptr);
+}
+
+// a ragged batch: the LPs order[0 .. a.B) of one cluster size a.S, each cluster its own shape (a.n, a.m, a.R, a.Q unused)
+__global__ void __launch_bounds__(CLUSTER_THREADS, 1)
+ragged_cluster_kernel(ClusterArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order) {
+    cluster_body<true>(a, lps, order);
 }
 
 // the per-CTA footprint of the header comment, for S CTAs per LP
@@ -324,6 +341,52 @@ cudaError_t solve_batched_cluster(double *T, int64_t B, int n, int m, int S, int
     if (e != cudaSuccess) return e;
     if (clusters <= 0) return cudaErrorInvalidClusterSize;
     e = cudaLaunchKernelEx(&cfg, cluster_kernel, a);
+    spx_host::count_launch();
+    if (e != cudaSuccess) return e;
+    return cudaGetLastError();
+}
+
+int64_t ragged_cluster_bytes(int n, int m, int S) { return cluster_bytes(n, m, S); }
+
+// one launch of a ragged plan: the l.count LPs order[l.first ..] at cluster size l.S, l.smem = the largest footprint
+// among them; cudaErrorInvalidClusterSize when the device cannot co-schedule one such cluster
+cudaError_t solve_ragged_cluster(const RaggedLaunch &l, const RaggedLp *lps, const int32_t *order, double *T, int rule,
+                                 double *x, double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab,
+                                 int32_t *collab, int32_t *trace, double *snap, cudaStream_t stream) {
+    if (l.count <= 0) return cudaSuccess;
+    static bool configured_dev[64] = {};
+    const int slot = spx_host::device_slot();
+    if (!configured_dev[slot]) {
+        cudaFuncAttributes fa;
+        cudaError_t e = cudaFuncGetAttributes(&fa, ragged_cluster_kernel);
+        if (e != cudaSuccess) return e;
+        if (fa.sharedSizeBytes > CLUSTER_STATIC) return cudaErrorInvalidValue;
+        e = cudaFuncSetAttribute(ragged_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)CLUSTER_DYN_BYTES);
+        if (e != cudaSuccess) return e;
+        e = cudaFuncSetAttribute(ragged_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+        if (e != cudaSuccess) return e;
+        configured_dev[slot] = true;
+    }
+    ClusterArgs a{T, l.count, 0, 0, rule, 0, l.S, 0, 0, x, obj, status, npiv, rowlab, collab, trace, snap};
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)(l.count * l.S));
+    cfg.blockDim = dim3(CLUSTER_THREADS);
+    cfg.dynamicSmemBytes = (size_t)l.smem;
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = (unsigned)l.S;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    int clusters = 0;
+    cudaError_t e = cudaOccupancyMaxActiveClusters(&clusters, ragged_cluster_kernel, &cfg);
+    if (e != cudaSuccess) return e;
+    if (clusters <= 0) return cudaErrorInvalidClusterSize;
+    const int32_t *ord = order + l.first;
+    e = cudaLaunchKernelEx(&cfg, ragged_cluster_kernel, a, lps, ord);
     spx_host::count_launch();
     if (e != cudaSuccess) return e;
     return cudaGetLastError();

@@ -4,7 +4,8 @@ Two partitionings, the two places where the pivot loop shards naturally
 (SURVEY.md §8e):
 
 * **Batches of independent small LPs** — contiguous split of the batch, no
-  data-path collective (``shard_range`` + ``solve_batched_sharded``).
+  data-path collective (``shard_range`` + ``solve_batched_sharded``; for LPs of
+  mixed shapes ``cells_range`` + ``solve_ragged_sharded``, balanced by cells).
 
 * **Column-sharded large tableau** — rank g owns a contiguous block of body
   columns as its own split matrix; the b column, labels and the 128-byte solver
@@ -660,4 +661,42 @@ def solve_batched_sharded(tables: np.ndarray, n: int, m: int, max_pivots: int = 
         from .batched import solve_batched as solver
     kw = {} if engine == "auto" else {"engine": engine}
     res = solver(tables[start:start + count], n, m, max_pivots=max_pivots, rule=rule, device=device, **kw)
+    return start, count, res
+
+
+def cells_range(cells, rank: int, world: int):
+    """Contiguous split of LPs with `cells` [B] cells each, balanced by cells: (start, count) of `rank`.
+
+    Rank r starts at the first LP whose prefix sum of cells reaches r/world of the total, so every
+    rank holds at most total/world + (the largest LP's cells) cells.
+    """
+    cells = np.asarray(cells, dtype=np.int64).reshape(-1)
+    prefix = np.concatenate([[0], np.cumsum(cells)])
+    total = int(prefix[-1])
+    bound = lambda r: int(np.searchsorted(prefix * world, r * total, side="left")) if r < world else cells.shape[0]  # noqa: E731
+    start = min(bound(rank), cells.shape[0])
+    return start, max(0, bound(rank + 1) - start)
+
+
+def solve_ragged_sharded(lps, max_pivots=64, rule: str = "reference", rank: Optional[int] = None,
+                         world: Optional[int] = None, device=None, solver=None, engine: str = "auto",
+                         trace: bool = True, snapshots: bool = False):
+    """Each rank solves its contiguous, cell-balanced share of a ragged batch; no collective on the data path.
+
+    `lps` and `max_pivots` as ``batched.solve_ragged``.  Returns (start, count, RaggedResult) for this
+    rank.  `solver` defaults to the CUDA ``solve_ragged``; tests pass a stand-in.
+    """
+    from .engine import as_rows_function
+    if rank is None:
+        rank = dist.get_rank() if dist.is_initialized() else 0
+    if world is None:
+        world = dist.get_world_size() if dist.is_initialized() else 1
+    lps = [as_rows_function(cons, fn) for cons, fn in lps]
+    start, count = cells_range([r.size + c.size for r, c in lps], rank, world)
+    caps = np.asarray(max_pivots, dtype=np.int64)
+    caps = int(caps) if caps.ndim == 0 else caps[start:start + count]
+    if solver is None:
+        from .batched import solve_ragged as solver
+    res = solver(lps[start:start + count], max_pivots=caps, rule=rule, trace=trace, snapshots=snapshots,
+                 device=device, engine=engine)
     return start, count, res

@@ -61,7 +61,8 @@ def solver_inputs(problem: Problem):
 def batch_tables(problems: Iterable[Problem]) -> tuple[np.ndarray, int, int]:
     """Problems of one shape -> the [B, cells] reference-flat array ``solve_batched`` takes.
 
-    Returns (tables, n, m).  Raises if the shapes differ (group by shape first).
+    Returns (tables, n, m).  Raises if the shapes differ: problems of mixed shapes go to
+    ``batched.solve_ragged([solver_inputs(p) for p in problems], ...)`` in one call.
     """
     flat, shape = [], None
     for p in problems:

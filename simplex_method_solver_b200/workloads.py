@@ -67,6 +67,40 @@ def gui_batch(B: int, seed: int = 0):
     return T, C
 
 
+def gui_ragged(B: int, seed: int = 0):
+    """GUI-like bounded polygons of 3 to 12 sides (k constraints, 2 variables): gui_batch's octagon construction with
+    the number of sides drawn per LP.  Returns a list of B (rows [k, 3], c [2]) pairs (10 shapes, all <= 38 cells)."""
+    g = np.random.default_rng([seed, 3])
+    sides = g.integers(3, 13, B)
+    out = []
+    for k in sides:
+        k = int(k)
+        th = 2 * np.pi * (np.arange(k) + g.uniform(0, 1, k)) / k
+        nx, ny = -np.cos(th), -np.sin(th)
+        r = g.uniform(1.0, 4.0, k)
+        p0 = 5.0
+        rows = np.round(np.stack([nx, ny, r - (nx * p0 + ny * p0)], axis=1), 2)
+        ph = g.uniform(0, 2 * np.pi)
+        out.append((rows, np.round(np.array([np.cos(ph), np.sin(ph)]), 2)))
+    return out
+
+
+def mixed_lps(B: int, seed: int = 0):
+    """B LPs of the dense and phase-1 families with n and m drawn log-uniformly from geometric grids of 24 values,
+    1..512 and 2..800 (a few hundred shapes), so they spread over K4 warp mode (<= 96 cells), K4 CTA mode
+    (<= 10,000 cells) and K7 at every cluster size; every shape fits one cluster (n <= 528 at m = 800).
+    Returns a list of B (rows [n, m+1], c [m]) pairs."""
+    g = np.random.default_rng([seed, 5])
+    ns = np.unique(np.round(np.geomspace(1, 512, 24)).astype(int))
+    ms = np.unique(np.round(np.geomspace(2, 800, 24)).astype(int))
+    out = []
+    for k in range(B):
+        n, m = int(g.choice(ns)), int(g.choice(ms))
+        fam = phase1_lp if g.random() < 0.5 else dense_lp
+        out.append(fam(n, m, seed * 1_000_003 + k))
+    return out
+
+
 def klee_minty(n: int):
     """KM(n): Klee-Minty cube, all floats (cfg5: n=20, 2^n - 1 pivots)."""
     rows = []
