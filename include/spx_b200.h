@@ -44,7 +44,7 @@
 extern "C" {
 #endif
 
-#define SPX_ABI_VERSION 6
+#define SPX_ABI_VERSION 7
 
 /* status codes == the outcomes of pick_element(), simplex.py:70-141 */
 #define SPX_PIVOT       1   /* (True, r, c, e)                                   :91,:141 */
@@ -107,7 +107,7 @@ int64_t     spx_launch_count(int reset);
 #define SPX_OPT_SHARD_CTAS       14 /* sharded / look-ahead pricing kernel: at most this many CTAs (0 = one per SM) */
 #define SPX_OPT_RESIDENT_VARIANT 15 /* L2-resident persistent loop: 0 default (price, sweep, one grid barrier per pivot), 1 = look-ahead pricing inside the CTA with the sweep rows prefetched by cp.async (bit-identical; measured slower on cfg2, kept selectable) */
 #define SPX_OPT_FUSE_PAIRS       12 /* fused update kernel: column pairs per lane, i.e. strip width / 64 (0 = default 2; 1 or 2) */
-#define SPX_OPT_CLUSTER_SIZE     16 /* K7 (spx_solve_batched_cluster): CTAs per LP, 1, 2, 4, 8 or 16 (0 = default: spx_cluster_size(n, m)); a size whose footprint does not fit is rejected */
+#define SPX_OPT_CLUSTER_SIZE     16 /* K7 (spx_solve_batched_cluster, ragged plans) and K8 (spx_solve_batched_global): CTAs per LP, 1, 2, 4, 8 or 16 (0 = default: spx_cluster_size(n, m) for K7, spx_global_cluster_size(n, m, B) for K8); a size whose footprint does not fit is rejected */
 int         spx_set_option(int32_t option, int64_t value);
 int64_t     spx_get_option(int32_t option);
 /* Device self-test of the hoisted-reciprocal division used by K3 against the
@@ -254,6 +254,36 @@ int spx_solve_batched_cluster(double *d_T, int64_t B, int32_t n, int32_t m, int3
  * fits, i.e. the cluster size K7 uses for an n x m LP unless SPX_OPT_CLUSTER_SIZE
  * forces one; 0 when the LP does not fit one cluster. */
 int32_t spx_cluster_size(int32_t n, int32_t m);
+
+/* ---- K8: batches of LPs too large for one cluster, the table in global memory -- */
+/* The loop of K7 with each LP's body rows left in d_T and updated there in place:
+ * a cluster of S CTAs solves one LP, CTA k owning body rows [k*R, k*R+R), R = ceil(n/S),
+ * and keeping only a copy of the f row, the old pivot row, its rows' old pivot-column
+ * entries and the labels in shared memory; two cluster barriers per pivot.  Arguments,
+ * NULL conventions, outputs and results are those of spx_solve_batched_cluster, bit for
+ * bit, for every shape either accepts.
+ * Capacity: with Q = ceil(m/S), one CTA needs
+ *     8*(2*m + 1 + R) + 4*(R + Q)  <=  230400 bytes
+ * for some S in {1, 2, 4, 8, 16} (m <= 11519 at S = 1 and m <= 14177 at S = 16; at
+ * m = 2000, n <= 15866 at S = 1 and n <= 263856 at S = 16).
+ * S: SPX_OPT_CLUSTER_SIZE when set, else spx_global_cluster_size(n, m, B).  Shape, rule,
+ * B, the non-null outputs, the capacity and B*S <= INT32_MAX are checked before the
+ * device is touched; B = 0 returns 0; a device that cannot co-schedule one cluster of
+ * S CTAs is an error, not a fall-back. */
+int spx_solve_batched_global(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule,
+                             int32_t max_pivots, double *d_x, double *d_obj,
+                             int32_t *d_status, int32_t *d_npiv,
+                             int32_t *d_rowlab, int32_t *d_collab,
+                             int32_t *d_trace, double *d_snap, void *stream);
+/* Host only (no device): S_min, the smallest S in {1, 2, 4, 8, 16} whose footprint
+ * above fits; 0 when the LP does not fit. */
+int32_t spx_global_min_cluster_size(int32_t n, int32_t m);
+/* The S a K8 solve of B such LPs launches on the current device: SPX_OPT_CLUSTER_SIZE
+ * when set (0 if it does not fit); else the S >= S_min that keeps the most SMs busy,
+ * min(B, cudaOccupancyMaxActiveClusters at S) * S, the smaller S on ties, so a single LP
+ * gets 16 CTAs and a batch that fills the device at S_min gets S_min; 0 when the LP does
+ * not fit, -1 on a CUDA error.  Queries occupancy, launches nothing. */
+int32_t spx_global_cluster_size(int32_t n, int32_t m, int64_t B);
 
 /* ---- ragged batches: LPs of any mix of shapes in one call (K4 and K7) ----------- */
 /* Each LP k has its own shape (n_k, m_k) and its own cap max_pivots_k.  Every buffer

@@ -13,7 +13,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "csrc", "libspx_b200.so")
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 LOOP_AUTO, LOOP_CLASSIC, LOOP_LOOKAHEAD, LOOP_RESIDENT, LOOP_FUSED = 0, 1, 2, 3, 4
 LOOP_MODES = {None: LOOP_AUTO, "auto": LOOP_AUTO, False: LOOP_CLASSIC, "classic": LOOP_CLASSIC,
               True: LOOP_LOOKAHEAD, "lookahead": LOOP_LOOKAHEAD, "resident": LOOP_RESIDENT,
@@ -88,6 +88,10 @@ SIGNATURES = {
     "spx_solve_batched_cluster": (ctypes.c_int, [_vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp,
                                                  _vp, _vp, _vp]),
     "spx_cluster_size": (_i32, [_i32, _i32]),
+    "spx_solve_batched_global": (ctypes.c_int, [_vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp,
+                                                _vp, _vp, _vp]),
+    "spx_global_min_cluster_size": (_i32, [_i32, _i32]),
+    "spx_global_cluster_size": (_i32, [_i32, _i32, _i64]),
     "spx_ragged_plan_bytes": (_i64, [_i64]),
     "spx_ragged_plan": (ctypes.c_int, [_vp, _i64, _i32, _vp, _i64, _vp]),
     "spx_solve_batched_ragged": (ctypes.c_int, [_vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

@@ -6,8 +6,11 @@ Each LP is the reference's whole get_solution() loop
   * "smem"    (K4, csrc/spx_batched.cu): one warp or one CTA per LP, up to
               ``spx_batched_max_cells()`` cells;
   * "cluster" (K7, csrc/spx_cluster.cu): one thread-block cluster of up to 16
-              CTAs per LP, for mid-size LPs up to ``spx_cluster_size() > 0``.
-``engine="auto"`` takes K4 for every shape K4 accepts and K7 above that.  Both
+              CTAs per LP, for mid-size LPs up to ``spx_cluster_size() > 0``;
+  * "global"  (K8, csrc/spx_global.cu): one cluster per LP with the table left in
+              global memory, for LPs up to ``spx_global_min_cluster_size() > 0``
+              (only when asked for: ``engine="auto"`` never routes to it).
+``engine="auto"`` takes K4 for every shape K4 accepts and K7 above that.  All three
 compute the same bits.  LPs never communicate, so a batch splits over GPUs by
 contiguous ranges with no collective (see parallel.shard_range).
 
@@ -37,7 +40,7 @@ class BatchResult(NamedTuple):
     snaps: Optional[np.ndarray]   # [B, max_pivots+1, cells]
 
 
-ENGINES = ("auto", "smem", "cluster")
+ENGINES = ("auto", "smem", "cluster", "global")
 _INT32_MAX = (1 << 31) - 1
 
 
@@ -52,14 +55,34 @@ def _cluster_capacity_text(n: int, m: int) -> str:
     return f"at m = {m} one cluster of 16 CTAs holds at most n = {lo} rows"
 
 
+def _global_capacity_text(n: int, m: int) -> str:
+    L = N.load()
+    if L.spx_global_min_cluster_size(1, m) == 0:
+        lo, hi = 1, m                          # largest m with spx_global_min_cluster_size(1, m) > 0
+        while lo < hi:
+            mid = (lo + hi + 1) // 2
+            lo, hi = (mid, hi) if L.spx_global_min_cluster_size(1, mid) else (lo, mid - 1)
+        return f"at most {lo} columns fit one cluster"
+    lo, hi = 1, n                              # largest n with spx_global_min_cluster_size(n, m) > 0
+    while lo < hi:
+        mid = (lo + hi + 1) // 2
+        lo, hi = (mid, hi) if L.spx_global_min_cluster_size(mid, m) else (lo, mid - 1)
+    return f"at m = {m} one cluster of 16 CTAs holds at most n = {lo} rows"
+
+
 def kernel_for(n: int, m: int, engine: str = "auto") -> str:
-    """"smem" (K4) or "cluster" (K7) for an n x m LP; ValueError when the engine cannot take it."""
+    """"smem" (K4), "cluster" (K7) or "global" (K8) for an n x m LP; ValueError when the engine cannot take it."""
     if engine not in ENGINES:
         raise ValueError(f"unknown engine {engine!r}; one of {ENGINES}")
     if not (1 <= n <= _INT32_MAX and 1 <= m <= _INT32_MAX):
         raise ValueError(f"bad shape {n} x {m}")
     L = N.load()
     cells = n * (m + 1) + m
+    if engine == "global":
+        if L.spx_global_min_cluster_size(n, m) == 0:
+            raise ValueError(f"a {n} x {m} LP ({cells} cells) exceeds the capacity of the global-memory cluster "
+                             f"solver: {_global_capacity_text(n, m)}; use SimplexMethod / DeviceTableau")
+        return "global"
     if engine == "smem" or (engine == "auto" and cells <= L.spx_batched_max_cells()):
         if cells > L.spx_batched_max_cells():
             raise ValueError(f"{cells} cells per LP exceed the shared-memory limit of one CTA "
@@ -67,14 +90,19 @@ def kernel_for(n: int, m: int, engine: str = "auto") -> str:
         return "smem"
     if L.spx_cluster_size(n, m) == 0:
         raise ValueError(f"a {n} x {m} LP ({cells} cells) exceeds the capacity of the cluster solver: "
-                         f"{_cluster_capacity_text(n, m)}; use SimplexMethod / DeviceTableau for large tableaus")
+                         f"{_cluster_capacity_text(n, m)}; use engine='global' (K8) up to its capacity, or "
+                         "SimplexMethod / DeviceTableau for large tableaus")
     return "cluster"
+
+
+_ENTRIES = {"smem": "spx_solve_batched", "cluster": "spx_solve_batched_cluster", "global": "spx_solve_batched_global"}
 
 
 class DeviceBatch:
     """Device buffers for one batch shape; reusable across solves (bench / serving).
 
-    ``kernel`` is "smem" (K4) or "cluster" (K7), chosen by ``kernel_for(n, m, engine)``.
+    ``kernel`` is "smem" (K4), "cluster" (K7) or "global" (K8), chosen by ``kernel_for(n, m, engine)``.
+    ``cluster_size`` is the CTAs per LP a K8 ``run`` launches on this device (None for K4 and K7).
     """
 
     def __init__(self, B: int, n: int, m: int, max_pivots: int = 64, trace: bool = True,
@@ -85,6 +113,12 @@ class DeviceBatch:
         self.cells = n * (m + 1) + m
         self.kernel = kernel_for(self.n, self.m, engine)
         dev = self.device
+        self.cluster_size = None
+        if self.kernel == "global":
+            with torch.cuda.device(dev):
+                self.cluster_size = int(N.lib().spx_global_cluster_size(self.n, self.m, self.B))
+            if self.cluster_size <= 0:
+                raise N.SpxError(f"spx_global_cluster_size failed: {N.lib().spx_last_error().decode(errors='replace')}")
         Bq = max(self.B, 1)
         self.T = torch.empty((Bq, self.cells), dtype=torch.float64, device=dev)
         self.x = torch.empty((Bq, m), dtype=torch.float64, device=dev)
@@ -106,7 +140,7 @@ class DeviceBatch:
     def run(self, rule: int = N.RULE_REFERENCE):
         """Launch the solver on the resident batch (asynchronous on the current stream)."""
         with torch.cuda.device(self.device):
-            entry = "spx_solve_batched" if self.kernel == "smem" else "spx_solve_batched_cluster"
+            entry = _ENTRIES[self.kernel]
             N.call(entry, self.T.data_ptr(), self.B, self.n, self.m, rule, self.max_pivots, self.x.data_ptr(), self.obj.data_ptr(), self.status.data_ptr(),
                    self.npiv.data_ptr(), self.rowlab.data_ptr(), self.collab.data_ptr(),
                    N.ptr(self.trace), N.ptr(self.snaps),
@@ -126,7 +160,7 @@ def solve_batched(tables, n: int, m: int, max_pivots: int = 64, rule: str = "ref
     tables: [B, cells] reference-flat fp64 (rows ``[a_1..a_m, b]`` x n, then the m
     function coefficients) — the flattened arguments of
     ``SimplexMethod(constraints, function)`` for each LP.
-    engine: "auto" (K4 when the LP fits one CTA, else K7), "smem" (K4) or "cluster" (K7).
+    engine: "auto" (K4 when the LP fits one CTA, else K7), "smem" (K4), "cluster" (K7) or "global" (K8).
     """
     tables = np.ascontiguousarray(np.asarray(tables, dtype=np.float64))
     if tables.ndim != 2 or tables.shape[1] != n * (m + 1) + m:
@@ -165,7 +199,7 @@ class RaggedPlan(NamedTuple):
 def ragged_plan(shapes, max_pivots, engine: str = "auto") -> RaggedPlan:
     """Host only: the library's plan for LPs of `shapes` [B, 2] (n, m) with caps `max_pivots` [B]."""
     if engine not in ENGINE_CODES:
-        raise ValueError(f"unknown engine {engine!r}; one of {ENGINES}")
+        raise ValueError(f"unknown engine {engine!r}; one of {tuple(ENGINE_CODES)}")
     L = N.load()
     shapes = np.asarray(shapes, dtype=np.int64).reshape(-1, 2)
     B = shapes.shape[0]

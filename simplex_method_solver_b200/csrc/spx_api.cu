@@ -53,6 +53,10 @@ int cluster_size(int64_t, int64_t);
 int cluster_size_for_solve(int64_t, int64_t);
 cudaError_t solve_batched_cluster(double *, int64_t, int, int, int, int, int, double *, double *, int32_t *,
                                   int32_t *, int32_t *, int32_t *, int32_t *, double *, cudaStream_t);
+int global_min_cluster_size(int64_t, int64_t);
+cudaError_t global_cluster_size(int64_t, int64_t, int64_t, int *);
+cudaError_t solve_batched_global(double *, int64_t, int, int, int, int, int, double *, double *, int32_t *,
+                                 int32_t *, int32_t *, int32_t *, int32_t *, double *, cudaStream_t);
 int64_t ragged_batched_bytes(int, int, int *);
 int ragged_cta_threads(int64_t);
 int ragged_warps_per_cta(int64_t, int64_t);
@@ -571,6 +575,48 @@ int spx_solve_batched_cluster(double *d_T, int64_t B, int32_t n, int32_t m, int3
         return -1;
     }
     return check(e, "cluster launch");
+}
+
+// ---- K8 -------------------------------------------------------------------------
+int32_t spx_global_min_cluster_size(int32_t n, int32_t m) { return spx_launch::global_min_cluster_size(n, m); }
+
+int32_t spx_global_cluster_size(int32_t n, int32_t m, int64_t B) {
+    int S = 0;
+    if (check(spx_launch::global_cluster_size(n, m, B < 0 ? 0 : B, &S), "spx_global_cluster_size")) return -1;
+    return S;
+}
+
+int spx_solve_batched_global(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule, int32_t max_pivots,
+                             double *d_x, double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab,
+                             int32_t *d_collab, int32_t *d_trace, double *d_snap, void *stream) {
+    SPX_REQUIRE(B >= 0 && n >= 1 && m >= 1 && max_pivots >= 0, "spx_solve_batched_global: bad arguments");
+    SPX_REQUIRE(B == 0 || (d_T && d_status && d_npiv), "spx_solve_batched_global: null T/status/npiv");
+    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_solve_batched_global: unknown rule %d",
+                rule);
+    const int smin = spx_launch::global_min_cluster_size(n, m);
+    SPX_REQUIRE(smin > 0,
+                "spx_solve_batched_global: a %d x %d LP exceeds the shared memory of one cluster (16 CTAs of 227 KB: "
+                "8*(2m+1+R) + 4*(R+Q) <= 230400 bytes with R = ceil(n/S), Q = ceil(m/S), S <= 16)", n, m);
+    const int forced = (int)spx_launch::get_option(SPX_OPT_CLUSTER_SIZE);
+    SPX_REQUIRE(forced == 0 || spx_global_min_cluster_size(n, m) <= forced,
+                "spx_solve_batched_global: a %d x %d LP does not fit a cluster of SPX_OPT_CLUSTER_SIZE = %d CTAs "
+                "(8*(2m+1+R) + 4*(R+Q) <= 230400 bytes; at least %d CTAs)", n, m, forced, smin);
+    // a default S above S_min is only chosen when all B clusters are co-resident, far below the grid limit
+    const int Smax = forced ? forced : smin;
+    SPX_REQUIRE(B <= INT32_MAX / Smax, "spx_solve_batched_global: B = %lld LPs x S = %d CTAs exceed one grid",
+                (long long)B, Smax);
+    if (B == 0) return 0;
+    int S = 0;
+    if (check(spx_launch::global_cluster_size(n, m, B, &S), "spx_solve_batched_global: occupancy")) return -1;
+    const cudaError_t e = spx_launch::solve_batched_global(d_T, B, n, m, S, rule, max_pivots, d_x, d_obj, d_status,
+                                                           d_npiv, d_rowlab, d_collab, d_trace, d_snap,
+                                                           as_stream(stream));
+    if (e == cudaErrorInvalidClusterSize) {
+        set_error("spx_solve_batched_global: the device cannot co-schedule one cluster of S = %d CTAs for a %d x %d "
+                  "LP (cudaOccupancyMaxActiveClusters = 0)", S, n, m);
+        return -1;
+    }
+    return check(e, "global launch");
 }
 
 // ---- ragged batches (K4 + K7) --------------------------------------------------------

@@ -28,9 +28,7 @@
 //             partials of pivot k+1 (written after B) from overwriting those of pivot k (read before B);
 //   update    the band and the f row in place, one division by the pivot (pivot_div, reciprocal hoisted).
 // A final cluster.sync() keeps every CTA's shared memory alive until no peer can read it any more.
-#include <cooperative_groups.h>
-
-#include "spx_block.cuh"
+#include "spx_cluster.cuh"
 
 namespace cg = cooperative_groups;
 
@@ -57,19 +55,6 @@ struct ClusterArgs {
     int32_t *collab;     // [B][n] or null
     int32_t *trace;      // [B][max_pivots][2] or null
     double  *snap;       // [B][max_pivots+1][cells] or null
-};
-
-// what one CTA knows about the pivot after folding its band
-struct Partial {
-    Ratio q;            // ratio scan of its rows for the f-row entering column (global row indices)
-    int   elig_key;     // 2 * (its first eligible row) + (that row's ratio is NaN); SPX_NONE none
-    int   bneg_row;     // its first row with b < 0 (global index); SPX_NONE none
-    int   bneg_col;     // the first positive cell of that row; SPX_NONE none
-};
-
-struct EqKey {          // Dantzig: the f cell whose orderable image is the minimum
-    unsigned long long key;
-    __device__ bool operator()(double v) const { return v < 0.0 && orderable(v) == key; }
 };
 
 // The body of both kernels.  RAGGED == false: shape, R, Q and offsets from the arguments (one shape per launch).
@@ -128,18 +113,7 @@ __device__ __forceinline__ void cluster_body(const ClusterArgs &a, const RaggedL
             if (rank == 0) for (int j = tid; j < m; j += nt) sg[fo + j] = f[j];
         }
         // ---- K1: entering column of the f row (:94-98), the same in every CTA
-        int cf;
-        if (a.rule == SPX_RULE_REFERENCE) {
-            cf = block_first_index(f, m, IsNeg(), sc);
-        } else {   // Dantzig: most negative, lowest index on ties
-            unsigned long long best = ~0ull;
-            for (int j = tid; j < m; j += nt) {
-                const double v = f[j];
-                if (v < 0.0) { const unsigned long long k = orderable(v); best = k < best ? k : best; }
-            }
-            best = block_min_u64(best, sc);
-            cf = (best == ~0ull) ? SPX_NONE : block_first_index(f, m, EqKey{best}, sc);
-        }
+        const int cf = f_row_entering(f, m, a.rule, sc);
         // ---- one pass over the band: phase-1 row (:72-76) and the ratio scan of column cf (:107-136)
         Ratio q = ratio_identity();
         int key = SPX_NONE, bneg = SPX_NONE;
@@ -165,27 +139,7 @@ __device__ __forceinline__ void cluster_body(const ClusterArgs &a, const RaggedL
         cluster.sync();                                    // A: every partial is published
 
         // ---- decision: each CTA merges the S partials itself
-        if (tid < 32) {
-            Partial p;
-            p.q = ratio_identity(); p.elig_key = SPX_NONE; p.bneg_row = SPX_NONE; p.bneg_col = SPX_NONE;
-            if (tid < S) p = *cluster.map_shared_rank(&s_part, tid);
-            const int r1 = warp_min_int(p.bneg_row);
-            const int c1 = warp_min_int(p.bneg_row == r1 ? p.bneg_col : SPX_NONE);
-            int st, r = -1, c = -1;
-            if (r1 != SPX_NONE) {                          // phase 1
-                if (c1 == SPX_NONE) st = SPX_INCORRECT;    // :88-89
-                else { st = SPX_PIVOT; r = r1; c = c1; }   // :91
-            } else if (cf == SPX_NONE) {
-                st = SPX_OPTIMAL;                          // :101-103
-            } else {
-                const Ratio g = warp_ratio_reduce(p.q);
-                const int k2 = warp_min_int(p.elig_key);
-                r = ratio_decide(g, k2 != SPX_NONE && (k2 & 1));
-                st = (r < 0) ? SPX_NOCONV : SPX_PIVOT;     // :138-139
-                c = cf;
-            }
-            if (tid == 0) { s_ctl[0] = st; s_ctl[1] = r; s_ctl[2] = c; }
-        }
+        if (tid < 32) cluster_decide(cluster, &s_part, S, cf, s_ctl);
         __syncthreads();
         status = s_ctl[0];
         const int r = s_ctl[1], c = s_ctl[2];
