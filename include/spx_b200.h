@@ -44,7 +44,7 @@
 extern "C" {
 #endif
 
-#define SPX_ABI_VERSION 7
+#define SPX_ABI_VERSION 8
 
 /* status codes == the outcomes of pick_element(), simplex.py:70-141 */
 #define SPX_PIVOT       1   /* (True, r, c, e)                                   :91,:141 */
@@ -107,7 +107,7 @@ int64_t     spx_launch_count(int reset);
 #define SPX_OPT_SHARD_CTAS       14 /* sharded / look-ahead pricing kernel: at most this many CTAs (0 = one per SM) */
 #define SPX_OPT_RESIDENT_VARIANT 15 /* L2-resident persistent loop: 0 default (price, sweep, one grid barrier per pivot), 1 = look-ahead pricing inside the CTA with the sweep rows prefetched by cp.async (bit-identical; measured slower on cfg2, kept selectable) */
 #define SPX_OPT_FUSE_PAIRS       12 /* fused update kernel: column pairs per lane, i.e. strip width / 64 (0 = default 2; 1 or 2) */
-#define SPX_OPT_CLUSTER_SIZE     16 /* K7 (spx_solve_batched_cluster, ragged plans) and K8 (spx_solve_batched_global): CTAs per LP, 1, 2, 4, 8 or 16 (0 = default: spx_cluster_size(n, m) for K7, spx_global_cluster_size(n, m, B) for K8); a size whose footprint does not fit is rejected */
+#define SPX_OPT_CLUSTER_SIZE     16 /* K7 and K8 (spx_solve_batched_cluster, spx_solve_batched_global, and ragged plans, read when the plan is made): CTAs per LP, 1, 2, 4, 8 or 16 (0 = default: spx_cluster_size(n, m) for K7, spx_global_cluster_size(n, m, B) for K8, spx_ragged_cluster_size for a ragged K8 launch); a size whose footprint does not fit is rejected */
 int         spx_set_option(int32_t option, int64_t value);
 int64_t     spx_get_option(int32_t option);
 /* Device self-test of the hoisted-reciprocal division used by K3 against the
@@ -285,24 +285,33 @@ int32_t spx_global_min_cluster_size(int32_t n, int32_t m);
  * not fit, -1 on a CUDA error.  Queries occupancy, launches nothing. */
 int32_t spx_global_cluster_size(int32_t n, int32_t m, int64_t B);
 
-/* ---- ragged batches: LPs of any mix of shapes in one call (K4 and K7) ----------- */
+/* ---- ragged batches: LPs of any mix of shapes in one call (K4, K7 and K8) ------- */
 /* Each LP k has its own shape (n_k, m_k) and its own cap max_pivots_k.  Every buffer
  * is packed in batch order: LP k's slice starts at the prefix sum over LPs 0..k-1 of
  *     d_T, d_snap-table   cells          d_x, d_rowlab   m
  *     d_collab            n              d_trace         max_pivots (pairs of int32)
  *     d_snap              (max_pivots+1)*cells
  * and d_obj, d_status, d_npiv hold one element per LP.  Each LP's results are those
- * of spx_solve_batched / spx_solve_batched_cluster for that LP alone, bit for bit.
+ * of spx_solve_batched / spx_solve_batched_cluster / spx_solve_batched_global for that
+ * LP alone, bit for bit.
  *
  * Routing: SPX_ENGINE_AUTO sends an LP to K4 when cells <= spx_batched_max_cells(),
- * else to K7 (at spx_cluster_size(n, m), or SPX_OPT_CLUSTER_SIZE when set); SMEM and
- * CLUSTER send every LP to that engine.  One solve makes at most 7 launches, in
+ * else to K7 (at spx_cluster_size(n, m), or SPX_OPT_CLUSTER_SIZE when set), and rejects
+ * an LP above K7's capacity; SMEM, CLUSTER and GLOBAL send every LP to that engine;
+ * AUTO_GLOBAL is AUTO with K8 for the LPs above K7's capacity (spx_cluster_size(n, m)
+ * == 0) up to K8's.  Code 3 is not an engine.  One solve makes at most 12 launches, in
  * sequence on `stream`: K4 warp mode (LPs of <= 96 cells) if any, K4 CTA mode if any,
- * one K7 launch per distinct cluster size.  Within a launch the LPs run largest first
- * (by cells, ties by batch index). */
-#define SPX_ENGINE_AUTO    0
-#define SPX_ENGINE_SMEM    1
-#define SPX_ENGINE_CLUSTER 2
+ * one K7 launch per distinct cluster size, then one K8 launch per distinct S_min
+ * (spx_global_min_cluster_size), or one at SPX_OPT_CLUSTER_SIZE when it is set when the
+ * plan is made.  Within a launch the LPs run largest first (by cells, ties by batch
+ * index).  A K8 launch planned without SPX_OPT_CLUSTER_SIZE runs at the S that
+ * spx_ragged_cluster_size reports: the rule of spx_global_cluster_size applied to the
+ * launch, over S >= its S_min, with the largest footprint of its LPs at each S. */
+#define SPX_ENGINE_AUTO        0
+#define SPX_ENGINE_SMEM        1
+#define SPX_ENGINE_CLUSTER     2
+#define SPX_ENGINE_GLOBAL      4
+#define SPX_ENGINE_AUTO_GLOBAL 5
 /* bytes of the plan of a batch of B LPs (-1 when B < 0) */
 int64_t spx_ragged_plan_bytes(int64_t B);
 /* Host only, no device.  h_shapes[B][3] = {n, m, max_pivots} in batch order.  Validates
@@ -317,11 +326,18 @@ int spx_ragged_plan(const int32_t *h_shapes, int64_t B, int32_t engine, void *h_
  * made by the caller (nothing allocates behind the caller's back and there is no hidden
  * synchronising copy).  The launches are read from h_plan, the descriptors from d_plan.
  * Plan header, rule and pointers are checked before the device is touched; a plan of
- * B = 0 returns 0.  Outputs and NULL conventions as spx_solve_batched. */
+ * B = 0 returns 0.  Outputs and NULL conventions as spx_solve_batched.  A K8 launch
+ * checks count * S <= INT32_MAX for the S it launches at; a device that cannot
+ * co-schedule one of its clusters is an error naming S and the footprint. */
 int spx_solve_batched_ragged(double *d_T, const void *h_plan, const void *d_plan, int32_t rule,
                              double *d_x, double *d_obj, int32_t *d_status, int32_t *d_npiv,
                              int32_t *d_rowlab, int32_t *d_collab, int32_t *d_trace, double *d_snap,
                              void *stream);
+/* The cluster size launch `launch` (0-based) of h_plan runs at on the current device: the
+ * planned S for K4 (1) and K7, and for K8 the planned S when SPX_OPT_CLUSTER_SIZE was set
+ * at plan time (no device needed), else the rule above (queries occupancy, launches
+ * nothing).  -1 on error. */
+int32_t spx_ragged_cluster_size(const void *h_plan, int32_t launch);
 
 /* ---- column-sharded large tableau (one process per GPU) ------------------- */
 /* Rank g owns global columns [col0, col0+m_loc) of the body as a local split

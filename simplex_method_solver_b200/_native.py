@@ -13,7 +13,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "csrc", "libspx_b200.so")
 
-ABI_VERSION = 7
+ABI_VERSION = 8
 LOOP_AUTO, LOOP_CLASSIC, LOOP_LOOKAHEAD, LOOP_RESIDENT, LOOP_FUSED = 0, 1, 2, 3, 4
 LOOP_MODES = {None: LOOP_AUTO, "auto": LOOP_AUTO, False: LOOP_CLASSIC, "classic": LOOP_CLASSIC,
               True: LOOP_LOOKAHEAD, "lookahead": LOOP_LOOKAHEAD, "resident": LOOP_RESIDENT,
@@ -24,7 +24,7 @@ OPT_UPDATE_KERNEL, OPT_TILED_MIN_BLOCKS, OPT_PIPE_ORDER, OPT_PIPE_GRID, OPT_TILE
 OPT_FUSE_MIN_BLOCKS, OPT_FUSE_PRICING, OPT_FUSE_LOOKAHEAD, OPT_FUSE_VARIANT, OPT_FUSE_TILE_ROWS, OPT_FUSE_PAIRS = 7, 8, 9, 10, 11, 12
 OPT_SHARD_THREADS, OPT_SHARD_CTAS, OPT_RESIDENT_VARIANT, OPT_CLUSTER_SIZE = 13, 14, 15, 16
 RULES = {"reference": RULE_REFERENCE, "bland": RULE_REFERENCE, "dantzig": RULE_DANTZIG}
-ENGINE_AUTO, ENGINE_SMEM, ENGINE_CLUSTER = 0, 1, 2
+ENGINE_AUTO, ENGINE_SMEM, ENGINE_CLUSTER, ENGINE_GLOBAL, ENGINE_AUTO_GLOBAL = 0, 1, 2, 4, 5
 
 # the two ValueError texts of pick_element(), /root/reference/src/simplex.py:89,139
 ERROR_TEXT = {INCORRECT: "incorrect system", NOCONV: "simplex method does not converge"}
@@ -95,6 +95,7 @@ SIGNATURES = {
     "spx_ragged_plan_bytes": (_i64, [_i64]),
     "spx_ragged_plan": (ctypes.c_int, [_vp, _i64, _i32, _vp, _i64, _vp]),
     "spx_solve_batched_ragged": (ctypes.c_int, [_vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "spx_ragged_cluster_size": (_i32, [_vp, _i32]),
     "spx_shard_msg_doubles": (_i64, [_i32]),
     "spx_shard_candidate": (ctypes.c_int, [_vp, _vp, _i32, _i32, _i64, _i64, _i32, _i32, _vp, _vp, _vp]),
     "spx_shard_select": (ctypes.c_int, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _vp, ctypes.c_uint64, _vp]),

@@ -10,13 +10,15 @@ Each LP is the reference's whole get_solution() loop
   * "global"  (K8, csrc/spx_global.cu): one cluster per LP with the table left in
               global memory, for LPs up to ``spx_global_min_cluster_size() > 0``
               (only when asked for: ``engine="auto"`` never routes to it).
-``engine="auto"`` takes K4 for every shape K4 accepts and K7 above that.  All three
+``engine="auto"`` takes K4 for every shape K4 accepts and K7 above that;
+``engine="auto_global"`` does the same and takes K8 above K7's capacity.  All three
 compute the same bits.  LPs never communicate, so a batch splits over GPUs by
 contiguous ranges with no collective (see parallel.shard_range).
 
 A ragged batch is packed in batch order (LP k's table, x, labels, trace and snapshots
 start at prefix sums over LPs 0..k-1, see include/spx_b200.h) and solved by one plan of
-at most seven launches: K4 warp mode, K4 CTA mode, one K7 launch per cluster size.
+at most twelve launches: K4 warp mode, K4 CTA mode, one K7 launch per cluster size, one
+K8 launch per smallest cluster size that holds its LPs.
 """
 from __future__ import annotations
 
@@ -40,7 +42,7 @@ class BatchResult(NamedTuple):
     snaps: Optional[np.ndarray]   # [B, max_pivots+1, cells]
 
 
-ENGINES = ("auto", "smem", "cluster", "global")
+ENGINES = ("auto", "smem", "cluster", "global", "auto_global")
 _INT32_MAX = (1 << 31) - 1
 
 
@@ -71,13 +73,21 @@ def _global_capacity_text(n: int, m: int) -> str:
 
 
 def kernel_for(n: int, m: int, engine: str = "auto") -> str:
-    """"smem" (K4), "cluster" (K7) or "global" (K8) for an n x m LP; ValueError when the engine cannot take it."""
+    """"smem" (K4), "cluster" (K7) or "global" (K8) for an n x m LP; ValueError when the engine cannot take it.
+
+    "auto_global" is "auto" with K8 above K7's capacity: K4 up to ``spx_batched_max_cells()`` cells, else K7 when
+    ``spx_cluster_size(n, m) > 0``, else K8 (the routing of ragged batches that mix every size).
+    """
     if engine not in ENGINES:
         raise ValueError(f"unknown engine {engine!r}; one of {ENGINES}")
     if not (1 <= n <= _INT32_MAX and 1 <= m <= _INT32_MAX):
         raise ValueError(f"bad shape {n} x {m}")
     L = N.load()
     cells = n * (m + 1) + m
+    if engine == "auto_global":
+        if cells <= L.spx_batched_max_cells():
+            return "smem"
+        engine = "cluster" if L.spx_cluster_size(n, m) else "global"
     if engine == "global":
         if L.spx_global_min_cluster_size(n, m) == 0:
             raise ValueError(f"a {n} x {m} LP ({cells} cells) exceeds the capacity of the global-memory cluster "
@@ -178,22 +188,24 @@ def solve_batched(tables, n: int, m: int, max_pivots: int = 64, rule: str = "ref
 
 
 # ---------------------------------------------------------------------------- ragged batches
-ENGINE_CODES = {"auto": N.ENGINE_AUTO, "smem": N.ENGINE_SMEM, "cluster": N.ENGINE_CLUSTER}
+ENGINE_CODES = {"auto": N.ENGINE_AUTO, "smem": N.ENGINE_SMEM, "cluster": N.ENGINE_CLUSTER, "global": N.ENGINE_GLOBAL,
+                "auto_global": N.ENGINE_AUTO_GLOBAL}
 # the plan spx_ragged_plan writes (csrc/spx_common.cuh: RaggedPlan, RaggedLaunch, RaggedLp)
 _LAUNCH = np.dtype([("kernel", "<i4"), ("S", "<i4"), ("threads", "<i4"), ("per_cta", "<i4"), ("smem", "<i8"),
-                    ("first", "<i8"), ("count", "<i8"), ("slot_doubles", "<i8")])
+                    ("first", "<i8"), ("count", "<i8"), ("slot_doubles", "<i8"), ("pick_S", "<i4"), ("reserved", "<i4")])
 _HEADER = np.dtype([("magic", "<u4"), ("abi", "<i4"), ("B", "<i8"), ("engine", "<i4"), ("nlaunch", "<i4"),
-                    ("totals", "<i8", 5), ("lp_offset", "<i8"), ("order_offset", "<i8"), ("launch", _LAUNCH, 7)])
+                    ("totals", "<i8", 5), ("lp_offset", "<i8"), ("order_offset", "<i8"), ("launch", _LAUNCH, 12)])
 _LP = np.dtype([("n", "<i4"), ("m", "<i4"), ("max_pivots", "<i4"), ("cells", "<i4"), ("t", "<i8"), ("xm", "<i8"),
                 ("xn", "<i8"), ("tr", "<i8"), ("sn", "<i8")])
-LAUNCH_KINDS = ("warp", "cta", "cluster")
+LAUNCH_KINDS = ("warp", "cta", "cluster", "global")
 
 
 class RaggedPlan(NamedTuple):
     plan: np.ndarray              # the plan bytes (uint8), as spx_ragged_plan wrote them
     totals: np.ndarray            # [5] packed lengths: T, x (= rowlab), collab, trace pairs, snap
     lps: np.ndarray               # [B] descriptors: n, m, max_pivots, cells and the offsets t, xm, xn, tr, sn
-    launches: list                # per launch: dict(kind, S, threads, smem, lps = LP indices in launch order)
+    launches: list                # per launch: dict(kind, S, threads, smem, lps = LP indices in launch order);
+    #                               for kind "global" S is the planned S (S_min, or SPX_OPT_CLUSTER_SIZE)
 
 
 def ragged_plan(shapes, max_pivots, engine: str = "auto") -> RaggedPlan:
@@ -286,7 +298,8 @@ class DeviceRaggedBatch:
     """Device buffers and the plan of one ragged batch; reusable across solves (as ``DeviceBatch``).
 
     shapes: [B] (n, m) pairs; max_pivots: an int or one int per LP.  ``kernels`` is each LP's
-    "smem" (K4) or "cluster" (K7) and ``launches`` the number of kernel launches of one ``run``.
+    "smem" (K4), "cluster" (K7) or "global" (K8), ``launches`` the number of kernel launches of one
+    ``run`` and ``cluster_sizes`` the CTAs per LP of each launch on this device (1 for K4).
     """
 
     def __init__(self, shapes, max_pivots: Union[int, Sequence[int]] = 64, trace: bool = True,
@@ -299,6 +312,12 @@ class DeviceRaggedBatch:
         self.kernels = kernels_for(self.shapes2, engine)
         self.plan = ragged_plan(self.shapes2, self.caps, engine)
         self.launches = len(self.plan.launches)
+        L = N.lib()
+        with torch.cuda.device(self.device):
+            self.cluster_sizes = [int(L.spx_ragged_cluster_size(self.plan.plan.ctypes.data, q))
+                                  for q in range(self.launches)]
+        if any(S <= 0 for S in self.cluster_sizes):
+            raise N.SpxError(f"spx_ragged_cluster_size failed: {L.spx_last_error().decode(errors='replace')}")
         self.shapes = np.concatenate([self.shapes2, self.caps[:, None]], axis=1)
         lp = self.plan.lps
         self.offsets = np.stack([lp["t"], lp["xm"], lp["xn"], lp["tr"], lp["sn"]], axis=1).astype(np.int64)
@@ -360,7 +379,8 @@ def solve_ragged(lps, max_pivots: Union[int, Sequence[int]] = 64, rule: str = "r
     ``[problem_io.solver_inputs(p) for p in problems]``); max_pivots: an int or one int per LP.
     Each LP's results are, bit for bit, those ``solve_batched`` returns for that LP alone
     (``RaggedResult.lp(k)``).  engine: "auto" (per LP, K4 when it fits one CTA, else K7),
-    "smem" or "cluster" for every LP.
+    "auto_global" (as "auto", and K8 above K7's capacity), or "smem", "cluster" or "global"
+    for every LP.
     """
     shapes, packed = pack_ragged(lps)
     db = DeviceRaggedBatch(shapes, max_pivots, trace, snapshots, device, engine)

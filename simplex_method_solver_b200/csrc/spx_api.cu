@@ -67,6 +67,11 @@ cudaError_t solve_ragged_batched(const spx::RaggedLaunch &, const spx::RaggedLp 
 cudaError_t solve_ragged_cluster(const spx::RaggedLaunch &, const spx::RaggedLp *, const int32_t *, double *, int,
                                  double *, double *, int32_t *, int32_t *, int32_t *, int32_t *, int32_t *, double *,
                                  cudaStream_t);
+int64_t ragged_global_bytes(int, int, int);
+cudaError_t ragged_global_size(const spx::RaggedLaunch &, const spx::RaggedLp *, const int32_t *, int *, int64_t *);
+cudaError_t solve_ragged_global(const spx::RaggedLaunch &, int, int64_t, const spx::RaggedLp *, const int32_t *,
+                                double *, int, double *, double *, int32_t *, int32_t *, int32_t *, int32_t *,
+                                int32_t *, double *, cudaStream_t);
 } // namespace spx_launch
 
 namespace spx_host {
@@ -619,7 +624,7 @@ int spx_solve_batched_global(double *d_T, int64_t B, int32_t n, int32_t m, int32
     return check(e, "global launch");
 }
 
-// ---- ragged batches (K4 + K7) --------------------------------------------------------
+// ---- ragged batches (K4 + K7 + K8) ---------------------------------------------------
 static int64_t ragged_lp_offset() { return ((int64_t)sizeof(spx::RaggedPlan) + 15) / 16 * 16; }
 
 int64_t spx_ragged_plan_bytes(int64_t B) {
@@ -631,14 +636,16 @@ int spx_ragged_plan(const int32_t *h_shapes, int64_t B, int32_t engine, void *h_
                     int64_t *h_totals) {
     using namespace spx;
     SPX_REQUIRE(B >= 0 && B <= INT32_MAX, "spx_ragged_plan: bad batch size B = %lld", (long long)B);
-    SPX_REQUIRE(engine >= SPX_ENGINE_AUTO && engine <= SPX_ENGINE_CLUSTER, "spx_ragged_plan: unknown engine %d", engine);
+    SPX_REQUIRE((engine >= SPX_ENGINE_AUTO && engine <= SPX_ENGINE_CLUSTER) || engine == SPX_ENGINE_GLOBAL ||
+                engine == SPX_ENGINE_AUTO_GLOBAL, "spx_ragged_plan: unknown engine %d", engine);
     SPX_REQUIRE(h_plan && h_totals && (B == 0 || h_shapes), "spx_ragged_plan: null shapes/plan/totals");
     SPX_REQUIRE(plan_bytes >= spx_ragged_plan_bytes(B), "spx_ragged_plan: plan_bytes = %lld < spx_ragged_plan_bytes(%lld) = %lld",
                 (long long)plan_bytes, (long long)B, (long long)spx_ragged_plan_bytes(B));
     RaggedPlan *P = static_cast<RaggedPlan *>(h_plan);
     RaggedLp *lps = reinterpret_cast<RaggedLp *>(static_cast<char *>(h_plan) + ragged_lp_offset());
     int32_t *order = reinterpret_cast<int32_t *>(lps + B);
-    // class of every LP: 0 warp mode, 1 CTA mode, 2 + log2(S) cluster; and its shared-memory footprint
+    // class of every LP: 0 warp mode, 1 CTA mode, 2 + log2(S) K7, 7 + log2(S) K8; and its shared-memory footprint
+    const int forced = (int)spx_launch::get_option(SPX_OPT_CLUSTER_SIZE);
     std::vector<int8_t> cls((size_t)B);
     std::vector<int64_t> bytes((size_t)B);
     int64_t tot[5] = {0, 0, 0, 0, 0};
@@ -647,8 +654,23 @@ int spx_ragged_plan(const int32_t *h_shapes, int64_t B, int32_t engine, void *h_
         SPX_REQUIRE(n >= 1 && m >= 1 && cap >= 0, "spx_ragged_plan: LP %lld: bad shape n=%d m=%d max_pivots=%d",
                     (long long)k, n, m, cap);
         const int64_t cells = spx_cells(n, m);
-        const bool k4 = engine == SPX_ENGINE_SMEM || (engine == SPX_ENGINE_AUTO && cells <= spx_batched_max_cells());
-        if (k4) {
+        const bool k4 = engine == SPX_ENGINE_SMEM ||
+                        ((engine == SPX_ENGINE_AUTO || engine == SPX_ENGINE_AUTO_GLOBAL) && cells <= spx_batched_max_cells());
+        const bool k8 = engine == SPX_ENGINE_GLOBAL ||
+                        (engine == SPX_ENGINE_AUTO_GLOBAL && !k4 && spx_launch::cluster_size(n, m) == 0);
+        if (k8) {
+            const int smin = spx_launch::global_min_cluster_size(n, m);
+            SPX_REQUIRE(smin > 0,
+                        "spx_ragged_plan: LP %lld: a %d x %d LP exceeds the shared memory of one cluster (16 CTAs of "
+                        "227 KB: 8*(2m+1+R) + 4*(R+Q) <= 230400 bytes with R = ceil(n/S), Q = ceil(m/S), S <= 16)",
+                        (long long)k, n, m);
+            SPX_REQUIRE(forced == 0 || smin <= forced,
+                        "spx_ragged_plan: LP %lld: a %d x %d LP does not fit a cluster of SPX_OPT_CLUSTER_SIZE = %d CTAs "
+                        "(8*(2m+1+R) + 4*(R+Q) <= 230400 bytes; at least %d CTAs)", (long long)k, n, m, forced, smin);
+            const int S = forced ? forced : smin;
+            bytes[k] = spx_launch::ragged_global_bytes(n, m, S);
+            cls[k] = (int8_t)(7 + __builtin_ctz((unsigned)S));
+        } else if (k4) {
             int kern = 0;
             bytes[k] = spx_launch::ragged_batched_bytes(n, m, &kern);
             SPX_REQUIRE(bytes[k] > 0 || cells > spx_batched_max_cells(),
@@ -675,7 +697,8 @@ int spx_ragged_plan(const int32_t *h_shapes, int64_t B, int32_t engine, void *h_
         tot[3] += cap;
         tot[4] += ((int64_t)cap + 1) * cells;
     }
-    // launches: warp mode, CTA mode, then K7 by cluster size; inside each, by cells descending, ties by index
+    // launches: warp mode, CTA mode, K7 by cluster size, then K8 by S_min (or the forced S); inside each, by cells
+    // descending, ties by index
     std::vector<int32_t> idx((size_t)B);
     for (int64_t k = 0; k < B; ++k) idx[k] = (int32_t)k;
     std::stable_sort(idx.begin(), idx.end(), [&](int32_t u, int32_t v) {
@@ -704,10 +727,11 @@ int spx_ragged_plan(const int32_t *h_shapes, int64_t B, int32_t engine, void *h_
             l.threads = spx_launch::ragged_cta_threads(lps[idx[q]].cells);     // the largest LP comes first
             l.smem = big;
         } else {
-            l.kernel = RAGGED_CLUSTER;
-            l.S = 1 << (c - 2);
+            l.kernel = c < 7 ? RAGGED_CLUSTER : RAGGED_GLOBAL;
+            l.S = 1 << (c < 7 ? c - 2 : c - 7);
             l.threads = 512;
             l.smem = big;
+            l.pick_S = (l.kernel == RAGGED_GLOBAL && forced == 0) ? 1 : 0;
             SPX_REQUIRE(l.count <= INT32_MAX / l.S, "spx_ragged_plan: %lld LPs x S = %d CTAs exceed one grid",
                         (long long)l.count, l.S);
         }
@@ -738,8 +762,8 @@ int spx_solve_batched_ragged(double *d_T, const void *h_plan, const void *d_plan
                 P->lp_offset == ragged_lp_offset() && P->order_offset == P->lp_offset + P->B * (int64_t)sizeof(RaggedLp);
     for (int i = 0; sane && i < P->nlaunch; ++i) {
         const RaggedLaunch &l = P->launch[i];
-        sane = l.first == counted && l.count >= 1 && l.kernel >= RAGGED_WARP && l.kernel <= RAGGED_CLUSTER &&
-               l.per_cta >= 1 && l.threads >= 32 && l.S >= 1 && l.S <= 16;
+        sane = l.first == counted && l.count >= 1 && l.kernel >= RAGGED_WARP && l.kernel <= RAGGED_GLOBAL &&
+               l.per_cta >= 1 && l.threads >= 32 && l.S >= 1 && l.S <= 16 && (l.pick_S == 0 || l.kernel == RAGGED_GLOBAL);
         counted += l.count;
     }
     SPX_REQUIRE(sane && counted == P->B, "spx_solve_batched_ragged: inconsistent plan header (B = %lld)", (long long)P->B);
@@ -748,9 +772,28 @@ int spx_solve_batched_ragged(double *d_T, const void *h_plan, const void *d_plan
     SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_solve_batched_ragged: unknown rule %d", rule);
     const RaggedLp *lps = reinterpret_cast<const RaggedLp *>(static_cast<const char *>(d_plan) + P->lp_offset);
     const int32_t *order = reinterpret_cast<const int32_t *>(static_cast<const char *>(d_plan) + P->order_offset);
+    const RaggedLp *h_lps = reinterpret_cast<const RaggedLp *>(static_cast<const char *>(h_plan) + P->lp_offset);
+    const int32_t *h_order = reinterpret_cast<const int32_t *>(static_cast<const char *>(h_plan) + P->order_offset);
     cudaStream_t s = as_stream(stream);
     for (int i = 0; i < P->nlaunch; ++i) {
         const RaggedLaunch &l = P->launch[i];
+        if (l.kernel == RAGGED_GLOBAL) {
+            int S = 0;
+            int64_t smem = 0;
+            if (check(spx_launch::ragged_global_size(l, h_lps, h_order, &S, &smem), "spx_solve_batched_ragged: occupancy"))
+                return -1;
+            SPX_REQUIRE(l.count <= INT32_MAX / S, "spx_solve_batched_ragged: %lld LPs x S = %d CTAs exceed one grid",
+                        (long long)l.count, S);
+            const cudaError_t e = spx_launch::solve_ragged_global(l, S, smem, lps, order, d_T, rule, d_x, d_obj, d_status,
+                                                                  d_npiv, d_rowlab, d_collab, d_trace, d_snap, s);
+            if (e == cudaErrorInvalidClusterSize) {
+                set_error("spx_solve_batched_ragged: the device cannot co-schedule one cluster of S = %d CTAs with %lld "
+                          "bytes of shared memory each (cudaOccupancyMaxActiveClusters = 0)", S, (long long)smem);
+                return -1;
+            }
+            if (check(e, "ragged global launch")) return -1;
+            continue;
+        }
         if (l.kernel != RAGGED_CLUSTER) {
             if (check(spx_launch::solve_ragged_batched(l, lps, order, d_T, rule, d_x, d_obj, d_status, d_npiv, d_rowlab,
                                                        d_collab, d_trace, d_snap, s), "ragged batched launch"))
@@ -767,6 +810,27 @@ int spx_solve_batched_ragged(double *d_T, const void *h_plan, const void *d_plan
         if (check(e, "ragged cluster launch")) return -1;
     }
     return 0;
+}
+
+int32_t spx_ragged_cluster_size(const void *h_plan, int32_t launch) {
+    using namespace spx;
+    const RaggedPlan *P = static_cast<const RaggedPlan *>(h_plan);
+    if (!P || P->magic != RAGGED_MAGIC || P->abi != SPX_ABI_VERSION) {
+        set_error("spx_ragged_cluster_size: h_plan is not a plan of this library (null, or magic / ABI version mismatch)");
+        return -1;
+    }
+    if (launch < 0 || launch >= P->nlaunch || P->nlaunch > RAGGED_MAX_LAUNCHES) {
+        set_error("spx_ragged_cluster_size: launch %d of a plan of %d launches", launch, P->nlaunch);
+        return -1;
+    }
+    const RaggedLaunch &l = P->launch[launch];
+    if (l.kernel != RAGGED_GLOBAL) return l.S;
+    const RaggedLp *h_lps = reinterpret_cast<const RaggedLp *>(static_cast<const char *>(h_plan) + P->lp_offset);
+    const int32_t *h_order = reinterpret_cast<const int32_t *>(static_cast<const char *>(h_plan) + P->order_offset);
+    int S = 0;
+    int64_t smem = 0;
+    if (check(spx_launch::ragged_global_size(l, h_lps, h_order, &S, &smem), "spx_ragged_cluster_size")) return -1;
+    return S;
 }
 
 // ---- column-sharded flow ----------------------------------------------------------

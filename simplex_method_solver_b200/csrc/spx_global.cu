@@ -30,6 +30,8 @@
 // in one place, the pivot row (owned by one CTA, read by all); the owner wrote it in the update of the previous
 // pivot, before its arrival at barrier A, whose release/acquire at cluster scope orders it before the read.  Every
 // other read of d_T is of the CTA's own band, ordered by __syncthreads().
+#include <algorithm>
+
 #include "spx_cluster.cuh"
 
 namespace cg = cooperative_groups;
@@ -74,7 +76,12 @@ __device__ __forceinline__ double2 ld_l2_v2(const double *p) {
     return v;
 }
 
-__global__ void __launch_bounds__(GLOBAL_THREADS, GLOBAL_MIN_CTAS) global_kernel(GlobalArgs a) {
+// The body of both kernels.  RAGGED == false: shape, R, Q and offsets from the arguments (one shape per launch).
+// RAGGED == true: LP order[blockIdx.x / S] of a ragged batch, its shape and offsets from lps[], R and Q from its shape
+// (as cluster_body in spx_cluster.cu).
+template <bool RAGGED>
+__device__ __forceinline__ void global_body(const GlobalArgs &a, const RaggedLp *__restrict__ lps,
+                                            const int32_t *__restrict__ order) {
     cg::cluster_group cluster = cg::this_cluster();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ Scratch sc;
@@ -82,9 +89,12 @@ __global__ void __launch_bounds__(GLOBAL_THREADS, GLOBAL_MIN_CTAS) global_kernel
     __shared__ int s_ctl[3];                               // {status, r, c} of the merged decision
     __shared__ double s_x01[2];                            // rank 0: b of the rows labelled x1, x2 (:49)
 
-    const int n = a.n, m = a.m, w1 = m + 1, S = a.S, R = a.R, Q = a.Q;
+    RaggedLp lpd;
+    if (RAGGED) lpd = lps[order[blockIdx.x / (unsigned)a.S]];
+    const int n = RAGGED ? lpd.n : a.n, m = RAGGED ? lpd.m : a.m, w1 = m + 1, S = a.S;
+    const int R = RAGGED ? (n + S - 1) / S : a.R, Q = RAGGED ? (m + S - 1) / S : a.Q;
     const int rank = (int)cluster.block_rank();
-    const int64_t lp = (int64_t)(blockIdx.x / (unsigned)S);
+    const int64_t lp = RAGGED ? (int64_t)order[blockIdx.x / (unsigned)S] : (int64_t)(blockIdx.x / (unsigned)S);
     const int tid = (int)threadIdx.x, nt = (int)blockDim.x;
     const int r0 = rank * R;                               // first body row of this band
     const int rows = max(0, min(R, n - r0));
@@ -100,7 +110,7 @@ __global__ void __launch_bounds__(GLOBAL_THREADS, GLOBAL_MIN_CTAS) global_kernel
 
     const int64_t cells = (int64_t)n * w1 + m;
     const int64_t fo = (int64_t)n * w1;                    // offset of the f row
-    double *Tg = a.T + lp * cells;
+    double *Tg = a.T + (RAGGED ? lpd.t : lp * cells);
     double *band = Tg + (int64_t)r0 * w1;                  // [rows][w1], in place
     // 16-byte accesses: a band starts at 8-byte alignment only, so a misaligned first cell and an odd last cell
     // are done one at a time
@@ -118,8 +128,8 @@ __global__ void __launch_bounds__(GLOBAL_THREADS, GLOBAL_MIN_CTAS) global_kernel
     const double f1 = (m >= 2) ? f[1] : 0.0;
 
     int npiv = 0, status;
-    double *snap = a.snap ? a.snap + lp * (int64_t)(a.max_pivots + 1) * cells : nullptr;
-    int32_t *trace = a.trace ? a.trace + lp * (int64_t)a.max_pivots * 2 : nullptr;
+    double *snap = a.snap ? a.snap + (RAGGED ? lpd.sn : lp * (int64_t)(a.max_pivots + 1) * cells) : nullptr;
+    int32_t *trace = a.trace ? a.trace + (RAGGED ? 2 * lpd.tr : lp * (int64_t)a.max_pivots * 2) : nullptr;
 
     for (;;) {
         if (snap) {
@@ -163,7 +173,7 @@ __global__ void __launch_bounds__(GLOBAL_THREADS, GLOBAL_MIN_CTAS) global_kernel
         status = s_ctl[0];
         const int r = s_ctl[1], c = s_ctl[2];
         if (status != SPX_PIVOT) break;
-        if (npiv >= a.max_pivots) { status = SPX_CAP; break; }
+        if (npiv >= (RAGGED ? lpd.max_pivots : a.max_pivots)) { status = SPX_CAP; break; }
 
         // ---- stash the old pivot row and the band's old pivot-column entries
         const int owner = r / R, holder = c / Q;           // owners of row r and of the header label of column c
@@ -245,7 +255,7 @@ __global__ void __launch_bounds__(GLOBAL_THREADS, GLOBAL_MIN_CTAS) global_kernel
 
     // ---- epilogue: the band is final in place; f row, labels, find_optimum()/f() (:48-68)
     if (rank == 0) for (int j = tid; j < m; j += nt) Tg[fo + j] = f[j];
-    double *xg = a.x ? a.x + lp * m : nullptr;
+    double *xg = a.x ? a.x + (RAGGED ? lpd.xm : lp * m) : nullptr;
     // labels are a permutation of 0..n+m-1: x_j is the b of the row labelled x_j, or 0 when a column carries it
     for (int i = tid; i < rows; i += nt) {
         const int lab = cl[i];
@@ -254,12 +264,12 @@ __global__ void __launch_bounds__(GLOBAL_THREADS, GLOBAL_MIN_CTAS) global_kernel
             if (xg) xg[lab] = v;
             if (lab < 2) *cluster.map_shared_rank(&s_x01[lab], 0) = v;
         }
-        if (a.collab) a.collab[lp * n + r0 + i] = lab;
+        if (a.collab) a.collab[(RAGGED ? lpd.xn : lp * n) + r0 + i] = lab;
     }
     for (int j = tid; j < cols; j += nt) {
         const int lab = rl[j];
         if (xg && lab < m) xg[lab] = 0.0;
-        if (a.rowlab) a.rowlab[lp * m + j0 + j] = lab;
+        if (a.rowlab) a.rowlab[(RAGGED ? lpd.xm : lp * m) + j0 + j] = lab;
     }
     cluster.sync();                                        // s_x01 complete; no CTA leaves while a peer may read it
     if (rank == 0 && tid == 0) {
@@ -267,6 +277,17 @@ __global__ void __launch_bounds__(GLOBAL_THREADS, GLOBAL_MIN_CTAS) global_kernel
         a.npiv[lp] = npiv;
         if (a.obj) a.obj[lp] = (m >= 2) ? __dadd_rn(__dmul_rn(f0, s_x01[0]), __dmul_rn(f1, s_x01[1])) : 0.0;
     }
+}
+
+__global__ void __launch_bounds__(GLOBAL_THREADS, GLOBAL_MIN_CTAS) global_kernel(GlobalArgs a) {
+    global_body<false>(a, nullptr, nullptr);
+}
+
+// a ragged batch: the LPs order[0 .. a.B) at one cluster size a.S, each cluster its own shape (a.n, a.m, a.R, a.Q,
+// a.max_pivots unused)
+__global__ void __launch_bounds__(GLOBAL_THREADS, GLOBAL_MIN_CTAS)
+ragged_global_kernel(GlobalArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order) {
+    global_body<true>(a, lps, order);
 }
 
 // the per-CTA footprint of the header comment, for S CTAs per LP
@@ -279,30 +300,41 @@ bool global_fits(int64_t n, int64_t m, int S) {
     return n >= 1 && m >= 1 && global_bytes(n, m, S) <= (int64_t)GLOBAL_DYN_BYTES;
 }
 
-// one-time per-device set-up of the kernel's shared memory and cluster size limits
-cudaError_t configure() {
-    static bool configured_dev[64] = {};
+// one-time per-device set-up of a K8 kernel's shared memory and cluster size limits
+template <typename Kernel>
+cudaError_t configure_kernel(Kernel kernel, bool (&configured_dev)[64]) {
     const int slot = spx_host::device_slot();
     if (configured_dev[slot]) return cudaSuccess;
     cudaFuncAttributes fa;
-    cudaError_t e = cudaFuncGetAttributes(&fa, global_kernel);
+    cudaError_t e = cudaFuncGetAttributes(&fa, kernel);
     if (e != cudaSuccess) return e;
     if (fa.sharedSizeBytes > GLOBAL_STATIC) return cudaErrorInvalidValue;
-    e = cudaFuncSetAttribute(global_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GLOBAL_DYN_BYTES);
+    e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GLOBAL_DYN_BYTES);
     if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(global_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+    e = cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
     if (e != cudaSuccess) return e;
     configured_dev[slot] = true;
     return cudaSuccess;
 }
 
-// launch configuration of `clusters` LPs at S CTAs each; attr must outlive cfg
-cudaLaunchConfig_t launch_config(int64_t n, int64_t m, int S, int64_t clusters, cudaLaunchAttribute *attr,
+cudaError_t configure() {
+    static bool configured_dev[64] = {};
+    return configure_kernel(global_kernel, configured_dev);
+}
+
+cudaError_t configure_ragged() {
+    static bool configured_dev[64] = {};
+    return configure_kernel(ragged_global_kernel, configured_dev);
+}
+
+// launch configuration of `clusters` LPs at S CTAs each with `smem` bytes of dynamic shared memory per CTA; attr must
+// outlive cfg
+cudaLaunchConfig_t launch_config(int64_t smem, int S, int64_t clusters, cudaLaunchAttribute *attr,
                                  cudaStream_t stream) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)(clusters * S));
     cfg.blockDim = dim3(GLOBAL_THREADS);
-    cfg.dynamicSmemBytes = (size_t)global_bytes(n, m, S);
+    cfg.dynamicSmemBytes = (size_t)smem;
     cfg.stream = stream;
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = (unsigned)S;
@@ -313,11 +345,34 @@ cudaLaunchConfig_t launch_config(int64_t n, int64_t m, int S, int64_t clusters, 
     return cfg;
 }
 
-// clusters of S CTAs for an n x m LP the current device co-schedules
-cudaError_t max_clusters(int64_t n, int64_t m, int S, int *clusters) {
-    cudaLaunchAttribute attr[1];
-    const cudaLaunchConfig_t cfg = launch_config(n, m, S, 1, attr, nullptr);
-    return cudaOccupancyMaxActiveClusters(clusters, global_kernel, &cfg);
+// The default cluster size of a K8 launch of `count` LPs on the current device: the S >= s_lo that keeps the most SMs
+// busy, min(count, co-resident clusters at S) * S, the smaller S on ties; bytes(S) is the launch's footprint at S
+// (which fits for every S >= s_lo: it does not grow with S).  A CTA streams its band at a rate bounded by its own
+// bytes in flight, so an idle SM is lost bandwidth, while a larger S costs barrier time per pivot: a single LP gets
+// 16 CTAs, a batch that fills the GPU at s_lo gets s_lo.
+template <typename Kernel, typename Bytes>
+cudaError_t busiest_cluster_size(Kernel kernel, int s_lo, int64_t count, Bytes bytes, int *S_out) {
+    int64_t best = -1;
+    for (int S = s_lo; S <= GLOBAL_MAX_S; S *= 2) {
+        cudaLaunchAttribute attr[1];
+        const cudaLaunchConfig_t cfg = launch_config(bytes(S), S, 1, attr, nullptr);
+        int clusters = 0;
+        const cudaError_t e = cudaOccupancyMaxActiveClusters(&clusters, kernel, &cfg);
+        if (e != cudaSuccess) return e;
+        const int64_t busy = (count < clusters ? count : (int64_t)clusters) * S;
+        if (busy > best) { best = busy; *S_out = S; }
+    }
+    return cudaSuccess;
+}
+
+// the largest footprint at S over the LPs of one ragged launch (host copies of the plan's descriptors)
+int64_t launch_bytes(const RaggedLaunch &l, const RaggedLp *lps, const int32_t *order, int S) {
+    int64_t big = 0;
+    for (int64_t q = l.first; q < l.first + l.count; ++q) {
+        const RaggedLp &d = lps[order[q]];
+        big = std::max(big, global_bytes(d.n, d.m, S));
+    }
+    return big;
 }
 
 } // namespace
@@ -333,11 +388,8 @@ int global_min_cluster_size(int64_t n, int64_t m) {
     return 0;
 }
 
-// S for a solve of B LPs on the current device: SPX_OPT_CLUSTER_SIZE when set (0 if that S does not fit); else the
-// S >= S_min that keeps the most SMs busy, min(B, co-resident clusters at S) * S, the smaller S on ties (0 when the
-// LP does not fit).  A CTA streams its band at a rate bounded by its own bytes in flight, so an idle SM is lost
-// bandwidth, while a larger S costs barrier time per pivot: a single LP gets 16 CTAs, a batch that fills the GPU
-// at S_min gets S_min.
+// S for a solve of B LPs on the current device: SPX_OPT_CLUSTER_SIZE when set (0 if that S does not fit); else
+// busiest_cluster_size() from S_min (0 when the LP does not fit)
 cudaError_t global_cluster_size(int64_t n, int64_t m, int64_t B, int *S_out) {
     *S_out = 0;
     const int forced = (int)get_option(SPX_OPT_CLUSTER_SIZE);
@@ -349,15 +401,7 @@ cudaError_t global_cluster_size(int64_t n, int64_t m, int64_t B, int *S_out) {
     if (smin == 0) return cudaSuccess;
     cudaError_t e = configure();
     if (e != cudaSuccess) return e;
-    int64_t best = -1;
-    for (int S = smin; S <= GLOBAL_MAX_S; S *= 2) {
-        int clusters = 0;
-        e = max_clusters(n, m, S, &clusters);
-        if (e != cudaSuccess) return e;
-        const int64_t busy = (B < clusters ? B : (int64_t)clusters) * S;
-        if (busy > best) { best = busy; *S_out = S; }
-    }
-    return cudaSuccess;
+    return busiest_cluster_size(global_kernel, smin, B, [&](int S) { return global_bytes(n, m, S); }, S_out);
 }
 
 // S CTAs per LP (validated by the caller); returns cudaErrorInvalidClusterSize when the device cannot co-schedule
@@ -371,12 +415,53 @@ cudaError_t solve_batched_global(double *T, int64_t B, int n, int m, int S, int 
     GlobalArgs a{T, B, n, m, rule, max_pivots, S, (n + S - 1) / S, (m + S - 1) / S,
                  x, obj, status, npiv, rowlab, collab, trace, snap};
     cudaLaunchAttribute attr[1];
-    const cudaLaunchConfig_t cfg = launch_config(n, m, S, B, attr, stream);
+    const cudaLaunchConfig_t cfg = launch_config(global_bytes(n, m, S), S, B, attr, stream);
     int clusters = 0;
     e = cudaOccupancyMaxActiveClusters(&clusters, global_kernel, &cfg);
     if (e != cudaSuccess) return e;
     if (clusters <= 0) return cudaErrorInvalidClusterSize;
     e = cudaLaunchKernelEx(&cfg, global_kernel, a);
+    spx_host::count_launch();
+    if (e != cudaSuccess) return e;
+    return cudaGetLastError();
+}
+
+int64_t ragged_global_bytes(int n, int m, int S) { return global_bytes(n, m, S); }
+
+// The S and footprint one K8 launch of a ragged plan runs at on the current device: as planned when l.pick_S == 0
+// (no device needed), else busiest_cluster_size() from the planned S over the launch's largest footprint at each S.
+// h_lps / h_order: the host plan's descriptors.
+cudaError_t ragged_global_size(const RaggedLaunch &l, const RaggedLp *h_lps, const int32_t *h_order, int *S_out,
+                               int64_t *smem_out) {
+    *S_out = l.S;
+    *smem_out = l.smem;
+    if (!l.pick_S) return cudaSuccess;
+    cudaError_t e = configure_ragged();
+    if (e != cudaSuccess) return e;
+    e = busiest_cluster_size(ragged_global_kernel, l.S, l.count,
+                             [&](int S) { return launch_bytes(l, h_lps, h_order, S); }, S_out);
+    if (e != cudaSuccess) return e;
+    *smem_out = launch_bytes(l, h_lps, h_order, *S_out);
+    return cudaSuccess;
+}
+
+// one K8 launch of a ragged plan: the l.count LPs order[l.first ..] at S CTAs each with smem bytes per CTA (from
+// ragged_global_size); cudaErrorInvalidClusterSize when the device cannot co-schedule one such cluster
+cudaError_t solve_ragged_global(const RaggedLaunch &l, int S, int64_t smem, const RaggedLp *lps, const int32_t *order,
+                                double *T, int rule, double *x, double *obj, int32_t *status, int32_t *npiv,
+                                int32_t *rowlab, int32_t *collab, int32_t *trace, double *snap, cudaStream_t stream) {
+    if (l.count <= 0) return cudaSuccess;
+    cudaError_t e = configure_ragged();
+    if (e != cudaSuccess) return e;
+    GlobalArgs a{T, l.count, 0, 0, rule, 0, S, 0, 0, x, obj, status, npiv, rowlab, collab, trace, snap};
+    cudaLaunchAttribute attr[1];
+    const cudaLaunchConfig_t cfg = launch_config(smem, S, l.count, attr, stream);
+    int clusters = 0;
+    e = cudaOccupancyMaxActiveClusters(&clusters, ragged_global_kernel, &cfg);
+    if (e != cudaSuccess) return e;
+    if (clusters <= 0) return cudaErrorInvalidClusterSize;
+    const int32_t *ord = order + l.first;
+    e = cudaLaunchKernelEx(&cfg, ragged_global_kernel, a, lps, ord);
     spx_host::count_launch();
     if (e != cudaSuccess) return e;
     return cudaGetLastError();

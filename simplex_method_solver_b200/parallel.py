@@ -683,8 +683,9 @@ def solve_ragged_sharded(lps, max_pivots=64, rule: str = "reference", rank: Opti
                          trace: bool = True, snapshots: bool = False):
     """Each rank solves its contiguous, cell-balanced share of a ragged batch; no collective on the data path.
 
-    `lps` and `max_pivots` as ``batched.solve_ragged``.  Returns (start, count, RaggedResult) for this
-    rank.  `solver` defaults to the CUDA ``solve_ragged``; tests pass a stand-in.
+    `lps`, `max_pivots` and `engine` (including "global" and "auto_global") as ``batched.solve_ragged``.
+    Returns (start, count, RaggedResult) for this rank.  `solver` defaults to the CUDA ``solve_ragged``;
+    tests pass a stand-in.
     """
     from .engine import as_rows_function
     if rank is None:

@@ -24,6 +24,10 @@ Differences from the reference, all opt-in or unavoidable:
     table in shared memory), which writes the per-pivot snapshots itself; for
     LPs above the one-CTA limit of ``engine="warp"``.  ``solve()`` keeps the
     streaming loop, as with ``"warp"``.
+  * ``engine="global"``: the same with the global-memory cluster kernel (K8,
+    the table stays in HBM and each CTA of the cluster updates its band of
+    rows in place), for LPs above K7's capacity up to K8's.  ``solve()`` keeps
+    the streaming loop.
   * ``engine="sharded"``: one process per GPU (torchrun); every rank constructs
     the same ``SimplexMethod`` and calls ``solve()`` — the body is split into
     column blocks over the ranks of ``group`` (the default process group) and
@@ -91,7 +95,7 @@ class SimplexMethod:
         self.column = ['y' + str(k) for k in range(1, self.n + 1)] + ['f']    # :31,:33
         if rule not in N.RULES:
             raise ValueError(f"unknown rule {rule!r}")
-        if engine not in ("auto", "warp", "stream", "sharded", "cluster"):
+        if engine not in ("auto", "warp", "stream", "sharded", "cluster", "global"):
             raise ValueError(f"unknown engine {engine!r}")
         self._rule = N.RULES[rule]
         self._engine = engine
@@ -234,8 +238,8 @@ class SimplexMethod:
     def _use_warp(self):
         if self._engine == "stream":
             return False
-        if self._engine == "cluster":
-            kernel_for(self.n, self.m, "cluster")        # ValueError above the cluster capacity
+        if self._engine in ("cluster", "global"):
+            kernel_for(self.n, self.m, self._engine)     # ValueError above the engine's capacity
             return True
         cells = self.n * (self.m + 1) + self.m
         fits = cells <= N.load().spx_batched_max_cells()
@@ -282,11 +286,17 @@ class SimplexMethod:
                            None, None, x1, x2, self.f(x1, x2)))   # :197-198
 
     def _solve_warp(self, result, budget, snapshots):
-        """Whole loop in one shared-memory-resident kernel launch (K4, or K7 with engine="cluster")
+        """Whole loop in one batched kernel launch (K4, K7 with engine="cluster", K8 with engine="global")
         per round of `cap` pivots."""
         n, m = self.n, self.m
-        engine = "cluster" if self._engine == "cluster" else "smem"
-        cap = 64
+        engine = self._engine if self._engine in ("cluster", "global") else "smem"
+        # rounds of up to `limit` pivots, so that one round's snapshots, (cap + 1) * cells doubles, stay under ~256 MB:
+        # K4 and K7 tables are small enough for rounds of 64 and more; a K8 table may allow fewer, down to one pivot
+        # (two snapshot tables) for the largest
+        cells = n * (m + 1) + m
+        limit = (256 << 20) // (8 * cells)
+        limit = max(1, limit - 1) if engine == "global" else max(64, limit)
+        cap = min(64, limit)
         while True:
             cap = min(cap, max(budget, 0))
             db = DeviceBatch(1, n, m, max_pivots=cap, trace=True, snapshots=True,
@@ -307,8 +317,7 @@ class SimplexMethod:
             budget -= k
             if status != N.CAP or budget <= 0:
                 return status
-            # grow the round, bounded so one round's snapshots stay under ~256 MB
-            cap = min(cap * 4, max(64, (256 << 20) // (8 * (n * (m + 1) + m))))
+            cap = min(cap * 4, limit)                        # grow the round up to the bound above
 
     def _push_labels(self):
         code = lambda s: int(s[1:]) - 1 if s[0] == 'x' else self.m + int(s[1:]) - 1  # noqa: E731

@@ -101,6 +101,23 @@ def mixed_lps(B: int, seed: int = 0):
     return out
 
 
+def mixed_large_lps(B: int = 1024, seed: int = 0):
+    """mixed_lps(B, seed) with cap 20,000 each, then 32 LPs above K7's capacity with cap 4,000 each: 8 each of
+    D(600, 800), phase-1 1000 x 1000, D(2000, 300) and D(64, 12000), in that order (seeds seed * 1_000_003 + B + q
+    for the q-th of them).  Every K4 class, every K7 cluster size and two K8 launches (S_min 1, and S_min 2 for
+    64 x 12000).  Returns (lps, caps): a list of B + 32 (rows [n, m+1], c [m]) pairs and the list of their caps."""
+    lps = mixed_lps(B, seed)
+    caps = [20000] * len(lps)
+    large = [(dense_lp, 600, 800), (phase1_lp, 1000, 1000), (dense_lp, 2000, 300), (dense_lp, 64, 12000)]
+    q = 0
+    for fam, n, m in large:
+        for _ in range(8):
+            lps.append(fam(n, m, seed * 1_000_003 + B + q))
+            caps.append(4000)
+            q += 1
+    return lps, caps
+
+
 def klee_minty(n: int):
     """KM(n): Klee-Minty cube, all floats (cfg5: n=20, 2^n - 1 pivots)."""
     rows = []
