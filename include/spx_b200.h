@@ -339,6 +339,43 @@ int spx_solve_batched_ragged(double *d_T, const void *h_plan, const void *d_plan
  * nothing).  -1 on error. */
 int32_t spx_ragged_cluster_size(const void *h_plan, int32_t launch);
 
+/* ---- sensitivity report of optimal final tables (csrc/spx_sensitivity.cu) ------- */
+/* The final table is a dictionary: x_B = b + T x_N, f = f0 + sum_j d_j x_N (recalculate_matrix,
+ * :143-177); the LP is: minimise c.x subject to b + A x >= 0, x >= 0.  Constraint k's slack is y_k.
+ * Per constraint k (n of each; ranges are [n][2] = (allowable decrease, allowable increase)):
+ *   y_k nonbasic in column j: dual = -d_j, slack = 0, rhs_range = (min over rows i with T[i][j] < 0
+ *                             of b_i / (-T[i][j]), min over rows with T[i][j] > 0 of b_i / T[i][j]);
+ *   y_k basic in row i:       dual = 0, slack = b_i, rhs_range = (b_i, +inf).
+ * Per variable k (m of each):
+ *   x_k nonbasic in column j: reduced_cost = d_j, cost_range = (d_j, +inf);
+ *   x_k basic in row i:       reduced_cost = 0, cost_range = (min over columns j with T[i][j] > 0 of
+ *                             d_j / T[i][j], min over columns with T[i][j] < 0 of d_j / (-T[i][j])).
+ * Each quotient is one IEEE division; a minimum over an empty set is +inf, a NaN quotient never
+ * wins, every zero is written as +0.0, and every output of an LP that is not optimal is NaN.  A
+ * minimum does not depend on the order of reduction, so the results equal a sequential statement
+ * bit for bit.  Labels and status are required; each output pointer may be NULL.  Arguments and
+ * shapes (and the plan header) are checked before the device is touched; B = 0 returns 0.
+ *
+ * Uniform batches: d_T [B][cells] final reference-flat tables (DeviceBatch after K4, K7 or K8),
+ * d_status [B], d_rowlab [B][m], d_collab [B][n]; d_dual, d_slack [B][n], d_rhs_range [B][n][2],
+ * d_redcost [B][m], d_cost_range [B][m][2].  An LP is optimal when d_status[k] == SPX_OPTIMAL. */
+int spx_sensitivity_batched(const double *d_T, int64_t B, int32_t n, int32_t m, const int32_t *d_status,
+                            const int32_t *d_rowlab, const int32_t *d_collab, double *d_dual, double *d_slack,
+                            double *d_redcost, double *d_rhs_range, double *d_cost_range, void *stream);
+/* Ragged batches packed as spx_solve_batched_ragged packs them: per-constraint outputs at the prefix
+ * sums of n (as d_collab; ranges twice that), per-variable outputs at the prefix sums of m (as d_x). */
+int spx_sensitivity_ragged(const double *d_T, const void *h_plan, const void *d_plan, const int32_t *d_status,
+                           const int32_t *d_rowlab, const int32_t *d_collab, double *d_dual, double *d_slack,
+                           double *d_redcost, double *d_rhs_range, double *d_cost_range, void *stream);
+/* One split table (d_A [(n+1)][ld], d_b [n]; d_rowlab [m], d_collab [n]), e.g. the current table of
+ * a streaming solve.  Optimality is decided from the table with pick_element's tests (:72-76 and
+ * :94-98: no b cell and no f cell negative), which copies b and the f row to the host and
+ * synchronises `stream`; *h_optimal = 1 when optimal, else 0 and every output is NaN. */
+int spx_sensitivity_split(const double *d_A, const double *d_b, int32_t n, int32_t m, int64_t ld,
+                          const int32_t *d_rowlab, const int32_t *d_collab, double *d_dual, double *d_slack,
+                          double *d_redcost, double *d_rhs_range, double *d_cost_range, int32_t *h_optimal,
+                          void *stream);
+
 /* ---- column-sharded large tableau (one process per GPU) ------------------- */
 /* Rank g owns global columns [col0, col0+m_loc) of the body as a local split
  * matrix d_A[(n+1)][ld_loc]; b, the labels and the state are replicated.  Per pivot:

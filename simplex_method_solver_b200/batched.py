@@ -42,6 +42,46 @@ class BatchResult(NamedTuple):
     snaps: Optional[np.ndarray]   # [B, max_pivots+1, cells]
 
 
+class Sensitivity(NamedTuple):
+    """Sensitivity report of optimal LPs (spx_sensitivity_*, include/spx_b200.h): the LP is "minimise c.x subject to
+    b + A x >= 0 and x >= 0", constraint k's slack is y_k.  Every output of an LP that is not optimal is NaN.
+    Ranges are (allowable decrease, allowable increase), +inf when unbounded."""
+    dual: np.ndarray              # [B, n] shadow price of each constraint, d f* / d b_k
+    slack: np.ndarray             # [B, n] value of each constraint's slack y_k at the optimum
+    reduced_cost: np.ndarray      # [B, m]
+    rhs_range: np.ndarray         # [B, n, 2] how far b_k may move before the optimal basis changes
+    cost_range: np.ndarray        # [B, m, 2] how far c_k may move before the optimal basis changes
+    optimal: np.ndarray           # [B] bool
+
+
+class _SensOut:
+    """Device outputs of one sensitivity call: nc per-constraint and nv per-variable entries."""
+
+    def __init__(self, nc: int, nv: int, device):
+        f64, q = torch.float64, (lambda k: max(k, 1))  # noqa: E731
+        self.nc, self.nv = nc, nv
+        self.t = [torch.empty(q(nc), dtype=f64, device=device), torch.empty(q(nc), dtype=f64, device=device),
+                  torch.empty(q(nv), dtype=f64, device=device), torch.empty(q(2 * nc), dtype=f64, device=device),
+                  torch.empty(q(2 * nv), dtype=f64, device=device)]
+
+    def ptrs(self):
+        return [t.data_ptr() for t in self.t]
+
+    def host(self):
+        nc, nv = self.nc, self.nv
+        return [t[:k].cpu().numpy() for t, k in zip(self.t, (nc, nc, nv, 2 * nc, 2 * nv))]
+
+
+def _sens_uniform(T, status, rowlab, collab, B: int, n: int, m: int, device) -> Sensitivity:
+    out = _SensOut(B * n, B * m, device)
+    with torch.cuda.device(device):
+        N.call("spx_sensitivity_batched", T.data_ptr(), B, n, m, status.data_ptr(), rowlab.data_ptr(),
+               collab.data_ptr(), *out.ptrs(), torch.cuda.current_stream(device).cuda_stream)
+    dual, slack, rc, rr, cr = out.host()
+    return Sensitivity(dual.reshape(B, n), slack.reshape(B, n), rc.reshape(B, m), rr.reshape(B, n, 2),
+                       cr.reshape(B, m, 2), status[:B].cpu().numpy() == N.OPTIMAL)
+
+
 ENGINES = ("auto", "smem", "cluster", "global", "auto_global")
 _INT32_MAX = (1 << 31) - 1
 
@@ -156,6 +196,10 @@ class DeviceBatch:
                    N.ptr(self.trace), N.ptr(self.snaps),
                    torch.cuda.current_stream(self.device).cuda_stream)
 
+    def sensitivity(self) -> Sensitivity:
+        """Sensitivity report of the final tables the last ``run`` left (K4, K7 and K8 alike); synchronises."""
+        return _sens_uniform(self.T, self.status, self.rowlab, self.collab, self.B, self.n, self.m, self.device)
+
     def result(self) -> BatchResult:
         B = self.B
         g = lambda t: None if t is None else t[:B].cpu().numpy()  # noqa: E731
@@ -266,6 +310,38 @@ class RaggedResult(NamedTuple):
                            None if self.snaps is None else self.snaps[sn: sn + (cap + 1) * cells].reshape(1, cap + 1, cells))
 
 
+class RaggedSensitivity(NamedTuple):
+    """Sensitivity report of a ragged batch, packed in batch order: per-constraint outputs at the prefix sums of n
+    (as ``collab``), per-variable outputs at the prefix sums of m (as ``x``)."""
+    dual: np.ndarray              # [sum n]
+    slack: np.ndarray             # [sum n]
+    reduced_cost: np.ndarray      # [sum m]
+    rhs_range: np.ndarray         # [sum n, 2]
+    cost_range: np.ndarray        # [sum m, 2]
+    optimal: np.ndarray           # [B] bool
+    shapes: np.ndarray            # [B, 3] int64: n, m, max_pivots
+    offsets: np.ndarray           # [B, 5] int64, as RaggedResult.offsets
+
+    def lp(self, k: int) -> Sensitivity:
+        """LP k alone, with the shapes ``DeviceBatch.sensitivity()`` gives for a batch of that one LP."""
+        n, m = int(self.shapes[k, 0]), int(self.shapes[k, 1])
+        xm, xn = int(self.offsets[k, 1]), int(self.offsets[k, 2])
+        return Sensitivity(self.dual[xn: xn + n][None], self.slack[xn: xn + n][None],
+                           self.reduced_cost[xm: xm + m][None], self.rhs_range[xn: xn + n][None],
+                           self.cost_range[xm: xm + m][None], self.optimal[k: k + 1])
+
+
+def _sens_ragged(T, h_plan: np.ndarray, d_plan, status, rowlab, collab, B: int, totals, shapes, offsets,
+                 device) -> RaggedSensitivity:
+    out = _SensOut(int(totals[2]), int(totals[1]), device)
+    with torch.cuda.device(device):
+        N.call("spx_sensitivity_ragged", T.data_ptr(), h_plan.ctypes.data, d_plan.data_ptr(), status.data_ptr(),
+               rowlab.data_ptr(), collab.data_ptr(), *out.ptrs(), torch.cuda.current_stream(device).cuda_stream)
+    dual, slack, rc, rr, cr = out.host()
+    return RaggedSensitivity(dual, slack, rc, rr.reshape(-1, 2), cr.reshape(-1, 2),
+                             status[:B].cpu().numpy() == N.OPTIMAL, shapes.copy(), offsets.copy())
+
+
 def _caps(max_pivots: Union[int, Sequence[int]], B: int) -> np.ndarray:
     caps = np.asarray(max_pivots, dtype=np.int64)
     if caps.ndim == 0:
@@ -351,6 +427,11 @@ class DeviceRaggedBatch:
                    self.rowlab.data_ptr(), self.collab.data_ptr(), N.ptr(self.trace), N.ptr(self.snaps),
                    torch.cuda.current_stream(self.device).cuda_stream)
 
+    def sensitivity(self) -> RaggedSensitivity:
+        """Sensitivity report of the final tables the last ``run`` left; synchronises."""
+        return _sens_ragged(self.T, self.plan.plan, self.d_plan, self.status, self.rowlab, self.collab, self.B,
+                            self.totals, self.shapes, self.offsets, self.device)
+
     def result(self) -> RaggedResult:
         B, tot = self.B, self.totals
         g = lambda t, k: None if t is None else t[:k].cpu().numpy()  # noqa: E731
@@ -388,3 +469,46 @@ def solve_ragged(lps, max_pivots: Union[int, Sequence[int]] = 64, rule: str = "r
         db.upload(packed)
         db.run(N.RULES[rule])
     return db.result()
+
+
+def sensitivity(result: Union[BatchResult, RaggedResult], device=None) -> Union[Sensitivity, RaggedSensitivity]:
+    """Sensitivity report of the final tables of a host ``BatchResult`` (``solve_batched``) or ``RaggedResult``
+    (``solve_ragged``): uploads the tables, labels and status and runs the report's kernels on ``device``."""
+    dev = torch.device(device if device is not None else "cuda")
+    up = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dtype=dt).reshape(-1)).to(dev)  # noqa: E731
+    if isinstance(result, RaggedResult):
+        shapes = np.asarray(result.shapes, dtype=np.int64).reshape(-1, 3)
+        B = shapes.shape[0]
+        plan = ragged_plan(shapes[:, :2], shapes[:, 2], "auto_global")
+        lp = plan.lps
+        offsets = np.stack([lp["t"], lp["xm"], lp["xn"], lp["tr"], lp["sn"]], axis=1).astype(np.int64)
+        if not np.array_equal(offsets, np.asarray(result.offsets, dtype=np.int64).reshape(-1, 5)):
+            raise ValueError("result.offsets are not the packing of result.shapes")
+        tot = [int(v) for v in plan.totals]
+        for name, a, k in (("tables", result.tables, tot[0]), ("rowlab", result.rowlab, tot[1]),
+                           ("collab", result.collab, tot[2]), ("status", result.status, B)):
+            if np.size(a) != k:
+                raise ValueError(f"result.{name} has {np.size(a)} entries, the shapes need {k}")
+        if B == 0:
+            z = np.zeros
+            return RaggedSensitivity(z(0), z(0), z(0), z((0, 2)), z((0, 2)), z(0, bool), shapes.copy(), offsets)
+        N.lib()
+        return _sens_ragged(up(result.tables, np.float64), plan.plan, torch.from_numpy(plan.plan).to(dev),
+                            up(result.status, np.int32), up(result.rowlab, np.int32), up(result.collab, np.int32),
+                            B, tot, shapes, offsets, dev)
+    if not isinstance(result, BatchResult):
+        raise TypeError(f"sensitivity() takes a BatchResult or a RaggedResult, not {type(result).__name__}")
+    rowlab, collab = np.asarray(result.rowlab), np.asarray(result.collab)
+    if rowlab.ndim != 2 or collab.ndim != 2 or rowlab.shape[0] != collab.shape[0]:
+        raise ValueError("result.rowlab must be [B, m] and result.collab [B, n]")
+    B, m, n = rowlab.shape[0], rowlab.shape[1], collab.shape[1]
+    if n < 1 or m < 1:
+        raise ValueError(f"bad shape {n} x {m}")
+    if np.shape(result.tables) != (B, n * (m + 1) + m) or np.shape(result.status) != (B,):
+        raise ValueError(f"result.tables must be [B, n*(m+1)+m] = [{B}, {n * (m + 1) + m}] and result.status [{B}]")
+    if B == 0:
+        z = np.zeros
+        return Sensitivity(z((0, n)), z((0, n)), z((0, m)), z((0, n, 2)), z((0, m, 2)), z(0, bool))
+    N.lib()
+    return _sens_uniform(up(result.tables, np.float64), up(result.status, np.int32), up(rowlab, np.int32),
+                         up(collab, np.int32), B, n, m, dev)

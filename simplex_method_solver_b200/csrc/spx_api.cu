@@ -72,6 +72,13 @@ cudaError_t ragged_global_size(const spx::RaggedLaunch &, const spx::RaggedLp *,
 cudaError_t solve_ragged_global(const spx::RaggedLaunch &, int, int64_t, const spx::RaggedLp *, const int32_t *,
                                 double *, int, double *, double *, int32_t *, int32_t *, int32_t *, int32_t *,
                                 int32_t *, double *, cudaStream_t);
+cudaError_t sensitivity_uniform(const double *, int64_t, int, int, const int32_t *, const int32_t *, const int32_t *,
+                                double *, double *, double *, double *, double *, cudaStream_t);
+cudaError_t sensitivity_ragged(const spx::RaggedPlan *, const spx::RaggedLp *, const int32_t *, const double *,
+                               const spx::RaggedLp *, const int32_t *, const int32_t *, const int32_t *,
+                               const int32_t *, double *, double *, double *, double *, double *, cudaStream_t);
+cudaError_t sensitivity_split(const double *, const double *, int, int, int64_t, int, const int32_t *, const int32_t *,
+                              double *, double *, double *, double *, double *, cudaStream_t);
 } // namespace spx_launch
 
 namespace spx_host {
@@ -749,14 +756,9 @@ int spx_ragged_plan(const int32_t *h_shapes, int64_t B, int32_t engine, void *h_
     return 0;
 }
 
-int spx_solve_batched_ragged(double *d_T, const void *h_plan, const void *d_plan, int32_t rule, double *d_x,
-                             double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab, int32_t *d_collab,
-                             int32_t *d_trace, double *d_snap, void *stream) {
+// the launch list of a plan covers its B LPs exactly once, in order
+static bool ragged_header_sane(const spx::RaggedPlan *P) {
     using namespace spx;
-    SPX_REQUIRE(h_plan, "spx_solve_batched_ragged: null plan");
-    const RaggedPlan *P = static_cast<const RaggedPlan *>(h_plan);
-    SPX_REQUIRE(P->magic == RAGGED_MAGIC && P->abi == SPX_ABI_VERSION,
-                "spx_solve_batched_ragged: h_plan is not a plan of this library (magic / ABI version mismatch)");
     int64_t counted = 0;
     bool sane = P->B >= 0 && P->nlaunch >= 0 && P->nlaunch <= RAGGED_MAX_LAUNCHES &&
                 P->lp_offset == ragged_lp_offset() && P->order_offset == P->lp_offset + P->B * (int64_t)sizeof(RaggedLp);
@@ -766,7 +768,18 @@ int spx_solve_batched_ragged(double *d_T, const void *h_plan, const void *d_plan
                l.per_cta >= 1 && l.threads >= 32 && l.S >= 1 && l.S <= 16 && (l.pick_S == 0 || l.kernel == RAGGED_GLOBAL);
         counted += l.count;
     }
-    SPX_REQUIRE(sane && counted == P->B, "spx_solve_batched_ragged: inconsistent plan header (B = %lld)", (long long)P->B);
+    return sane && counted == P->B;
+}
+
+int spx_solve_batched_ragged(double *d_T, const void *h_plan, const void *d_plan, int32_t rule, double *d_x,
+                             double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab, int32_t *d_collab,
+                             int32_t *d_trace, double *d_snap, void *stream) {
+    using namespace spx;
+    SPX_REQUIRE(h_plan, "spx_solve_batched_ragged: null plan");
+    const RaggedPlan *P = static_cast<const RaggedPlan *>(h_plan);
+    SPX_REQUIRE(P->magic == RAGGED_MAGIC && P->abi == SPX_ABI_VERSION,
+                "spx_solve_batched_ragged: h_plan is not a plan of this library (magic / ABI version mismatch)");
+    SPX_REQUIRE(ragged_header_sane(P), "spx_solve_batched_ragged: inconsistent plan header (B = %lld)", (long long)P->B);
     if (P->B == 0) return 0;
     SPX_REQUIRE(d_plan && d_T && d_status && d_npiv, "spx_solve_batched_ragged: null d_plan/T/status/npiv");
     SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_solve_batched_ragged: unknown rule %d", rule);
@@ -831,6 +844,65 @@ int32_t spx_ragged_cluster_size(const void *h_plan, int32_t launch) {
     int64_t smem = 0;
     if (check(spx_launch::ragged_global_size(l, h_lps, h_order, &S, &smem), "spx_ragged_cluster_size")) return -1;
     return S;
+}
+
+// ---- sensitivity report of optimal final tables (csrc/spx_sensitivity.cu) -------------
+int spx_sensitivity_batched(const double *d_T, int64_t B, int32_t n, int32_t m, const int32_t *d_status,
+                            const int32_t *d_rowlab, const int32_t *d_collab, double *d_dual, double *d_slack,
+                            double *d_redcost, double *d_rhs_range, double *d_cost_range, void *stream) {
+    SPX_REQUIRE(B >= 0 && n >= 1 && m >= 1, "spx_sensitivity_batched: bad arguments (B = %lld, n = %d, m = %d)",
+                (long long)B, n, m);
+    if (B == 0) return 0;
+    SPX_REQUIRE(d_T && d_status && d_rowlab && d_collab, "spx_sensitivity_batched: null T/status/rowlab/collab");
+    return check(spx_launch::sensitivity_uniform(d_T, B, n, m, d_status, d_rowlab, d_collab, d_dual, d_slack,
+                                                 d_redcost, d_rhs_range, d_cost_range, as_stream(stream)),
+                 "sensitivity launch");
+}
+
+int spx_sensitivity_ragged(const double *d_T, const void *h_plan, const void *d_plan, const int32_t *d_status,
+                           const int32_t *d_rowlab, const int32_t *d_collab, double *d_dual, double *d_slack,
+                           double *d_redcost, double *d_rhs_range, double *d_cost_range, void *stream) {
+    using namespace spx;
+    SPX_REQUIRE(h_plan, "spx_sensitivity_ragged: null plan");
+    const RaggedPlan *P = static_cast<const RaggedPlan *>(h_plan);
+    SPX_REQUIRE(P->magic == RAGGED_MAGIC && P->abi == SPX_ABI_VERSION,
+                "spx_sensitivity_ragged: h_plan is not a plan of this library (magic / ABI version mismatch)");
+    SPX_REQUIRE(ragged_header_sane(P), "spx_sensitivity_ragged: inconsistent plan header (B = %lld)", (long long)P->B);
+    if (P->B == 0) return 0;
+    SPX_REQUIRE(d_plan && d_T && d_status && d_rowlab && d_collab,
+                "spx_sensitivity_ragged: null d_plan/T/status/rowlab/collab");
+    const char *h = static_cast<const char *>(h_plan), *d = static_cast<const char *>(d_plan);
+    return check(spx_launch::sensitivity_ragged(P, reinterpret_cast<const RaggedLp *>(h + P->lp_offset),
+                                                reinterpret_cast<const int32_t *>(h + P->order_offset), d_T,
+                                                reinterpret_cast<const RaggedLp *>(d + P->lp_offset),
+                                                reinterpret_cast<const int32_t *>(d + P->order_offset), d_status,
+                                                d_rowlab, d_collab, d_dual, d_slack, d_redcost, d_rhs_range,
+                                                d_cost_range, as_stream(stream)),
+                 "ragged sensitivity launch");
+}
+
+int spx_sensitivity_split(const double *d_A, const double *d_b, int32_t n, int32_t m, int64_t ld,
+                          const int32_t *d_rowlab, const int32_t *d_collab, double *d_dual, double *d_slack,
+                          double *d_redcost, double *d_rhs_range, double *d_cost_range, int32_t *h_optimal,
+                          void *stream) {
+    SPX_REQUIRE(n >= 1 && m >= 1 && ld >= m, "spx_sensitivity_split: bad arguments (n = %d, m = %d, ld = %lld)", n, m,
+                (long long)ld);
+    SPX_REQUIRE(d_A && d_b && d_rowlab && d_collab && h_optimal, "spx_sensitivity_split: null A/b/rowlab/collab/optimal");
+    // pick_element's tests, simplex.py:72-76 and :94-98: optimal when no b cell and no f cell is negative
+    cudaStream_t s = as_stream(stream);
+    std::vector<double> hb((size_t)n), hf((size_t)m);
+    if (check(cudaMemcpyAsync(hb.data(), d_b, sizeof(double) * n, cudaMemcpyDeviceToHost, s), "spx_sensitivity_split: copy b") ||
+        check(cudaMemcpyAsync(hf.data(), d_A + (int64_t)n * ld, sizeof(double) * m, cudaMemcpyDeviceToHost, s),
+              "spx_sensitivity_split: copy f") ||
+        check(cudaStreamSynchronize(s), "spx_sensitivity_split: synchronize"))
+        return -1;
+    int optimal = 1;
+    for (double v : hb) optimal &= !(v < 0);
+    for (double v : hf) optimal &= !(v < 0);
+    *h_optimal = optimal;
+    return check(spx_launch::sensitivity_split(d_A, d_b, n, m, ld, optimal, d_rowlab, d_collab, d_dual, d_slack,
+                                               d_redcost, d_rhs_range, d_cost_range, s),
+                 "split sensitivity launch");
 }
 
 // ---- column-sharded flow ----------------------------------------------------------

@@ -40,11 +40,13 @@ Differences from the reference, all opt-in or unavoidable:
 """
 from __future__ import annotations
 
+import ctypes
+
 import numpy as np
 import torch
 
 from . import _native as N
-from .batched import DeviceBatch, kernel_for
+from .batched import DeviceBatch, Sensitivity, _SensOut, kernel_for
 from .engine import DeviceTableau, Solution, as_rows_function
 
 CAP_TEXT = "pivot limit reached"
@@ -385,6 +387,23 @@ class SimplexMethod:
         sol = dev.solution(status, self._npiv)
         self._labels_from_codes(sol.rowlab, sol.collab)
         return sol
+
+    def sensitivity(self) -> Sensitivity:
+        """Sensitivity report of the current table, which must be optimal: after ``solve()``, ``get_solution()``
+        or step-API pivots.  Arrays without the batch axis: dual, slack [n], reduced_cost [m], rhs_range [n, 2],
+        cost_range [m, 2]; ``optimal`` is True.  ValueError when the current table is not optimal."""
+        self._not_sharded("sensitivity()")
+        dev, n, m = self._dev, self.n, self.m
+        c = dev.cur(self._npiv)
+        out = _SensOut(n, m, dev.device)
+        optimal = ctypes.c_int32(0)
+        dev._call("spx_sensitivity_split", dev.A[c].data_ptr(), dev.b[c].data_ptr(), n, m, dev.ld,
+                  dev.rowlab.data_ptr(), dev.collab.data_ptr(), *out.ptrs(), ctypes.byref(optimal))
+        if not optimal.value:
+            raise ValueError("sensitivity() needs an optimal table: the current table has a negative b or f cell "
+                             "(solve the LP to optimality first)")
+        dual, slack, rc, rr, cr = out.host()
+        return Sensitivity(dual, slack, rc, rr.reshape(n, 2), cr.reshape(m, 2), True)
 
     def _labels_from_codes(self, rowlab, collab):
         name = lambda v: f"x{v + 1}" if v < self.m else f"y{v - self.m + 1}"  # noqa: E731
