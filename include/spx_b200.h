@@ -92,20 +92,17 @@ int         spx_device_info(int32_t *sm_count, int32_t *cc_major, int32_t *cc_mi
 int64_t     spx_launch_count(int reset);
 
 /* process-wide tuning knobs; every setting computes bit-identical results */
-#define SPX_OPT_UPDATE_KERNEL    1  /* 0 auto (by body size), 1 tiled, 2 persistent TMA-pipelined */
+/* Keys 1, 3, 4, 10 and 15 are retired: they selected kernel variants that measured slower than the defaults and
+ * were removed.  spx_set_option rejects them with any value and spx_get_option reads 0; the numbers are never reused. */
 #define SPX_OPT_TILED_MIN_BLOCKS 2  /* tiled kernel: resident CTAs per SM the register budget targets (1..4) */
-#define SPX_OPT_PIPE_ORDER       3  /* pipelined kernel tile order: 0 chunked column-major, 1 interleaved row-major */
-#define SPX_OPT_PIPE_GRID        4  /* pipelined kernel CTAs (0 = one per SM) */
 #define SPX_OPT_TILED_ROWS       5  /* tiled kernel rows per tile (0 = auto; else a multiple of 8 <= 64) */
 #define SPX_OPT_FUSE_DEPTH       6  /* fused loop: pivots applied per pass over the body (0 = default 8, max 8) */
 #define SPX_OPT_FUSE_MIN_BLOCKS  7  /* fused update kernel: resident CTAs per SM its register budget targets (2..4, 0 = default 3) */
 #define SPX_OPT_FUSE_PRICING     8  /* fused loop pricing kernel: 0 auto, 1 one CTA, 2 whole-GPU cooperative */
 #define SPX_OPT_FUSE_LOOKAHEAD   9  /* fused loop in spx_solve: 1 = price pass q+1 on a side stream during update q, 2 = the same with the persistent pricing engine (see spx_fshard_set_lookahead); default 0: off on one GPU */
-#define SPX_OPT_FUSE_VARIANT     10 /* fused update kernel: 0 default (lazy range guard: one range test per cell per PASS), 1 = round 1's kernel (range test per cell per level) */
 #define SPX_OPT_FUSE_TILE_ROWS   11 /* fused update kernel: rows of the strip one warp walks (0 = 128; a multiple of 8 <= 4096) */
 #define SPX_OPT_SHARD_THREADS    13 /* sharded / look-ahead pricing kernel: threads per CTA, one CTA per SM (0 = default 512; 64..512, multiple of 32) */
 #define SPX_OPT_SHARD_CTAS       14 /* sharded / look-ahead pricing kernel: at most this many CTAs (0 = one per SM) */
-#define SPX_OPT_RESIDENT_VARIANT 15 /* L2-resident persistent loop: 0 default (price, sweep, one grid barrier per pivot), 1 = look-ahead pricing inside the CTA with the sweep rows prefetched by cp.async (bit-identical; measured slower on cfg2, kept selectable) */
 #define SPX_OPT_FUSE_PAIRS       12 /* fused update kernel: column pairs per lane, i.e. strip width / 64 (0 = default 2; 1 or 2) */
 #define SPX_OPT_CLUSTER_SIZE     16 /* K7 and K8 (spx_solve_batched_cluster, spx_solve_batched_global, and ragged plans, read when the plan is made): CTAs per LP, 1, 2, 4, 8 or 16 (0 = default: spx_cluster_size(n, m) for K7, spx_global_cluster_size(n, m, B) for K8, spx_ragged_cluster_size for a ragged K8 launch); a size whose footprint does not fit is rejected */
 int         spx_set_option(int32_t option, int64_t value);
@@ -490,7 +487,7 @@ int spx_fshard_close(spx_fshard *h);
  * stored on every rank, keys exchanged over NVLink, ratio partials in (grid barrier 2), level recorded}.
  * Synchronises `stream`.  No reference counterpart. */
 int spx_fused_debug_stamps(const void *d_work, int32_t n, int64_t ld, uint64_t *h_out, int32_t capacity, void *stream);
-/* Developer aid: with SPX_RESIDENT_STAMPS=1 in the environment the L2-resident persistent kernels accumulate clock64()
+/* Developer aid: with SPX_RESIDENT_STAMPS=1 in the environment the L2-resident persistent kernel accumulates clock64()
  * cycles per phase of a pivot (thread 0 of CTA 0); h_out16[0..14] = the sums over the last launch in the order of the
  * kernel's pc.mark(k) calls (csrc/spx_resident.cu), h_out16[15] = pivots applied.  No reference counterpart. */
 int spx_resident_debug(uint64_t *h_out16);

@@ -20,9 +20,10 @@ LOOP_MODES = {None: LOOP_AUTO, "auto": LOOP_AUTO, False: LOOP_CLASSIC, "classic"
               "fused": LOOP_FUSED}
 PIVOT, OPTIMAL, INCORRECT, NOCONV, CAP, PEER_TIMEOUT = 1, 0, -1, -2, -3, -4
 RULE_REFERENCE, RULE_DANTZIG = 0, 1
-OPT_UPDATE_KERNEL, OPT_TILED_MIN_BLOCKS, OPT_PIPE_ORDER, OPT_PIPE_GRID, OPT_TILED_ROWS, OPT_FUSE_DEPTH = 1, 2, 3, 4, 5, 6
-OPT_FUSE_MIN_BLOCKS, OPT_FUSE_PRICING, OPT_FUSE_LOOKAHEAD, OPT_FUSE_VARIANT, OPT_FUSE_TILE_ROWS, OPT_FUSE_PAIRS = 7, 8, 9, 10, 11, 12
-OPT_SHARD_THREADS, OPT_SHARD_CTAS, OPT_RESIDENT_VARIANT, OPT_CLUSTER_SIZE = 13, 14, 15, 16
+# keys 1, 3, 4, 10 and 15 are retired (include/spx_b200.h)
+OPT_TILED_MIN_BLOCKS, OPT_TILED_ROWS, OPT_FUSE_DEPTH = 2, 5, 6
+OPT_FUSE_MIN_BLOCKS, OPT_FUSE_PRICING, OPT_FUSE_LOOKAHEAD, OPT_FUSE_TILE_ROWS, OPT_FUSE_PAIRS = 7, 8, 9, 11, 12
+OPT_SHARD_THREADS, OPT_SHARD_CTAS, OPT_CLUSTER_SIZE = 13, 14, 16
 RULES = {"reference": RULE_REFERENCE, "bland": RULE_REFERENCE, "dantzig": RULE_DANTZIG}
 ENGINE_AUTO, ENGINE_SMEM, ENGINE_CLUSTER, ENGINE_GLOBAL, ENGINE_AUTO_GLOBAL = 0, 1, 2, 4, 5
 

@@ -242,259 +242,15 @@ resident_loop_kernel(ResidentArgs a) {
     }
 }
 
-// ---- K5b: the same loop with LOOK-AHEAD PRICING inside the CTA -------------------------------------------
-// In resident_loop_kernel a pivot is a chain of dependent L2 round trips: f row -> (reduce) -> column gather ->
-// (reduce) -> pivot row + tile loads -> update -> grid barrier: 11.2 us at cfg2, of which the sweep is ~4.  But pivot
-// k+1 does not need table k+1: the b column, the f row (or the phase-1 row) and the entering column of table k+1 are
-// O(n + m) cells that follow from table k and pivot k by the update's own arithmetic (apply_level: same operations,
-// same roundings — the idea of the fused loop K6, one level deep).  So, per pivot, every CTA
-//   1. starts the loads of ITS slice of sweep k: cp.async (16 B per thread per row, L2 -> shared memory, the
-//      thread's own slots, nobody else reads them) — in flight while it prices;
-//   2. prices pivot k+1 from table k through the pending level k (redundantly in every CTA, as before): running
-//      b column in place, f head / phase-1 row / Dantzig scan on lazily evaluated cells, lazy column gather into
-//      the other s_col buffer, ratio test;
-//   3. finishes sweep k from shared memory (rows beyond the prefetch capacity: plain batched loads) and stores;
-//   4. one grid barrier: table k+1 is complete — and its pivot is already chosen.
-// The critical path of a pivot drops from (pricing + sweep + barrier) to (pricing with the sweep's loads underneath
-// + the sweep's arithmetic + barrier).
-constexpr int RES_PF_ROW_BYTES = RES_THREADS * 16;       // one prefetched row of a slice: a double2 per thread
-constexpr int RES_PASS_AHEAD   = 8;                      // rows per batch of the rows that were not prefetched
-
-template <bool STAMPS>
-__global__ void __launch_bounds__(RES_THREADS, 1)
-resident_ahead_kernel(ResidentArgs a, int pf_rows) {
-    cg::grid_group grid = cg::this_grid();
-    extern __shared__ __align__(16) double res_smem[];
-    __shared__ Scratch s;
-    const int n = a.n, m = a.m;
-    const int64_t ld = a.ld;
-    const int colw = (n + 2) & ~1;
-    double *s_colv[2] = {res_smem, res_smem + colw};            // [n + 1] pivot column of the current / next table
-    double *s_b = res_smem + 2 * colw;                          // [n] this CTA's replica of the '-b' column
-    double2 *s_pf = reinterpret_cast<double2 *>(res_smem + 2 * colw + ((n + 1) & ~1));   // [pf_rows][RES_THREADS]
-    const int tid = threadIdx.x, nt = blockDim.x;
-
-    int64_t npiv = a.st->npiv;
-    const int64_t cap = a.st->max_pivots;
-    if (a.st->status != SPX_PIVOT) return;          // uniform over the grid: nobody reaches a barrier
-    int cur = (int)(npiv & 1);
-    for (int i = tid; i < n; i += nt) s_b[i] = __ldcg(a.b[cur] + i);
-    __syncthreads();
-
-    const int n_ct = (m + RES_TC - 1) / RES_TC;
-    const int per_ct = max(1, (int)gridDim.x / n_ct);          // CTAs that share one column tile
-    const int rpc = (n + 1 + per_ct - 1) / per_ct;             // rows per CTA
-    const int head = min(m, 4 * nt);
-
-    int status = SPX_PIVOT, r = -1, r1 = -1, cl = SPX_NONE, c = 0;
-    double p = 0.0;
-    int64_t steps = 0;
-    bool have = false;                              // a chosen pivot (r, cl, p, s_colv[c]) waits to be applied
-    __shared__ unsigned long long s_acc[STAMPS ? RES_DBG : 1];
-    PhaseClock<STAMPS> pc; pc.start(s_acc, blockIdx.x == 0 && tid == 0);
-    for (;;) {
-        pc.mark(0);                                 // (loop overhead, exit checks)
-        const double *A = a.A[cur];
-        double *An = a.A[cur ^ 1];
-        LevelDiv L; L.r = r; L.c = cl; L.d = pivot_div_prepare(have ? p : 1.0);
-        const double *s_col = s_colv[c];            // column cl of table k (valid when have)
-        double *s_new = s_colv[have ? (c ^ 1) : c]; // receives the entering column of the table being priced
-        const double *ROWk = A + (int64_t)(have ? r : 0) * ld;
-
-        // ---------------- 1. this CTA's first unit of sweep k: rows into shared memory, asynchronously
-        const int unit0 = blockIdx.x;
-        const bool own0 = have && unit0 < n_ct * per_ct && (unit0 % n_ct) * RES_TC + 2 * tid < m;
-        int pf = 0;
-        double2 rj0 = make_double2(0.0, 0.0);
-        if (own0) {
-            const int j = (unit0 % n_ct) * RES_TC + 2 * tid, i0 = (unit0 / n_ct) * rpc;
-            pf = max(0, min(pf_rows, min(n + 1, i0 + rpc) - i0));
-            for (int u = 0; u < pf; ++u)
-                asm volatile("cp.async.cg.shared.global [%0], [%1], 16;"
-                             :: "r"(smem_u32(s_pf + (size_t)u * RES_THREADS + tid)), "l"(A + (int64_t)(i0 + u) * ld + j) : "memory");
-            rj0 = ldcg2(ROWk + j);
-        }
-        asm volatile("cp.async.commit_group;" ::: "memory");
-        pc.mark(1);                                 // prefetch issued
-        // ---------------- 2. price the next pivot: from table k directly (!have) or through level k (have)
-        // cell (t, j) of the table being priced, from its stored value
-        auto cellv = [&](double raw, int t, int j, double rowj) -> double {
-            return have ? apply_level(raw, t, j, L, rowj, s_col[t]) : raw;
-        };
-        int nstatus = SPX_PIVOT, nr = r, nr1 = -1, ncl = SPX_NONE;
-        double np_ = p;
-        {
-            int bneg = SPX_NONE, fneg = SPX_NONE;
-            const double *frow = A + (int64_t)n * ld;
-            double fv[4], rv[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int j = u * nt + tid;
-                fv[u] = (j < head) ? __ldcg(frow + j) : 0.0;
-                rv[u] = (have && j < head) ? __ldcg(ROWk + j) : 0.0;
-            }
-            if (have) {                                   // running b column, in place (:155-156, :166-175 on the last column)
-                const double br = s_b[r];
-                __syncthreads();
-                for (int i = tid; i < n; i += nt) {
-                    const double bi = s_b[i];
-                    const double v = (i == r) ? pivot_div(-bi, L.d) : cell_update(bi, L.d, br, s_col[i]);
-                    s_b[i] = v;
-                    if (v < 0.0) bneg = min(bneg, i);
-                }
-            } else {
-                for (int i = tid; i < n; i += nt) if (s_b[i] < 0.0) { bneg = i; break; }
-            }
-#pragma unroll
-            for (int u = 3; u >= 0; --u) {
-                const int j = u * nt + tid;
-                if (j < head && cellv(fv[u], n, j, rv[u]) < 0.0) fneg = j;
-            }
-            pc.mark(2);                                   // running b + f head (loads, lazy evaluation)
-            block_min_int2(bneg, fneg, s);                // (its barriers also publish the new s_b)
-            pc.mark(3);                                   // first reduction
-            nr1 = (bneg == SPX_NONE) ? -1 : bneg;
-            if (nr1 >= 0) {
-                const double *row = A + (int64_t)nr1 * ld;
-                ncl = block_first_index_fn(m, [&](int j) { return cellv(__ldcg(row + j), nr1, j, have ? __ldcg(ROWk + j) : 0.0); },
-                                           IsPos(), s);                                             // :82-85
-            } else if (a.rule == SPX_RULE_REFERENCE) {
-                ncl = fneg;                                                                         // :94-98
-                if (ncl == SPX_NONE && m > head) {
-                    const int rest = block_first_index_fn(m - head, [&](int j) {
-                        return cellv(__ldcg(frow + head + j), n, head + j, have ? __ldcg(ROWk + head + j) : 0.0); }, IsNeg(), s);
-                    ncl = (rest == SPX_NONE) ? SPX_NONE : head + rest;
-                }
-            } else {                                      // Dantzig: most negative, lowest index on ties
-                unsigned long long best = ~0ull;
-                for (int j = tid; j < m; j += nt) {
-                    const double v = cellv(__ldcg(frow + j), n, j, have ? __ldcg(ROWk + j) : 0.0);
-                    if (v < 0.0) { const unsigned long long k = orderable(v); best = k < best ? k : best; }
-                }
-                best = block_min_u64(best, s);
-                int loc = SPX_NONE;
-                if (best != ~0ull)
-                    for (int j = tid; j < m; j += nt) {
-                        const double v = cellv(__ldcg(frow + j), n, j, have ? __ldcg(ROWk + j) : 0.0);
-                        if (v < 0.0 && orderable(v) == best) { loc = j; break; }
-                    }
-                ncl = block_min_int(loc, s);
-            }
-            pc.mark(4);                                   // entering column decided
-            if (ncl == SPX_NONE) {
-                nstatus = (nr1 >= 0) ? SPX_INCORRECT : SPX_OPTIMAL;                                 // :88-89, :101-103
-            } else {
-                // the entering column of the priced table into s_new, ratio test against the running b
-                const double rc = have ? __ldcg(ROWk + ncl) : 0.0;
-                Ratio q = ratio_identity();
-                for (int i = tid; i <= n; i += nt) {
-                    const double v = cellv(__ldcg(A + (int64_t)i * ld + ncl), i, ncl, rc);
-                    s_new[i] = v;
-                    if (nr1 < 0 && i < n) ratio_accumulate(q, i, v, s_b[i]);
-                }
-                pc.mark(5);                               // lazy column gather + ratios
-                if (nr1 >= 0) {
-                    nr = nr1;                                                                       // :91
-                    __syncthreads();
-                } else {
-                    q = block_ratio_reduce(q, s);                                                   // syncs: s_new is complete
-                    bool elig_nan = false;
-                    if (q.elig_row != SPX_NONE) {
-                        const double v = __ddiv_rn(s_b[q.elig_row], s_new[q.elig_row]);
-                        elig_nan = (v != v);
-                    }
-                    nr = ratio_decide(q, elig_nan);                                                 // :138-141
-                    if (nr < 0) nstatus = SPX_NOCONV;
-                }
-                if (nstatus == SPX_PIVOT) np_ = s_new[nr];
-            }
-        }
-
-        pc.mark(6);                                 // ratio reduction + decision
-        // ---------------- 3. finish sweep k: this CTA's slices of the out-of-place update
-        if (have) {
-            asm volatile("cp.async.wait_group 0;" ::: "memory");
-            pc.mark(7);                             // wait for the prefetched rows
-            const PivotDiv d = L.d;
-            for (int unit = blockIdx.x; unit < n_ct * per_ct; unit += gridDim.x) {
-                const int ct = unit % n_ct, slice = unit / n_ct;
-                const int j = ct * RES_TC + 2 * tid;
-                if (j >= m) continue;
-                const int row_end = min(n + 1, (slice + 1) * rpc);
-                int i0 = slice * rpc;
-                const double2 rj = (unit == unit0) ? rj0 : ldcg2(ROWk + j);
-                const int jc = (cl >= j && cl < j + 2) ? cl - j : -1;
-                if (unit == unit0) {
-                    for (int u = 0; u < pf; ++u)
-                        stcg2(An + (int64_t)(i0 + u) * ld + j,
-                              generic_pair(s_pf[(size_t)u * RES_THREADS + tid], i0 + u, r, jc, rj, s_col[i0 + u], d));
-                    i0 += pf;
-                }
-                for (; i0 < row_end; i0 += RES_PASS_AHEAD) {     // rows beyond the prefetch capacity
-                    double2 tv[RES_PASS_AHEAD];
-#pragma unroll
-                    for (int u = 0; u < RES_PASS_AHEAD; ++u)
-                        if (i0 + u < row_end) tv[u] = ldcg2(A + (int64_t)(i0 + u) * ld + j);
-#pragma unroll
-                    for (int u = 0; u < RES_PASS_AHEAD; ++u)
-                        if (i0 + u < row_end)
-                            stcg2(An + (int64_t)(i0 + u) * ld + j,
-                                  generic_pair(tv[u], i0 + u, r, jc, rj, s_col[i0 + u], d));
-                }
-            }
-            if (blockIdx.x == 0 && tid == 0) {                 // labels (:152) and the pivot trace
-                const int32_t tmp = a.rowlab[cl]; a.rowlab[cl] = a.collab[r]; a.collab[r] = tmp;
-                if (a.trace) { a.trace[2 * npiv] = r; a.trace[2 * npiv + 1] = cl; }
-            }
-            ++npiv; ++steps; cur ^= 1; c ^= 1;
-            pc.mark(8);                             // sweep arithmetic + stores issued, labels
-            grid.sync();                                       // table k+1 is complete and visible in L2
-            pc.mark(9);                             // grid barrier
-        }
-        // ---------------- the priced pivot becomes the pending one
-        status = nstatus; r1 = nr1; cl = ncl;
-        if (ncl != SPX_NONE) r = nr;
-        p = np_;
-        if (status != SPX_PIVOT) break;
-        if (npiv >= cap) { status = SPX_CAP; break; }
-        if (steps >= a.max_steps) break;                   // priced, not applied: status stays SPX_PIVOT
-        have = true;
-    }
-
-    pc.finish((unsigned long long)steps);
-    // ---------------- exit (uniform): CTA 0 publishes the state, the b column and the priced column
-    if (blockIdx.x == 0) {
-        const double *s_col = s_colv[c];
-        __syncthreads();
-        for (int i = tid; i < n; i += nt) a.b[cur][i] = s_b[i];
-        if (status == SPX_PIVOT || status == SPX_CAP)
-            for (int i = tid; i <= n; i += nt) a.colbuf[i] = s_col[i];
-        if (tid == 0) {
-            spx_state o;
-            o.status = status; o.r = r; o.c = (cl == SPX_NONE) ? -1 : cl; o.p = p;
-            o.npiv = npiv; o.max_pivots = cap; o.phase1 = (r1 >= 0) ? 1 : 0; o.slot = 0;
-            o.hint_tag[0] = o.hint_tag[1] = -1;
-            o.hint_bneg[0] = o.hint_bneg[1] = SPX_NONE;
-            o.hint_fneg[0] = o.hint_fneg[1] = SPX_NONE;
-            for (int k = 0; k < 6; ++k) o.reserved[k] = 0;
-            *a.st = o;
-        }
-    }
-}
-
 int g_res_grid = -1;     // co-resident CTAs on this device (0: cooperative launch unsupported)
-constexpr int RES_SMEM_MAX = 227 * 1024 - 4096;          // opt-in dynamic shared memory per CTA, less the static part
 
 } // namespace
 
 namespace spx_launch {
 
 int sm_count();
-int64_t get_option(int key);
 
 size_t resident_smem(int n) { return (size_t)(((n + 2) & ~1) + n + 2) * sizeof(double); }
-// look-ahead kernel: two column buffers, the b replica, then the prefetch rows
-size_t resident_ahead_vectors(int n) { return (size_t)(2 * ((n + 2) & ~1) + ((n + 1) & ~1)) * sizeof(double); }
 
 // Can this tableau run in the resident loop?  (fits the shared-memory replicas and ~L2)
 bool resident_fits(int n, int m, int64_t ld) {
@@ -519,17 +275,12 @@ bool resident_fits(int n, int m, int64_t ld) {
     if (g_res_grid > 0 && !attr) {
         cudaFuncSetAttribute(resident_loop_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)resident_smem(RES_MAX_N));
         cudaFuncSetAttribute(resident_loop_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)resident_smem(RES_MAX_N));
-        cudaFuncSetAttribute(resident_ahead_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, RES_SMEM_MAX);
-        cudaFuncSetAttribute(resident_ahead_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, RES_SMEM_MAX);
         attr = true;
     }
     return g_res_grid > 0;
 }
 
 // Apply at most `max_steps` pivots in one persistent launch; the outcome is in *st.
-// SPX_OPT_RESIDENT_VARIANT 0 (default): resident_loop_kernel (price, sweep, barrier); 1: resident_ahead_kernel
-// (look-ahead pricing inside the CTA) — bit-identical, measured SLOWER on cfg2 (12.1 vs 11.2 us/pivot,
-// profiles/r2/r2n_resident_kernels_phase_cycles.md), kept selectable.
 cudaError_t resident_loop(double *A0, double *A1, double *b0, double *b1, int n, int m, int64_t ld, int rule,
                           int64_t max_steps, spx_state *st, double *colbuf, int32_t *rowlab, int32_t *collab,
                           int32_t *trace, cudaStream_t stream) {
@@ -545,23 +296,10 @@ cudaError_t resident_loop(double *A0, double *A1, double *b0, double *b1, int n,
     int grid = g_res_grid;
     if (units < grid) grid = (int)units;
     if (grid < 1) grid = 1;
-    cudaError_t e;
-    if ((int)get_option(SPX_OPT_RESIDENT_VARIANT) != 1) {
-        void *args[] = {&a};
-        e = cudaLaunchCooperativeKernel(stamps ? (const void *)resident_loop_kernel<true> : (const void *)resident_loop_kernel<false>,
-                                        dim3(grid), dim3(RES_THREADS), args, resident_smem(n), stream);
-    } else {
-        // rows of a CTA's slice that fit shared memory next to the vectors are prefetched during the pricing
-        const int per_ct = (int)((int64_t)grid / n_ct > 0 ? (int64_t)grid / n_ct : 1);
-        const int rpc = (n + 1 + per_ct - 1) / per_ct;
-        const size_t vec = resident_ahead_vectors(n);
-        int pf_rows = (int)(((size_t)RES_SMEM_MAX - vec) / RES_PF_ROW_BYTES);
-        if (pf_rows > rpc) pf_rows = rpc;
-        if (pf_rows < 0) pf_rows = 0;
-        void *args[] = {&a, &pf_rows};
-        e = cudaLaunchCooperativeKernel(stamps ? (const void *)resident_ahead_kernel<true> : (const void *)resident_ahead_kernel<false>,
-                                        dim3(grid), dim3(RES_THREADS), args, vec + (size_t)pf_rows * RES_PF_ROW_BYTES, stream);
-    }
+    void *args[] = {&a};
+    const cudaError_t e = cudaLaunchCooperativeKernel(
+        stamps ? (const void *)resident_loop_kernel<true> : (const void *)resident_loop_kernel<false>, dim3(grid),
+        dim3(RES_THREADS), args, resident_smem(n), stream);
     spx_host::count_launch();
     return e;
 }

@@ -8,24 +8,12 @@
 // 1 DMUL + 2 DFMA for the division by the pivot (reciprocal hoisted, see
 // pivot_div in spx_common.cuh) = 6 fp64 issues against 16 B of traffic.
 //
-// Two kernels, same arithmetic, same results:
-//
-//  update_tiled_kernel      one CTA per tile of TR (default 8) rows x 512 columns; a thread
-//      owns two adjacent columns (one 128-bit access per row) and walks down the
-//      rows: fully coalesced 512-byte line groups, the thread's two pivot-row
-//      values in registers, the column multiplier a shared-memory broadcast.  The
-//      pivot-row slice and the pivot-column slice are staged with two
-//      cp.async.bulk (TMA, SASS UBLKCP) copies on one mbarrier.  The default at every
-//      size: 8 rows in flight per thread, 4 CTAs per SM (64 registers), 6.8 TB/s at cfg4.
-//
-//  update_pipelined_kernel  persistent, warp-specialised, one CTA per SM: a
-//      producer lane streams tiles of 8 rows x 512 columns (32 KB) into a 6-stage
-//      shared-memory ring with cp.async.bulk (each stage also carries its slice of
-//      the pivot column and, when the column tile changes, of the pivot row);
-//      8 consumer warps read the stage with conflict-free 128-bit LDS, release it,
-//      compute and store straight to HBM with 128-bit streaming stores.  Up to
-//      ~190 KB of reads in flight per SM independent of register count.  Measured
-//      slower than the tiled kernel (5.5 vs 6.8 TB/s); selectable with spx_set_option.
+// update_tiled_kernel: one CTA per tile of TR (default 8) rows x 512 columns; a thread
+// owns two adjacent columns (one 128-bit access per row) and walks down the rows: fully
+// coalesced 512-byte line groups, the thread's two pivot-row values in registers, the
+// column multiplier a shared-memory broadcast.  The pivot-row slice and the pivot-column
+// slice are staged with two cp.async.bulk (TMA, SASS UBLKCP) copies on one mbarrier.
+// 8 rows in flight per thread, 4 CTAs per SM (64 registers): 6.8 TB/s at cfg4.
 //
 // Fused into the same pass: the b ('-b') column update, the label swap
 // (:152), the pivot trace, and the pricing of the NEXT pivot (first negative
@@ -171,170 +159,6 @@ update_tiled_kernel(const double *__restrict__ Ain, double *__restrict__ Aout,
     }
 }
 
-// ---- persistent TMA-pipelined kernel --------------------------------------------
-constexpr int PIPE_CONSUMERS = 256;                    // 8 consumer warps
-constexpr int PIPE_THREADS   = PIPE_CONSUMERS + 32;    // + 1 producer warp
-constexpr int PIPE_TC        = 2 * PIPE_CONSUMERS;     // 512 columns per tile
-constexpr int PIPE_TR        = 8;                      // rows per tile / stage
-constexpr int PIPE_STAGES    = 6;
-
-struct alignas(128) PipeStage {
-    double body[PIPE_TR][PIPE_TC];   // 32 KB
-    double row[PIPE_TC];             // pivot-row slice (valid when the column tile changed)
-    double col[16];                  // pivot-column slice of the tile's rows
-};
-constexpr size_t PIPE_SMEM = PIPE_STAGES * sizeof(PipeStage) + 2 * PIPE_STAGES * sizeof(uint64_t);
-
-struct TileIter {
-    // order 0: contiguous chunk per CTA, column tile major (pivot-row slice reloaded rarely)
-    // order 1: interleaved, row-tile major (neighbouring CTAs read neighbouring 4 KB pieces)
-    int64_t t, t_end, step;
-    int n_ct, n_rt, order;
-    __device__ __forceinline__ bool valid() const { return t < t_end; }
-    __device__ __forceinline__ void next() { t += step; }
-    __device__ __forceinline__ int ct() const { return order == 0 ? (int)(t / n_rt) : (int)(t % n_ct); }
-    __device__ __forceinline__ int rt() const { return order == 0 ? (int)(t % n_rt) : (int)(t / n_ct); }
-};
-
-__device__ __forceinline__ TileIter make_iter(int n_ct, int n_rt, int order) {
-    TileIter it;
-    it.n_ct = n_ct; it.n_rt = n_rt; it.order = order;
-    const int64_t total = (int64_t)n_ct * n_rt;
-    if (order == 0) {
-        const int64_t per = (total + gridDim.x - 1) / gridDim.x;
-        it.t = (int64_t)blockIdx.x * per;
-        it.t_end = min(total, it.t + per);
-        it.step = 1;
-    } else {
-        it.t = blockIdx.x; it.t_end = total; it.step = gridDim.x;
-    }
-    return it;
-}
-
-__global__ void __launch_bounds__(PIPE_THREADS, 1)
-update_pipelined_kernel(const double *__restrict__ Ain, double *__restrict__ Aout,
-                        const double *__restrict__ bin, double *__restrict__ bout,
-                        int n, int m_loc, int64_t ld, int64_t col0, int order, int ahead,
-                        spx_state *st, const double *__restrict__ colbuf,
-                        int32_t *__restrict__ rowlab, int32_t *__restrict__ collab,
-                        int32_t *__restrict__ trace) {
-    if (st->status != SPX_PIVOT) return;
-
-    extern __shared__ __align__(128) unsigned char pipe_smem[];
-    PipeStage *stg  = reinterpret_cast<PipeStage *>(pipe_smem);
-    uint64_t *full  = reinterpret_cast<uint64_t *>(pipe_smem + PIPE_STAGES * sizeof(PipeStage));
-    uint64_t *empty = full + PIPE_STAGES;
-
-    const int     r    = st->r;
-    const int64_t cg   = st->c;
-    const int     slot = st->slot;
-    const double  p    = st->p;
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    if (tid == 0) {
-        for (int s = 0; s < PIPE_STAGES; ++s) {
-            mbar_init(&full[s], 1);                          // the producer's expect_tx arrive
-            mbar_init(&empty[s], PIPE_CONSUMERS / 32);       // one arrive per consumer warp
-        }
-        mbar_fence_init();
-    }
-    __syncthreads();
-
-    const int n_ct = (m_loc + PIPE_TC - 1) / PIPE_TC;
-    const int n_rt = (n + 1 + PIPE_TR - 1) / PIPE_TR;
-    TileIter it = make_iter(n_ct, n_rt, order);
-
-    if (warp == PIPE_CONSUMERS / 32) {
-        // ---------------- producer warp: lane u < 8 copies row u of the tile, lane 8 the
-        // pivot-column slice, lane 9 the pivot-row slice; lane 0 posts the byte count
-        int prev_ct = -1;
-        for (int k = 0; it.valid(); it.next(), ++k) {
-            const int s = k % PIPE_STAGES;
-            const int use = k / PIPE_STAGES;
-            if (use > 0) mbar_wait(&empty[s], (uint32_t)((use - 1) & 1));
-            const int ct = it.ct(), rt = it.rt();
-            const int j0 = ct * PIPE_TC, i0 = rt * PIPE_TR;
-            const int rows = min(PIPE_TR, n + 1 - i0);
-            const uint32_t row_bytes = (uint32_t)(min((int64_t)PIPE_TC, ld - j0) * 8);
-            const bool new_ct = (ct != prev_ct);
-            if (lane == 0)
-                mbar_expect_tx(&full[s], rows * row_bytes + PIPE_TR * 8 + (new_ct ? row_bytes : 0u));
-            if (lane < rows)
-                bulk_g2s(stg[s].body[lane], Ain + (int64_t)(i0 + lane) * ld + j0, row_bytes, &full[s]);
-            else if (lane == PIPE_TR)
-                bulk_g2s(stg[s].col, colbuf + i0, PIPE_TR * 8, &full[s]);
-            else if (lane == PIPE_TR + 1 && new_ct)
-                bulk_g2s(stg[s].row, Ain + (int64_t)r * ld + j0, row_bytes, &full[s]);
-            prev_ct = ct;
-        }
-        return;
-    }
-
-    // ---------------- consumers
-    const PivotDiv d = pivot_div_prepare(p);
-    const int64_t cl = cg - col0;
-    int prev_ct = -1;
-    double2 rj = make_double2(0.0, 0.0);
-    int fneg = SPX_NONE;
-    bool saw_f = false;
-    for (int k = 0; it.valid(); it.next(), ++k) {
-        const int s = k % PIPE_STAGES;
-        const int ct = it.ct(), rt = it.rt();
-        const int j0 = ct * PIPE_TC, i0 = rt * PIPE_TR;
-        const int rows = min(PIPE_TR, n + 1 - i0);
-        mbar_wait(&full[s], (uint32_t)((k / PIPE_STAGES) & 1));
-        if (ct != prev_ct) { rj = *reinterpret_cast<const double2 *>(&stg[s].row[2 * tid]); prev_ct = ct; }
-        double2 t[PIPE_TR];
-        double  ci[PIPE_TR];
-#pragma unroll
-        for (int u = 0; u < PIPE_TR; ++u) {
-            t[u]  = *reinterpret_cast<const double2 *>(&stg[s].body[u][2 * tid]);
-            ci[u] = stg[s].col[u];
-        }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&empty[s]);             // stage is in registers: release it
-
-        const int  j      = j0 + 2 * tid;
-        const bool active = j < m_loc;
-        const bool has_c  = (cl >= j0) && (cl < j0 + PIPE_TC);
-        const bool has_r  = (r >= i0) && (r < i0 + rows);
-        const bool has_f  = (i0 + rows == n + 1);
-        double *dst = Aout + (int64_t)i0 * ld + j;
-        if (!active) continue;                              // (never diverges inside a warp's barrier use)
-        if (!has_c && !has_r && !has_f) {                   // interior tile, full height
-#pragma unroll
-            for (int u = 0; u < PIPE_TR; ++u) {
-                double2 o;
-                o.x = cell_update(t[u].x, d, rj.x, ci[u]);
-                o.y = cell_update(t[u].y, d, rj.y, ci[u]);
-                st_stream(dst + (int64_t)u * ld, o);
-            }
-        } else {
-            const int jc = has_c ? (int)(cl - j) : -1;
-#pragma unroll
-            for (int u = 0; u < PIPE_TR; ++u) {
-                if (u < rows) {
-                    const int i = i0 + u;
-                    const double2 o = generic_pair(t[u], i, r, jc, rj, ci[u], d);
-                    st_stream(dst + (int64_t)u * ld, o);
-                    if (i == n) {
-                        saw_f = true;
-                        if (o.x < 0.0) fneg = min(fneg, j);
-                        else if (o.y < 0.0 && j + 1 < m_loc) fneg = min(fneg, j + 1);
-                    }
-                }
-            }
-        }
-    }
-    if (saw_f && fneg != SPX_NONE && !ahead) atomicMin(&st->hint_fneg[slot], fneg);
-
-    // ---- the '-b' column, spread over the consumer threads of all CTAs
-    if (!ahead)
-        for (int base = blockIdx.x * PIPE_CONSUMERS; base < n; base += gridDim.x * PIPE_CONSUMERS)
-            update_b_rows(bin, bout, colbuf, n, r, d, base + tid, true, &st->hint_bneg[slot]);
-    if (blockIdx.x == 0 && tid == 0) commit_pivot(st, r, cg, slot, rowlab, collab, trace, ahead);
-}
-
 // a / p for arrays: the self-test of pivot_div against the compiler's div.rn.f64
 __global__ void division_selftest_kernel(const double *__restrict__ a, const double *__restrict__ p,
                                          int64_t count, int64_t np, unsigned long long *mismatches,
@@ -345,7 +169,7 @@ __global__ void division_selftest_kernel(const double *__restrict__ a, const dou
         const PivotDiv d = pivot_div_prepare(pv);
         const double q = pivot_div(a[k], d);
         const double e = __ddiv_rn(a[k], pv);
-        // the fused kernel's form: guards accumulated, exact redo when one tripped
+        // pivot_div_unchecked: guards accumulated, exact redo when one tripped
         bool ok = true;
         double q2 = pivot_div_unchecked(a[k], d, ok);
         if (!ok) q2 = pivot_div(a[k], d);
@@ -433,21 +257,16 @@ static int pick_tr(int n, int m_loc) {
 int64_t get_option(int key) { return (key >= 0 && key < 17) ? g_opt[key] : -1; }
 int set_option(int key, int64_t value) {
     switch (key) {
-    case SPX_OPT_UPDATE_KERNEL:    if (value < 0 || value > 2) return -1; break;
     case SPX_OPT_TILED_MIN_BLOCKS: if (value < 1 || value > 4) return -1; break;
-    case SPX_OPT_PIPE_ORDER:       if (value < 0 || value > 1) return -1; break;
-    case SPX_OPT_PIPE_GRID:        if (value < 0 || value > 4096) return -1; break;
     case SPX_OPT_TILED_ROWS:       if (value < 0 || value > UPD_TR_MAX || value % 8) return -1; break;
     case SPX_OPT_FUSE_DEPTH:       if (value < 0 || value > 8) return -1; break;
     case SPX_OPT_FUSE_MIN_BLOCKS:  if (value < 0 || value > 4) return -1; break;
     case SPX_OPT_FUSE_PRICING:     if (value < 0 || value > 2) return -1; break;
     case SPX_OPT_FUSE_LOOKAHEAD:   if (value < 0 || value > 2) return -1; break;
-    case SPX_OPT_FUSE_VARIANT:     if (value < 0 || value > 1) return -1; break;
     case SPX_OPT_FUSE_TILE_ROWS:   if (value < 0 || value > 4096 || value % 8) return -1; break;
     case SPX_OPT_FUSE_PAIRS:       if (value < 0 || value > 2) return -1; break;
     case SPX_OPT_SHARD_THREADS:    if (value < 0 || value > 512 || value % 32 || value == 32) return -1; break;
     case SPX_OPT_SHARD_CTAS:       if (value < 0 || value > 4096) return -1; break;
-    case SPX_OPT_RESIDENT_VARIANT: if (value < 0 || value > 1) return -1; break;
     case SPX_OPT_CLUSTER_SIZE:     if (value < 0 || value > 16 || (value & (value - 1))) return -1; break;
     default: return -1;
     }
@@ -458,29 +277,6 @@ int set_option(int key, int64_t value) {
 cudaError_t update(const double *Ain, double *Aout, const double *bin, double *bout, int n,
                    int m_loc, int64_t ld, int64_t col0, spx_state *st, const double *colbuf,
                    int32_t *rowlab, int32_t *collab, int32_t *trace, int ahead, cudaStream_t stream) {
-    int kernel = (int)g_opt[SPX_OPT_UPDATE_KERNEL];
-    // measured on B200 (profiles/): the tiled kernel streams at the copy rate already; the
-    // pipelined kernel stays selectable for experiments
-    if (kernel == 0) kernel = 1;
-    if (kernel == 2) {
-        static bool configured_dev[64] = {};
-        bool &configured = configured_dev[spx_host::device_slot()];
-        if (!configured) {
-            cudaError_t e = cudaFuncSetAttribute(update_pipelined_kernel,
-                                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PIPE_SMEM);
-            if (e != cudaSuccess) return e;
-            configured = true;
-        }
-        const int64_t tiles = (((int64_t)m_loc + PIPE_TC - 1) / PIPE_TC) * (((int64_t)n + 1 + PIPE_TR - 1) / PIPE_TR);
-        int64_t grid = g_opt[SPX_OPT_PIPE_GRID] > 0 ? g_opt[SPX_OPT_PIPE_GRID] : sm_count();
-        if (tiles < grid) grid = tiles;
-        if (grid < 1) grid = 1;                       // a shard with no columns still updates b
-        update_pipelined_kernel<<<(unsigned)grid, PIPE_THREADS, PIPE_SMEM, stream>>>(
-            Ain, Aout, bin, bout, n, m_loc, ld, col0, (int)g_opt[SPX_OPT_PIPE_ORDER], ahead, st, colbuf,
-            rowlab, collab, trace);
-        spx_host::count_launch();
-        return cudaGetLastError();
-    }
     const int tr = pick_tr(n, m_loc);
     dim3 grid((unsigned)((m_loc + UPD_TC - 1) / UPD_TC), (unsigned)((n + 1 + tr - 1) / tr));
     if (grid.x == 0) grid.x = 1;      // a shard with no columns still updates b

@@ -81,19 +81,19 @@ def test_host_side_layout_helpers_agree_with_python(native):
     assert native.LOOP_MODES[None] == 0 and native.LOOP_MODES["fused"] == 4 and native.LOOP_MODES[True] == 2
 
 
-def test_options_validate_their_ranges(native):
+def test_options_validate_ranges_and_reject_retired_keys(native):
     L = native.load()
     try:
-        assert L.spx_get_option(10) == 0 and L.spx_get_option(11) == 0 and L.spx_get_option(7) == 0   # defaults
-        assert L.spx_get_option(12) == 0
-        assert L.spx_set_option(10, 1) == 0 and L.spx_get_option(10) == 1          # round 1's fused update kernel
-        assert L.spx_set_option(10, 2) != 0 and L.spx_set_option(10, -1) != 0
+        assert L.spx_get_option(11) == 0 and L.spx_get_option(7) == 0 and L.spx_get_option(12) == 0   # defaults
+        for k in (1, 3, 4, 10, 15):                                                  # retired keys: rejected, read 0
+            for v in (0, 1, 2):
+                assert L.spx_set_option(k, v) != 0
+            assert L.spx_get_option(k) == 0
         assert L.spx_set_option(11, 40) == 0 and L.spx_get_option(11) == 40        # rows per warp strip: multiples of 8
         assert L.spx_set_option(11, 12) != 0 and L.spx_set_option(11, 4104) != 0
         assert L.spx_set_option(12, 2) == 0 and L.spx_set_option(12, 3) != 0       # column pairs per lane: 1 or 2
         assert L.spx_set_option(6, 9) != 0 and L.spx_set_option(99, 0) != 0
     finally:
-        L.spx_set_option(10, 0)
         L.spx_set_option(11, 0)
         L.spx_set_option(12, 0)
 

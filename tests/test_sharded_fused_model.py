@@ -1,4 +1,4 @@
-"""CPU model of the column-sharded FUSED loop (csrc/spx_fused.cu: shard_price_kernel + update_fused_kernel),
+"""CPU model of the column-sharded FUSED loop (csrc/spx_fused.cu: shard_price_kernel + update_lazy_kernel),
 checked bit for bit against the oracle.  It restates, in numpy and rank by rank, WHAT every rank computes in
 a pass — not the CUDA code — so that the algorithm the kernels implement is pinned on the inputs the hardware
 tests could not cover in round 1 (entering columns owned by the LAST ranks, phase-1 pivots, degenerate ties,
@@ -72,7 +72,7 @@ def run_model(rows, c, splits, F, cap, lookahead):
         return (lvl["r"], cl if 0 <= cl < rk.m else -1, lvl["p"])
 
     def sweep(levels, row_planes_per_rank):
-        """update_fused_kernel: every rank applies `levels` to its stored columns (and f row shard)"""
+        """update_lazy_kernel: every rank applies `levels` to its stored columns (and f row shard)"""
         for rk, planes in zip(ranks, row_planes_per_rank):
             if rk.m == 0:
                 continue

@@ -18,8 +18,6 @@ def main():
     modes = sys.argv[3].split(",") if len(sys.argv) > 3 else ["resident", "classic", "lookahead"]
     from simplex_method_solver_b200 import _native as N
     for mode in modes:
-        N.lib().spx_set_option(N.OPT_RESIDENT_VARIANT, 1 if mode == "resident-ahead" else 0)
-        mode = "resident" if mode == "resident-ahead" else mode
         tab = DeviceTableau(n, m, trace_capacity=200000)
         tab.load(rows, c, max_pivots=200000)
         tab.solve(stop_after=50, lookahead=mode)

@@ -25,8 +25,7 @@ def main():
     ap.add_argument("--minb", default="3")
     ap.add_argument("--items", default="0", help="fused update kernel: column pairs per lane (0 = default, 1, 2)")
     ap.add_argument("--variants", default="0",
-                    help="update kernel schedules as variant:tile_rows, e.g. 0:32,0:64,1 (0 = update_lazy_kernel, the default; "
-                         "1 = round 1's update_fused_kernel)")
+                    help="update kernel schedules as rows per warp strip, e.g. 0,32,64 (0 = the default)")
     a = ap.parse_args()
     L = N.lib()
     rows, c = W.dense_lp(a.n, a.m, 0)
@@ -36,16 +35,15 @@ def main():
             gold = np.asarray(json.load(fh)["cfg4"]["trace"], dtype=np.int32)
     cells = a.n * (a.m + 1) + a.m
     tab = DeviceTableau(a.n, a.m, trace_capacity=4 * a.pivots + 64)
-    variants = [(int(v.split(":")[0]), int(v.split(":")[1]) if ":" in v else 0) for v in a.variants.split(",")]
-    for mode, F, mb, (var, trows), items in [("lookahead", 0, 0, (0, 0), 0)] + [("fused", int(x), int(y), v, int(z))
-                                                                                for v in variants
-                                                                                for z in a.items.split(",")
-                                                                                for y in a.minb.split(",")
-                                                                                for x in a.depths.split(",")]:
+    for mode, F, mb, trows, items in [("lookahead", 0, 0, 0, 0)] + [("fused", int(x), int(y), int(v), int(z))
+                                                                    for v in a.variants.split(",")
+                                                                    for z in a.items.split(",")
+                                                                    for y in a.minb.split(",")
+                                                                    for x in a.depths.split(",")]:
         if F:
             assert L.spx_set_option(N.OPT_FUSE_DEPTH, F) == 0
             assert L.spx_set_option(7, mb) == 0
-            assert L.spx_set_option(10, var) == 0 and L.spx_set_option(11, trows) == 0
+            assert L.spx_set_option(11, trows) == 0
             assert L.spx_set_option(12, items) == 0
         tab.load(rows, c, max_pivots=4 * a.pivots + 32)
         tab.solve(stop_after=a.pivots, chunk=a.pivots, lookahead=mode)          # warm-up
@@ -60,7 +58,7 @@ def main():
             tr = tab.trace[:npiv].cpu().numpy()
             k = min(len(gold), npiv)
             ok = f" golden[{k}]={'OK' if (tr[:k] == gold[:k]).all() else 'MISMATCH'}"
-        print(f"{mode:9s} F={F} minb={mb} variant={var}:{trows} pairs={items}: {a.pivots} pivots in {ms:8.2f} ms  {a.pivots / ms * 1e3:8.1f} pivots/s  "
+        print(f"{mode:9s} F={F} minb={mb} rows={trows} pairs={items}: {a.pivots} pivots in {ms:8.2f} ms  {a.pivots / ms * 1e3:8.1f} pivots/s  "
               f"{ms / a.pivots * 1e3:7.1f} us/pivot  north-star {16.0 * cells * a.pivots / ms / 1e6:8.0f} GB/s  "
               f"status={st} npiv={npiv}{ok}", flush=True)
 
