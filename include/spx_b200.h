@@ -219,13 +219,20 @@ int spx_extract(const double *d_b, int32_t n, int32_t m, const int32_t *d_collab
  *   d_status [B], d_npiv [B], d_rowlab [B][m], d_collab [B][n],
  *   d_trace [B][max_pivots][2], d_snap [B][max_pivots+1][cells] (the Info.table
  *   sequence of get_solution(), simplex.py:181,198: slot k = table before pivot k).
- * cells is limited by shared memory: spx_batched_max_cells(). */
+ * The LP must fit one CTA's shared memory: spx_batched_fits(n, m). */
 int spx_solve_batched(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule,
                       int32_t max_pivots, double *d_x, double *d_obj,
                       int32_t *d_status, int32_t *d_npiv,
                       int32_t *d_rowlab, int32_t *d_collab,
                       int32_t *d_trace, double *d_snap, void *stream);
 int64_t spx_batched_max_cells(void);
+/* Host only (no device): 1 when spx_solve_batched takes an n x m LP, else 0.  With
+ * cells = n*(m+1) + m: cells <= spx_batched_max_cells(), and above 96 cells (one CTA per
+ * LP) the cell lookup table and the LP's two tables, x and labels fit the shared memory
+ * of a CTA beside the kernel's 16 static bytes:
+ *     ceil16(4*cells) + ceil16(8*(2*cells + m) + 4*(n + m))  <=  232448 - 16 bytes.
+ * E.g. 72 x 136 (10,000 cells) fits; 1 x 4470 (8,941 cells) and 2 x 3228 do not. */
+int32_t spx_batched_fits(int32_t n, int32_t m);
 
 /* ---- K7: batches of independent mid-size LPs, one thread-block cluster per LP -- */
 /* The whole loop of get_solution(), simplex.py:179-199 (pick_element :70-141 and
@@ -292,7 +299,7 @@ int32_t spx_global_cluster_size(int32_t n, int32_t m, int64_t B);
  * of spx_solve_batched / spx_solve_batched_cluster / spx_solve_batched_global for that
  * LP alone, bit for bit.
  *
- * Routing: SPX_ENGINE_AUTO sends an LP to K4 when cells <= spx_batched_max_cells(),
+ * Routing: SPX_ENGINE_AUTO sends an LP to K4 when spx_batched_fits(n, m),
  * else to K7 (at spx_cluster_size(n, m), or SPX_OPT_CLUSTER_SIZE when set), and rejects
  * an LP above K7's capacity; SMEM, CLUSTER and GLOBAL send every LP to that engine;
  * AUTO_GLOBAL is AUTO with K8 for the LPs above K7's capacity (spx_cluster_size(n, m)

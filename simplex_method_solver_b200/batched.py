@@ -115,8 +115,9 @@ def _global_capacity_text(n: int, m: int) -> str:
 def kernel_for(n: int, m: int, engine: str = "auto") -> str:
     """"smem" (K4), "cluster" (K7) or "global" (K8) for an n x m LP; ValueError when the engine cannot take it.
 
-    "auto_global" is "auto" with K8 above K7's capacity: K4 up to ``spx_batched_max_cells()`` cells, else K7 when
-    ``spx_cluster_size(n, m) > 0``, else K8 (the routing of ragged batches that mix every size).
+    "auto" is K4 when ``spx_batched_fits(n, m)`` (at most ``spx_batched_max_cells()`` cells, and one CTA's shared
+    memory holds the LP), else K7.  "auto_global" is "auto" with K8 above K7's capacity: K4 when it fits, else K7
+    when ``spx_cluster_size(n, m) > 0``, else K8 (the routing of ragged batches that mix every size).
     """
     if engine not in ENGINES:
         raise ValueError(f"unknown engine {engine!r}; one of {ENGINES}")
@@ -124,8 +125,9 @@ def kernel_for(n: int, m: int, engine: str = "auto") -> str:
         raise ValueError(f"bad shape {n} x {m}")
     L = N.load()
     cells = n * (m + 1) + m
+    fits = bool(L.spx_batched_fits(n, m))
     if engine == "auto_global":
-        if cells <= L.spx_batched_max_cells():
+        if fits:
             return "smem"
         engine = "cluster" if L.spx_cluster_size(n, m) else "global"
     if engine == "global":
@@ -133,10 +135,13 @@ def kernel_for(n: int, m: int, engine: str = "auto") -> str:
             raise ValueError(f"a {n} x {m} LP ({cells} cells) exceeds the capacity of the global-memory cluster "
                              f"solver: {_global_capacity_text(n, m)}; use SimplexMethod / DeviceTableau")
         return "global"
-    if engine == "smem" or (engine == "auto" and cells <= L.spx_batched_max_cells()):
+    if engine == "smem" or (engine == "auto" and fits):
         if cells > L.spx_batched_max_cells():
             raise ValueError(f"{cells} cells per LP exceed the shared-memory limit of one CTA "
                              f"({L.spx_batched_max_cells()}); use engine='cluster' or 'auto'")
+        if not fits:
+            raise ValueError(f"a {n} x {m} LP ({cells} cells) does not fit the shared memory of one CTA; "
+                             "use engine='cluster' or 'auto'")
         return "smem"
     if L.spx_cluster_size(n, m) == 0:
         raise ValueError(f"a {n} x {m} LP ({cells} cells) exceeds the capacity of the cluster solver: "

@@ -16,6 +16,7 @@ int     sm_count();
 int64_t colbuf_doubles(int n);
 int64_t shard_msg_doubles(int n);
 int64_t batched_max_cells();
+bool batched_fits(int, int);
 cudaError_t pick(const double *, const double *, int, int, int64_t, int, int, spx_state *, double *,
                  cudaStream_t);
 cudaError_t shard_candidate(const double *, const double *, int, int, int64_t, int64_t, int, int,
@@ -545,6 +546,7 @@ int spx_extract(const double *d_b, int32_t n, int32_t m, const int32_t *d_collab
 
 // ---- K4 -------------------------------------------------------------------------
 int64_t spx_batched_max_cells(void) { return spx_launch::batched_max_cells(); }
+int32_t spx_batched_fits(int32_t n, int32_t m) { return spx_launch::batched_fits(n, m) ? 1 : 0; }
 
 int spx_solve_batched(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule, int32_t max_pivots,
                       double *d_x, double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab,
@@ -555,6 +557,9 @@ int spx_solve_batched(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule
     SPX_REQUIRE(spx_cells(n, m) <= spx_batched_max_cells(),
                 "spx_solve_batched: %lld cells per LP exceed the shared-memory resident limit %lld; use spx_solve",
                 (long long)spx_cells(n, m), (long long)spx_batched_max_cells());
+    SPX_REQUIRE(spx_launch::batched_fits(n, m),
+                "spx_solve_batched: a %d x %d LP (%lld cells) does not fit the shared memory of one CTA; "
+                "use spx_solve_batched_cluster", n, m, (long long)spx_cells(n, m));
     cudaError_t e = spx_launch::solve_batched(d_T, B, n, m, rule, max_pivots, d_x, d_obj, d_status, d_npiv,
                                               d_rowlab, d_collab, d_trace, d_snap, as_stream(stream));
     return check(e, "batched launch");
@@ -662,7 +667,7 @@ int spx_ragged_plan(const int32_t *h_shapes, int64_t B, int32_t engine, void *h_
                     (long long)k, n, m, cap);
         const int64_t cells = spx_cells(n, m);
         const bool k4 = engine == SPX_ENGINE_SMEM ||
-                        ((engine == SPX_ENGINE_AUTO || engine == SPX_ENGINE_AUTO_GLOBAL) && cells <= spx_batched_max_cells());
+                        ((engine == SPX_ENGINE_AUTO || engine == SPX_ENGINE_AUTO_GLOBAL) && spx_launch::batched_fits(n, m));
         const bool k8 = engine == SPX_ENGINE_GLOBAL ||
                         (engine == SPX_ENGINE_AUTO_GLOBAL && !k4 && spx_launch::cluster_size(n, m) == 0);
         if (k8) {

@@ -22,7 +22,8 @@ constexpr size_t SMEM_LIMIT = 227 * 1024;
 constexpr int64_t CTA_MODE_MIN_CELLS = 96;    // above this one CTA (not one warp) solves an LP
 constexpr int     CTA_CELLS_PER_WARP = 32;    // CTA mode: cells per warp (2..8 warps)
 constexpr size_t  WARP_LUT_BYTES = CTA_MODE_MIN_CELLS * 4;   // ragged warp mode: per-warp lookup table (384 B)
-constexpr size_t  RAGGED_STATIC = 16;         // ragged kernels: static shared memory (s_ctl), checked at launch
+constexpr size_t  K4_STATIC = 16;             // every K4 kernel: static shared memory (s_ctl), checked at launch
+constexpr size_t  K4_DYN_LIMIT = SMEM_LIMIT - K4_STATIC;   // the dynamic and the static bytes of a CTA share SMEM_LIMIT
 
 struct BatchedArgs {
     double  *T;          // [B][cells] in/out
@@ -392,20 +393,47 @@ size_t lut_bytes(int n, int m) {
     return (cells * 4 + 15) / 16 * 16;
 }
 
+// Sets the dynamic shared-memory limit of a K4 kernel to K4_DYN_LIMIT once per device, after checking that its static
+// bytes are the K4_STATIC the capacity rule reserves.  A failure is returned once: the runtime's last error is cleared,
+// so that the next launch's cudaGetLastError() does not report it again.
+template <class K>
+cudaError_t configure_k4(K kernel, size_t &configured) {
+    if (configured) return cudaSuccess;
+    cudaFuncAttributes fa;
+    cudaError_t e = cudaFuncGetAttributes(&fa, kernel);
+    if (e == cudaSuccess && fa.sharedSizeBytes > K4_STATIC) return cudaErrorInvalidValue;
+    if (e == cudaSuccess)
+        e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K4_DYN_LIMIT);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return e;
+    }
+    configured = K4_DYN_LIMIT;
+    return cudaSuccess;
+}
+
 } // namespace
 
 namespace spx_launch {
 
 int64_t batched_max_cells() { return 10000; }
 
+// K4's capacity, one rule for the uniform and the ragged entries: at most batched_max_cells() cells, and in CTA mode
+// (above 96 cells) the lookup table and the LP's tables within K4_DYN_LIMIT; warp mode always fits
+bool batched_fits(int n, int m) {
+    if (n < 1 || m < 1 || n > 65535 || m > 65534) return false;
+    const int64_t cells = (int64_t)n * (m + 1) + m;
+    if (cells > batched_max_cells()) return false;
+    return cells <= CTA_MODE_MIN_CELLS || lut_bytes(n, m) + warp_bytes(n, m) <= K4_DYN_LIMIT;
+}
+
 // returns cudaErrorInvalidValue when one LP does not fit shared memory
 cudaError_t solve_batched(double *T, int64_t B, int n, int m, int rule, int max_pivots, double *x,
                           double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab,
                           int32_t *collab, int32_t *trace, double *snap, cudaStream_t stream) {
     if (B <= 0) return cudaSuccess;
-    if (n > 65535 || m > 65534) return cudaErrorInvalidValue;
+    if (!batched_fits(n, m)) return cudaErrorInvalidValue;
     const size_t wb = warp_bytes(n, m), lb = lut_bytes(n, m);
-    if (lb + wb > SMEM_LIMIT) return cudaErrorInvalidValue;
     const int64_t cells = (int64_t)n * (m + 1) + m;
     BatchedArgs a{T, B, n, m, rule, max_pivots, x, obj, status, npiv, rowlab, collab, trace, snap};
     static size_t configured_dev[64][2] = {};
@@ -416,11 +444,9 @@ cudaError_t solve_batched(double *T, int64_t B, int n, int m, int rule, int max_
         int warps = (int)((cells + CTA_CELLS_PER_WARP - 1) / CTA_CELLS_PER_WARP);
         warps = warps < 2 ? 2 : (warps > 16 ? 16 : warps);
         const size_t smem = lb + wb;
-        if (smem > 48 * 1024 && smem > configured[1]) {
-            cudaError_t e = cudaFuncSetAttribute(batched_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                 (int)SMEM_LIMIT);
+        if (smem > 48 * 1024) {
+            const cudaError_t e = configure_k4(batched_kernel<true>, configured[1]);
             if (e != cudaSuccess) return e;
-            configured[1] = SMEM_LIMIT;
         }
         batched_kernel<true><<<(unsigned)B, warps * 32, smem, stream>>>(a, 1, (int)(wb / sizeof(double)));
         spx_host::count_launch();
@@ -433,11 +459,9 @@ cudaError_t solve_batched(double *T, int64_t B, int n, int m, int rule, int max_
     if (wpc < 1) wpc = 1;
     if ((int64_t)wpc > B) wpc = (int)B;
     const size_t smem = lb + (size_t)wpc * wb;
-    if (smem > 48 * 1024 && smem > configured[0]) {
-        cudaError_t e = cudaFuncSetAttribute(batched_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (int)SMEM_LIMIT);
+    if (smem > 48 * 1024) {
+        const cudaError_t e = configure_k4(batched_kernel<false>, configured[0]);
         if (e != cudaSuccess) return e;
-        configured[0] = SMEM_LIMIT;
     }
     const int64_t ctas = (B + wpc - 1) / wpc;
     batched_kernel<false><<<(unsigned)ctas, wpc * 32, smem, stream>>>(a, wpc, (int)(wb / sizeof(double)));
@@ -447,12 +471,10 @@ cudaError_t solve_batched(double *T, int64_t B, int n, int m, int rule, int max_
 
 // ---- ragged batches: the plan's numbers for K4 ----
 // shared memory of one LP: CTA mode lookup table + tables, or warp mode slot (no table); -1 when K4 cannot take it
-// (the uniform entry's limits)
+// (batched_fits, the uniform entry's rule)
 int64_t ragged_batched_bytes(int n, int m, int *kernel) {
-    if (n < 1 || m < 1 || n > 65535 || m > 65534) return -1;
+    if (!batched_fits(n, m)) return -1;
     const int64_t cells = (int64_t)n * (m + 1) + m;
-    // the dynamic and the static shared memory of a CTA share SMEM_LIMIT
-    if (cells > batched_max_cells() || lut_bytes(n, m) + warp_bytes(n, m) > SMEM_LIMIT - RAGGED_STATIC) return -1;
     *kernel = cells > CTA_MODE_MIN_CELLS ? RAGGED_CTA : RAGGED_WARP;
     return cells > CTA_MODE_MIN_CELLS ? (int64_t)(lut_bytes(n, m) + warp_bytes(n, m))
                                       : (int64_t)(WARP_LUT_BYTES + warp_bytes(n, m));
@@ -477,17 +499,10 @@ cudaError_t solve_ragged_batched(const RaggedLaunch &l, const RaggedLp *lps, con
     static size_t configured_dev[64][2] = {};
     size_t *configured = configured_dev[spx_host::device_slot()];
     const bool cta = (l.kernel == RAGGED_CTA);
-    if (l.smem > 48 * 1024 && (size_t)l.smem > configured[cta]) {
-        cudaFuncAttributes fa;
-        cudaError_t e = cta ? cudaFuncGetAttributes(&fa, ragged_batched_kernel<true>)
-                            : cudaFuncGetAttributes(&fa, ragged_batched_kernel<false>);
+    if (l.smem > 48 * 1024) {
+        const cudaError_t e = cta ? configure_k4(ragged_batched_kernel<true>, configured[1])
+                                  : configure_k4(ragged_batched_kernel<false>, configured[0]);
         if (e != cudaSuccess) return e;
-        if (fa.sharedSizeBytes > RAGGED_STATIC) return cudaErrorInvalidValue;
-        const int dyn = (int)(SMEM_LIMIT - RAGGED_STATIC);
-        e = cta ? cudaFuncSetAttribute(ragged_batched_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn)
-                : cudaFuncSetAttribute(ragged_batched_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn);
-        if (e != cudaSuccess) return e;
-        configured[cta] = SMEM_LIMIT - RAGGED_STATIC;
     }
     const int64_t ctas = (l.count + l.per_cta - 1) / l.per_cta;
     if (cta)

@@ -61,6 +61,8 @@ def test_abi_constants_and_state_layout(native):
     assert L.spx_colbuf_doubles(16384) >= 16385
     assert L.spx_shard_msg_doubles(16384) % 16 == 0 and L.spx_shard_msg_doubles(16384) >= 16389
     assert L.spx_batched_max_cells() >= 440
+    assert L.spx_batched_fits(4, 2) == 1 and L.spx_batched_fits(72, 136) == 1 and L.spx_batched_fits(1, 4470) == 0
+    assert L.spx_batched_fits(0, 2) == 0 and L.spx_batched_fits(100, 100) == 0
     assert L.spx_launch_count(1) >= 0 and L.spx_launch_count(0) == 0
 
 

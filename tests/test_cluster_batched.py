@@ -105,12 +105,17 @@ def test_cluster_size_option_values(lib):
     assert lib.spx_get_option(OPT_CLUSTER_SIZE) == 0
 
 
-def test_engine_routing_needs_no_device(lib):
+def test_engine_routing_by_k4_footprint_needs_no_device(lib):
     from simplex_method_solver_b200.batched import kernel_for
-    for n, m in ((8, 2), (4, 2), (20, 20), (64, 33), (99, 99), (1, 4999)):
+    for n, m in ((8, 2), (4, 2), (20, 20), (64, 33), (99, 99), (1, 4469), (72, 136)):
         assert n * (m + 1) + m <= lib.spx_batched_max_cells()
         assert kernel_for(n, m) == "smem" and kernel_for(n, m, "smem") == "smem"
         assert kernel_for(n, m, "cluster") == "cluster"
+    for n, m in ((1, 4470), (1, 4999), (2, 3228)):          # within 10,000 cells, but wider than one CTA holds
+        assert n * (m + 1) + m <= lib.spx_batched_max_cells() and not lib.spx_batched_fits(n, m)
+        assert kernel_for(n, m) == "cluster" and kernel_for(n, m, "auto_global") == "cluster"
+        with pytest.raises(ValueError, match=f"a {n} x {m} LP .*does not fit the shared memory of one CTA"):
+            kernel_for(n, m, "smem")
     for n, m in ((100, 100), (128, 256), (512, 800), (3, 9000)):
         assert kernel_for(n, m) == "cluster" and kernel_for(n, m, "cluster") == "cluster"
         with pytest.raises(ValueError):

@@ -45,16 +45,6 @@ def expected_launches(L, shapes, engine="auto"):
     return len({expected_class(L, n, m, engine) for n, m in shapes})
 
 
-def uniform_engine(n, m):
-    """The engine solve_batched can solve an n x m LP alone with: "auto", except for K4 CTA-mode shapes of more than
-    48 KB of shared memory, which spx_solve_batched cannot launch (it asks for 227 KB of dynamic shared memory on top
-    of the kernel's static bytes); K7 gives them the same bits."""
-    cells = cells_of(n, m)
-    lut = (cells * 4 + 15) // 16 * 16
-    wb = ((2 * cells + m) * 8 + (n + m) * 4 + 15) // 16 * 16
-    return "cluster" if 96 < cells <= 10000 and lut + wb > 48 * 1024 else "auto"
-
-
 def random_shapes(rng, B):
     """Shapes across warp mode, CTA mode and every cluster size."""
     out = []
@@ -141,7 +131,7 @@ def _plan_raw(L, shapes, engine=0, nbytes=None):
     return rc, ctypes.string_at(L.spx_last_error()), buf
 
 
-def test_plan_validation_names_the_lp(lib):
+def test_plan_validation_names_the_lp_and_sends_wide_k4_shapes_to_k7(lib):
     for bad, text in (([(4, 2, 10), (0, 2, 10)], b"LP 1: bad shape n=0"),
                       ([(4, 2, 10), (4, 2, 10), (4, 0, 10)], b"LP 2: bad shape n=4 m=0"),
                       ([(4, 2, -1)], b"LP 0: bad shape n=4 m=2 max_pivots=-1"),
@@ -155,8 +145,10 @@ def test_plan_validation_names_the_lp(lib):
     with cluster_size(lib, 1):
         rc, err, _ = _plan_raw(lib, [(100, 100, 5), (128, 256, 5)])
         assert rc < 0 and b"LP 1: a 128 x 256 LP does not fit a cluster of SPX_OPT_CLUSTER_SIZE = 1 CTAs" in err, err
-    rc, err, _ = _plan_raw(lib, [(8, 2, 5), (1, 4999, 5)])       # 9,999 cells, 260 KB: K4 cannot hold it
+    rc, err, _ = _plan_raw(lib, [(8, 2, 5), (1, 4999, 5)], engine=1)   # 9,999 cells, 260 KB: K4 cannot hold it
     assert rc < 0 and b"LP 1: a 1 x 4999 LP (9999 cells) does not fit the shared memory of one CTA" in err, err
+    rc, err, _ = _plan_raw(lib, [(8, 2, 5), (1, 4999, 5)])              # "auto" gives it to K7
+    assert rc == 0, err
     rc, err, _ = _plan_raw(lib, [(8, 2, 5)] * 3, nbytes=lib.spx_ragged_plan_bytes(3) - 1)
     assert rc < 0 and b"plan_bytes" in err
     rc, err, _ = _plan_raw(lib, [(8, 2, 5)], engine=3)
@@ -367,8 +359,7 @@ def test_independence_and_order(spx):
     res = spx.batched.solve_ragged(lps, max_pivots=caps)
     for k, (rows, c) in enumerate(lps):
         n, m = rows.shape[0], c.shape[0]
-        alone = spx.batched.solve_batched(flat_of(rows, c)[None, :], n, m, max_pivots=caps[k],
-                                          engine=uniform_engine(n, m))
+        alone = spx.batched.solve_batched(flat_of(rows, c)[None, :], n, m, max_pivots=caps[k])
         for f, a, b in zip(alone._fields, alone, res.lp(k)):
             if a is None:
                 assert b is None, f

@@ -15,7 +15,7 @@ import oracle
 from simplex_method_solver_b200 import workloads as W
 from test_cluster_batched import _family, cluster_size
 from test_global_batched import expected_min_size
-from test_ragged_batched import _check_case, _golden_lps, _plan_raw, random_shapes, uniform_engine
+from test_ragged_batched import _check_case, _golden_lps, _plan_raw, random_shapes
 from util import END_TO_STATUS, bits, flat_of, label_codes, table_sha
 
 SIZES = (1, 2, 4, 8, 16)
@@ -298,7 +298,6 @@ def _same(a_res, b_res, what):
 
 @pytest.mark.gpu
 def test_auto_global_batch_against_oracle_and_per_lp(spx):
-    from simplex_method_solver_b200.batched import kernel_for
     lps, caps = _mixed_large(1)
     shapes = [(r.shape[0], c.shape[0]) for r, c in lps]
     db = spx.batched.DeviceRaggedBatch(shapes, caps, engine="auto_global")
@@ -318,9 +317,7 @@ def test_auto_global_batch_against_oracle_and_per_lp(spx):
         assert np.array_equal(bits(one.tables[0]), bits(o.table)), k
         assert one.rowlab[0].tolist() == o.rowlab.tolist() and one.collab[0].tolist() == o.collab.tolist(), k
         assert np.array_equal(bits(one.x[0]), bits(o.x)) and bits(one.obj[0]) == bits(o.obj2), k
-        kind = kernel_for(n, m, "auto_global")
-        engine = uniform_engine(n, m) if kind == "smem" else kind
-        alone = spx.batched.solve_batched(flat_of(rows, c)[None, :], n, m, max_pivots=caps[k], engine=engine)
+        alone = spx.batched.solve_batched(flat_of(rows, c)[None, :], n, m, max_pivots=caps[k], engine="auto_global")
         _same(alone, one, k)
     assert {oracle.CAP, oracle.OPTIMAL, oracle.INCORRECT, oracle.NOCONV} <= ends
 
