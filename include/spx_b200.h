@@ -299,11 +299,8 @@ int32_t spx_global_cluster_size(int32_t n, int32_t m, int64_t B);
  * of spx_solve_batched / spx_solve_batched_cluster / spx_solve_batched_global for that
  * LP alone, bit for bit.
  *
- * Routing: SPX_ENGINE_AUTO sends an LP to K4 when spx_batched_fits(n, m),
- * else to K7 (at spx_cluster_size(n, m), or SPX_OPT_CLUSTER_SIZE when set), and rejects
- * an LP above K7's capacity; SMEM, CLUSTER and GLOBAL send every LP to that engine;
- * AUTO_GLOBAL is AUTO with K8 for the LPs above K7's capacity (spx_cluster_size(n, m)
- * == 0) up to K8's.  Code 3 is not an engine.  One solve makes at most 12 launches, in
+ * Routing: each LP goes where spx_batched_route sends it, K7 at spx_cluster_size(n, m)
+ * or SPX_OPT_CLUSTER_SIZE when set.  One solve makes at most 12 launches, in
  * sequence on `stream`: K4 warp mode (LPs of <= 96 cells) if any, K4 CTA mode if any,
  * one K7 launch per distinct cluster size, then one K8 launch per distinct S_min
  * (spx_global_min_cluster_size), or one at SPX_OPT_CLUSTER_SIZE when it is set when the
@@ -316,6 +313,17 @@ int32_t spx_global_cluster_size(int32_t n, int32_t m, int64_t B);
 #define SPX_ENGINE_CLUSTER     2
 #define SPX_ENGINE_GLOBAL      4
 #define SPX_ENGINE_AUTO_GLOBAL 5
+/* Host only (no device): the engine that takes an n x m LP under `engine`, the rule of
+ * spx_ragged_plan and of the uniform entries: SPX_ENGINE_SMEM (K4), SPX_ENGINE_CLUSTER
+ * (K7) or SPX_ENGINE_GLOBAL (K8).  SPX_ENGINE_AUTO sends an LP to K4 when
+ * spx_batched_fits(n, m), else to K7, and rejects an LP above K7's capacity
+ * (spx_cluster_size(n, m) == 0); SMEM, CLUSTER and GLOBAL send every LP to that engine;
+ * AUTO_GLOBAL is AUTO with K8 for the LPs above K7's capacity, up to K8's.  Code 3 is
+ * not an engine.  -1 when the engine cannot take the LP (spx_last_error() names the
+ * capacity it exceeds), the shape is not n, m >= 1, or the code is unknown.
+ * SPX_OPT_CLUSTER_SIZE is not read: the plan and the uniform entries also refuse an LP
+ * that does not fit the cluster size it forces. */
+int32_t spx_batched_route(int32_t n, int32_t m, int32_t engine);
 /* bytes of the plan of a batch of B LPs (-1 when B < 0) */
 int64_t spx_ragged_plan_bytes(int64_t B);
 /* Host only, no device.  h_shapes[B][3] = {n, m, max_pivots} in batch order.  Validates

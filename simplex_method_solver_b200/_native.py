@@ -87,6 +87,7 @@ SIGNATURES = {
                                          _vp, _vp, _vp]),
     "spx_batched_max_cells": (_i64, []),
     "spx_batched_fits": (_i32, [_i32, _i32]),
+    "spx_batched_route": (_i32, [_i32, _i32, _i32]),
     "spx_solve_batched_cluster": (ctypes.c_int, [_vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp,
                                                  _vp, _vp, _vp]),
     "spx_cluster_size": (_i32, [_i32, _i32]),

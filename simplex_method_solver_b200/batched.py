@@ -83,71 +83,28 @@ def _sens_uniform(T, status, rowlab, collab, B: int, n: int, m: int, device) -> 
 
 
 ENGINES = ("auto", "smem", "cluster", "global", "auto_global")
+ENGINE_CODES = {"auto": N.ENGINE_AUTO, "smem": N.ENGINE_SMEM, "cluster": N.ENGINE_CLUSTER, "global": N.ENGINE_GLOBAL,
+                "auto_global": N.ENGINE_AUTO_GLOBAL}
 _INT32_MAX = (1 << 31) - 1
-
-
-def _cluster_capacity_text(n: int, m: int) -> str:
-    L = N.load()
-    if L.spx_cluster_size(1, m) == 0:
-        return f"at most {max(k for k in range(1, m + 1) if L.spx_cluster_size(1, k))} columns fit one cluster"
-    lo, hi = 1, 1 << 20                        # largest n with spx_cluster_size(n, m) > 0
-    while lo < hi:
-        mid = (lo + hi + 1) // 2
-        lo, hi = (mid, hi) if L.spx_cluster_size(mid, m) else (lo, mid - 1)
-    return f"at m = {m} one cluster of 16 CTAs holds at most n = {lo} rows"
-
-
-def _global_capacity_text(n: int, m: int) -> str:
-    L = N.load()
-    if L.spx_global_min_cluster_size(1, m) == 0:
-        lo, hi = 1, m                          # largest m with spx_global_min_cluster_size(1, m) > 0
-        while lo < hi:
-            mid = (lo + hi + 1) // 2
-            lo, hi = (mid, hi) if L.spx_global_min_cluster_size(1, mid) else (lo, mid - 1)
-        return f"at most {lo} columns fit one cluster"
-    lo, hi = 1, n                              # largest n with spx_global_min_cluster_size(n, m) > 0
-    while lo < hi:
-        mid = (lo + hi + 1) // 2
-        lo, hi = (mid, hi) if L.spx_global_min_cluster_size(mid, m) else (lo, mid - 1)
-    return f"at m = {m} one cluster of 16 CTAs holds at most n = {lo} rows"
 
 
 def kernel_for(n: int, m: int, engine: str = "auto") -> str:
     """"smem" (K4), "cluster" (K7) or "global" (K8) for an n x m LP; ValueError when the engine cannot take it.
 
-    "auto" is K4 when ``spx_batched_fits(n, m)`` (at most ``spx_batched_max_cells()`` cells, and one CTA's shared
-    memory holds the LP), else K7.  "auto_global" is "auto" with K8 above K7's capacity: K4 when it fits, else K7
-    when ``spx_cluster_size(n, m) > 0``, else K8 (the routing of ragged batches that mix every size).
+    The library's routing rule, ``spx_batched_route`` (include/spx_b200.h): "auto" is K4 when
+    ``spx_batched_fits(n, m)`` (at most ``spx_batched_max_cells()`` cells, and one CTA's shared memory holds the LP),
+    else K7.  "auto_global" is "auto" with K8 above K7's capacity: K4 when it fits, else K7 when
+    ``spx_cluster_size(n, m) > 0``, else K8 (the routing of ragged batches that mix every size).
     """
     if engine not in ENGINES:
         raise ValueError(f"unknown engine {engine!r}; one of {ENGINES}")
     if not (1 <= n <= _INT32_MAX and 1 <= m <= _INT32_MAX):
         raise ValueError(f"bad shape {n} x {m}")
     L = N.load()
-    cells = n * (m + 1) + m
-    fits = bool(L.spx_batched_fits(n, m))
-    if engine == "auto_global":
-        if fits:
-            return "smem"
-        engine = "cluster" if L.spx_cluster_size(n, m) else "global"
-    if engine == "global":
-        if L.spx_global_min_cluster_size(n, m) == 0:
-            raise ValueError(f"a {n} x {m} LP ({cells} cells) exceeds the capacity of the global-memory cluster "
-                             f"solver: {_global_capacity_text(n, m)}; use SimplexMethod / DeviceTableau")
-        return "global"
-    if engine == "smem" or (engine == "auto" and fits):
-        if cells > L.spx_batched_max_cells():
-            raise ValueError(f"{cells} cells per LP exceed the shared-memory limit of one CTA "
-                             f"({L.spx_batched_max_cells()}); use engine='cluster' or 'auto'")
-        if not fits:
-            raise ValueError(f"a {n} x {m} LP ({cells} cells) does not fit the shared memory of one CTA; "
-                             "use engine='cluster' or 'auto'")
-        return "smem"
-    if L.spx_cluster_size(n, m) == 0:
-        raise ValueError(f"a {n} x {m} LP ({cells} cells) exceeds the capacity of the cluster solver: "
-                         f"{_cluster_capacity_text(n, m)}; use engine='global' (K8) up to its capacity, or "
-                         "SimplexMethod / DeviceTableau for large tableaus")
-    return "cluster"
+    code = L.spx_batched_route(n, m, ENGINE_CODES[engine])
+    if code < 0:
+        raise ValueError(L.spx_last_error().decode(errors="replace"))
+    return {N.ENGINE_SMEM: "smem", N.ENGINE_CLUSTER: "cluster", N.ENGINE_GLOBAL: "global"}[code]
 
 
 _ENTRIES = {"smem": "spx_solve_batched", "cluster": "spx_solve_batched_cluster", "global": "spx_solve_batched_global"}
@@ -237,8 +194,6 @@ def solve_batched(tables, n: int, m: int, max_pivots: int = 64, rule: str = "ref
 
 
 # ---------------------------------------------------------------------------- ragged batches
-ENGINE_CODES = {"auto": N.ENGINE_AUTO, "smem": N.ENGINE_SMEM, "cluster": N.ENGINE_CLUSTER, "global": N.ENGINE_GLOBAL,
-                "auto_global": N.ENGINE_AUTO_GLOBAL}
 # the plan spx_ragged_plan writes (csrc/spx_common.cuh: RaggedPlan, RaggedLaunch, RaggedLp)
 _LAUNCH = np.dtype([("kernel", "<i4"), ("S", "<i4"), ("threads", "<i4"), ("per_cta", "<i4"), ("smem", "<i8"),
                     ("first", "<i8"), ("count", "<i8"), ("slot_doubles", "<i8"), ("pick_S", "<i4"), ("reserved", "<i4")])

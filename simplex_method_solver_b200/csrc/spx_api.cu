@@ -50,10 +50,11 @@ cudaError_t lazy_guard_selftest(const double *, const double *, const double *, 
 cudaError_t init_state(spx_state *, int32_t *, int32_t *, int, int, int64_t, cudaStream_t);
 cudaError_t solve_batched(double *, int64_t, int, int, int, int, double *, double *, int32_t *,
                           int32_t *, int32_t *, int32_t *, int32_t *, double *, cudaStream_t);
+bool cluster_fits(int64_t, int64_t, int);
 int cluster_size(int64_t, int64_t);
-int cluster_size_for_solve(int64_t, int64_t);
 cudaError_t solve_batched_cluster(double *, int64_t, int, int, int, int, int, double *, double *, int32_t *,
                                   int32_t *, int32_t *, int32_t *, int32_t *, double *, cudaStream_t);
+bool global_fits(int64_t, int64_t, int);
 int global_min_cluster_size(int64_t, int64_t);
 cudaError_t global_cluster_size(int64_t, int64_t, int64_t, int *);
 cudaError_t solve_batched_global(double *, int64_t, int, int, int, int, int, double *, double *, int32_t *,
@@ -100,11 +101,23 @@ int check(cudaError_t e, const char *what) {
     return -1;
 }
 
+// puts printf-style text in front of the current error message
+void prefix_error(const char *fmt, ...) {
+    char msg[sizeof(g_err)];
+    std::memcpy(msg, g_err, sizeof(msg));
+    va_list ap;
+    va_start(ap, fmt);
+    const int k = vsnprintf(g_err, sizeof(g_err), fmt, ap);
+    va_end(ap);
+    if (k >= 0 && k < (int)sizeof(g_err)) snprintf(g_err + k, sizeof(g_err) - k, "%s", msg);
+}
+
 void count_launch(int k) { g_launches.fetch_add(k, std::memory_order_relaxed); }
 
 } // namespace spx_host
 
 using spx_host::check;
+using spx_host::prefix_error;
 using spx_host::set_error;
 
 #define SPX_REQUIRE(cond, ...)            \
@@ -116,6 +129,110 @@ using spx_host::set_error;
     } while (0)
 
 static inline cudaStream_t as_stream(void *s) { return reinterpret_cast<cudaStream_t>(s); }
+
+// ---- batched routing: which kernel takes an n x m LP under an engine code (K4, K7, K8) ------------------------
+namespace {
+
+bool known_engine(int engine) {
+    return (engine >= SPX_ENGINE_AUTO && engine <= SPX_ENGINE_CLUSTER) || engine == SPX_ENGINE_GLOBAL ||
+           engine == SPX_ENGINE_AUTO_GLOBAL;
+}
+
+// The capacity a one-cluster solver's footprint test `fits` (cluster_fits, global_fits) denies an n x m LP.  A
+// footprint grows with n and m and shrinks as S grows, so the limits are those of S = 16, found by bisection.
+void capacity_text(char *buf, size_t len, int64_t n, int64_t m, bool (*fits)(int64_t, int64_t, int)) {
+    auto last = [](int64_t lo, int64_t hi, auto ok) {     // the largest v in [lo, hi) with ok(v), given ok(lo), !ok(hi)
+        while (hi - lo > 1) {
+            const int64_t mid = lo + (hi - lo) / 2;
+            (ok(mid) ? lo : hi) = mid;
+        }
+        return lo;
+    };
+    const int64_t cols = last(1, (int64_t)INT32_MAX + 1, [&](int64_t v) { return fits(1, v, 16); });
+    if (m > cols) {
+        snprintf(buf, len, "capacity: at most %lld columns fit one cluster", (long long)cols);
+        return;
+    }
+    snprintf(buf, len, "capacity: at m = %lld one cluster of 16 CTAs holds at most n = %lld rows, and at most %lld "
+             "columns fit one cluster", (long long)m, (long long)last(1, n, [&](int64_t v) { return fits(v, m, 16); }),
+             (long long)cols);
+}
+
+// Where one LP runs: the kernel, its cluster size and its dynamic shared memory per CTA at that size.
+struct Route {
+    int     kernel;     // spx::RaggedKernel: RAGGED_WARP or RAGGED_CTA (K4), RAGGED_CLUSTER (K7), RAGGED_GLOBAL (K8)
+    int     S;          // K7: the cluster size; K8: S_min, or the forced size; K4: 1
+    int64_t bytes;      // at S; K4 warp mode: the LP's slot
+};
+
+// The one routing rule of the batched engines, for an n x m LP (n, m >= 1) under a known engine code, with
+// `forced` the cluster size SPX_OPT_CLUSTER_SIZE forces (0: none).  AUTO: K4 when batched_fits, else K7; SMEM,
+// CLUSTER, GLOBAL: that engine; AUTO_GLOBAL: AUTO, with K8 above K7's capacity.  False, with the error message
+// naming the capacity the LP exceeds, when that engine cannot take it.
+bool route_lp(int n, int m, int engine, int forced, Route *r) {
+    using namespace spx;
+    const int64_t cells = spx_cells(n, m);
+    const bool k4 = engine == SPX_ENGINE_SMEM ||
+                    ((engine == SPX_ENGINE_AUTO || engine == SPX_ENGINE_AUTO_GLOBAL) && spx_launch::batched_fits(n, m));
+    const bool k8 = engine == SPX_ENGINE_GLOBAL ||
+                    (engine == SPX_ENGINE_AUTO_GLOBAL && !k4 && spx_launch::cluster_size(n, m) == 0);
+    char cap[192];
+    r->S = 1;
+    if (k4) {
+        r->bytes = spx_launch::ragged_batched_bytes(n, m, &r->kernel);
+        if (r->bytes > 0) return true;
+        if (cells > spx_launch::batched_max_cells())
+            set_error("%lld cells per LP exceed the shared-memory resident limit %lld", (long long)cells,
+                      (long long)spx_launch::batched_max_cells());
+        else
+            set_error("a %d x %d LP (%lld cells) does not fit the shared memory of one CTA", n, m, (long long)cells);
+        return false;
+    }
+    if (k8) {
+        const int smin = spx_launch::global_min_cluster_size(n, m);
+        if (smin == 0) {
+            capacity_text(cap, sizeof(cap), n, m, spx_launch::global_fits);
+            set_error("a %d x %d LP exceeds the shared memory of one cluster (16 CTAs of 227 KB: 8*(2m+1+R) + 4*(R+Q) "
+                      "<= 230400 bytes with R = ceil(n/S), Q = ceil(m/S), S <= 16); %s", n, m, cap);
+            return false;
+        }
+        if (forced && smin > forced) {
+            set_error("a %d x %d LP does not fit a cluster of SPX_OPT_CLUSTER_SIZE = %d CTAs (8*(2m+1+R) + 4*(R+Q) "
+                      "<= 230400 bytes; at least %d CTAs)", n, m, forced, smin);
+            return false;
+        }
+        r->kernel = RAGGED_GLOBAL;
+        r->S = forced ? forced : smin;
+        r->bytes = spx_launch::ragged_global_bytes(n, m, r->S);
+        return true;
+    }
+    if (spx_launch::cluster_size(n, m) == 0) {
+        capacity_text(cap, sizeof(cap), n, m, spx_launch::cluster_fits);
+        set_error("a %d x %d LP exceeds one cluster (16 CTAs of 227 KB shared memory: 8*(R*(m+2)+2m+1) + 4*(R+Q) "
+                  "<= 230400 bytes with R = ceil(n/16), Q = ceil(m/16)); %s", n, m, cap);
+        return false;
+    }
+    if (forced && !spx_launch::cluster_fits(n, m, forced)) {
+        set_error("a %d x %d LP does not fit a cluster of SPX_OPT_CLUSTER_SIZE = %d CTAs", n, m, forced);
+        return false;
+    }
+    r->kernel = RAGGED_CLUSTER;
+    r->S = forced ? forced : spx_launch::cluster_size(n, m);
+    r->bytes = spx_launch::ragged_cluster_bytes(n, m, r->S);
+    return true;
+}
+
+int forced_cluster_size() { return (int)spx_launch::get_option(SPX_OPT_CLUSTER_SIZE); }
+
+// the result of a K7 or K8 launch, with the refusal of a device that cannot co-schedule one cluster spelled out
+int check_cluster_launch(cudaError_t e, const char *who, int S, int64_t smem) {
+    if (e != cudaErrorInvalidClusterSize) return check(e, who);
+    set_error("%s: the device cannot co-schedule one cluster of S = %d CTAs with %lld bytes of shared memory each "
+              "(cudaOccupancyMaxActiveClusters = 0)", who, S, (long long)smem);
+    return -1;
+}
+
+} // namespace
 
 extern "C" {
 
@@ -544,6 +661,22 @@ int spx_extract(const double *d_b, int32_t n, int32_t m, const int32_t *d_collab
                  "extract launch");
 }
 
+// ---- routing of the batched engines (route_lp) ---------------------------------------
+int32_t spx_batched_route(int32_t n, int32_t m, int32_t engine) {
+    if (!known_engine(engine)) {
+        set_error("unknown engine %d", engine);
+        return -1;
+    }
+    if (n < 1 || m < 1) {
+        set_error("bad shape %d x %d", n, m);
+        return -1;
+    }
+    Route r;
+    if (!route_lp(n, m, engine, 0, &r)) return -1;
+    return r.kernel == spx::RAGGED_GLOBAL ? SPX_ENGINE_GLOBAL
+                                          : (r.kernel == spx::RAGGED_CLUSTER ? SPX_ENGINE_CLUSTER : SPX_ENGINE_SMEM);
+}
+
 // ---- K4 -------------------------------------------------------------------------
 int64_t spx_batched_max_cells(void) { return spx_launch::batched_max_cells(); }
 int32_t spx_batched_fits(int32_t n, int32_t m) { return spx_launch::batched_fits(n, m) ? 1 : 0; }
@@ -554,12 +687,11 @@ int spx_solve_batched(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule
     SPX_REQUIRE(B >= 0 && n >= 1 && m >= 1 && max_pivots >= 0, "spx_solve_batched: bad arguments");
     SPX_REQUIRE(B == 0 || (d_T && d_status && d_npiv), "spx_solve_batched: null T/status/npiv");
     SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_solve_batched: unknown rule %d", rule);
-    SPX_REQUIRE(spx_cells(n, m) <= spx_batched_max_cells(),
-                "spx_solve_batched: %lld cells per LP exceed the shared-memory resident limit %lld; use spx_solve",
-                (long long)spx_cells(n, m), (long long)spx_batched_max_cells());
-    SPX_REQUIRE(spx_launch::batched_fits(n, m),
-                "spx_solve_batched: a %d x %d LP (%lld cells) does not fit the shared memory of one CTA; "
-                "use spx_solve_batched_cluster", n, m, (long long)spx_cells(n, m));
+    Route r;
+    if (!route_lp(n, m, SPX_ENGINE_SMEM, 0, &r)) {
+        prefix_error("spx_solve_batched: ");
+        return -2;
+    }
     cudaError_t e = spx_launch::solve_batched(d_T, B, n, m, rule, max_pivots, d_x, d_obj, d_status, d_npiv,
                                               d_rowlab, d_collab, d_trace, d_snap, as_stream(stream));
     return check(e, "batched launch");
@@ -575,23 +707,17 @@ int spx_solve_batched_cluster(double *d_T, int64_t B, int32_t n, int32_t m, int3
     SPX_REQUIRE(B == 0 || (d_T && d_status && d_npiv), "spx_solve_batched_cluster: null T/status/npiv");
     SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_solve_batched_cluster: unknown rule %d",
                 rule);
-    SPX_REQUIRE(spx_launch::cluster_size(n, m) > 0,
-                "spx_solve_batched_cluster: a %d x %d LP exceeds one cluster (16 CTAs of 227 KB shared memory: "
-                "8*(R*(m+2)+2m+1) + 4*(R+Q) <= 230400 bytes with R = ceil(n/16), Q = ceil(m/16))", n, m);
-    const int S = spx_launch::cluster_size_for_solve(n, m);
-    SPX_REQUIRE(S > 0, "spx_solve_batched_cluster: a %d x %d LP does not fit a cluster of SPX_OPT_CLUSTER_SIZE = %d CTAs",
-                n, m, (int)spx_launch::get_option(SPX_OPT_CLUSTER_SIZE));
-    SPX_REQUIRE(B <= INT32_MAX / S, "spx_solve_batched_cluster: B = %lld LPs x S = %d CTAs exceed one grid",
-                (long long)B, S);
-    const cudaError_t e = spx_launch::solve_batched_cluster(d_T, B, n, m, S, rule, max_pivots, d_x, d_obj, d_status,
-                                                            d_npiv, d_rowlab, d_collab, d_trace, d_snap,
-                                                            as_stream(stream));
-    if (e == cudaErrorInvalidClusterSize) {
-        set_error("spx_solve_batched_cluster: the device cannot co-schedule one cluster of S = %d CTAs for a %d x %d "
-                  "LP (cudaOccupancyMaxActiveClusters = 0)", S, n, m);
-        return -1;
+    Route r;
+    if (!route_lp(n, m, SPX_ENGINE_CLUSTER, forced_cluster_size(), &r)) {
+        prefix_error("spx_solve_batched_cluster: ");
+        return -2;
     }
-    return check(e, "cluster launch");
+    SPX_REQUIRE(B <= INT32_MAX / r.S, "spx_solve_batched_cluster: B = %lld LPs x S = %d CTAs exceed one grid",
+                (long long)B, r.S);
+    return check_cluster_launch(spx_launch::solve_batched_cluster(d_T, B, n, m, r.S, rule, max_pivots, d_x, d_obj,
+                                                                  d_status, d_npiv, d_rowlab, d_collab, d_trace,
+                                                                  d_snap, as_stream(stream)),
+                                "spx_solve_batched_cluster", r.S, r.bytes);
 }
 
 // ---- K8 -------------------------------------------------------------------------
@@ -610,30 +736,21 @@ int spx_solve_batched_global(double *d_T, int64_t B, int32_t n, int32_t m, int32
     SPX_REQUIRE(B == 0 || (d_T && d_status && d_npiv), "spx_solve_batched_global: null T/status/npiv");
     SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_solve_batched_global: unknown rule %d",
                 rule);
-    const int smin = spx_launch::global_min_cluster_size(n, m);
-    SPX_REQUIRE(smin > 0,
-                "spx_solve_batched_global: a %d x %d LP exceeds the shared memory of one cluster (16 CTAs of 227 KB: "
-                "8*(2m+1+R) + 4*(R+Q) <= 230400 bytes with R = ceil(n/S), Q = ceil(m/S), S <= 16)", n, m);
-    const int forced = (int)spx_launch::get_option(SPX_OPT_CLUSTER_SIZE);
-    SPX_REQUIRE(forced == 0 || spx_global_min_cluster_size(n, m) <= forced,
-                "spx_solve_batched_global: a %d x %d LP does not fit a cluster of SPX_OPT_CLUSTER_SIZE = %d CTAs "
-                "(8*(2m+1+R) + 4*(R+Q) <= 230400 bytes; at least %d CTAs)", n, m, forced, smin);
+    Route r;
+    if (!route_lp(n, m, SPX_ENGINE_GLOBAL, forced_cluster_size(), &r)) {
+        prefix_error("spx_solve_batched_global: ");
+        return -2;
+    }
     // a default S above S_min is only chosen when all B clusters are co-resident, far below the grid limit
-    const int Smax = forced ? forced : smin;
-    SPX_REQUIRE(B <= INT32_MAX / Smax, "spx_solve_batched_global: B = %lld LPs x S = %d CTAs exceed one grid",
-                (long long)B, Smax);
+    SPX_REQUIRE(B <= INT32_MAX / r.S, "spx_solve_batched_global: B = %lld LPs x S = %d CTAs exceed one grid",
+                (long long)B, r.S);
     if (B == 0) return 0;
     int S = 0;
     if (check(spx_launch::global_cluster_size(n, m, B, &S), "spx_solve_batched_global: occupancy")) return -1;
-    const cudaError_t e = spx_launch::solve_batched_global(d_T, B, n, m, S, rule, max_pivots, d_x, d_obj, d_status,
-                                                           d_npiv, d_rowlab, d_collab, d_trace, d_snap,
-                                                           as_stream(stream));
-    if (e == cudaErrorInvalidClusterSize) {
-        set_error("spx_solve_batched_global: the device cannot co-schedule one cluster of S = %d CTAs for a %d x %d "
-                  "LP (cudaOccupancyMaxActiveClusters = 0)", S, n, m);
-        return -1;
-    }
-    return check(e, "global launch");
+    return check_cluster_launch(spx_launch::solve_batched_global(d_T, B, n, m, S, rule, max_pivots, d_x, d_obj,
+                                                                 d_status, d_npiv, d_rowlab, d_collab, d_trace,
+                                                                 d_snap, as_stream(stream)),
+                                "spx_solve_batched_global", S, spx_launch::ragged_global_bytes(n, m, S));
 }
 
 // ---- ragged batches (K4 + K7 + K8) ---------------------------------------------------
@@ -648,8 +765,7 @@ int spx_ragged_plan(const int32_t *h_shapes, int64_t B, int32_t engine, void *h_
                     int64_t *h_totals) {
     using namespace spx;
     SPX_REQUIRE(B >= 0 && B <= INT32_MAX, "spx_ragged_plan: bad batch size B = %lld", (long long)B);
-    SPX_REQUIRE((engine >= SPX_ENGINE_AUTO && engine <= SPX_ENGINE_CLUSTER) || engine == SPX_ENGINE_GLOBAL ||
-                engine == SPX_ENGINE_AUTO_GLOBAL, "spx_ragged_plan: unknown engine %d", engine);
+    SPX_REQUIRE(known_engine(engine), "spx_ragged_plan: unknown engine %d", engine);
     SPX_REQUIRE(h_plan && h_totals && (B == 0 || h_shapes), "spx_ragged_plan: null shapes/plan/totals");
     SPX_REQUIRE(plan_bytes >= spx_ragged_plan_bytes(B), "spx_ragged_plan: plan_bytes = %lld < spx_ragged_plan_bytes(%lld) = %lld",
                 (long long)plan_bytes, (long long)B, (long long)spx_ragged_plan_bytes(B));
@@ -657,7 +773,7 @@ int spx_ragged_plan(const int32_t *h_shapes, int64_t B, int32_t engine, void *h_
     RaggedLp *lps = reinterpret_cast<RaggedLp *>(static_cast<char *>(h_plan) + ragged_lp_offset());
     int32_t *order = reinterpret_cast<int32_t *>(lps + B);
     // class of every LP: 0 warp mode, 1 CTA mode, 2 + log2(S) K7, 7 + log2(S) K8; and its shared-memory footprint
-    const int forced = (int)spx_launch::get_option(SPX_OPT_CLUSTER_SIZE);
+    const int forced = forced_cluster_size();
     std::vector<int8_t> cls((size_t)B);
     std::vector<int64_t> bytes((size_t)B);
     int64_t tot[5] = {0, 0, 0, 0, 0};
@@ -665,43 +781,15 @@ int spx_ragged_plan(const int32_t *h_shapes, int64_t B, int32_t engine, void *h_
         const int32_t n = h_shapes[3 * k], m = h_shapes[3 * k + 1], cap = h_shapes[3 * k + 2];
         SPX_REQUIRE(n >= 1 && m >= 1 && cap >= 0, "spx_ragged_plan: LP %lld: bad shape n=%d m=%d max_pivots=%d",
                     (long long)k, n, m, cap);
-        const int64_t cells = spx_cells(n, m);
-        const bool k4 = engine == SPX_ENGINE_SMEM ||
-                        ((engine == SPX_ENGINE_AUTO || engine == SPX_ENGINE_AUTO_GLOBAL) && spx_launch::batched_fits(n, m));
-        const bool k8 = engine == SPX_ENGINE_GLOBAL ||
-                        (engine == SPX_ENGINE_AUTO_GLOBAL && !k4 && spx_launch::cluster_size(n, m) == 0);
-        if (k8) {
-            const int smin = spx_launch::global_min_cluster_size(n, m);
-            SPX_REQUIRE(smin > 0,
-                        "spx_ragged_plan: LP %lld: a %d x %d LP exceeds the shared memory of one cluster (16 CTAs of "
-                        "227 KB: 8*(2m+1+R) + 4*(R+Q) <= 230400 bytes with R = ceil(n/S), Q = ceil(m/S), S <= 16)",
-                        (long long)k, n, m);
-            SPX_REQUIRE(forced == 0 || smin <= forced,
-                        "spx_ragged_plan: LP %lld: a %d x %d LP does not fit a cluster of SPX_OPT_CLUSTER_SIZE = %d CTAs "
-                        "(8*(2m+1+R) + 4*(R+Q) <= 230400 bytes; at least %d CTAs)", (long long)k, n, m, forced, smin);
-            const int S = forced ? forced : smin;
-            bytes[k] = spx_launch::ragged_global_bytes(n, m, S);
-            cls[k] = (int8_t)(7 + __builtin_ctz((unsigned)S));
-        } else if (k4) {
-            int kern = 0;
-            bytes[k] = spx_launch::ragged_batched_bytes(n, m, &kern);
-            SPX_REQUIRE(bytes[k] > 0 || cells > spx_batched_max_cells(),
-                        "spx_ragged_plan: LP %lld: a %d x %d LP (%lld cells) does not fit the shared memory of one CTA; "
-                        "use engine auto or cluster", (long long)k, n, m, (long long)cells);
-            SPX_REQUIRE(bytes[k] > 0, "spx_ragged_plan: LP %lld: %lld cells per LP exceed the shared-memory resident "
-                        "limit %lld; use spx_solve", (long long)k, (long long)cells, (long long)spx_batched_max_cells());
-            cls[k] = (int8_t)kern;
-        } else {
-            SPX_REQUIRE(spx_launch::cluster_size(n, m) > 0,
-                        "spx_ragged_plan: LP %lld: a %d x %d LP exceeds one cluster (16 CTAs of 227 KB shared memory: "
-                        "8*(R*(m+2)+2m+1) + 4*(R+Q) <= 230400 bytes with R = ceil(n/16), Q = ceil(m/16))",
-                        (long long)k, n, m);
-            const int S = spx_launch::cluster_size_for_solve(n, m);
-            SPX_REQUIRE(S > 0, "spx_ragged_plan: LP %lld: a %d x %d LP does not fit a cluster of SPX_OPT_CLUSTER_SIZE = %d CTAs",
-                        (long long)k, n, m, (int)spx_launch::get_option(SPX_OPT_CLUSTER_SIZE));
-            bytes[k] = spx_launch::ragged_cluster_bytes(n, m, S);
-            cls[k] = (int8_t)(2 + __builtin_ctz((unsigned)S));
+        Route r;
+        if (!route_lp(n, m, engine, forced, &r)) {
+            prefix_error("spx_ragged_plan: LP %lld: ", (long long)k);
+            return -2;
         }
+        bytes[k] = r.bytes;
+        cls[k] = (int8_t)(r.kernel == RAGGED_CLUSTER ? 2 + __builtin_ctz((unsigned)r.S)
+                          : r.kernel == RAGGED_GLOBAL ? 7 + __builtin_ctz((unsigned)r.S) : r.kernel);
+        const int64_t cells = spx_cells(n, m);
         lps[k] = RaggedLp{n, m, cap, (int32_t)cells, tot[0], tot[1], tot[2], tot[3], tot[4]};
         tot[0] += cells;
         tot[1] += m;
@@ -802,30 +890,21 @@ int spx_solve_batched_ragged(double *d_T, const void *h_plan, const void *d_plan
                 return -1;
             SPX_REQUIRE(l.count <= INT32_MAX / S, "spx_solve_batched_ragged: %lld LPs x S = %d CTAs exceed one grid",
                         (long long)l.count, S);
-            const cudaError_t e = spx_launch::solve_ragged_global(l, S, smem, lps, order, d_T, rule, d_x, d_obj, d_status,
-                                                                  d_npiv, d_rowlab, d_collab, d_trace, d_snap, s);
-            if (e == cudaErrorInvalidClusterSize) {
-                set_error("spx_solve_batched_ragged: the device cannot co-schedule one cluster of S = %d CTAs with %lld "
-                          "bytes of shared memory each (cudaOccupancyMaxActiveClusters = 0)", S, (long long)smem);
+            if (check_cluster_launch(spx_launch::solve_ragged_global(l, S, smem, lps, order, d_T, rule, d_x, d_obj,
+                                                                     d_status, d_npiv, d_rowlab, d_collab, d_trace,
+                                                                     d_snap, s),
+                                     "spx_solve_batched_ragged", S, smem))
                 return -1;
-            }
-            if (check(e, "ragged global launch")) return -1;
-            continue;
-        }
-        if (l.kernel != RAGGED_CLUSTER) {
-            if (check(spx_launch::solve_ragged_batched(l, lps, order, d_T, rule, d_x, d_obj, d_status, d_npiv, d_rowlab,
-                                                       d_collab, d_trace, d_snap, s), "ragged batched launch"))
+        } else if (l.kernel == RAGGED_CLUSTER) {
+            if (check_cluster_launch(spx_launch::solve_ragged_cluster(l, lps, order, d_T, rule, d_x, d_obj, d_status,
+                                                                      d_npiv, d_rowlab, d_collab, d_trace, d_snap, s),
+                                     "spx_solve_batched_ragged", l.S, l.smem))
                 return -1;
-            continue;
-        }
-        const cudaError_t e = spx_launch::solve_ragged_cluster(l, lps, order, d_T, rule, d_x, d_obj, d_status, d_npiv,
-                                                               d_rowlab, d_collab, d_trace, d_snap, s);
-        if (e == cudaErrorInvalidClusterSize) {
-            set_error("spx_solve_batched_ragged: the device cannot co-schedule one cluster of S = %d CTAs with %lld bytes "
-                      "of shared memory each (cudaOccupancyMaxActiveClusters = 0)", l.S, (long long)l.smem);
+        } else if (check(spx_launch::solve_ragged_batched(l, lps, order, d_T, rule, d_x, d_obj, d_status, d_npiv,
+                                                            d_rowlab, d_collab, d_trace, d_snap, s),
+                         "ragged batched launch")) {
             return -1;
         }
-        if (check(e, "ragged cluster launch")) return -1;
     }
     return 0;
 }

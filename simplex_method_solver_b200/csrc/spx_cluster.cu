@@ -36,12 +36,6 @@ namespace {
 
 using namespace spx;
 
-constexpr int    CLUSTER_THREADS   = 512;
-constexpr int    CLUSTER_MAX_S     = 16;
-constexpr size_t CLUSTER_SMEM      = 227 * 1024;                    // shared memory of one CTA, static + dynamic
-constexpr size_t CLUSTER_STATIC    = 2048;                          // reserved for the kernel's static scratch
-constexpr size_t CLUSTER_DYN_BYTES = CLUSTER_SMEM - CLUSTER_STATIC;  // 230,400 bytes for the footprint above
-
 struct ClusterArgs {
     double  *T;          // [B][cells] in/out
     int64_t  B;
@@ -233,15 +227,13 @@ int64_t cluster_bytes(int64_t n, int64_t m, int S) {
     return 8 * (R * (m + 2) + 2 * m + 1) + 4 * (R + Q);
 }
 
-bool cluster_fits(int64_t n, int64_t m, int S) {
-    return n >= 1 && m >= 1 && cluster_bytes(n, m, S) <= (int64_t)CLUSTER_DYN_BYTES;
-}
-
 } // namespace
 
 namespace spx_launch {
 
-int64_t get_option(int key);
+bool cluster_fits(int64_t n, int64_t m, int S) {
+    return n >= 1 && m >= 1 && cluster_bytes(n, m, S) <= (int64_t)CLUSTER_DYN_BYTES;
+}
 
 // smallest S in {1, 2, 4, 8, 16} whose footprint fits, 0 when none does
 int cluster_size(int64_t n, int64_t m) {
@@ -250,54 +242,14 @@ int cluster_size(int64_t n, int64_t m) {
     return 0;
 }
 
-// S for a solve: SPX_OPT_CLUSTER_SIZE when set (0 if that S does not fit), else cluster_size()
-int cluster_size_for_solve(int64_t n, int64_t m) {
-    const int forced = (int)get_option(SPX_OPT_CLUSTER_SIZE);
-    if (forced > 0) return cluster_fits(n, m, forced) ? forced : 0;
-    return cluster_size(n, m);
-}
-
 // S CTAs per LP (validated by the caller); returns cudaErrorInvalidClusterSize when the device cannot co-schedule
 // one cluster of this size and footprint
 cudaError_t solve_batched_cluster(double *T, int64_t B, int n, int m, int S, int rule, int max_pivots, double *x,
                                   double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab, int32_t *collab,
                                   int32_t *trace, double *snap, cudaStream_t stream) {
-    if (B <= 0) return cudaSuccess;
-    static bool configured_dev[64] = {};
-    const int slot = spx_host::device_slot();
-    if (!configured_dev[slot]) {
-        cudaFuncAttributes fa;
-        cudaError_t e = cudaFuncGetAttributes(&fa, cluster_kernel);
-        if (e != cudaSuccess) return e;
-        if (fa.sharedSizeBytes > CLUSTER_STATIC) return cudaErrorInvalidValue;
-        e = cudaFuncSetAttribute(cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLUSTER_DYN_BYTES);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-        if (e != cudaSuccess) return e;
-        configured_dev[slot] = true;
-    }
     ClusterArgs a{T, B, n, m, rule, max_pivots, S, (n + S - 1) / S, (m + S - 1) / S,
                   x, obj, status, npiv, rowlab, collab, trace, snap};
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(B * S));
-    cfg.blockDim = dim3(CLUSTER_THREADS);
-    cfg.dynamicSmemBytes = (size_t)cluster_bytes(n, m, S);
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = (unsigned)S;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    int clusters = 0;
-    cudaError_t e = cudaOccupancyMaxActiveClusters(&clusters, cluster_kernel, &cfg);
-    if (e != cudaSuccess) return e;
-    if (clusters <= 0) return cudaErrorInvalidClusterSize;
-    e = cudaLaunchKernelEx(&cfg, cluster_kernel, a);
-    spx_host::count_launch();
-    if (e != cudaSuccess) return e;
-    return cudaGetLastError();
+    return launch_cluster_kernel<cluster_kernel>(S, B, cluster_bytes(n, m, S), stream, a);
 }
 
 int64_t ragged_cluster_bytes(int n, int m, int S) { return cluster_bytes(n, m, S); }
@@ -307,43 +259,8 @@ int64_t ragged_cluster_bytes(int n, int m, int S) { return cluster_bytes(n, m, S
 cudaError_t solve_ragged_cluster(const RaggedLaunch &l, const RaggedLp *lps, const int32_t *order, double *T, int rule,
                                  double *x, double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab,
                                  int32_t *collab, int32_t *trace, double *snap, cudaStream_t stream) {
-    if (l.count <= 0) return cudaSuccess;
-    static bool configured_dev[64] = {};
-    const int slot = spx_host::device_slot();
-    if (!configured_dev[slot]) {
-        cudaFuncAttributes fa;
-        cudaError_t e = cudaFuncGetAttributes(&fa, ragged_cluster_kernel);
-        if (e != cudaSuccess) return e;
-        if (fa.sharedSizeBytes > CLUSTER_STATIC) return cudaErrorInvalidValue;
-        e = cudaFuncSetAttribute(ragged_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)CLUSTER_DYN_BYTES);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(ragged_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-        if (e != cudaSuccess) return e;
-        configured_dev[slot] = true;
-    }
     ClusterArgs a{T, l.count, 0, 0, rule, 0, l.S, 0, 0, x, obj, status, npiv, rowlab, collab, trace, snap};
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(l.count * l.S));
-    cfg.blockDim = dim3(CLUSTER_THREADS);
-    cfg.dynamicSmemBytes = (size_t)l.smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = (unsigned)l.S;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    int clusters = 0;
-    cudaError_t e = cudaOccupancyMaxActiveClusters(&clusters, ragged_cluster_kernel, &cfg);
-    if (e != cudaSuccess) return e;
-    if (clusters <= 0) return cudaErrorInvalidClusterSize;
-    const int32_t *ord = order + l.first;
-    e = cudaLaunchKernelEx(&cfg, ragged_cluster_kernel, a, lps, ord);
-    spx_host::count_launch();
-    if (e != cudaSuccess) return e;
-    return cudaGetLastError();
+    return launch_cluster_kernel<ragged_cluster_kernel>(l.S, l.count, l.smem, stream, a, lps, order + l.first);
 }
 
 } // namespace spx_launch

@@ -1,12 +1,18 @@
-// spx_cluster.cuh — the pricing steps shared by the two one-cluster-per-LP solvers, K7 (spx_cluster.cu, table in
-// shared memory) and K8 (spx_global.cu, table in global memory): the entering column of the replicated f row and
-// the merge of the S per-CTA partials into one pivot decision that every CTA reaches on its own.
+// spx_cluster.cuh — what the two one-cluster-per-LP solvers, K7 (spx_cluster.cu, table in shared memory) and K8
+// (spx_global.cu, table in global memory), share: the pricing steps (the entering column of the replicated f row and
+// the merge of the S per-CTA partials into one pivot decision that every CTA reaches on its own), and the host launch.
 #pragma once
 #include <cooperative_groups.h>
 
 #include "spx_block.cuh"
 
 namespace spx {
+
+constexpr int    CLUSTER_THREADS   = 512;
+constexpr int    CLUSTER_MAX_S     = 16;
+constexpr size_t CLUSTER_SMEM      = 227 * 1024;                    // shared memory of one CTA, static + dynamic
+constexpr size_t CLUSTER_STATIC    = 2048;                          // reserved for the kernel's static scratch
+constexpr size_t CLUSTER_DYN_BYTES = CLUSTER_SMEM - CLUSTER_STATIC;  // 230,400 bytes for the per-CTA footprint
 
 // what one CTA knows about the pivot after folding its band
 struct Partial {
@@ -58,6 +64,62 @@ __device__ __forceinline__ void cluster_decide(cooperative_groups::cluster_group
         c = cf;
     }
     if (tid == 0) { ctl[0] = st; ctl[1] = r; ctl[2] = c; }
+}
+
+// ---- host: the launch of a K7 or K8 kernel ----
+// launch configuration of `clusters` LPs at S CTAs each with `smem` bytes of dynamic shared memory per CTA; attr must
+// outlive cfg
+inline cudaLaunchConfig_t cluster_launch_config(int64_t smem, int S, int64_t clusters, cudaLaunchAttribute *attr,
+                                                cudaStream_t stream) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)(clusters * S));
+    cfg.blockDim = dim3(CLUSTER_THREADS);
+    cfg.dynamicSmemBytes = (size_t)smem;
+    cfg.stream = stream;
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = (unsigned)S;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cfg;
+}
+
+// one-time per-device set-up of Kernel's shared memory and cluster size limits
+template <auto Kernel>
+cudaError_t configure_cluster_kernel() {
+    static bool configured_dev[64] = {};
+    const int slot = spx_host::device_slot();
+    if (configured_dev[slot]) return cudaSuccess;
+    cudaFuncAttributes fa;
+    cudaError_t e = cudaFuncGetAttributes(&fa, Kernel);
+    if (e != cudaSuccess) return e;
+    if (fa.sharedSizeBytes > CLUSTER_STATIC) return cudaErrorInvalidValue;
+    e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CLUSTER_DYN_BYTES);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+    if (e != cudaSuccess) return e;
+    configured_dev[slot] = true;
+    return cudaSuccess;
+}
+
+// Kernel(args...) on `clusters` LPs at S CTAs each (validated by the caller) with `smem` bytes per CTA; returns
+// cudaErrorInvalidClusterSize when the device cannot co-schedule one such cluster
+template <auto Kernel, typename... Args>
+cudaError_t launch_cluster_kernel(int S, int64_t clusters, int64_t smem, cudaStream_t stream, Args... args) {
+    if (clusters <= 0) return cudaSuccess;
+    cudaError_t e = configure_cluster_kernel<Kernel>();
+    if (e != cudaSuccess) return e;
+    cudaLaunchAttribute attr[1];
+    const cudaLaunchConfig_t cfg = cluster_launch_config(smem, S, clusters, attr, stream);
+    int active = 0;
+    e = cudaOccupancyMaxActiveClusters(&active, Kernel, &cfg);
+    if (e != cudaSuccess) return e;
+    if (active <= 0) return cudaErrorInvalidClusterSize;
+    e = cudaLaunchKernelEx(&cfg, Kernel, args...);
+    spx_host::count_launch();
+    if (e != cudaSuccess) return e;
+    return cudaGetLastError();
 }
 
 } // namespace spx

@@ -9,7 +9,7 @@
 // band's old pivot-column entries, the band's row labels cl and a slice of Q = ceil(m/S) header labels rl.  Per CTA,
 // in bytes:
 //     8 * (m + (m+1) + R)  +  4 * (R + Q)                f row, pivot row, pivot column; cl, rl slice
-// which must fit GLOBAL_DYN_BYTES (227 KB minus the static reduction scratch): m <= 11,519 at S = 1 and 14,177 at
+// which must fit CLUSTER_DYN_BYTES (227 KB minus the static reduction scratch): m <= 11,519 at S = 1 and 14,177 at
 // S = 16; at m = 2,000, n <= 15,866 at S = 1 and 263,856 at S = 16.
 //
 // One pivot, per CTA (K7's protocol):
@@ -40,15 +40,10 @@ namespace {
 
 using namespace spx;
 
-constexpr int    GLOBAL_THREADS   = 512;
 // one CTA of 512 threads per SM: the pricing and the division's slow path need more than the 64 registers two would
 // leave (spills); six 16-byte loads in flight per thread keep 48 KB per SM in flight for the update
 constexpr int    GLOBAL_MIN_CTAS  = 1;
 constexpr int    GLOBAL_UNROLL    = 6;
-constexpr int    GLOBAL_MAX_S     = 16;
-constexpr size_t GLOBAL_SMEM      = 227 * 1024;                    // shared memory of one CTA, static + dynamic
-constexpr size_t GLOBAL_STATIC    = 2048;                          // reserved for the kernel's static scratch
-constexpr size_t GLOBAL_DYN_BYTES = GLOBAL_SMEM - GLOBAL_STATIC;   // 230,400 bytes for the footprint above
 
 struct GlobalArgs {
     double  *T;          // [B][cells] in/out
@@ -279,13 +274,13 @@ __device__ __forceinline__ void global_body(const GlobalArgs &a, const RaggedLp 
     }
 }
 
-__global__ void __launch_bounds__(GLOBAL_THREADS, GLOBAL_MIN_CTAS) global_kernel(GlobalArgs a) {
+__global__ void __launch_bounds__(CLUSTER_THREADS, GLOBAL_MIN_CTAS) global_kernel(GlobalArgs a) {
     global_body<false>(a, nullptr, nullptr);
 }
 
 // a ragged batch: the LPs order[0 .. a.B) at one cluster size a.S, each cluster its own shape (a.n, a.m, a.R, a.Q,
 // a.max_pivots unused)
-__global__ void __launch_bounds__(GLOBAL_THREADS, GLOBAL_MIN_CTAS)
+__global__ void __launch_bounds__(CLUSTER_THREADS, GLOBAL_MIN_CTAS)
 ragged_global_kernel(GlobalArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order) {
     global_body<true>(a, lps, order);
 }
@@ -296,68 +291,21 @@ int64_t global_bytes(int64_t n, int64_t m, int S) {
     return 8 * (2 * m + 1 + R) + 4 * (R + Q);
 }
 
-bool global_fits(int64_t n, int64_t m, int S) {
-    return n >= 1 && m >= 1 && global_bytes(n, m, S) <= (int64_t)GLOBAL_DYN_BYTES;
-}
-
-// one-time per-device set-up of a K8 kernel's shared memory and cluster size limits
-template <typename Kernel>
-cudaError_t configure_kernel(Kernel kernel, bool (&configured_dev)[64]) {
-    const int slot = spx_host::device_slot();
-    if (configured_dev[slot]) return cudaSuccess;
-    cudaFuncAttributes fa;
-    cudaError_t e = cudaFuncGetAttributes(&fa, kernel);
-    if (e != cudaSuccess) return e;
-    if (fa.sharedSizeBytes > GLOBAL_STATIC) return cudaErrorInvalidValue;
-    e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GLOBAL_DYN_BYTES);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-    if (e != cudaSuccess) return e;
-    configured_dev[slot] = true;
-    return cudaSuccess;
-}
-
-cudaError_t configure() {
-    static bool configured_dev[64] = {};
-    return configure_kernel(global_kernel, configured_dev);
-}
-
-cudaError_t configure_ragged() {
-    static bool configured_dev[64] = {};
-    return configure_kernel(ragged_global_kernel, configured_dev);
-}
-
-// launch configuration of `clusters` LPs at S CTAs each with `smem` bytes of dynamic shared memory per CTA; attr must
-// outlive cfg
-cudaLaunchConfig_t launch_config(int64_t smem, int S, int64_t clusters, cudaLaunchAttribute *attr,
-                                 cudaStream_t stream) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(clusters * S));
-    cfg.blockDim = dim3(GLOBAL_THREADS);
-    cfg.dynamicSmemBytes = (size_t)smem;
-    cfg.stream = stream;
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = (unsigned)S;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    return cfg;
-}
-
 // The default cluster size of a K8 launch of `count` LPs on the current device: the S >= s_lo that keeps the most SMs
 // busy, min(count, co-resident clusters at S) * S, the smaller S on ties; bytes(S) is the launch's footprint at S
 // (which fits for every S >= s_lo: it does not grow with S).  A CTA streams its band at a rate bounded by its own
 // bytes in flight, so an idle SM is lost bandwidth, while a larger S costs barrier time per pivot: a single LP gets
 // 16 CTAs, a batch that fills the GPU at s_lo gets s_lo.
-template <typename Kernel, typename Bytes>
-cudaError_t busiest_cluster_size(Kernel kernel, int s_lo, int64_t count, Bytes bytes, int *S_out) {
+template <auto Kernel, typename Bytes>
+cudaError_t busiest_cluster_size(int s_lo, int64_t count, Bytes bytes, int *S_out) {
+    cudaError_t e = configure_cluster_kernel<Kernel>();
+    if (e != cudaSuccess) return e;
     int64_t best = -1;
-    for (int S = s_lo; S <= GLOBAL_MAX_S; S *= 2) {
+    for (int S = s_lo; S <= CLUSTER_MAX_S; S *= 2) {
         cudaLaunchAttribute attr[1];
-        const cudaLaunchConfig_t cfg = launch_config(bytes(S), S, 1, attr, nullptr);
+        const cudaLaunchConfig_t cfg = cluster_launch_config(bytes(S), S, 1, attr, nullptr);
         int clusters = 0;
-        const cudaError_t e = cudaOccupancyMaxActiveClusters(&clusters, kernel, &cfg);
+        e = cudaOccupancyMaxActiveClusters(&clusters, Kernel, &cfg);
         if (e != cudaSuccess) return e;
         const int64_t busy = (count < clusters ? count : (int64_t)clusters) * S;
         if (busy > best) { best = busy; *S_out = S; }
@@ -381,9 +329,13 @@ namespace spx_launch {
 
 int64_t get_option(int key);
 
+bool global_fits(int64_t n, int64_t m, int S) {
+    return n >= 1 && m >= 1 && global_bytes(n, m, S) <= (int64_t)CLUSTER_DYN_BYTES;
+}
+
 // smallest S in {1, 2, 4, 8, 16} whose footprint fits, 0 when none does
 int global_min_cluster_size(int64_t n, int64_t m) {
-    for (int S = 1; S <= GLOBAL_MAX_S; S *= 2)
+    for (int S = 1; S <= CLUSTER_MAX_S; S *= 2)
         if (global_fits(n, m, S)) return S;
     return 0;
 }
@@ -399,9 +351,7 @@ cudaError_t global_cluster_size(int64_t n, int64_t m, int64_t B, int *S_out) {
     }
     const int smin = global_min_cluster_size(n, m);
     if (smin == 0) return cudaSuccess;
-    cudaError_t e = configure();
-    if (e != cudaSuccess) return e;
-    return busiest_cluster_size(global_kernel, smin, B, [&](int S) { return global_bytes(n, m, S); }, S_out);
+    return busiest_cluster_size<global_kernel>(smin, B, [&](int S) { return global_bytes(n, m, S); }, S_out);
 }
 
 // S CTAs per LP (validated by the caller); returns cudaErrorInvalidClusterSize when the device cannot co-schedule
@@ -409,21 +359,9 @@ cudaError_t global_cluster_size(int64_t n, int64_t m, int64_t B, int *S_out) {
 cudaError_t solve_batched_global(double *T, int64_t B, int n, int m, int S, int rule, int max_pivots, double *x,
                                  double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab, int32_t *collab,
                                  int32_t *trace, double *snap, cudaStream_t stream) {
-    if (B <= 0) return cudaSuccess;
-    cudaError_t e = configure();
-    if (e != cudaSuccess) return e;
     GlobalArgs a{T, B, n, m, rule, max_pivots, S, (n + S - 1) / S, (m + S - 1) / S,
                  x, obj, status, npiv, rowlab, collab, trace, snap};
-    cudaLaunchAttribute attr[1];
-    const cudaLaunchConfig_t cfg = launch_config(global_bytes(n, m, S), S, B, attr, stream);
-    int clusters = 0;
-    e = cudaOccupancyMaxActiveClusters(&clusters, global_kernel, &cfg);
-    if (e != cudaSuccess) return e;
-    if (clusters <= 0) return cudaErrorInvalidClusterSize;
-    e = cudaLaunchKernelEx(&cfg, global_kernel, a);
-    spx_host::count_launch();
-    if (e != cudaSuccess) return e;
-    return cudaGetLastError();
+    return launch_cluster_kernel<global_kernel>(S, B, global_bytes(n, m, S), stream, a);
 }
 
 int64_t ragged_global_bytes(int n, int m, int S) { return global_bytes(n, m, S); }
@@ -436,10 +374,8 @@ cudaError_t ragged_global_size(const RaggedLaunch &l, const RaggedLp *h_lps, con
     *S_out = l.S;
     *smem_out = l.smem;
     if (!l.pick_S) return cudaSuccess;
-    cudaError_t e = configure_ragged();
-    if (e != cudaSuccess) return e;
-    e = busiest_cluster_size(ragged_global_kernel, l.S, l.count,
-                             [&](int S) { return launch_bytes(l, h_lps, h_order, S); }, S_out);
+    const cudaError_t e = busiest_cluster_size<ragged_global_kernel>(
+        l.S, l.count, [&](int S) { return launch_bytes(l, h_lps, h_order, S); }, S_out);
     if (e != cudaSuccess) return e;
     *smem_out = launch_bytes(l, h_lps, h_order, *S_out);
     return cudaSuccess;
@@ -450,21 +386,8 @@ cudaError_t ragged_global_size(const RaggedLaunch &l, const RaggedLp *h_lps, con
 cudaError_t solve_ragged_global(const RaggedLaunch &l, int S, int64_t smem, const RaggedLp *lps, const int32_t *order,
                                 double *T, int rule, double *x, double *obj, int32_t *status, int32_t *npiv,
                                 int32_t *rowlab, int32_t *collab, int32_t *trace, double *snap, cudaStream_t stream) {
-    if (l.count <= 0) return cudaSuccess;
-    cudaError_t e = configure_ragged();
-    if (e != cudaSuccess) return e;
     GlobalArgs a{T, l.count, 0, 0, rule, 0, S, 0, 0, x, obj, status, npiv, rowlab, collab, trace, snap};
-    cudaLaunchAttribute attr[1];
-    const cudaLaunchConfig_t cfg = launch_config(smem, S, l.count, attr, stream);
-    int clusters = 0;
-    e = cudaOccupancyMaxActiveClusters(&clusters, ragged_global_kernel, &cfg);
-    if (e != cudaSuccess) return e;
-    if (clusters <= 0) return cudaErrorInvalidClusterSize;
-    const int32_t *ord = order + l.first;
-    e = cudaLaunchKernelEx(&cfg, ragged_global_kernel, a, lps, ord);
-    spx_host::count_launch();
-    if (e != cudaSuccess) return e;
-    return cudaGetLastError();
+    return launch_cluster_kernel<ragged_global_kernel>(S, l.count, smem, stream, a, lps, order + l.first);
 }
 
 } // namespace spx_launch

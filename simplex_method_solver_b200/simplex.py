@@ -245,7 +245,7 @@ class SimplexMethod:
             return True
         cells = self.n * (self.m + 1) + self.m
         L = N.load()
-        fits = cells <= L.spx_batched_max_cells() and bool(L.spx_batched_fits(self.n, self.m))
+        fits = bool(L.spx_batched_fits(self.n, self.m))
         if self._engine == "warp" and not fits:
             raise ValueError("engine='warp' needs the LP to fit shared memory")
         return fits and (self._engine == "warp" or cells <= 2048)

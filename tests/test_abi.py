@@ -63,6 +63,11 @@ def test_abi_constants_and_state_layout(native):
     assert L.spx_batched_max_cells() >= 440
     assert L.spx_batched_fits(4, 2) == 1 and L.spx_batched_fits(72, 136) == 1 and L.spx_batched_fits(1, 4470) == 0
     assert L.spx_batched_fits(0, 2) == 0 and L.spx_batched_fits(100, 100) == 0
+    smem, cluster, glob = native.ENGINE_SMEM, native.ENGINE_CLUSTER, native.ENGINE_GLOBAL
+    assert L.spx_batched_route(4, 2, native.ENGINE_AUTO) == smem and L.spx_batched_route(1, 4470, 0) == cluster
+    assert L.spx_batched_route(529, 800, native.ENGINE_AUTO_GLOBAL) == glob and L.spx_batched_route(4, 2, glob) == glob
+    for n, m, engine in ((529, 800, 0), (0, 2, 0), (4, 2, 3), (4, 2, 6)):
+        assert L.spx_batched_route(n, m, engine) == -1 and L.spx_last_error()
     assert L.spx_launch_count(1) >= 0 and L.spx_launch_count(0) == 0
 
 

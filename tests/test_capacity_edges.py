@@ -173,6 +173,70 @@ def test_edge_table_follows_the_footprints(lib):
     assert 8 * (2 * 14177 + 1 + 1) + 4 * (1 + 887) == K8_BYTES == 8 * (2 * 11519 + 1 + 1) + 4 * (1 + 11519)
 
 
+def _route_grid():
+    """The edge shapes, the K8 row limits at m = 2,000 (S = 1 and 16), and every shape one row or column away."""
+    base = set(EDGES) | {(15866, 2000), (263856, 2000)}
+    return sorted({(n + dn, m + dm) for n, m in base for dn in (-1, 0, 1) for dm in (-1, 0, 1) if n + dn and m + dm})
+
+
+def test_route_agrees_with_kernel_for_the_plan_and_the_uniform_entries(lib):
+    """spx_batched_route, kernel_for, the kind the ragged plan gives the LP and the uniform entry of that engine (B = 0,
+    so nothing reaches the device) accept and refuse the same LPs, send them to the same kernel, and (without a forced
+    cluster size) refuse with the same text; a forced size only adds the refusals of LPs that do not fit it."""
+    from simplex_method_solver_b200 import _native as N
+    from simplex_method_solver_b200.batched import ENGINE_CODES, kernel_for, ragged_plan
+    from test_cluster_batched import footprint_fits
+    entries = {"smem": lib.spx_solve_batched, "cluster": lib.spx_solve_batched_cluster,
+               "global": lib.spx_solve_batched_global}
+    kind_of = {N.ENGINE_SMEM: "smem", N.ENGINE_CLUSTER: "cluster", N.ENGINE_GLOBAL: "global"}
+    plan_kind = {"warp": "smem", "cta": "smem", "cluster": "cluster", "global": "global"}
+    routed = set()
+    for forced in (0, 1, 16):
+        with cluster_size(lib, forced):
+            for n, m in _route_grid():
+                for engine, code in ENGINE_CODES.items():
+                    got = lib.spx_batched_route(n, m, code)
+                    why = lib.spx_last_error().decode()
+                    kind = kind_of.get(got)
+                    assert (kind is None) == (got == -1), (n, m, engine, got)
+                    if forced == 0:
+                        routed.add((engine, kind))
+                        try:
+                            assert kernel_for(n, m, engine) == kind, (n, m, engine)
+                        except ValueError as e:
+                            assert kind is None and str(e) == why, (n, m, engine, str(e), why)
+                    # a forced size refuses K7 and K8 LPs that do not fit it, and sets S
+                    fits_forced = (forced == 0 or kind == "smem" or
+                                   (kind == "cluster" and footprint_fits(n, m, forced)) or
+                                   (kind == "global" and 0 < k8_min_size(n, m) <= forced))
+                    accept = kind is not None and fits_forced
+                    try:
+                        plan = ragged_plan([(n, m)], 0, engine)
+                        assert accept, (n, m, engine, forced)
+                        (la,) = plan.launches
+                        assert plan_kind[la["kind"]] == kind, (n, m, engine, forced)
+                        if forced and kind != "smem":
+                            assert la["S"] == forced
+                        elif kind == "cluster":
+                            assert la["S"] == expected_size(n, m)
+                        elif kind == "global":
+                            assert la["S"] == k8_min_size(n, m)
+                    except ValueError as e:
+                        assert not accept, (n, m, engine, forced, str(e))
+                        assert forced or str(e) == f"spx_ragged_plan: LP 0: {why}", (str(e), why)
+                    # the uniform entry of the engine the LP is routed to, or of the engine asked for
+                    entry = entries[kind or engine] if engine in entries or kind else None
+                    if entry is None:
+                        continue
+                    rc = entry(None, 0, n, m, 0, 10, None, None, None, None, None, None, None, None, None)
+                    assert (rc == 0) == accept, (n, m, engine, forced, rc, lib.spx_last_error())
+                    if rc != 0 and forced == 0:
+                        assert lib.spx_last_error().decode() == f"{entry.__name__}: {why}"
+    assert routed == {(e, k) for e in ENGINE_CODES for k in (None, "smem", "cluster", "global")} - {
+        ("auto", "global"), ("smem", "cluster"), ("smem", "global"), ("cluster", "smem"), ("cluster", "global"),
+        ("global", "smem"), ("global", "cluster")}
+
+
 # --------------------------------------------------------------------------- the adversarial LPs
 def band_rows(n):
     """Rows at band edges of every cluster size: k*R - 1 and k*R for the second and the last band (R = ceil(n/S))
