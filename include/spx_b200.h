@@ -388,6 +388,49 @@ int spx_sensitivity_split(const double *d_A, const double *d_b, int32_t n, int32
                           double *d_redcost, double *d_rhs_range, double *d_cost_range, int32_t *h_optimal,
                           void *stream);
 
+/* ---- warm start: change and resume final tables (csrc/spx_warm.cu) ---------------- */
+/* The final table of a batched solve is a dictionary (conventions of the sensitivity report above;
+ * label codes x_k -> k, y_k -> m + k, w1 = m + 1, b_i = T[i*w1 + m], d_j = T[n*w1 + j]).  The change
+ * entries apply new right-hand sides b + db and costs c + dc to final tables IN PLACE, per LP and in
+ * exactly this order (every product and sum rounded on its own, no FMA; the body cells are never
+ * written):
+ *   for each row i in [0, n):      v = b_i;  L = collab[i];  if m <= L < m+n and db[L-m] != 0: v = v + db[L-m];
+ *                                  for j = 0 .. m-1 ascending: H = rowlab[j];
+ *                                      if m <= H < m+n and (d = db[H-m]) != 0: v = v - d*T[i][j];
+ *                                  b_i = v
+ *   for each column j in [0, m):   v = d_j;  H = rowlab[j];  if 0 <= H < m and dc[H] != 0: v = v + dc[H];
+ *                                  for i = 0 .. n-1 ascending: L = collab[i];
+ *                                      if 0 <= L < m and (d = dc[L]) != 0: v = v + d*T[i][j];
+ *                                  d_j = v
+ * A zero delta (-0.0 included) leaves the table bit for bit; a label outside its range is skipped.  The
+ * b update reads only body columns j < m and the f update only body rows, so both run in one launch.
+ * Uniform: d_T [B][cells], d_rowlab [B][m], d_collab [B][n], d_delta_b [B][n], d_delta_c [B][m].  Ragged
+ * (packed as spx_solve_batched_ragged): d_delta_b at the prefix sums of n (as d_collab), d_delta_c at
+ * those of m (as d_x).  Either delta may be NULL; with both NULL, or B = 0, nothing is done and 0 is
+ * returned.  Labels are required.  Arguments (and the plan header) are checked before the device is
+ * touched.  No workspace. */
+int spx_warm_change_batched(double *d_T, int64_t B, int32_t n, int32_t m, const int32_t *d_rowlab,
+                            const int32_t *d_collab, const double *d_delta_b, const double *d_delta_c, void *stream);
+int spx_warm_change_ragged(double *d_T, const void *h_plan, const void *d_plan, const int32_t *d_rowlab,
+                           const int32_t *d_collab, const double *d_delta_b, const double *d_delta_c, void *stream);
+/* Continue every LP for up to max_pivots (ragged: the plan's caps) more pivots from the table in d_T and
+ * the labels in d_rowlab / d_collab, which are required and in/out; the pivot loop is that of the solve
+ * entries, and the trace and snapshots count from 0 in each call.  Uniform: engine as spx_batched_route
+ * (AUTO, SMEM, CLUSTER, GLOBAL, AUTO_GLOBAL) with the routing, cluster-size rules and SPX_OPT_CLUSTER_SIZE
+ * of spx_solve_batched / _cluster / _global; a resume may run on another engine or cluster size than the
+ * solve before it and computes the same bits.  d_function ([B][m], ragged packed as d_x) holds the LPs'
+ * current costs, used only for d_obj = function[0]*x1 + function[1]*x2; required when d_obj != NULL.
+ * Outputs, NULL conventions and errors otherwise as spx_solve_batched / spx_solve_batched_ragged; B = 0
+ * returns 0. */
+int spx_warm_solve_batched(int32_t engine, double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule,
+                           int32_t max_pivots, const double *d_function, double *d_x, double *d_obj,
+                           int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab, int32_t *d_collab,
+                           int32_t *d_trace, double *d_snap, void *stream);
+int spx_warm_solve_ragged(double *d_T, const void *h_plan, const void *d_plan, int32_t rule,
+                          const double *d_function, double *d_x, double *d_obj, int32_t *d_status,
+                          int32_t *d_npiv, int32_t *d_rowlab, int32_t *d_collab, int32_t *d_trace,
+                          double *d_snap, void *stream);
+
 /* ---- column-sharded large tableau (one process per GPU) ------------------- */
 /* Rank g owns global columns [col0, col0+m_loc) of the body as a local split
  * matrix d_A[(n+1)][ld_loc]; b, the labels and the state are replicated.  Per pivot:

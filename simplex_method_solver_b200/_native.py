@@ -103,6 +103,11 @@ SIGNATURES = {
     "spx_sensitivity_ragged": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "spx_sensitivity_split": (ctypes.c_int, [_vp, _vp, _i32, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _pi32,
                                              _vp]),
+    "spx_warm_change_batched": (ctypes.c_int, [_vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "spx_warm_change_ragged": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "spx_warm_solve_batched": (ctypes.c_int, [_i32, _vp, _i64, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp,
+                                              _vp, _vp, _vp, _vp, _vp]),
+    "spx_warm_solve_ragged": (ctypes.c_int, [_vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "spx_shard_msg_doubles": (_i64, [_i32]),
     "spx_shard_candidate": (ctypes.c_int, [_vp, _vp, _i32, _i32, _i64, _i64, _i32, _i32, _vp, _vp, _vp]),
     "spx_shard_select": (ctypes.c_int, [_vp, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _vp, ctypes.c_uint64, _vp]),

@@ -19,6 +19,10 @@ A ragged batch is packed in batch order (LP k's table, x, labels, trace and snap
 start at prefix sums over LPs 0..k-1, see include/spx_b200.h) and solved by one plan of
 at most twelve launches: K4 warp mode, K4 CTA mode, one K7 launch per cluster size, one
 K8 launch per smallest cluster size that holds its LPs.
+
+Warm start: a batch's final tables are dictionaries, so they can be continued (``resume``, e.g. after
+``SPX_CAP``) or re-optimised after new right-hand sides and costs (``change`` then ``resume``; ``resolve``
+does both from a host result).  The change is exact to the bit (include/spx_b200.h, spx_warm_change_*).
 """
 from __future__ import annotations
 
@@ -110,6 +114,48 @@ def kernel_for(n: int, m: int, engine: str = "auto") -> str:
 _ENTRIES = {"smem": "spx_solve_batched", "cluster": "spx_solve_batched_cluster", "global": "spx_solve_batched_global"}
 
 
+_ENGINE_OF_KERNEL = {"smem": N.ENGINE_SMEM, "cluster": N.ENGINE_CLUSTER, "global": N.ENGINE_GLOBAL}
+
+
+def _per_lp(a, B: int, k: int, name: str) -> np.ndarray:
+    """[B, k] or [k] (broadcast over the batch) -> contiguous fp64 [B, k]."""
+    a = np.asarray(a, dtype=np.float64)
+    if a.shape == (k,):
+        a = np.broadcast_to(a, (B, k))
+    if a.shape != (B, k):
+        raise ValueError(f"{name} must be [{B}, {k}] or [{k}], got shape {a.shape}")
+    return np.ascontiguousarray(a)
+
+
+def _first_bad_lp(bad_rows: np.ndarray, what: str) -> None:
+    bad = np.flatnonzero(bad_rows)
+    if bad.size:
+        raise ValueError(f"LP {int(bad[0])}: {what}")
+
+
+def _check_labels(rowlab: np.ndarray, collab: np.ndarray) -> None:
+    """rowlab [B, m], collab [B, n]: each LP's labels must be a permutation of 0..n+m-1."""
+    n, m = collab.shape[1], rowlab.shape[1]
+    lab = np.sort(np.concatenate([rowlab, collab], axis=1), axis=1)
+    _first_bad_lp((lab != np.arange(n + m)).any(axis=1), f"labels are not a permutation of 0..{n + m - 1}")
+
+
+def _check_ragged_labels(rowlab: np.ndarray, collab: np.ndarray, shapes: np.ndarray, xm, xn) -> None:
+    """packed labels: LP k's rowlab at xm[k], collab at xn[k] must be a permutation of 0..n_k+m_k-1"""
+    for k, (n, m) in enumerate(np.asarray(shapes, dtype=np.int64).reshape(-1, 2)):
+        n, m, a, b = int(n), int(m), int(xm[k]), int(xn[k])
+        lab = np.sort(np.concatenate([rowlab[a: a + m], collab[b: b + n]]))
+        if not np.array_equal(lab, np.arange(n + m)):
+            raise ValueError(f"LP {k}: labels are not a permutation of 0..{n + m - 1}")
+
+
+def _empty_batch(n: int, m: int, max_pivots: int, trace: bool, snapshots: bool) -> BatchResult:
+    z, cells = np.zeros, n * (m + 1) + m
+    return BatchResult(z(0, np.int32), z(0, np.int32), z((0, m)), z(0), z((0, cells)), z((0, m), np.int32),
+                       z((0, n), np.int32), z((0, max_pivots, 2), np.int32) if trace else None,
+                       z((0, max_pivots + 1, cells)) if snapshots else None)
+
+
 class DeviceBatch:
     """Device buffers for one batch shape; reusable across solves (bench / serving).
 
@@ -158,6 +204,50 @@ class DeviceBatch:
                    N.ptr(self.trace), N.ptr(self.snaps),
                    torch.cuda.current_stream(self.device).cuda_stream)
 
+    def upload_labels(self, rowlab, collab, non_blocking: bool = False):
+        """Set the labels a ``change`` and a ``resume`` start from: rowlab [B, m] and collab [B, n] int label codes
+        of final tables (e.g. a host ``BatchResult``'s).  Labels that are not a permutation of 0..n+m-1 are a
+        ValueError naming the LP."""
+        rowlab = np.ascontiguousarray(rowlab, dtype=np.int32)
+        collab = np.ascontiguousarray(collab, dtype=np.int32)
+        if rowlab.shape != (self.B, self.m) or collab.shape != (self.B, self.n):
+            raise ValueError(f"rowlab must be [{self.B}, {self.m}] and collab [{self.B}, {self.n}], got "
+                             f"{rowlab.shape} and {collab.shape}")
+        _check_labels(rowlab, collab)
+        self.rowlab[: self.B].copy_(torch.from_numpy(rowlab), non_blocking=non_blocking)
+        self.collab[: self.B].copy_(torch.from_numpy(collab), non_blocking=non_blocking)
+
+    def change(self, rhs_delta=None, cost_delta=None):
+        """Apply new right-hand sides b + rhs_delta and costs c + cost_delta to the resident final tables, in
+        place, with the labels the last ``run``, ``resume`` or ``upload_labels`` left (``spx_warm_change_batched``, exact to the bit).
+        rhs_delta: [B, n] or [n] (broadcast over the batch); cost_delta: [B, m] or [m]; either may be None.
+        A non-finite delta is a ValueError naming the LP.  Asynchronous on the current stream."""
+        B, n, m = self.B, self.n, self.m
+        db = None if rhs_delta is None else _per_lp(rhs_delta, B, n, "rhs_delta")
+        dc = None if cost_delta is None else _per_lp(cost_delta, B, m, "cost_delta")
+        for name, d in (("rhs_delta", db), ("cost_delta", dc)):
+            if d is not None:
+                _first_bad_lp(~np.isfinite(d).all(axis=1), f"{name} is not finite")
+        if B == 0 or (db is None and dc is None):
+            return
+        up = lambda a: None if a is None else torch.from_numpy(a).to(self.device)  # noqa: E731
+        d_db, d_dc = up(db), up(dc)
+        with torch.cuda.device(self.device):
+            N.call("spx_warm_change_batched", self.T.data_ptr(), B, n, m, self.rowlab.data_ptr(),
+                   self.collab.data_ptr(), N.ptr(d_db), N.ptr(d_dc), torch.cuda.current_stream(self.device).cuda_stream)
+
+    def resume(self, function, rule: int = N.RULE_REFERENCE):
+        """Continue every LP from its resident table and labels for up to ``max_pivots`` more pivots, on this
+        batch's engine (``spx_warm_solve_batched``).  function: [B, m] or [m], the LPs' current costs, used only
+        for ``obj``.  Trace and snapshots count from 0 again.  Asynchronous on the current stream."""
+        fn = _per_lp(function, self.B, self.m, "function")
+        self._function = torch.from_numpy(fn).to(self.device) if self.B else None    # alive until the kernel ran
+        with torch.cuda.device(self.device):
+            N.call("spx_warm_solve_batched", _ENGINE_OF_KERNEL[self.kernel], self.T.data_ptr(), self.B, self.n,
+                   self.m, rule, self.max_pivots, N.ptr(self._function), self.x.data_ptr(), self.obj.data_ptr(),
+                   self.status.data_ptr(), self.npiv.data_ptr(), self.rowlab.data_ptr(), self.collab.data_ptr(),
+                   N.ptr(self.trace), N.ptr(self.snaps), torch.cuda.current_stream(self.device).cuda_stream)
+
     def sensitivity(self) -> Sensitivity:
         """Sensitivity report of the final tables the last ``run`` left (K4, K7 and K8 alike); synchronises."""
         return _sens_uniform(self.T, self.status, self.rowlab, self.collab, self.B, self.n, self.m, self.device)
@@ -183,11 +273,7 @@ def solve_batched(tables, n: int, m: int, max_pivots: int = 64, rule: str = "ref
         raise ValueError("tables must be [B, n*(m+1)+m]")
     db = DeviceBatch(tables.shape[0], n, m, max_pivots, trace, snapshots, device, engine)
     if db.B == 0:
-        z = np.zeros
-        return BatchResult(z(0, np.int32), z(0, np.int32), z((0, m)), z(0), z((0, db.cells)),
-                           z((0, m), np.int32), z((0, n), np.int32),
-                           z((0, max_pivots, 2), np.int32) if trace else None,
-                           z((0, max_pivots + 1, db.cells)) if snapshots else None)
+        return _empty_batch(n, m, max_pivots, trace, snapshots)
     db.upload(tables)
     db.run(N.RULES[rule])
     return db.result()
@@ -387,6 +473,56 @@ class DeviceRaggedBatch:
                    self.rowlab.data_ptr(), self.collab.data_ptr(), N.ptr(self.trace), N.ptr(self.snaps),
                    torch.cuda.current_stream(self.device).cuda_stream)
 
+    def _packed(self, a, total: int, k: int, name: str) -> np.ndarray:
+        """a packed [total] fp64 array; a non-finite entry is a ValueError naming its LP (k: the column of
+        ``offsets``, 1 for per-variable arrays, 2 for per-constraint arrays)"""
+        a = np.ascontiguousarray(np.asarray(a, dtype=np.float64).reshape(-1))
+        if a.shape != (total,):
+            raise ValueError(f"{name} must be packed [{total}], got {a.shape[0]} entries")
+        bad = np.flatnonzero(~np.isfinite(a))
+        if bad.size:
+            lp = int(np.searchsorted(self.offsets[:, k], bad[0], side="right")) - 1    # n, m >= 1: no empty slice
+            raise ValueError(f"LP {lp}: {name} is not finite")
+        return a
+
+    def upload_labels(self, rowlab, collab, non_blocking: bool = False):
+        """As ``DeviceBatch.upload_labels``, packed: rowlab [sum m] (as ``x``) and collab [sum n]."""
+        rowlab = np.ascontiguousarray(rowlab, dtype=np.int32).reshape(-1)
+        collab = np.ascontiguousarray(collab, dtype=np.int32).reshape(-1)
+        if rowlab.shape != (self.totals[1],) or collab.shape != (self.totals[2],):
+            raise ValueError(f"rowlab must be packed [{self.totals[1]}] and collab [{self.totals[2]}]")
+        _check_ragged_labels(rowlab, collab, self.shapes2, self.offsets[:, 1], self.offsets[:, 2])
+        self.rowlab[: self.totals[1]].copy_(torch.from_numpy(rowlab), non_blocking=non_blocking)
+        self.collab[: self.totals[2]].copy_(torch.from_numpy(collab), non_blocking=non_blocking)
+
+    def change(self, rhs_delta=None, cost_delta=None):
+        """As ``DeviceBatch.change``, with rhs_delta packed [sum n] (as ``collab``) and cost_delta packed
+        [sum m] (as ``x``) (``spx_warm_change_ragged``)."""
+        tot = self.totals
+        db = None if rhs_delta is None else self._packed(rhs_delta, tot[2], 2, "rhs_delta")
+        dc = None if cost_delta is None else self._packed(cost_delta, tot[1], 1, "cost_delta")
+        if self.B == 0 or (db is None and dc is None):
+            return
+        up = lambda a: None if a is None else torch.from_numpy(a).to(self.device)  # noqa: E731
+        d_db, d_dc = up(db), up(dc)
+        with torch.cuda.device(self.device):
+            N.call("spx_warm_change_ragged", self.T.data_ptr(), self.plan.plan.ctypes.data, self.d_plan.data_ptr(),
+                   self.rowlab.data_ptr(), self.collab.data_ptr(), N.ptr(d_db), N.ptr(d_dc),
+                   torch.cuda.current_stream(self.device).cuda_stream)
+
+    def resume(self, function, rule: int = N.RULE_REFERENCE):
+        """As ``DeviceBatch.resume``, each LP for up to its own cap; function packed [sum m] (as ``x``)
+        (``spx_warm_solve_ragged``)."""
+        fn = np.ascontiguousarray(np.asarray(function, dtype=np.float64).reshape(-1))
+        if fn.shape != (self.totals[1],):
+            raise ValueError(f"function must be packed [{self.totals[1]}], got {fn.shape[0]} entries")
+        self._function = torch.from_numpy(fn).to(self.device) if self.B else None    # alive until the kernels ran
+        with torch.cuda.device(self.device):
+            N.call("spx_warm_solve_ragged", self.T.data_ptr(), self.plan.plan.ctypes.data, self.d_plan.data_ptr(),
+                   rule, N.ptr(self._function), self.x.data_ptr(), self.obj.data_ptr(), self.status.data_ptr(),
+                   self.npiv.data_ptr(), self.rowlab.data_ptr(), self.collab.data_ptr(), N.ptr(self.trace),
+                   N.ptr(self.snaps), torch.cuda.current_stream(self.device).cuda_stream)
+
     def sensitivity(self) -> RaggedSensitivity:
         """Sensitivity report of the final tables the last ``run`` left; synchronises."""
         return _sens_ragged(self.T, self.plan.plan, self.d_plan, self.status, self.rowlab, self.collab, self.B,
@@ -472,3 +608,114 @@ def sensitivity(result: Union[BatchResult, RaggedResult], device=None) -> Union[
     N.lib()
     return _sens_uniform(up(result.tables, np.float64), up(result.status, np.int32), up(rowlab, np.int32),
                          up(collab, np.int32), B, n, m, dev)
+
+
+def _new_values(new, old: np.ndarray, name: str):
+    """(new values, delta = new - old) of [B, k] `old`; new None: unchanged, no delta."""
+    if new is None:
+        return old, None
+    new = _per_lp(new, old.shape[0], old.shape[1], name)
+    return new, new - old
+
+
+def _packed_values(new, sizes: np.ndarray, name: str) -> Optional[np.ndarray]:
+    """a packed array, or one array per LP -> packed fp64; None stays None"""
+    if new is None:
+        return None
+    if isinstance(new, (list, tuple)) and len(new) == len(sizes) and len(new) and np.ndim(new[0]) == 1:
+        for k, (v, s) in enumerate(zip(new, sizes)):
+            if np.shape(v) != (int(s),):
+                raise ValueError(f"LP {k}: {name} must have {int(s)} entries, got shape {np.shape(v)}")
+        new = np.concatenate([np.asarray(v, dtype=np.float64) for v in new])
+    new = np.asarray(new, dtype=np.float64).reshape(-1)
+    if new.shape != (int(sizes.sum()),):
+        raise ValueError(f"{name} must be packed [{int(sizes.sum())}] or one array per LP")
+    return new
+
+
+def resolve(result: Union[BatchResult, RaggedResult], data, rhs=None, cost=None, max_pivots=64,
+            rule: str = "reference", trace: bool = True, snapshots: bool = False, device=None,
+            engine: str = "auto") -> Union[BatchResult, RaggedResult]:
+    """Re-optimise solved LPs after new right-hand sides and/or costs, from their final tables.
+
+    result: a host ``BatchResult`` (``solve_batched``) with data = the [B, cells] tables it was solved from,
+    or a ``RaggedResult`` (``solve_ragged``) with data = its ``(constraints, function)`` pairs.  data must hold
+    the b and c the final tables currently belong to: to chain, pass the result of an earlier ``resolve`` with
+    the tables (or pairs) carrying that call's new b and c, not the original ones, or the deltas are wrong.
+    rhs / cost: the new b ([B, n] or [n]) and c ([B, m] or [m]); for a ragged result packed ([sum n],
+    [sum m]) or one array per LP.  None keeps the old values; with neither, the LPs simply continue.
+    The final tables and labels are uploaded, changed by delta = new - old (``change``) and resumed for up
+    to max_pivots more pivots with function = the new costs (``resume``).  Returns the result type given.
+    Non-finite deltas, labels that are not a permutation of 0..n+m-1 and shapes that do not match are
+    ValueErrors naming the LP.
+    """
+    if isinstance(result, RaggedResult):
+        return _resolve_ragged(result, data, rhs, cost, max_pivots, rule, trace, snapshots, device, engine)
+    if not isinstance(result, BatchResult):
+        raise TypeError(f"resolve() takes a BatchResult or a RaggedResult, not {type(result).__name__}")
+    rowlab = np.ascontiguousarray(result.rowlab, dtype=np.int32)
+    collab = np.ascontiguousarray(result.collab, dtype=np.int32)
+    if rowlab.ndim != 2 or collab.ndim != 2 or rowlab.shape[0] != collab.shape[0]:
+        raise ValueError("result.rowlab must be [B, m] and result.collab [B, n]")
+    B, m, n = rowlab.shape[0], rowlab.shape[1], collab.shape[1]
+    if n < 1 or m < 1:
+        raise ValueError(f"bad shape {n} x {m}")
+    cells = n * (m + 1) + m
+    tables = np.ascontiguousarray(result.tables, dtype=np.float64)
+    data = np.asarray(data, dtype=np.float64)
+    if tables.shape != (B, cells) or data.shape != (B, cells):
+        raise ValueError(f"result.tables and data must be [B, n*(m+1)+m] = [{B}, {cells}], got "
+                         f"{tables.shape} and {data.shape}")
+    _check_labels(rowlab, collab)
+    new_c, dc = _new_values(cost, data[:, n * (m + 1):], "cost")
+    _, db = _new_values(rhs, data[:, : n * (m + 1)].reshape(B, n, m + 1)[:, :, m], "rhs")
+    for name, d in (("rhs - old rhs", db), ("cost - old cost", dc)):
+        if d is not None:
+            _first_bad_lp(~np.isfinite(d).all(axis=1), f"{name} is not finite")
+    db_ = DeviceBatch(B, n, m, int(max_pivots), trace, snapshots, device, engine)
+    if B == 0:
+        return _empty_batch(n, m, int(max_pivots), trace, snapshots)
+    db_.upload(tables)
+    db_.upload_labels(rowlab, collab)
+    db_.change(db, dc)
+    db_.resume(new_c, N.RULES[rule])
+    return db_.result()
+
+
+def _resolve_ragged(result: RaggedResult, data, rhs, cost, max_pivots, rule, trace, snapshots, device,
+                    engine) -> RaggedResult:
+    shapes, packed = pack_ragged(data)
+    rshapes = np.asarray(result.shapes, dtype=np.int64).reshape(-1, 3)
+    if not np.array_equal(shapes, rshapes[:, :2]):
+        raise ValueError("data are not the LPs of result (their shapes differ from result.shapes)")
+    B = shapes.shape[0]
+    plan = ragged_plan(shapes, _caps(max_pivots, B), engine)
+    offsets = np.stack([plan.lps["t"], plan.lps["xm"], plan.lps["xn"]], axis=1).astype(np.int64)
+    tot = [int(v) for v in plan.totals]
+    for name, a, k in (("tables", result.tables, tot[0]), ("rowlab", result.rowlab, tot[1]),
+                       ("collab", result.collab, tot[2])):
+        if np.size(a) != k:
+            raise ValueError(f"result.{name} has {np.size(a)} entries, the shapes need {k}")
+    rowlab = np.ascontiguousarray(result.rowlab, dtype=np.int32).reshape(-1)
+    collab = np.ascontiguousarray(result.collab, dtype=np.int32).reshape(-1)
+    old_b, old_c = np.empty(tot[2]), np.empty(tot[1])
+    _check_ragged_labels(rowlab, collab, shapes, offsets[:, 1], offsets[:, 2])
+    for k in range(B):
+        n, m = (int(v) for v in shapes[k])
+        t, xm, xn = (int(v) for v in offsets[k])
+        old_b[xn: xn + n] = packed[t: t + n * (m + 1)].reshape(n, m + 1)[:, m]
+        old_c[xm: xm + m] = packed[t + n * (m + 1): t + n * (m + 1) + m]
+    new_b = _packed_values(rhs, shapes[:, 0], "rhs")
+    new_c = _packed_values(cost, shapes[:, 1], "cost")
+    deltas = [None if v is None else v - old for v, old in ((new_b, old_b), (new_c, old_c))]
+    for name, d, col in (("rhs - old rhs", deltas[0], 2), ("cost - old cost", deltas[1], 1)):
+        bad = np.flatnonzero(~np.isfinite(d)) if d is not None else []
+        if len(bad):
+            raise ValueError(f"LP {int(np.searchsorted(offsets[:, col], bad[0], side='right')) - 1}: {name} is not finite")
+    db_ = DeviceRaggedBatch(shapes, max_pivots, trace, snapshots, device, engine)
+    if B:
+        db_.upload(np.ascontiguousarray(result.tables, dtype=np.float64).reshape(-1))
+        db_.upload_labels(rowlab, collab)
+        db_.change(*deltas)
+        db_.resume(old_c if new_c is None else new_c, N.RULES[rule])
+    return db_.result()

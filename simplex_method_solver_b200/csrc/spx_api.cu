@@ -49,31 +49,33 @@ cudaError_t lazy_guard_selftest(const double *, const double *, const double *, 
                                 double *, double *, unsigned long long *, cudaStream_t);
 cudaError_t init_state(spx_state *, int32_t *, int32_t *, int, int, int64_t, cudaStream_t);
 cudaError_t solve_batched(double *, int64_t, int, int, int, int, double *, double *, int32_t *,
-                          int32_t *, int32_t *, int32_t *, int32_t *, double *, cudaStream_t);
+                          int32_t *, int32_t *, int32_t *, int32_t *, double *, bool, const double *, cudaStream_t);
 bool cluster_fits(int64_t, int64_t, int);
 int cluster_size(int64_t, int64_t);
 cudaError_t solve_batched_cluster(double *, int64_t, int, int, int, int, int, double *, double *, int32_t *,
-                                  int32_t *, int32_t *, int32_t *, int32_t *, double *, cudaStream_t);
+                                  int32_t *, int32_t *, int32_t *, int32_t *, double *, bool, const double *,
+                                  cudaStream_t);
 bool global_fits(int64_t, int64_t, int);
 int global_min_cluster_size(int64_t, int64_t);
 cudaError_t global_cluster_size(int64_t, int64_t, int64_t, int *);
 cudaError_t solve_batched_global(double *, int64_t, int, int, int, int, int, double *, double *, int32_t *,
-                                 int32_t *, int32_t *, int32_t *, int32_t *, double *, cudaStream_t);
+                                 int32_t *, int32_t *, int32_t *, int32_t *, double *, bool, const double *,
+                                 cudaStream_t);
 int64_t ragged_batched_bytes(int, int, int *);
 int ragged_cta_threads(int64_t);
 int ragged_warps_per_cta(int64_t, int64_t);
 int64_t ragged_cluster_bytes(int, int, int);
 cudaError_t solve_ragged_batched(const spx::RaggedLaunch &, const spx::RaggedLp *, const int32_t *, double *, int,
                                  double *, double *, int32_t *, int32_t *, int32_t *, int32_t *, int32_t *, double *,
-                                 cudaStream_t);
+                                 bool, const double *, cudaStream_t);
 cudaError_t solve_ragged_cluster(const spx::RaggedLaunch &, const spx::RaggedLp *, const int32_t *, double *, int,
                                  double *, double *, int32_t *, int32_t *, int32_t *, int32_t *, int32_t *, double *,
-                                 cudaStream_t);
+                                 bool, const double *, cudaStream_t);
 int64_t ragged_global_bytes(int, int, int);
 cudaError_t ragged_global_size(const spx::RaggedLaunch &, const spx::RaggedLp *, const int32_t *, int *, int64_t *);
 cudaError_t solve_ragged_global(const spx::RaggedLaunch &, int, int64_t, const spx::RaggedLp *, const int32_t *,
                                 double *, int, double *, double *, int32_t *, int32_t *, int32_t *, int32_t *,
-                                int32_t *, double *, cudaStream_t);
+                                int32_t *, double *, bool, const double *, cudaStream_t);
 cudaError_t sensitivity_uniform(const double *, int64_t, int, int, const int32_t *, const int32_t *, const int32_t *,
                                 double *, double *, double *, double *, double *, cudaStream_t);
 cudaError_t sensitivity_ragged(const spx::RaggedPlan *, const spx::RaggedLp *, const int32_t *, const double *,
@@ -81,6 +83,11 @@ cudaError_t sensitivity_ragged(const spx::RaggedPlan *, const spx::RaggedLp *, c
                                const int32_t *, double *, double *, double *, double *, double *, cudaStream_t);
 cudaError_t sensitivity_split(const double *, const double *, int, int, int64_t, int, const int32_t *, const int32_t *,
                               double *, double *, double *, double *, double *, cudaStream_t);
+cudaError_t warm_change_uniform(double *, int64_t, int, int, const int32_t *, const int32_t *, const double *,
+                                const double *, cudaStream_t);
+cudaError_t warm_change_ragged(const spx::RaggedPlan *, const spx::RaggedLp *, const int32_t *, double *,
+                               const spx::RaggedLp *, const int32_t *, const int32_t *, const int32_t *, const double *,
+                               const double *, cudaStream_t);
 } // namespace spx_launch
 
 namespace spx_host {
@@ -230,6 +237,47 @@ int check_cluster_launch(cudaError_t e, const char *who, int S, int64_t smem) {
     set_error("%s: the device cannot co-schedule one cluster of S = %d CTAs with %lld bytes of shared memory each "
               "(cudaOccupancyMaxActiveClusters = 0)", who, S, (long long)smem);
     return -1;
+}
+
+// One uniform solve (warm == false) or resume (warm == true) on the engine route_lp gives `engine`: the body of
+// spx_solve_batched, spx_solve_batched_cluster, spx_solve_batched_global and spx_warm_solve_batched.  K4 reads no
+// forced cluster size; K7 and K8 check the grid limit, and K8 launches at spx_global_cluster_size.
+int solve_uniform(const char *who, int engine, bool warm, double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule,
+                  int32_t max_pivots, const double *d_function, double *d_x, double *d_obj, int32_t *d_status,
+                  int32_t *d_npiv, int32_t *d_rowlab, int32_t *d_collab, int32_t *d_trace, double *d_snap,
+                  void *stream) {
+    SPX_REQUIRE(known_engine(engine), "%s: unknown engine %d", who, engine);
+    SPX_REQUIRE(B >= 0 && n >= 1 && m >= 1 && max_pivots >= 0, "%s: bad arguments", who);
+    SPX_REQUIRE(B == 0 || (d_T && d_status && d_npiv), "%s: null T/status/npiv", who);
+    SPX_REQUIRE(!warm || B == 0 || (d_rowlab && d_collab), "%s: null rowlab/collab (the labels to resume from)", who);
+    SPX_REQUIRE(!warm || B == 0 || !d_obj || d_function, "%s: null function with obj", who);
+    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "%s: unknown rule %d", who, rule);
+    Route r;
+    if (!route_lp(n, m, engine, forced_cluster_size(), &r)) {
+        prefix_error("%s: ", who);
+        return -2;
+    }
+    cudaStream_t s = as_stream(stream);
+    if (r.kernel == spx::RAGGED_WARP || r.kernel == spx::RAGGED_CTA)
+        return check(spx_launch::solve_batched(d_T, B, n, m, rule, max_pivots, d_x, d_obj, d_status, d_npiv, d_rowlab,
+                                               d_collab, d_trace, d_snap, warm, d_function, s),
+                     "batched launch");
+    // K8: a default S above S_min is only chosen when all B clusters are co-resident, far below the grid limit
+    SPX_REQUIRE(B <= INT32_MAX / r.S, "%s: B = %lld LPs x S = %d CTAs exceed one grid", who, (long long)B, r.S);
+    if (r.kernel == spx::RAGGED_CLUSTER)
+        return check_cluster_launch(spx_launch::solve_batched_cluster(d_T, B, n, m, r.S, rule, max_pivots, d_x, d_obj,
+                                                                      d_status, d_npiv, d_rowlab, d_collab, d_trace,
+                                                                      d_snap, warm, d_function, s),
+                                    who, r.S, r.bytes);
+    if (B == 0) return 0;
+    int S = 0;
+    char what[96];
+    snprintf(what, sizeof(what), "%s: occupancy", who);
+    if (check(spx_launch::global_cluster_size(n, m, B, &S), what)) return -1;
+    return check_cluster_launch(spx_launch::solve_batched_global(d_T, B, n, m, S, rule, max_pivots, d_x, d_obj,
+                                                                 d_status, d_npiv, d_rowlab, d_collab, d_trace,
+                                                                 d_snap, warm, d_function, s),
+                                who, S, spx_launch::ragged_global_bytes(n, m, S));
 }
 
 } // namespace
@@ -684,17 +732,8 @@ int32_t spx_batched_fits(int32_t n, int32_t m) { return spx_launch::batched_fits
 int spx_solve_batched(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule, int32_t max_pivots,
                       double *d_x, double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab,
                       int32_t *d_collab, int32_t *d_trace, double *d_snap, void *stream) {
-    SPX_REQUIRE(B >= 0 && n >= 1 && m >= 1 && max_pivots >= 0, "spx_solve_batched: bad arguments");
-    SPX_REQUIRE(B == 0 || (d_T && d_status && d_npiv), "spx_solve_batched: null T/status/npiv");
-    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_solve_batched: unknown rule %d", rule);
-    Route r;
-    if (!route_lp(n, m, SPX_ENGINE_SMEM, 0, &r)) {
-        prefix_error("spx_solve_batched: ");
-        return -2;
-    }
-    cudaError_t e = spx_launch::solve_batched(d_T, B, n, m, rule, max_pivots, d_x, d_obj, d_status, d_npiv,
-                                              d_rowlab, d_collab, d_trace, d_snap, as_stream(stream));
-    return check(e, "batched launch");
+    return solve_uniform("spx_solve_batched", SPX_ENGINE_SMEM, false, d_T, B, n, m, rule, max_pivots, nullptr, d_x,
+                         d_obj, d_status, d_npiv, d_rowlab, d_collab, d_trace, d_snap, stream);
 }
 
 // ---- K7 -------------------------------------------------------------------------
@@ -703,21 +742,8 @@ int32_t spx_cluster_size(int32_t n, int32_t m) { return spx_launch::cluster_size
 int spx_solve_batched_cluster(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule, int32_t max_pivots,
                               double *d_x, double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab,
                               int32_t *d_collab, int32_t *d_trace, double *d_snap, void *stream) {
-    SPX_REQUIRE(B >= 0 && n >= 1 && m >= 1 && max_pivots >= 0, "spx_solve_batched_cluster: bad arguments");
-    SPX_REQUIRE(B == 0 || (d_T && d_status && d_npiv), "spx_solve_batched_cluster: null T/status/npiv");
-    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_solve_batched_cluster: unknown rule %d",
-                rule);
-    Route r;
-    if (!route_lp(n, m, SPX_ENGINE_CLUSTER, forced_cluster_size(), &r)) {
-        prefix_error("spx_solve_batched_cluster: ");
-        return -2;
-    }
-    SPX_REQUIRE(B <= INT32_MAX / r.S, "spx_solve_batched_cluster: B = %lld LPs x S = %d CTAs exceed one grid",
-                (long long)B, r.S);
-    return check_cluster_launch(spx_launch::solve_batched_cluster(d_T, B, n, m, r.S, rule, max_pivots, d_x, d_obj,
-                                                                  d_status, d_npiv, d_rowlab, d_collab, d_trace,
-                                                                  d_snap, as_stream(stream)),
-                                "spx_solve_batched_cluster", r.S, r.bytes);
+    return solve_uniform("spx_solve_batched_cluster", SPX_ENGINE_CLUSTER, false, d_T, B, n, m, rule, max_pivots,
+                         nullptr, d_x, d_obj, d_status, d_npiv, d_rowlab, d_collab, d_trace, d_snap, stream);
 }
 
 // ---- K8 -------------------------------------------------------------------------
@@ -732,25 +758,8 @@ int32_t spx_global_cluster_size(int32_t n, int32_t m, int64_t B) {
 int spx_solve_batched_global(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule, int32_t max_pivots,
                              double *d_x, double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab,
                              int32_t *d_collab, int32_t *d_trace, double *d_snap, void *stream) {
-    SPX_REQUIRE(B >= 0 && n >= 1 && m >= 1 && max_pivots >= 0, "spx_solve_batched_global: bad arguments");
-    SPX_REQUIRE(B == 0 || (d_T && d_status && d_npiv), "spx_solve_batched_global: null T/status/npiv");
-    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_solve_batched_global: unknown rule %d",
-                rule);
-    Route r;
-    if (!route_lp(n, m, SPX_ENGINE_GLOBAL, forced_cluster_size(), &r)) {
-        prefix_error("spx_solve_batched_global: ");
-        return -2;
-    }
-    // a default S above S_min is only chosen when all B clusters are co-resident, far below the grid limit
-    SPX_REQUIRE(B <= INT32_MAX / r.S, "spx_solve_batched_global: B = %lld LPs x S = %d CTAs exceed one grid",
-                (long long)B, r.S);
-    if (B == 0) return 0;
-    int S = 0;
-    if (check(spx_launch::global_cluster_size(n, m, B, &S), "spx_solve_batched_global: occupancy")) return -1;
-    return check_cluster_launch(spx_launch::solve_batched_global(d_T, B, n, m, S, rule, max_pivots, d_x, d_obj,
-                                                                 d_status, d_npiv, d_rowlab, d_collab, d_trace,
-                                                                 d_snap, as_stream(stream)),
-                                "spx_solve_batched_global", S, spx_launch::ragged_global_bytes(n, m, S));
+    return solve_uniform("spx_solve_batched_global", SPX_ENGINE_GLOBAL, false, d_T, B, n, m, rule, max_pivots,
+                         nullptr, d_x, d_obj, d_status, d_npiv, d_rowlab, d_collab, d_trace, d_snap, stream);
 }
 
 // ---- ragged batches (K4 + K7 + K8) ---------------------------------------------------
@@ -864,49 +873,79 @@ static bool ragged_header_sane(const spx::RaggedPlan *P) {
     return sane && counted == P->B;
 }
 
-int spx_solve_batched_ragged(double *d_T, const void *h_plan, const void *d_plan, int32_t rule, double *d_x,
-                             double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab, int32_t *d_collab,
-                             int32_t *d_trace, double *d_snap, void *stream) {
+// The plan header of `who`'s h_plan, checked: magic, ABI version and launch list
+static const spx::RaggedPlan *checked_plan(const char *who, const void *h_plan) {
     using namespace spx;
-    SPX_REQUIRE(h_plan, "spx_solve_batched_ragged: null plan");
+    if (!h_plan) {
+        set_error("%s: null plan", who);
+        return nullptr;
+    }
     const RaggedPlan *P = static_cast<const RaggedPlan *>(h_plan);
-    SPX_REQUIRE(P->magic == RAGGED_MAGIC && P->abi == SPX_ABI_VERSION,
-                "spx_solve_batched_ragged: h_plan is not a plan of this library (magic / ABI version mismatch)");
-    SPX_REQUIRE(ragged_header_sane(P), "spx_solve_batched_ragged: inconsistent plan header (B = %lld)", (long long)P->B);
+    if (P->magic != RAGGED_MAGIC || P->abi != SPX_ABI_VERSION) {
+        set_error("%s: h_plan is not a plan of this library (magic / ABI version mismatch)", who);
+        return nullptr;
+    }
+    if (!ragged_header_sane(P)) {
+        set_error("%s: inconsistent plan header (B = %lld)", who, (long long)P->B);
+        return nullptr;
+    }
+    return P;
+}
+
+// One ragged solve (warm == false) or resume (warm == true): the body of spx_solve_batched_ragged and
+// spx_warm_solve_ragged
+static int solve_ragged(const char *who, bool warm, double *d_T, const void *h_plan, const void *d_plan, int32_t rule,
+                        const double *d_function, double *d_x, double *d_obj, int32_t *d_status, int32_t *d_npiv,
+                        int32_t *d_rowlab, int32_t *d_collab, int32_t *d_trace, double *d_snap, void *stream) {
+    using namespace spx;
+    const RaggedPlan *P = checked_plan(who, h_plan);
+    if (!P) return -2;
     if (P->B == 0) return 0;
-    SPX_REQUIRE(d_plan && d_T && d_status && d_npiv, "spx_solve_batched_ragged: null d_plan/T/status/npiv");
-    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_solve_batched_ragged: unknown rule %d", rule);
+    SPX_REQUIRE(d_plan && d_T && d_status && d_npiv, "%s: null d_plan/T/status/npiv", who);
+    SPX_REQUIRE(!warm || (d_rowlab && d_collab), "%s: null rowlab/collab (the labels to resume from)", who);
+    SPX_REQUIRE(!warm || !d_obj || d_function, "%s: null function with obj", who);
+    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "%s: unknown rule %d", who, rule);
     const RaggedLp *lps = reinterpret_cast<const RaggedLp *>(static_cast<const char *>(d_plan) + P->lp_offset);
     const int32_t *order = reinterpret_cast<const int32_t *>(static_cast<const char *>(d_plan) + P->order_offset);
     const RaggedLp *h_lps = reinterpret_cast<const RaggedLp *>(static_cast<const char *>(h_plan) + P->lp_offset);
     const int32_t *h_order = reinterpret_cast<const int32_t *>(static_cast<const char *>(h_plan) + P->order_offset);
     cudaStream_t s = as_stream(stream);
+    char what[96];
     for (int i = 0; i < P->nlaunch; ++i) {
         const RaggedLaunch &l = P->launch[i];
         if (l.kernel == RAGGED_GLOBAL) {
             int S = 0;
             int64_t smem = 0;
-            if (check(spx_launch::ragged_global_size(l, h_lps, h_order, &S, &smem), "spx_solve_batched_ragged: occupancy"))
+            snprintf(what, sizeof(what), "%s: occupancy", who);
+            if (check(spx_launch::ragged_global_size(l, h_lps, h_order, &S, &smem), what))
                 return -1;
-            SPX_REQUIRE(l.count <= INT32_MAX / S, "spx_solve_batched_ragged: %lld LPs x S = %d CTAs exceed one grid",
+            SPX_REQUIRE(l.count <= INT32_MAX / S, "%s: %lld LPs x S = %d CTAs exceed one grid", who,
                         (long long)l.count, S);
             if (check_cluster_launch(spx_launch::solve_ragged_global(l, S, smem, lps, order, d_T, rule, d_x, d_obj,
                                                                      d_status, d_npiv, d_rowlab, d_collab, d_trace,
-                                                                     d_snap, s),
-                                     "spx_solve_batched_ragged", S, smem))
+                                                                     d_snap, warm, d_function, s),
+                                     who, S, smem))
                 return -1;
         } else if (l.kernel == RAGGED_CLUSTER) {
             if (check_cluster_launch(spx_launch::solve_ragged_cluster(l, lps, order, d_T, rule, d_x, d_obj, d_status,
-                                                                      d_npiv, d_rowlab, d_collab, d_trace, d_snap, s),
-                                     "spx_solve_batched_ragged", l.S, l.smem))
+                                                                      d_npiv, d_rowlab, d_collab, d_trace, d_snap,
+                                                                      warm, d_function, s),
+                                     who, l.S, l.smem))
                 return -1;
         } else if (check(spx_launch::solve_ragged_batched(l, lps, order, d_T, rule, d_x, d_obj, d_status, d_npiv,
-                                                            d_rowlab, d_collab, d_trace, d_snap, s),
+                                                            d_rowlab, d_collab, d_trace, d_snap, warm, d_function, s),
                          "ragged batched launch")) {
             return -1;
         }
     }
     return 0;
+}
+
+int spx_solve_batched_ragged(double *d_T, const void *h_plan, const void *d_plan, int32_t rule, double *d_x,
+                             double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab, int32_t *d_collab,
+                             int32_t *d_trace, double *d_snap, void *stream) {
+    return solve_ragged("spx_solve_batched_ragged", false, d_T, h_plan, d_plan, rule, nullptr, d_x, d_obj, d_status,
+                        d_npiv, d_rowlab, d_collab, d_trace, d_snap, stream);
 }
 
 int32_t spx_ragged_cluster_size(const void *h_plan, int32_t launch) {
@@ -987,6 +1026,50 @@ int spx_sensitivity_split(const double *d_A, const double *d_b, int32_t n, int32
     return check(spx_launch::sensitivity_split(d_A, d_b, n, m, ld, optimal, d_rowlab, d_collab, d_dual, d_slack,
                                                d_redcost, d_rhs_range, d_cost_range, s),
                  "split sensitivity launch");
+}
+
+// ---- warm start: change and resume final tables (csrc/spx_warm.cu) ------------------
+int spx_warm_change_batched(double *d_T, int64_t B, int32_t n, int32_t m, const int32_t *d_rowlab,
+                            const int32_t *d_collab, const double *d_delta_b, const double *d_delta_c, void *stream) {
+    SPX_REQUIRE(B >= 0 && n >= 1 && m >= 1, "spx_warm_change_batched: bad arguments (B = %lld, n = %d, m = %d)",
+                (long long)B, n, m);
+    if (B == 0 || (!d_delta_b && !d_delta_c)) return 0;
+    SPX_REQUIRE(d_T && d_rowlab && d_collab, "spx_warm_change_batched: null T/rowlab/collab");
+    return check(spx_launch::warm_change_uniform(d_T, B, n, m, d_rowlab, d_collab, d_delta_b, d_delta_c,
+                                                 as_stream(stream)),
+                 "warm change launch");
+}
+
+int spx_warm_change_ragged(double *d_T, const void *h_plan, const void *d_plan, const int32_t *d_rowlab,
+                           const int32_t *d_collab, const double *d_delta_b, const double *d_delta_c, void *stream) {
+    using namespace spx;
+    const RaggedPlan *P = checked_plan("spx_warm_change_ragged", h_plan);
+    if (!P) return -2;
+    if (P->B == 0 || (!d_delta_b && !d_delta_c)) return 0;
+    SPX_REQUIRE(d_plan && d_T && d_rowlab && d_collab, "spx_warm_change_ragged: null d_plan/T/rowlab/collab");
+    const char *h = static_cast<const char *>(h_plan), *d = static_cast<const char *>(d_plan);
+    return check(spx_launch::warm_change_ragged(P, reinterpret_cast<const RaggedLp *>(h + P->lp_offset),
+                                                reinterpret_cast<const int32_t *>(h + P->order_offset), d_T,
+                                                reinterpret_cast<const RaggedLp *>(d + P->lp_offset),
+                                                reinterpret_cast<const int32_t *>(d + P->order_offset), d_rowlab,
+                                                d_collab, d_delta_b, d_delta_c, as_stream(stream)),
+                 "ragged warm change launch");
+}
+
+int spx_warm_solve_batched(int32_t engine, double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule,
+                           int32_t max_pivots, const double *d_function, double *d_x, double *d_obj,
+                           int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab, int32_t *d_collab,
+                           int32_t *d_trace, double *d_snap, void *stream) {
+    return solve_uniform("spx_warm_solve_batched", engine, true, d_T, B, n, m, rule, max_pivots, d_function, d_x,
+                         d_obj, d_status, d_npiv, d_rowlab, d_collab, d_trace, d_snap, stream);
+}
+
+int spx_warm_solve_ragged(double *d_T, const void *h_plan, const void *d_plan, int32_t rule,
+                          const double *d_function, double *d_x, double *d_obj, int32_t *d_status,
+                          int32_t *d_npiv, int32_t *d_rowlab, int32_t *d_collab, int32_t *d_trace,
+                          double *d_snap, void *stream) {
+    return solve_ragged("spx_warm_solve_ragged", true, d_T, h_plan, d_plan, rule, d_function, d_x, d_obj, d_status,
+                        d_npiv, d_rowlab, d_collab, d_trace, d_snap, stream);
 }
 
 // ---- column-sharded flow ----------------------------------------------------------

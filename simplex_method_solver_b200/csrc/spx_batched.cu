@@ -123,9 +123,21 @@ __device__ __forceinline__ int warp_pick(const double *cur, int n, int m, int ru
 // CTA == true : one CTA per LP for tables of hundreds of cells (Klee-Minty n=20: 440 cells, 2^20-1
 //               strictly sequential pivots): warp 0 prices the pivot, every warp updates its share
 //               of the cells, two block barriers per pivot.
-template <bool CTA>
-__global__ void __launch_bounds__(CTA ? 512 : 256, CTA ? 1 : 6)
-batched_kernel(BatchedArgs a, int warps_per_cta, int warp_doubles) {
+// is `lab` the label of a variable x_(lab+1)?  A resume also rejects negative labels (it never indexes with one)
+template <bool WARM>
+__device__ __forceinline__ bool x_label(int lab, int m) {
+    if constexpr (WARM) return lab >= 0 && lab < m;
+    else return lab < m;
+}
+
+// CTA == false / true as above.
+// WARM == false: a solve from the loaded table, labels 'x1'..'xm' / 'y1'..'yn', f0 and f1 from its f row.
+// WARM == true:  a resume (spx_warm_solve_batched): labels read from a.rowlab / a.collab, f0 and f1 for obj from
+//                `function` [B][m], and no label outside [0, m) indexes xs.
+
+template <bool CTA, bool WARM>
+__device__ __forceinline__ void batched_solve(const BatchedArgs &a, const double *function, int warps_per_cta,
+                                              int warp_doubles) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ int s_ctl[4];                               // CTA mode: {status, r, c} of warp 0's pick
     const int n = a.n, m = a.m, w1 = m + 1;
@@ -144,6 +156,10 @@ batched_kernel(BatchedArgs a, int warps_per_cta, int warp_doubles) {
 
     const int64_t lp = CTA ? (int64_t)blockIdx.x : (int64_t)blockIdx.x * warps_per_cta + warp;
     if (!CTA && (warp >= warps_per_cta || lp >= a.B)) return;
+    // a resume: the current costs for obj, read before anything else (read later, around the label loads or in the
+    // epilogue, they cost warp mode, at the register cap of its launch bounds, more spills than the solve has)
+    const double c0 = (WARM && function && m >= 2) ? function[lp * m] : 0.0;
+    const double c1 = (WARM && function && m >= 2) ? function[lp * m + 1] : 0.0;
     const int tl = CTA ? (int)threadIdx.x : lane;          // thread index within the LP's group
     const int nl = CTA ? (int)blockDim.x : 32;             // threads of the group
     auto group_sync = [&]() { if (CTA) __syncthreads(); else __syncwarp(); };
@@ -158,8 +174,13 @@ batched_kernel(BatchedArgs a, int warps_per_cta, int warp_doubles) {
 
     double *Tg = a.T + lp * (int64_t)cells;
     for (int k = tl; k < cells; k += nl) cur[k] = Tg[k];
-    for (int j = tl; j < m; j += nl) rl[j] = j;           // 'x1'..'xm'  :30
-    for (int i = tl; i < n; i += nl) cl[i] = m + i;       // 'y1'..'yn'  :31
+    if constexpr (WARM) {
+        for (int j = tl; j < m; j += nl) rl[j] = a.rowlab[lp * m + j];
+        for (int i = tl; i < n; i += nl) cl[i] = a.collab[lp * n + i];
+    } else {
+        for (int j = tl; j < m; j += nl) rl[j] = j;       // 'x1'..'xm'  :30
+        for (int i = tl; i < n; i += nl) cl[i] = m + i;   // 'y1'..'yn'  :31
+    }
     group_sync();
     const int fo = n * w1;                                // offset of the f row
     const double f0 = (m >= 1) ? cur[fo] : 0.0;           // self.function is never mutated (:29,:49)
@@ -218,7 +239,7 @@ batched_kernel(BatchedArgs a, int warps_per_cta, int warp_doubles) {
     group_sync();
     for (int i = tl; i < n; i += nl) {
         const int lab = cl[i];
-        if (lab < m) xs[lab] = cur[i * w1 + m];
+        if (x_label<WARM>(lab, m)) xs[lab] = cur[i * w1 + m];
     }
     group_sync();
     if (a.x) for (int j = tl; j < m; j += nl) a.x[lp * m + j] = xs[j];
@@ -227,8 +248,21 @@ batched_kernel(BatchedArgs a, int warps_per_cta, int warp_doubles) {
     if (tl == 0) {
         a.status[lp] = status;
         a.npiv[lp] = npiv;
-        if (a.obj) a.obj[lp] = (m >= 2) ? __dadd_rn(__dmul_rn(f0, xs[0]), __dmul_rn(f1, xs[1])) : 0.0;
+        if (a.obj) a.obj[lp] = (m >= 2) ? __dadd_rn(__dmul_rn(WARM ? c0 : f0, xs[0]), __dmul_rn(WARM ? c1 : f1, xs[1])) : 0.0;
     }
+}
+
+template <bool CTA>
+__global__ void __launch_bounds__(CTA ? 512 : 256, CTA ? 1 : 6)
+batched_kernel(BatchedArgs a, int warps_per_cta, int warp_doubles) {
+    batched_solve<CTA, false>(a, nullptr, warps_per_cta, warp_doubles);
+}
+
+// the resume of batched_kernel (spx_warm_solve_batched); function [B][m], the LPs' current costs, or null without obj
+template <bool CTA>
+__global__ void __launch_bounds__(CTA ? 512 : 256, CTA ? 1 : 6)
+batched_warm_kernel(BatchedArgs a, const double *function, int warps_per_cta, int warp_doubles) {
+    batched_solve<CTA, true>(a, function, warps_per_cta, warp_doubles);
 }
 
 // One LP of a ragged batch, start to finish: batched_kernel's loop with the shape and the offsets taken from the LP's
@@ -237,10 +271,12 @@ batched_kernel(BatchedArgs a, int warps_per_cta, int warp_doubles) {
 // CTA have different shapes, so each warp has its own cell -> (row, col) lookup table (cell_i, cell_j) instead of a
 // CTA-wide one; in CTA mode the group synchronises with a named barrier of its own nl threads.
 // (batched_kernel keeps its own copy of the loop: it runs at the 40-register cap of its launch bounds in warp mode,
-// and any restructuring of its code moves its spills.)
-template <bool CTA>
+// and any restructuring of its code moves its spills.)  WARM: the resume, as batched_solve's; gd: LP lp's descriptor
+// in global memory (d is its copy).
+template <bool CTA, bool WARM>
 __device__ __forceinline__ void ragged_body(const BatchedArgs &a, const RaggedLp &d, int64_t lp, const uint16_t *cell_i,
-                                             const uint16_t *cell_j, double *base, int *s_ctl, int tl, int nl) {
+                                             const uint16_t *cell_j, double *base, int *s_ctl, int tl, int nl,
+                                             const double *function, const RaggedLp *gd) {
     const int n = d.n, m = d.m, w1 = m + 1;
     const int cells = n * w1 + m;
     const int max_pivots = d.max_pivots;
@@ -258,8 +294,19 @@ __device__ __forceinline__ void ragged_body(const BatchedArgs &a, const RaggedLp
 
     double *Tg = a.T + d.t;
     for (int k = tl; k < cells; k += nl) cur[k] = Tg[k];
-    for (int j = tl; j < m; j += nl) rl[j] = j;           // 'x1'..'xm'  :30
-    for (int i = tl; i < n; i += nl) cl[i] = m + i;       // 'y1'..'yn'  :31
+    double c0 = 0.0, c1 = 0.0;                            // a resume: the current costs for obj
+    if constexpr (WARM) {
+        // The offsets come from the descriptor in global memory (gd, read once each), not from d: warp mode runs at
+        // the register cap of its launch bounds and keeps d's offsets in local memory, so reading them there would
+        // cost more spill loads than the solve has.
+        const int64_t xm = *(volatile const int64_t *)&gd->xm, xn = *(volatile const int64_t *)&gd->xn;
+        for (int j = tl; j < m; j += nl) rl[j] = a.rowlab[xm + j];
+        if (function && m >= 2) { c0 = function[xm]; c1 = function[xm + 1]; }
+        for (int i = tl; i < n; i += nl) cl[i] = a.collab[xn + i];
+    } else {
+        for (int j = tl; j < m; j += nl) rl[j] = j;       // 'x1'..'xm'  :30
+        for (int i = tl; i < n; i += nl) cl[i] = m + i;   // 'y1'..'yn'  :31
+    }
     group_sync();
     const int fo = n * w1;                                // offset of the f row
     const double f0 = (m >= 1) ? cur[fo] : 0.0;           // self.function is never mutated (:29,:49)
@@ -318,7 +365,7 @@ __device__ __forceinline__ void ragged_body(const BatchedArgs &a, const RaggedLp
     group_sync();
     for (int i = tl; i < n; i += nl) {
         const int lab = cl[i];
-        if (lab < m) xs[lab] = cur[i * w1 + m];
+        if (x_label<WARM>(lab, m)) xs[lab] = cur[i * w1 + m];
     }
     group_sync();
     if (a.x) for (int j = tl; j < m; j += nl) a.x[d.xm + j] = xs[j];
@@ -327,7 +374,7 @@ __device__ __forceinline__ void ragged_body(const BatchedArgs &a, const RaggedLp
     if (tl == 0) {
         a.status[lp] = status;
         a.npiv[lp] = npiv;
-        if (a.obj) a.obj[lp] = (m >= 2) ? __dadd_rn(__dmul_rn(f0, xs[0]), __dmul_rn(f1, xs[1])) : 0.0;
+        if (a.obj) a.obj[lp] = (m >= 2) ? __dadd_rn(__dmul_rn(WARM ? c0 : f0, xs[0]), __dmul_rn(WARM ? c1 : f1, xs[1])) : 0.0;
     }
 }
 
@@ -336,10 +383,10 @@ __device__ __forceinline__ void ragged_body(const BatchedArgs &a, const RaggedLp
 // bounds as batched_kernel<false>.  CTA mode: slot = CTA; the CTA is launched at the warp count of
 // the largest LP of the launch, builds the lookup table of its own LP, and only the warps its LP needs stay (the
 // warp count the uniform entry gives that shape: 32 cells per warp, 2..16 warps).
-template <bool CTA>
-__global__ void __launch_bounds__(CTA ? 512 : 256, CTA ? 1 : 6)
-ragged_batched_kernel(BatchedArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
-                      int warps_per_cta, int warp_doubles) {
+template <bool CTA, bool WARM>
+__device__ __forceinline__ void ragged_batched(const BatchedArgs &a, const RaggedLp *__restrict__ lps,
+                                               const int32_t *__restrict__ order, int warps_per_cta, int warp_doubles,
+                                               const double *function) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ int s_ctl[4];
     const int warp = threadIdx.x >> 5;
@@ -360,7 +407,7 @@ ragged_batched_kernel(BatchedArgs a, const RaggedLp *__restrict__ lps, const int
         }
         __syncwarp();
         double *base = reinterpret_cast<double *>(slot_raw + WARP_LUT_BYTES);
-        ragged_body<false>(a, d, lp, cell_i, cell_j, base, s_ctl, lane, 32);
+        ragged_body<false, WARM>(a, d, lp, cell_i, cell_j, base, s_ctl, lane, 32, function, lps + lp);
         return;
     }
     const int64_t lp = order[slot];
@@ -380,7 +427,22 @@ ragged_batched_kernel(BatchedArgs a, const RaggedLp *__restrict__ lps, const int
     if ((int)threadIdx.x >= nl) return;
     const size_t lut_bytes = ((size_t)cells * 4 + 15) / 16 * 16;
     double *base = reinterpret_cast<double *>(smem_raw + lut_bytes);
-    ragged_body<true>(a, d, lp, cell_i, cell_j, base, s_ctl, (int)threadIdx.x, nl);
+    ragged_body<true, WARM>(a, d, lp, cell_i, cell_j, base, s_ctl, (int)threadIdx.x, nl, function, lps + lp);
+}
+
+template <bool CTA>
+__global__ void __launch_bounds__(CTA ? 512 : 256, CTA ? 1 : 6)
+ragged_batched_kernel(BatchedArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
+                      int warps_per_cta, int warp_doubles) {
+    ragged_batched<CTA, false>(a, lps, order, warps_per_cta, warp_doubles, nullptr);
+}
+
+// the resume of ragged_batched_kernel (spx_warm_solve_ragged); function packed as x, or null without obj
+template <bool CTA>
+__global__ void __launch_bounds__(CTA ? 512 : 256, CTA ? 1 : 6)
+ragged_batched_warm_kernel(BatchedArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
+                           int warps_per_cta, int warp_doubles, const double *function) {
+    ragged_batched<CTA, true>(a, lps, order, warps_per_cta, warp_doubles, function);
 }
 
 size_t warp_bytes(int n, int m) {
@@ -427,16 +489,17 @@ bool batched_fits(int n, int m) {
     return cells <= CTA_MODE_MIN_CELLS || lut_bytes(n, m) + warp_bytes(n, m) <= K4_DYN_LIMIT;
 }
 
-// returns cudaErrorInvalidValue when one LP does not fit shared memory
+// returns cudaErrorInvalidValue when one LP does not fit shared memory; warm: the resume (batched_warm_kernel)
 cudaError_t solve_batched(double *T, int64_t B, int n, int m, int rule, int max_pivots, double *x,
                           double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab,
-                          int32_t *collab, int32_t *trace, double *snap, cudaStream_t stream) {
+                          int32_t *collab, int32_t *trace, double *snap, bool warm, const double *function,
+                          cudaStream_t stream) {
     if (B <= 0) return cudaSuccess;
     if (!batched_fits(n, m)) return cudaErrorInvalidValue;
     const size_t wb = warp_bytes(n, m), lb = lut_bytes(n, m);
     const int64_t cells = (int64_t)n * (m + 1) + m;
     BatchedArgs a{T, B, n, m, rule, max_pivots, x, obj, status, npiv, rowlab, collab, trace, snap};
-    static size_t configured_dev[64][2] = {};
+    static size_t configured_dev[64][4] = {};
     size_t *configured = configured_dev[spx_host::device_slot()];
     if (cells > CTA_MODE_MIN_CELLS) {
         // one CTA per LP: one cell per thread where possible (measured on Klee-Minty n=20: 32 cells per warp
@@ -445,10 +508,14 @@ cudaError_t solve_batched(double *T, int64_t B, int n, int m, int rule, int max_
         warps = warps < 2 ? 2 : (warps > 16 ? 16 : warps);
         const size_t smem = lb + wb;
         if (smem > 48 * 1024) {
-            const cudaError_t e = configure_k4(batched_kernel<true>, configured[1]);
+            const cudaError_t e = warm ? configure_k4(batched_warm_kernel<true>, configured[3])
+                                       : configure_k4(batched_kernel<true>, configured[1]);
             if (e != cudaSuccess) return e;
         }
-        batched_kernel<true><<<(unsigned)B, warps * 32, smem, stream>>>(a, 1, (int)(wb / sizeof(double)));
+        if (warm)
+            batched_warm_kernel<true><<<(unsigned)B, warps * 32, smem, stream>>>(a, function, 1, (int)(wb / sizeof(double)));
+        else
+            batched_kernel<true><<<(unsigned)B, warps * 32, smem, stream>>>(a, 1, (int)(wb / sizeof(double)));
         spx_host::count_launch();
         return cudaGetLastError();
     }
@@ -460,11 +527,15 @@ cudaError_t solve_batched(double *T, int64_t B, int n, int m, int rule, int max_
     if ((int64_t)wpc > B) wpc = (int)B;
     const size_t smem = lb + (size_t)wpc * wb;
     if (smem > 48 * 1024) {
-        const cudaError_t e = configure_k4(batched_kernel<false>, configured[0]);
+        const cudaError_t e = warm ? configure_k4(batched_warm_kernel<false>, configured[2])
+                                   : configure_k4(batched_kernel<false>, configured[0]);
         if (e != cudaSuccess) return e;
     }
     const int64_t ctas = (B + wpc - 1) / wpc;
-    batched_kernel<false><<<(unsigned)ctas, wpc * 32, smem, stream>>>(a, wpc, (int)(wb / sizeof(double)));
+    if (warm)
+        batched_warm_kernel<false><<<(unsigned)ctas, wpc * 32, smem, stream>>>(a, function, wpc, (int)(wb / sizeof(double)));
+    else
+        batched_kernel<false><<<(unsigned)ctas, wpc * 32, smem, stream>>>(a, wpc, (int)(wb / sizeof(double)));
     spx_host::count_launch();
     return cudaGetLastError();
 }
@@ -493,19 +564,29 @@ int ragged_warps_per_cta(int64_t slot, int64_t count) {
 
 cudaError_t solve_ragged_batched(const RaggedLaunch &l, const RaggedLp *lps, const int32_t *order, double *T, int rule,
                                  double *x, double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab,
-                                 int32_t *collab, int32_t *trace, double *snap, cudaStream_t stream) {
+                                 int32_t *collab, int32_t *trace, double *snap, bool warm, const double *function,
+                                 cudaStream_t stream) {
     if (l.count <= 0) return cudaSuccess;
     BatchedArgs a{T, l.count, 0, 0, rule, 0, x, obj, status, npiv, rowlab, collab, trace, snap};
-    static size_t configured_dev[64][2] = {};
+    static size_t configured_dev[64][4] = {};
     size_t *configured = configured_dev[spx_host::device_slot()];
     const bool cta = (l.kernel == RAGGED_CTA);
     if (l.smem > 48 * 1024) {
-        const cudaError_t e = cta ? configure_k4(ragged_batched_kernel<true>, configured[1])
-                                  : configure_k4(ragged_batched_kernel<false>, configured[0]);
+        const cudaError_t e = warm ? (cta ? configure_k4(ragged_batched_warm_kernel<true>, configured[3])
+                                          : configure_k4(ragged_batched_warm_kernel<false>, configured[2]))
+                                   : (cta ? configure_k4(ragged_batched_kernel<true>, configured[1])
+                                          : configure_k4(ragged_batched_kernel<false>, configured[0]));
         if (e != cudaSuccess) return e;
     }
     const int64_t ctas = (l.count + l.per_cta - 1) / l.per_cta;
-    if (cta)
+    const int per_cta = cta ? 1 : l.per_cta, slot_doubles = cta ? 0 : (int)l.slot_doubles;
+    if (warm && cta)
+        ragged_batched_warm_kernel<true><<<(unsigned)ctas, l.threads, (size_t)l.smem, stream>>>(
+            a, lps, order + l.first, per_cta, slot_doubles, function);
+    else if (warm)
+        ragged_batched_warm_kernel<false><<<(unsigned)ctas, l.threads, (size_t)l.smem, stream>>>(
+            a, lps, order + l.first, per_cta, slot_doubles, function);
+    else if (cta)
         ragged_batched_kernel<true><<<(unsigned)ctas, l.threads, (size_t)l.smem, stream>>>(a, lps, order + l.first, 1, 0);
     else
         ragged_batched_kernel<false><<<(unsigned)ctas, l.threads, (size_t)l.smem, stream>>>(a, lps, order + l.first,

@@ -53,9 +53,12 @@ struct ClusterArgs {
 
 // The body of both kernels.  RAGGED == false: shape, R, Q and offsets from the arguments (one shape per launch).
 // RAGGED == true: LP order[blockIdx.x / S] of a ragged batch, its shape and offsets from lps[], R and Q from its shape.
-template <bool RAGGED>
+// WARM == true: a resume (spx_warm_solve_*): each CTA reads the labels of its band and of its header slice from
+// a.rowlab / a.collab, f0 and f1 for obj come from `function` (packed as x) in the epilogue, and no label outside
+// [0, m) indexes x or s_x01.
+template <bool RAGGED, bool WARM>
 __device__ __forceinline__ void cluster_body(const ClusterArgs &a, const RaggedLp *__restrict__ lps,
-                                             const int32_t *__restrict__ order) {
+                                             const int32_t *__restrict__ order, const double *function) {
     cg::cluster_group cluster = cg::this_cluster();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ Scratch sc;
@@ -88,8 +91,13 @@ __device__ __forceinline__ void cluster_body(const ClusterArgs &a, const RaggedL
     double *Tg = a.T + (RAGGED ? d.t : lp * cells);
     for (int k = tid; k < bandcells; k += nt) band[k] = Tg[(int64_t)r0 * w1 + k];
     for (int j = tid; j < m; j += nt) f[j] = Tg[fo + j];
-    for (int i = tid; i < rows; i += nt) cl[i] = m + r0 + i;
-    for (int j = tid; j < cols; j += nt) rl[j] = j0 + j;
+    if constexpr (WARM) {
+        for (int i = tid; i < rows; i += nt) cl[i] = a.collab[(RAGGED ? d.xn : lp * n) + r0 + i];
+        for (int j = tid; j < cols; j += nt) rl[j] = a.rowlab[(RAGGED ? d.xm : lp * m) + j0 + j];
+    } else {
+        for (int i = tid; i < rows; i += nt) cl[i] = m + r0 + i;
+        for (int j = tid; j < cols; j += nt) rl[j] = j0 + j;
+    }
     if (tid < 2) s_x01[tid] = 0.0;
     cluster.sync();                                        // every CTA runs and is loaded before any DSMEM access
     const double f0 = (m >= 1) ? f[0] : 0.0;               // self.function is never mutated (:29,:49)
@@ -191,7 +199,7 @@ __device__ __forceinline__ void cluster_body(const ClusterArgs &a, const RaggedL
     // labels are a permutation of 0..n+m-1: x_j is the b of the row labelled x_j, or 0 when a column carries it
     for (int i = tid; i < rows; i += nt) {
         const int lab = cl[i];
-        if (lab < m) {
+        if ((!WARM || lab >= 0) && lab < m) {
             const double v = band[i * w1 + m];
             if (xg) xg[lab] = v;
             if (lab < 2) *cluster.map_shared_rank(&s_x01[lab], 0) = v;
@@ -200,25 +208,40 @@ __device__ __forceinline__ void cluster_body(const ClusterArgs &a, const RaggedL
     }
     for (int j = tid; j < cols; j += nt) {
         const int lab = rl[j];
-        if (xg && lab < m) xg[lab] = 0.0;
+        if (xg && (!WARM || lab >= 0) && lab < m) xg[lab] = 0.0;
         if (a.rowlab) a.rowlab[(RAGGED ? d.xm : lp * m) + j0 + j] = lab;
     }
     cluster.sync();                                        // s_x01 complete; no CTA leaves while a peer may read it
     if (rank == 0 && tid == 0) {
         a.status[lp] = status;
         a.npiv[lp] = npiv;
-        if (a.obj) a.obj[lp] = (m >= 2) ? __dadd_rn(__dmul_rn(f0, s_x01[0]), __dmul_rn(f1, s_x01[1])) : 0.0;
+        if (a.obj) {
+            const double *fn = function + (RAGGED ? d.xm : lp * m);
+            const double g0 = WARM ? fn[0] : f0, g1 = WARM && m >= 2 ? fn[1] : f1;
+            a.obj[lp] = (m >= 2) ? __dadd_rn(__dmul_rn(g0, s_x01[0]), __dmul_rn(g1, s_x01[1])) : 0.0;
+        }
     }
 }
 
 __global__ void __launch_bounds__(CLUSTER_THREADS, 1) cluster_kernel(ClusterArgs a) {
-    cluster_body<false>(a, nullptr, nullptr);
+    cluster_body<false, false>(a, nullptr, nullptr, nullptr);
 }
 
 // a ragged batch: the LPs order[0 .. a.B) of one cluster size a.S, each cluster its own shape (a.n, a.m, a.R, a.Q unused)
 __global__ void __launch_bounds__(CLUSTER_THREADS, 1)
 ragged_cluster_kernel(ClusterArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order) {
-    cluster_body<true>(a, lps, order);
+    cluster_body<true, false>(a, lps, order, nullptr);
+}
+
+// the resumes of the two kernels above (spx_warm_solve_*): function [B][m] or packed as x, null without obj
+__global__ void __launch_bounds__(CLUSTER_THREADS, 1) cluster_warm_kernel(ClusterArgs a, const double *function) {
+    cluster_body<false, true>(a, nullptr, nullptr, function);
+}
+
+__global__ void __launch_bounds__(CLUSTER_THREADS, 1)
+ragged_cluster_warm_kernel(ClusterArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
+                           const double *function) {
+    cluster_body<true, true>(a, lps, order, function);
 }
 
 // the per-CTA footprint of the header comment, for S CTAs per LP
@@ -246,9 +269,11 @@ int cluster_size(int64_t n, int64_t m) {
 // one cluster of this size and footprint
 cudaError_t solve_batched_cluster(double *T, int64_t B, int n, int m, int S, int rule, int max_pivots, double *x,
                                   double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab, int32_t *collab,
-                                  int32_t *trace, double *snap, cudaStream_t stream) {
+                                  int32_t *trace, double *snap, bool warm, const double *function,
+                                  cudaStream_t stream) {
     ClusterArgs a{T, B, n, m, rule, max_pivots, S, (n + S - 1) / S, (m + S - 1) / S,
                   x, obj, status, npiv, rowlab, collab, trace, snap};
+    if (warm) return launch_cluster_kernel<cluster_warm_kernel>(S, B, cluster_bytes(n, m, S), stream, a, function);
     return launch_cluster_kernel<cluster_kernel>(S, B, cluster_bytes(n, m, S), stream, a);
 }
 
@@ -258,8 +283,12 @@ int64_t ragged_cluster_bytes(int n, int m, int S) { return cluster_bytes(n, m, S
 // among them; cudaErrorInvalidClusterSize when the device cannot co-schedule one such cluster
 cudaError_t solve_ragged_cluster(const RaggedLaunch &l, const RaggedLp *lps, const int32_t *order, double *T, int rule,
                                  double *x, double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab,
-                                 int32_t *collab, int32_t *trace, double *snap, cudaStream_t stream) {
+                                 int32_t *collab, int32_t *trace, double *snap, bool warm, const double *function,
+                                 cudaStream_t stream) {
     ClusterArgs a{T, l.count, 0, 0, rule, 0, l.S, 0, 0, x, obj, status, npiv, rowlab, collab, trace, snap};
+    if (warm)
+        return launch_cluster_kernel<ragged_cluster_warm_kernel>(l.S, l.count, l.smem, stream, a, lps, order + l.first,
+                                                                 function);
     return launch_cluster_kernel<ragged_cluster_kernel>(l.S, l.count, l.smem, stream, a, lps, order + l.first);
 }
 

@@ -73,10 +73,10 @@ __device__ __forceinline__ double2 ld_l2_v2(const double *p) {
 
 // The body of both kernels.  RAGGED == false: shape, R, Q and offsets from the arguments (one shape per launch).
 // RAGGED == true: LP order[blockIdx.x / S] of a ragged batch, its shape and offsets from lps[], R and Q from its shape
-// (as cluster_body in spx_cluster.cu).
-template <bool RAGGED>
+// (as cluster_body in spx_cluster.cu).  WARM == true: a resume, as cluster_body's.
+template <bool RAGGED, bool WARM>
 __device__ __forceinline__ void global_body(const GlobalArgs &a, const RaggedLp *__restrict__ lps,
-                                            const int32_t *__restrict__ order) {
+                                            const int32_t *__restrict__ order, const double *function) {
     cg::cluster_group cluster = cg::this_cluster();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ Scratch sc;
@@ -115,8 +115,13 @@ __device__ __forceinline__ void global_body(const GlobalArgs &a, const RaggedLp 
     const double inv_w1 = 1.0 / (double)w1;
 
     for (int j = tid; j < m; j += nt) f[j] = ld_l2(Tg + fo + j);
-    for (int i = tid; i < rows; i += nt) cl[i] = m + r0 + i;
-    for (int j = tid; j < cols; j += nt) rl[j] = j0 + j;
+    if constexpr (WARM) {
+        for (int i = tid; i < rows; i += nt) cl[i] = a.collab[(RAGGED ? lpd.xn : lp * n) + r0 + i];
+        for (int j = tid; j < cols; j += nt) rl[j] = a.rowlab[(RAGGED ? lpd.xm : lp * m) + j0 + j];
+    } else {
+        for (int i = tid; i < rows; i += nt) cl[i] = m + r0 + i;
+        for (int j = tid; j < cols; j += nt) rl[j] = j0 + j;
+    }
     if (tid < 2) s_x01[tid] = 0.0;
     cluster.sync();                                        // every CTA runs and is loaded before any DSMEM access
     const double f0 = (m >= 1) ? f[0] : 0.0;               // self.function is never mutated (:29,:49)
@@ -254,7 +259,7 @@ __device__ __forceinline__ void global_body(const GlobalArgs &a, const RaggedLp 
     // labels are a permutation of 0..n+m-1: x_j is the b of the row labelled x_j, or 0 when a column carries it
     for (int i = tid; i < rows; i += nt) {
         const int lab = cl[i];
-        if (lab < m) {
+        if ((!WARM || lab >= 0) && lab < m) {
             const double v = ld_l2(band + (int64_t)i * w1 + m);
             if (xg) xg[lab] = v;
             if (lab < 2) *cluster.map_shared_rank(&s_x01[lab], 0) = v;
@@ -263,26 +268,41 @@ __device__ __forceinline__ void global_body(const GlobalArgs &a, const RaggedLp 
     }
     for (int j = tid; j < cols; j += nt) {
         const int lab = rl[j];
-        if (xg && lab < m) xg[lab] = 0.0;
+        if (xg && (!WARM || lab >= 0) && lab < m) xg[lab] = 0.0;
         if (a.rowlab) a.rowlab[(RAGGED ? lpd.xm : lp * m) + j0 + j] = lab;
     }
     cluster.sync();                                        // s_x01 complete; no CTA leaves while a peer may read it
     if (rank == 0 && tid == 0) {
         a.status[lp] = status;
         a.npiv[lp] = npiv;
-        if (a.obj) a.obj[lp] = (m >= 2) ? __dadd_rn(__dmul_rn(f0, s_x01[0]), __dmul_rn(f1, s_x01[1])) : 0.0;
+        if (a.obj) {
+            const double *fn = function + (RAGGED ? lpd.xm : lp * m);
+            const double g0 = WARM ? fn[0] : f0, g1 = WARM && m >= 2 ? fn[1] : f1;
+            a.obj[lp] = (m >= 2) ? __dadd_rn(__dmul_rn(g0, s_x01[0]), __dmul_rn(g1, s_x01[1])) : 0.0;
+        }
     }
 }
 
 __global__ void __launch_bounds__(CLUSTER_THREADS, GLOBAL_MIN_CTAS) global_kernel(GlobalArgs a) {
-    global_body<false>(a, nullptr, nullptr);
+    global_body<false, false>(a, nullptr, nullptr, nullptr);
 }
 
 // a ragged batch: the LPs order[0 .. a.B) at one cluster size a.S, each cluster its own shape (a.n, a.m, a.R, a.Q,
 // a.max_pivots unused)
 __global__ void __launch_bounds__(CLUSTER_THREADS, GLOBAL_MIN_CTAS)
 ragged_global_kernel(GlobalArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order) {
-    global_body<true>(a, lps, order);
+    global_body<true, false>(a, lps, order, nullptr);
+}
+
+// the resumes of the two kernels above (spx_warm_solve_*): function [B][m] or packed as x, null without obj
+__global__ void __launch_bounds__(CLUSTER_THREADS, GLOBAL_MIN_CTAS) global_warm_kernel(GlobalArgs a, const double *function) {
+    global_body<false, true>(a, nullptr, nullptr, function);
+}
+
+__global__ void __launch_bounds__(CLUSTER_THREADS, GLOBAL_MIN_CTAS)
+ragged_global_warm_kernel(GlobalArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
+                          const double *function) {
+    global_body<true, true>(a, lps, order, function);
 }
 
 // the per-CTA footprint of the header comment, for S CTAs per LP
@@ -358,9 +378,11 @@ cudaError_t global_cluster_size(int64_t n, int64_t m, int64_t B, int *S_out) {
 // one cluster of this size and footprint
 cudaError_t solve_batched_global(double *T, int64_t B, int n, int m, int S, int rule, int max_pivots, double *x,
                                  double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab, int32_t *collab,
-                                 int32_t *trace, double *snap, cudaStream_t stream) {
+                                 int32_t *trace, double *snap, bool warm, const double *function,
+                                 cudaStream_t stream) {
     GlobalArgs a{T, B, n, m, rule, max_pivots, S, (n + S - 1) / S, (m + S - 1) / S,
                  x, obj, status, npiv, rowlab, collab, trace, snap};
+    if (warm) return launch_cluster_kernel<global_warm_kernel>(S, B, global_bytes(n, m, S), stream, a, function);
     return launch_cluster_kernel<global_kernel>(S, B, global_bytes(n, m, S), stream, a);
 }
 
@@ -385,8 +407,12 @@ cudaError_t ragged_global_size(const RaggedLaunch &l, const RaggedLp *h_lps, con
 // ragged_global_size); cudaErrorInvalidClusterSize when the device cannot co-schedule one such cluster
 cudaError_t solve_ragged_global(const RaggedLaunch &l, int S, int64_t smem, const RaggedLp *lps, const int32_t *order,
                                 double *T, int rule, double *x, double *obj, int32_t *status, int32_t *npiv,
-                                int32_t *rowlab, int32_t *collab, int32_t *trace, double *snap, cudaStream_t stream) {
+                                int32_t *rowlab, int32_t *collab, int32_t *trace, double *snap, bool warm,
+                                const double *function, cudaStream_t stream) {
     GlobalArgs a{T, l.count, 0, 0, rule, 0, S, 0, 0, x, obj, status, npiv, rowlab, collab, trace, snap};
+    if (warm)
+        return launch_cluster_kernel<ragged_global_warm_kernel>(S, l.count, smem, stream, a, lps, order + l.first,
+                                                                function);
     return launch_cluster_kernel<ragged_global_kernel>(S, l.count, smem, stream, a, lps, order + l.first);
 }
 
