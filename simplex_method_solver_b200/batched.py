@@ -127,17 +127,22 @@ def _per_lp(a, B: int, k: int, name: str) -> np.ndarray:
     return np.ascontiguousarray(a)
 
 
-def _first_bad_lp(bad_rows: np.ndarray, what: str) -> None:
-    bad = np.flatnonzero(bad_rows)
-    if bad.size:
-        raise ValueError(f"LP {int(bad[0])}: {what}")
+def _check_finite(a: Optional[np.ndarray], what: str, starts: Optional[np.ndarray] = None) -> None:
+    """A non-finite entry of `a` is a ValueError naming its LP: a is [B, k], one row per LP, or with `starts` packed,
+    LP k's entries from starts[k] on (n, m >= 1: no LP's slice is empty).  None passes."""
+    bad = np.flatnonzero(~np.isfinite(a)) if a is not None else []
+    if len(bad):
+        lp = bad[0] // a.shape[1] if starts is None else np.searchsorted(starts, bad[0], side="right") - 1
+        raise ValueError(f"LP {int(lp)}: {what} is not finite")
 
 
 def _check_labels(rowlab: np.ndarray, collab: np.ndarray) -> None:
     """rowlab [B, m], collab [B, n]: each LP's labels must be a permutation of 0..n+m-1."""
     n, m = collab.shape[1], rowlab.shape[1]
     lab = np.sort(np.concatenate([rowlab, collab], axis=1), axis=1)
-    _first_bad_lp((lab != np.arange(n + m)).any(axis=1), f"labels are not a permutation of 0..{n + m - 1}")
+    bad = np.flatnonzero((lab != np.arange(n + m)).any(axis=1))
+    if bad.size:
+        raise ValueError(f"LP {int(bad[0])}: labels are not a permutation of 0..{n + m - 1}")
 
 
 def _check_ragged_labels(rowlab: np.ndarray, collab: np.ndarray, shapes: np.ndarray, xm, xn) -> None:
@@ -225,9 +230,8 @@ class DeviceBatch:
         B, n, m = self.B, self.n, self.m
         db = None if rhs_delta is None else _per_lp(rhs_delta, B, n, "rhs_delta")
         dc = None if cost_delta is None else _per_lp(cost_delta, B, m, "cost_delta")
-        for name, d in (("rhs_delta", db), ("cost_delta", dc)):
-            if d is not None:
-                _first_bad_lp(~np.isfinite(d).all(axis=1), f"{name} is not finite")
+        _check_finite(db, "rhs_delta")
+        _check_finite(dc, "cost_delta")
         if B == 0 or (db is None and dc is None):
             return
         up = lambda a: None if a is None else torch.from_numpy(a).to(self.device)  # noqa: E731
@@ -294,6 +298,7 @@ class RaggedPlan(NamedTuple):
     plan: np.ndarray              # the plan bytes (uint8), as spx_ragged_plan wrote them
     totals: np.ndarray            # [5] packed lengths: T, x (= rowlab), collab, trace pairs, snap
     lps: np.ndarray               # [B] descriptors: n, m, max_pivots, cells and the offsets t, xm, xn, tr, sn
+    offsets: np.ndarray           # [B, 5] int64: the offsets t, xm, xn, tr, sn of each LP (RaggedResult.offsets)
     launches: list                # per launch: dict(kind, S, threads, smem, lps = LP indices in launch order);
     #                               for kind "global" S is the planned S (S_min, or SPX_OPT_CLUSTER_SIZE)
 
@@ -325,7 +330,8 @@ def ragged_plan(shapes, max_pivots, engine: str = "auto") -> RaggedPlan:
         f, c = int(la["first"]), int(la["count"])
         launches.append({"kind": LAUNCH_KINDS[int(la["kernel"])], "S": int(la["S"]), "threads": int(la["threads"]),
                          "smem": int(la["smem"]), "lps": order[f: f + c].copy()})
-    return RaggedPlan(plan, totals, lps, launches)
+    offsets = np.stack([lps["t"], lps["xm"], lps["xn"], lps["tr"], lps["sn"]], axis=1).astype(np.int64)
+    return RaggedPlan(plan, totals, lps, offsets, launches)
 
 
 class RaggedResult(NamedTuple):
@@ -441,8 +447,7 @@ class DeviceRaggedBatch:
         if any(S <= 0 for S in self.cluster_sizes):
             raise N.SpxError(f"spx_ragged_cluster_size failed: {L.spx_last_error().decode(errors='replace')}")
         self.shapes = np.concatenate([self.shapes2, self.caps[:, None]], axis=1)
-        lp = self.plan.lps
-        self.offsets = np.stack([lp["t"], lp["xm"], lp["xn"], lp["tr"], lp["sn"]], axis=1).astype(np.int64)
+        self.offsets = self.plan.offsets
         tot = [int(v) for v in self.plan.totals]
         dev, f64, i32 = self.device, torch.float64, torch.int32
         q = lambda k: max(k, 1)  # noqa: E731
@@ -479,10 +484,7 @@ class DeviceRaggedBatch:
         a = np.ascontiguousarray(np.asarray(a, dtype=np.float64).reshape(-1))
         if a.shape != (total,):
             raise ValueError(f"{name} must be packed [{total}], got {a.shape[0]} entries")
-        bad = np.flatnonzero(~np.isfinite(a))
-        if bad.size:
-            lp = int(np.searchsorted(self.offsets[:, k], bad[0], side="right")) - 1    # n, m >= 1: no empty slice
-            raise ValueError(f"LP {lp}: {name} is not finite")
+        _check_finite(a, name, self.offsets[:, k])
         return a
 
     def upload_labels(self, rowlab, collab, non_blocking: bool = False):
@@ -567,6 +569,29 @@ def solve_ragged(lps, max_pivots: Union[int, Sequence[int]] = 64, rule: str = "r
     return db.result()
 
 
+def _uniform_labels(result: BatchResult, fn: str):
+    """(rowlab [B, m], collab [B, n], B, n, m) of a host BatchResult given to `fn`, with n, m >= 1"""
+    if not isinstance(result, BatchResult):
+        raise TypeError(f"{fn}() takes a BatchResult or a RaggedResult, not {type(result).__name__}")
+    rowlab = np.ascontiguousarray(result.rowlab, dtype=np.int32)
+    collab = np.ascontiguousarray(result.collab, dtype=np.int32)
+    if rowlab.ndim != 2 or collab.ndim != 2 or rowlab.shape[0] != collab.shape[0]:
+        raise ValueError("result.rowlab must be [B, m] and result.collab [B, n]")
+    B, m, n = rowlab.shape[0], rowlab.shape[1], collab.shape[1]
+    if n < 1 or m < 1:
+        raise ValueError(f"bad shape {n} x {m}")
+    return rowlab, collab, B, n, m
+
+
+def _check_packing(result: RaggedResult, plan: RaggedPlan) -> None:
+    """the packed tables, labels and status of a host RaggedResult have the sizes of the LPs of `plan`"""
+    tot = plan.totals
+    for name, a, k in (("tables", result.tables, tot[0]), ("rowlab", result.rowlab, tot[1]),
+                       ("collab", result.collab, tot[2]), ("status", result.status, len(plan.lps))):
+        if np.size(a) != k:
+            raise ValueError(f"result.{name} has {np.size(a)} entries, the shapes need {k}")
+
+
 def sensitivity(result: Union[BatchResult, RaggedResult], device=None) -> Union[Sensitivity, RaggedSensitivity]:
     """Sensitivity report of the final tables of a host ``BatchResult`` (``solve_batched``) or ``RaggedResult``
     (``solve_ragged``): uploads the tables, labels and status and runs the report's kernels on ``device``."""
@@ -576,30 +601,17 @@ def sensitivity(result: Union[BatchResult, RaggedResult], device=None) -> Union[
         shapes = np.asarray(result.shapes, dtype=np.int64).reshape(-1, 3)
         B = shapes.shape[0]
         plan = ragged_plan(shapes[:, :2], shapes[:, 2], "auto_global")
-        lp = plan.lps
-        offsets = np.stack([lp["t"], lp["xm"], lp["xn"], lp["tr"], lp["sn"]], axis=1).astype(np.int64)
-        if not np.array_equal(offsets, np.asarray(result.offsets, dtype=np.int64).reshape(-1, 5)):
+        if not np.array_equal(plan.offsets, np.asarray(result.offsets, dtype=np.int64).reshape(-1, 5)):
             raise ValueError("result.offsets are not the packing of result.shapes")
-        tot = [int(v) for v in plan.totals]
-        for name, a, k in (("tables", result.tables, tot[0]), ("rowlab", result.rowlab, tot[1]),
-                           ("collab", result.collab, tot[2]), ("status", result.status, B)):
-            if np.size(a) != k:
-                raise ValueError(f"result.{name} has {np.size(a)} entries, the shapes need {k}")
+        _check_packing(result, plan)
         if B == 0:
             z = np.zeros
-            return RaggedSensitivity(z(0), z(0), z(0), z((0, 2)), z((0, 2)), z(0, bool), shapes.copy(), offsets)
+            return RaggedSensitivity(z(0), z(0), z(0), z((0, 2)), z((0, 2)), z(0, bool), shapes.copy(), plan.offsets)
         N.lib()
         return _sens_ragged(up(result.tables, np.float64), plan.plan, torch.from_numpy(plan.plan).to(dev),
                             up(result.status, np.int32), up(result.rowlab, np.int32), up(result.collab, np.int32),
-                            B, tot, shapes, offsets, dev)
-    if not isinstance(result, BatchResult):
-        raise TypeError(f"sensitivity() takes a BatchResult or a RaggedResult, not {type(result).__name__}")
-    rowlab, collab = np.asarray(result.rowlab), np.asarray(result.collab)
-    if rowlab.ndim != 2 or collab.ndim != 2 or rowlab.shape[0] != collab.shape[0]:
-        raise ValueError("result.rowlab must be [B, m] and result.collab [B, n]")
-    B, m, n = rowlab.shape[0], rowlab.shape[1], collab.shape[1]
-    if n < 1 or m < 1:
-        raise ValueError(f"bad shape {n} x {m}")
+                            B, plan.totals, shapes, plan.offsets, dev)
+    rowlab, collab, B, n, m = _uniform_labels(result, "sensitivity")
     if np.shape(result.tables) != (B, n * (m + 1) + m) or np.shape(result.status) != (B,):
         raise ValueError(f"result.tables must be [B, n*(m+1)+m] = [{B}, {n * (m + 1) + m}] and result.status [{B}]")
     if B == 0:
@@ -651,15 +663,7 @@ def resolve(result: Union[BatchResult, RaggedResult], data, rhs=None, cost=None,
     """
     if isinstance(result, RaggedResult):
         return _resolve_ragged(result, data, rhs, cost, max_pivots, rule, trace, snapshots, device, engine)
-    if not isinstance(result, BatchResult):
-        raise TypeError(f"resolve() takes a BatchResult or a RaggedResult, not {type(result).__name__}")
-    rowlab = np.ascontiguousarray(result.rowlab, dtype=np.int32)
-    collab = np.ascontiguousarray(result.collab, dtype=np.int32)
-    if rowlab.ndim != 2 or collab.ndim != 2 or rowlab.shape[0] != collab.shape[0]:
-        raise ValueError("result.rowlab must be [B, m] and result.collab [B, n]")
-    B, m, n = rowlab.shape[0], rowlab.shape[1], collab.shape[1]
-    if n < 1 or m < 1:
-        raise ValueError(f"bad shape {n} x {m}")
+    rowlab, collab, B, n, m = _uniform_labels(result, "resolve")
     cells = n * (m + 1) + m
     tables = np.ascontiguousarray(result.tables, dtype=np.float64)
     data = np.asarray(data, dtype=np.float64)
@@ -669,9 +673,8 @@ def resolve(result: Union[BatchResult, RaggedResult], data, rhs=None, cost=None,
     _check_labels(rowlab, collab)
     new_c, dc = _new_values(cost, data[:, n * (m + 1):], "cost")
     _, db = _new_values(rhs, data[:, : n * (m + 1)].reshape(B, n, m + 1)[:, :, m], "rhs")
-    for name, d in (("rhs - old rhs", db), ("cost - old cost", dc)):
-        if d is not None:
-            _first_bad_lp(~np.isfinite(d).all(axis=1), f"{name} is not finite")
+    _check_finite(db, "rhs - old rhs")
+    _check_finite(dc, "cost - old cost")
     db_ = DeviceBatch(B, n, m, int(max_pivots), trace, snapshots, device, engine)
     if B == 0:
         return _empty_batch(n, m, int(max_pivots), trace, snapshots)
@@ -690,28 +693,22 @@ def _resolve_ragged(result: RaggedResult, data, rhs, cost, max_pivots, rule, tra
         raise ValueError("data are not the LPs of result (their shapes differ from result.shapes)")
     B = shapes.shape[0]
     plan = ragged_plan(shapes, _caps(max_pivots, B), engine)
-    offsets = np.stack([plan.lps["t"], plan.lps["xm"], plan.lps["xn"]], axis=1).astype(np.int64)
-    tot = [int(v) for v in plan.totals]
-    for name, a, k in (("tables", result.tables, tot[0]), ("rowlab", result.rowlab, tot[1]),
-                       ("collab", result.collab, tot[2])):
-        if np.size(a) != k:
-            raise ValueError(f"result.{name} has {np.size(a)} entries, the shapes need {k}")
+    offsets = plan.offsets
+    _check_packing(result, plan)
     rowlab = np.ascontiguousarray(result.rowlab, dtype=np.int32).reshape(-1)
     collab = np.ascontiguousarray(result.collab, dtype=np.int32).reshape(-1)
-    old_b, old_c = np.empty(tot[2]), np.empty(tot[1])
+    old_b, old_c = np.empty(int(plan.totals[2])), np.empty(int(plan.totals[1]))
     _check_ragged_labels(rowlab, collab, shapes, offsets[:, 1], offsets[:, 2])
     for k in range(B):
         n, m = (int(v) for v in shapes[k])
-        t, xm, xn = (int(v) for v in offsets[k])
+        t, xm, xn = (int(v) for v in offsets[k, :3])
         old_b[xn: xn + n] = packed[t: t + n * (m + 1)].reshape(n, m + 1)[:, m]
         old_c[xm: xm + m] = packed[t + n * (m + 1): t + n * (m + 1) + m]
     new_b = _packed_values(rhs, shapes[:, 0], "rhs")
     new_c = _packed_values(cost, shapes[:, 1], "cost")
     deltas = [None if v is None else v - old for v, old in ((new_b, old_b), (new_c, old_c))]
-    for name, d, col in (("rhs - old rhs", deltas[0], 2), ("cost - old cost", deltas[1], 1)):
-        bad = np.flatnonzero(~np.isfinite(d)) if d is not None else []
-        if len(bad):
-            raise ValueError(f"LP {int(np.searchsorted(offsets[:, col], bad[0], side='right')) - 1}: {name} is not finite")
+    _check_finite(deltas[0], "rhs - old rhs", offsets[:, 2])
+    _check_finite(deltas[1], "cost - old cost", offsets[:, 1])
     db_ = DeviceRaggedBatch(shapes, max_pivots, trace, snapshots, device, engine)
     if B:
         db_.upload(np.ascontiguousarray(result.tables, dtype=np.float64).reshape(-1))

@@ -9,86 +9,7 @@
 #include <cstring>
 #include <vector>
 
-#include "spx_common.cuh"
-
-namespace spx_launch {
-int     sm_count();
-int64_t colbuf_doubles(int n);
-int64_t shard_msg_doubles(int n);
-int64_t batched_max_cells();
-bool batched_fits(int, int);
-cudaError_t pick(const double *, const double *, int, int, int64_t, int, int, spx_state *, double *,
-                 cudaStream_t);
-cudaError_t shard_candidate(const double *, const double *, int, int, int64_t, int64_t, int, int,
-                            const spx_state *, double *, cudaStream_t);
-cudaError_t shard_select(const double *, int, const double *, int, int, spx_state *, double *,
-                         const unsigned long long *, unsigned long long, cudaStream_t);
-cudaError_t update(const double *, double *, const double *, double *, int, int, int64_t, int64_t,
-                   spx_state *, const double *, int32_t *, int32_t *, int32_t *, int, cudaStream_t);
-cudaError_t ahead_candidate(const double *, const double *, double *, int, int, int64_t, int64_t, int,
-                            const spx_state *, const double *, double *, cudaStream_t);
-cudaError_t ahead_select(const double *, int, const double *, int, const spx_state *, spx_state *,
-                         double *, const unsigned long long *, unsigned long long, cudaStream_t);
-cudaError_t extract(const double *, int, int, const int32_t *, const double *, double *, double *,
-                    cudaStream_t);
-bool resident_fits(int, int, int64_t);
-cudaError_t resident_loop(double *, double *, double *, double *, int, int, int64_t, int, int64_t, spx_state *,
-                          double *, int32_t *, int32_t *, int32_t *, cudaStream_t);
-int fuse_max();
-int64_t fused_workspace_bytes(int, int64_t);
-cudaError_t fused_pass(double *, double *, double *, double *, int, int, int64_t, int, int, int, int, int, spx_state *,
-                       void *, int32_t *, int32_t *, int32_t *, cudaStream_t);
-cudaError_t fused_solve_passes(double *, double *, double *, double *, int, int, int64_t, int, spx_state *, void *,
-                               int32_t *, int32_t *, int32_t *, int64_t, int, int, int, cudaStream_t);
-cudaError_t fused_solo_sync();
-int64_t get_option(int);
-int     set_option(int, int64_t);
-cudaError_t selftest_division(const double *, const double *, int64_t, int64_t, unsigned long long *,
-                              double *, cudaStream_t);
-cudaError_t lazy_guard_selftest(const double *, const double *, const double *, const double *, int, int64_t,
-                                double *, double *, unsigned long long *, cudaStream_t);
-cudaError_t init_state(spx_state *, int32_t *, int32_t *, int, int, int64_t, cudaStream_t);
-cudaError_t solve_batched(double *, int64_t, int, int, int, int, double *, double *, int32_t *,
-                          int32_t *, int32_t *, int32_t *, int32_t *, double *, bool, const double *, cudaStream_t);
-bool cluster_fits(int64_t, int64_t, int);
-int cluster_size(int64_t, int64_t);
-cudaError_t solve_batched_cluster(double *, int64_t, int, int, int, int, int, double *, double *, int32_t *,
-                                  int32_t *, int32_t *, int32_t *, int32_t *, double *, bool, const double *,
-                                  cudaStream_t);
-bool global_fits(int64_t, int64_t, int);
-int global_min_cluster_size(int64_t, int64_t);
-cudaError_t global_cluster_size(int64_t, int64_t, int64_t, int *);
-cudaError_t solve_batched_global(double *, int64_t, int, int, int, int, int, double *, double *, int32_t *,
-                                 int32_t *, int32_t *, int32_t *, int32_t *, double *, bool, const double *,
-                                 cudaStream_t);
-int64_t ragged_batched_bytes(int, int, int *);
-int ragged_cta_threads(int64_t);
-int ragged_warps_per_cta(int64_t, int64_t);
-int64_t ragged_cluster_bytes(int, int, int);
-cudaError_t solve_ragged_batched(const spx::RaggedLaunch &, const spx::RaggedLp *, const int32_t *, double *, int,
-                                 double *, double *, int32_t *, int32_t *, int32_t *, int32_t *, int32_t *, double *,
-                                 bool, const double *, cudaStream_t);
-cudaError_t solve_ragged_cluster(const spx::RaggedLaunch &, const spx::RaggedLp *, const int32_t *, double *, int,
-                                 double *, double *, int32_t *, int32_t *, int32_t *, int32_t *, int32_t *, double *,
-                                 bool, const double *, cudaStream_t);
-int64_t ragged_global_bytes(int, int, int);
-cudaError_t ragged_global_size(const spx::RaggedLaunch &, const spx::RaggedLp *, const int32_t *, int *, int64_t *);
-cudaError_t solve_ragged_global(const spx::RaggedLaunch &, int, int64_t, const spx::RaggedLp *, const int32_t *,
-                                double *, int, double *, double *, int32_t *, int32_t *, int32_t *, int32_t *,
-                                int32_t *, double *, bool, const double *, cudaStream_t);
-cudaError_t sensitivity_uniform(const double *, int64_t, int, int, const int32_t *, const int32_t *, const int32_t *,
-                                double *, double *, double *, double *, double *, cudaStream_t);
-cudaError_t sensitivity_ragged(const spx::RaggedPlan *, const spx::RaggedLp *, const int32_t *, const double *,
-                               const spx::RaggedLp *, const int32_t *, const int32_t *, const int32_t *,
-                               const int32_t *, double *, double *, double *, double *, double *, cudaStream_t);
-cudaError_t sensitivity_split(const double *, const double *, int, int, int64_t, int, const int32_t *, const int32_t *,
-                              double *, double *, double *, double *, double *, cudaStream_t);
-cudaError_t warm_change_uniform(double *, int64_t, int, int, const int32_t *, const int32_t *, const double *,
-                                const double *, cudaStream_t);
-cudaError_t warm_change_ragged(const spx::RaggedPlan *, const spx::RaggedLp *, const int32_t *, double *,
-                               const spx::RaggedLp *, const int32_t *, const int32_t *, const int32_t *, const double *,
-                               const double *, cudaStream_t);
-} // namespace spx_launch
+#include "spx_launch.cuh"
 
 namespace spx_host {
 
@@ -239,19 +160,18 @@ int check_cluster_launch(cudaError_t e, const char *who, int S, int64_t smem) {
     return -1;
 }
 
-// One uniform solve (warm == false) or resume (warm == true) on the engine route_lp gives `engine`: the body of
+// One uniform solve (io.warm == false) or resume (io.warm == true) on the engine route_lp gives `engine`: the body of
 // spx_solve_batched, spx_solve_batched_cluster, spx_solve_batched_global and spx_warm_solve_batched.  K4 reads no
 // forced cluster size; K7 and K8 check the grid limit, and K8 launches at spx_global_cluster_size.
-int solve_uniform(const char *who, int engine, bool warm, double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule,
-                  int32_t max_pivots, const double *d_function, double *d_x, double *d_obj, int32_t *d_status,
-                  int32_t *d_npiv, int32_t *d_rowlab, int32_t *d_collab, int32_t *d_trace, double *d_snap,
-                  void *stream) {
+int solve_uniform(const char *who, int engine, int64_t B, int32_t n, int32_t m, int32_t max_pivots,
+                  const spx::BatchIO &io, void *stream) {
     SPX_REQUIRE(known_engine(engine), "%s: unknown engine %d", who, engine);
     SPX_REQUIRE(B >= 0 && n >= 1 && m >= 1 && max_pivots >= 0, "%s: bad arguments", who);
-    SPX_REQUIRE(B == 0 || (d_T && d_status && d_npiv), "%s: null T/status/npiv", who);
-    SPX_REQUIRE(!warm || B == 0 || (d_rowlab && d_collab), "%s: null rowlab/collab (the labels to resume from)", who);
-    SPX_REQUIRE(!warm || B == 0 || !d_obj || d_function, "%s: null function with obj", who);
-    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "%s: unknown rule %d", who, rule);
+    SPX_REQUIRE(B == 0 || (io.T && io.status && io.npiv), "%s: null T/status/npiv", who);
+    SPX_REQUIRE(!io.warm || B == 0 || (io.rowlab && io.collab), "%s: null rowlab/collab (the labels to resume from)",
+                who);
+    SPX_REQUIRE(!io.warm || B == 0 || !io.obj || io.function, "%s: null function with obj", who);
+    SPX_REQUIRE(io.rule == SPX_RULE_REFERENCE || io.rule == SPX_RULE_DANTZIG, "%s: unknown rule %d", who, io.rule);
     Route r;
     if (!route_lp(n, m, engine, forced_cluster_size(), &r)) {
         prefix_error("%s: ", who);
@@ -259,25 +179,19 @@ int solve_uniform(const char *who, int engine, bool warm, double *d_T, int64_t B
     }
     cudaStream_t s = as_stream(stream);
     if (r.kernel == spx::RAGGED_WARP || r.kernel == spx::RAGGED_CTA)
-        return check(spx_launch::solve_batched(d_T, B, n, m, rule, max_pivots, d_x, d_obj, d_status, d_npiv, d_rowlab,
-                                               d_collab, d_trace, d_snap, warm, d_function, s),
-                     "batched launch");
+        return check(spx_launch::solve_batched(B, n, m, max_pivots, io, s), "batched launch");
     // K8: a default S above S_min is only chosen when all B clusters are co-resident, far below the grid limit
     SPX_REQUIRE(B <= INT32_MAX / r.S, "%s: B = %lld LPs x S = %d CTAs exceed one grid", who, (long long)B, r.S);
     if (r.kernel == spx::RAGGED_CLUSTER)
-        return check_cluster_launch(spx_launch::solve_batched_cluster(d_T, B, n, m, r.S, rule, max_pivots, d_x, d_obj,
-                                                                      d_status, d_npiv, d_rowlab, d_collab, d_trace,
-                                                                      d_snap, warm, d_function, s),
-                                    who, r.S, r.bytes);
+        return check_cluster_launch(spx_launch::solve_batched_cluster(B, n, m, r.S, max_pivots, io, s), who, r.S,
+                                    r.bytes);
     if (B == 0) return 0;
     int S = 0;
     char what[96];
     snprintf(what, sizeof(what), "%s: occupancy", who);
     if (check(spx_launch::global_cluster_size(n, m, B, &S), what)) return -1;
-    return check_cluster_launch(spx_launch::solve_batched_global(d_T, B, n, m, S, rule, max_pivots, d_x, d_obj,
-                                                                 d_status, d_npiv, d_rowlab, d_collab, d_trace,
-                                                                 d_snap, warm, d_function, s),
-                                who, S, spx_launch::ragged_global_bytes(n, m, S));
+    return check_cluster_launch(spx_launch::solve_batched_global(B, n, m, S, max_pivots, io, s), who, S,
+                                spx_launch::ragged_global_bytes(n, m, S));
 }
 
 } // namespace
@@ -732,8 +646,9 @@ int32_t spx_batched_fits(int32_t n, int32_t m) { return spx_launch::batched_fits
 int spx_solve_batched(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule, int32_t max_pivots,
                       double *d_x, double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab,
                       int32_t *d_collab, int32_t *d_trace, double *d_snap, void *stream) {
-    return solve_uniform("spx_solve_batched", SPX_ENGINE_SMEM, false, d_T, B, n, m, rule, max_pivots, nullptr, d_x,
-                         d_obj, d_status, d_npiv, d_rowlab, d_collab, d_trace, d_snap, stream);
+    return solve_uniform("spx_solve_batched", SPX_ENGINE_SMEM, B, n, m, max_pivots,
+                         {d_T, nullptr, d_x, d_obj, d_status, d_npiv, d_rowlab, d_collab, d_trace, d_snap, rule, false},
+                         stream);
 }
 
 // ---- K7 -------------------------------------------------------------------------
@@ -742,8 +657,9 @@ int32_t spx_cluster_size(int32_t n, int32_t m) { return spx_launch::cluster_size
 int spx_solve_batched_cluster(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule, int32_t max_pivots,
                               double *d_x, double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab,
                               int32_t *d_collab, int32_t *d_trace, double *d_snap, void *stream) {
-    return solve_uniform("spx_solve_batched_cluster", SPX_ENGINE_CLUSTER, false, d_T, B, n, m, rule, max_pivots,
-                         nullptr, d_x, d_obj, d_status, d_npiv, d_rowlab, d_collab, d_trace, d_snap, stream);
+    return solve_uniform("spx_solve_batched_cluster", SPX_ENGINE_CLUSTER, B, n, m, max_pivots,
+                         {d_T, nullptr, d_x, d_obj, d_status, d_npiv, d_rowlab, d_collab, d_trace, d_snap, rule, false},
+                         stream);
 }
 
 // ---- K8 -------------------------------------------------------------------------
@@ -758,8 +674,9 @@ int32_t spx_global_cluster_size(int32_t n, int32_t m, int64_t B) {
 int spx_solve_batched_global(double *d_T, int64_t B, int32_t n, int32_t m, int32_t rule, int32_t max_pivots,
                              double *d_x, double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab,
                              int32_t *d_collab, int32_t *d_trace, double *d_snap, void *stream) {
-    return solve_uniform("spx_solve_batched_global", SPX_ENGINE_GLOBAL, false, d_T, B, n, m, rule, max_pivots,
-                         nullptr, d_x, d_obj, d_status, d_npiv, d_rowlab, d_collab, d_trace, d_snap, stream);
+    return solve_uniform("spx_solve_batched_global", SPX_ENGINE_GLOBAL, B, n, m, max_pivots,
+                         {d_T, nullptr, d_x, d_obj, d_status, d_npiv, d_rowlab, d_collab, d_trace, d_snap, rule, false},
+                         stream);
 }
 
 // ---- ragged batches (K4 + K7 + K8) ---------------------------------------------------
@@ -873,68 +790,63 @@ static bool ragged_header_sane(const spx::RaggedPlan *P) {
     return sane && counted == P->B;
 }
 
-// The plan header of `who`'s h_plan, checked: magic, ABI version and launch list
-static const spx::RaggedPlan *checked_plan(const char *who, const void *h_plan) {
+// The plan `who` was given, checked (magic, ABI version and launch list), as a view of its host copy h_plan and of its
+// device copy d_plan (null: the view's device arrays are null); false, with the error set, when it is not a plan
+static bool checked_plan(const char *who, const void *h_plan, const void *d_plan, spx::PlanView *v) {
     using namespace spx;
     if (!h_plan) {
         set_error("%s: null plan", who);
-        return nullptr;
+        return false;
     }
     const RaggedPlan *P = static_cast<const RaggedPlan *>(h_plan);
     if (P->magic != RAGGED_MAGIC || P->abi != SPX_ABI_VERSION) {
         set_error("%s: h_plan is not a plan of this library (magic / ABI version mismatch)", who);
-        return nullptr;
+        return false;
     }
     if (!ragged_header_sane(P)) {
         set_error("%s: inconsistent plan header (B = %lld)", who, (long long)P->B);
-        return nullptr;
+        return false;
     }
-    return P;
+    auto at = [](const void *plan, int64_t offset) {
+        return plan ? static_cast<const char *>(plan) + offset : nullptr;
+    };
+    *v = PlanView{P, reinterpret_cast<const RaggedLp *>(at(h_plan, P->lp_offset)),
+                  reinterpret_cast<const int32_t *>(at(h_plan, P->order_offset)),
+                  reinterpret_cast<const RaggedLp *>(at(d_plan, P->lp_offset)),
+                  reinterpret_cast<const int32_t *>(at(d_plan, P->order_offset))};
+    return true;
 }
 
-// One ragged solve (warm == false) or resume (warm == true): the body of spx_solve_batched_ragged and
+// One ragged solve (io.warm == false) or resume (io.warm == true): the body of spx_solve_batched_ragged and
 // spx_warm_solve_ragged
-static int solve_ragged(const char *who, bool warm, double *d_T, const void *h_plan, const void *d_plan, int32_t rule,
-                        const double *d_function, double *d_x, double *d_obj, int32_t *d_status, int32_t *d_npiv,
-                        int32_t *d_rowlab, int32_t *d_collab, int32_t *d_trace, double *d_snap, void *stream) {
+static int solve_ragged(const char *who, const void *h_plan, const void *d_plan, const spx::BatchIO &io,
+                        void *stream) {
     using namespace spx;
-    const RaggedPlan *P = checked_plan(who, h_plan);
-    if (!P) return -2;
-    if (P->B == 0) return 0;
-    SPX_REQUIRE(d_plan && d_T && d_status && d_npiv, "%s: null d_plan/T/status/npiv", who);
-    SPX_REQUIRE(!warm || (d_rowlab && d_collab), "%s: null rowlab/collab (the labels to resume from)", who);
-    SPX_REQUIRE(!warm || !d_obj || d_function, "%s: null function with obj", who);
-    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "%s: unknown rule %d", who, rule);
-    const RaggedLp *lps = reinterpret_cast<const RaggedLp *>(static_cast<const char *>(d_plan) + P->lp_offset);
-    const int32_t *order = reinterpret_cast<const int32_t *>(static_cast<const char *>(d_plan) + P->order_offset);
-    const RaggedLp *h_lps = reinterpret_cast<const RaggedLp *>(static_cast<const char *>(h_plan) + P->lp_offset);
-    const int32_t *h_order = reinterpret_cast<const int32_t *>(static_cast<const char *>(h_plan) + P->order_offset);
+    PlanView v;
+    if (!checked_plan(who, h_plan, d_plan, &v)) return -2;
+    if (v.P->B == 0) return 0;
+    SPX_REQUIRE(d_plan && io.T && io.status && io.npiv, "%s: null d_plan/T/status/npiv", who);
+    SPX_REQUIRE(!io.warm || (io.rowlab && io.collab), "%s: null rowlab/collab (the labels to resume from)", who);
+    SPX_REQUIRE(!io.warm || !io.obj || io.function, "%s: null function with obj", who);
+    SPX_REQUIRE(io.rule == SPX_RULE_REFERENCE || io.rule == SPX_RULE_DANTZIG, "%s: unknown rule %d", who, io.rule);
     cudaStream_t s = as_stream(stream);
     char what[96];
-    for (int i = 0; i < P->nlaunch; ++i) {
-        const RaggedLaunch &l = P->launch[i];
+    for (int i = 0; i < v.P->nlaunch; ++i) {
+        const RaggedLaunch &l = v.P->launch[i];
         if (l.kernel == RAGGED_GLOBAL) {
             int S = 0;
             int64_t smem = 0;
             snprintf(what, sizeof(what), "%s: occupancy", who);
-            if (check(spx_launch::ragged_global_size(l, h_lps, h_order, &S, &smem), what))
+            if (check(spx_launch::ragged_global_size(v, l, &S, &smem), what))
                 return -1;
             SPX_REQUIRE(l.count <= INT32_MAX / S, "%s: %lld LPs x S = %d CTAs exceed one grid", who,
                         (long long)l.count, S);
-            if (check_cluster_launch(spx_launch::solve_ragged_global(l, S, smem, lps, order, d_T, rule, d_x, d_obj,
-                                                                     d_status, d_npiv, d_rowlab, d_collab, d_trace,
-                                                                     d_snap, warm, d_function, s),
-                                     who, S, smem))
+            if (check_cluster_launch(spx_launch::solve_ragged_global(v, l, S, smem, io, s), who, S, smem))
                 return -1;
         } else if (l.kernel == RAGGED_CLUSTER) {
-            if (check_cluster_launch(spx_launch::solve_ragged_cluster(l, lps, order, d_T, rule, d_x, d_obj, d_status,
-                                                                      d_npiv, d_rowlab, d_collab, d_trace, d_snap,
-                                                                      warm, d_function, s),
-                                     who, l.S, l.smem))
+            if (check_cluster_launch(spx_launch::solve_ragged_cluster(v, l, io, s), who, l.S, l.smem))
                 return -1;
-        } else if (check(spx_launch::solve_ragged_batched(l, lps, order, d_T, rule, d_x, d_obj, d_status, d_npiv,
-                                                            d_rowlab, d_collab, d_trace, d_snap, warm, d_function, s),
-                         "ragged batched launch")) {
+        } else if (check(spx_launch::solve_ragged_batched(v, l, io, s), "ragged batched launch")) {
             return -1;
         }
     }
@@ -944,28 +856,23 @@ static int solve_ragged(const char *who, bool warm, double *d_T, const void *h_p
 int spx_solve_batched_ragged(double *d_T, const void *h_plan, const void *d_plan, int32_t rule, double *d_x,
                              double *d_obj, int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab, int32_t *d_collab,
                              int32_t *d_trace, double *d_snap, void *stream) {
-    return solve_ragged("spx_solve_batched_ragged", false, d_T, h_plan, d_plan, rule, nullptr, d_x, d_obj, d_status,
-                        d_npiv, d_rowlab, d_collab, d_trace, d_snap, stream);
+    return solve_ragged("spx_solve_batched_ragged", h_plan, d_plan,
+                        {d_T, nullptr, d_x, d_obj, d_status, d_npiv, d_rowlab, d_collab, d_trace, d_snap, rule, false},
+                        stream);
 }
 
 int32_t spx_ragged_cluster_size(const void *h_plan, int32_t launch) {
-    using namespace spx;
-    const RaggedPlan *P = static_cast<const RaggedPlan *>(h_plan);
-    if (!P || P->magic != RAGGED_MAGIC || P->abi != SPX_ABI_VERSION) {
-        set_error("spx_ragged_cluster_size: h_plan is not a plan of this library (null, or magic / ABI version mismatch)");
+    spx::PlanView v;
+    if (!checked_plan("spx_ragged_cluster_size", h_plan, nullptr, &v)) return -1;
+    if (launch < 0 || launch >= v.P->nlaunch) {
+        set_error("spx_ragged_cluster_size: launch %d of a plan of %d launches", launch, v.P->nlaunch);
         return -1;
     }
-    if (launch < 0 || launch >= P->nlaunch || P->nlaunch > RAGGED_MAX_LAUNCHES) {
-        set_error("spx_ragged_cluster_size: launch %d of a plan of %d launches", launch, P->nlaunch);
-        return -1;
-    }
-    const RaggedLaunch &l = P->launch[launch];
-    if (l.kernel != RAGGED_GLOBAL) return l.S;
-    const RaggedLp *h_lps = reinterpret_cast<const RaggedLp *>(static_cast<const char *>(h_plan) + P->lp_offset);
-    const int32_t *h_order = reinterpret_cast<const int32_t *>(static_cast<const char *>(h_plan) + P->order_offset);
+    const spx::RaggedLaunch &l = v.P->launch[launch];
+    if (l.kernel != spx::RAGGED_GLOBAL) return l.S;
     int S = 0;
     int64_t smem = 0;
-    if (check(spx_launch::ragged_global_size(l, h_lps, h_order, &S, &smem), "spx_ragged_cluster_size")) return -1;
+    if (check(spx_launch::ragged_global_size(v, l, &S, &smem), "spx_ragged_cluster_size")) return -1;
     return S;
 }
 
@@ -985,22 +892,13 @@ int spx_sensitivity_batched(const double *d_T, int64_t B, int32_t n, int32_t m, 
 int spx_sensitivity_ragged(const double *d_T, const void *h_plan, const void *d_plan, const int32_t *d_status,
                            const int32_t *d_rowlab, const int32_t *d_collab, double *d_dual, double *d_slack,
                            double *d_redcost, double *d_rhs_range, double *d_cost_range, void *stream) {
-    using namespace spx;
-    SPX_REQUIRE(h_plan, "spx_sensitivity_ragged: null plan");
-    const RaggedPlan *P = static_cast<const RaggedPlan *>(h_plan);
-    SPX_REQUIRE(P->magic == RAGGED_MAGIC && P->abi == SPX_ABI_VERSION,
-                "spx_sensitivity_ragged: h_plan is not a plan of this library (magic / ABI version mismatch)");
-    SPX_REQUIRE(ragged_header_sane(P), "spx_sensitivity_ragged: inconsistent plan header (B = %lld)", (long long)P->B);
-    if (P->B == 0) return 0;
+    spx::PlanView v;
+    if (!checked_plan("spx_sensitivity_ragged", h_plan, d_plan, &v)) return -2;
+    if (v.P->B == 0) return 0;
     SPX_REQUIRE(d_plan && d_T && d_status && d_rowlab && d_collab,
                 "spx_sensitivity_ragged: null d_plan/T/status/rowlab/collab");
-    const char *h = static_cast<const char *>(h_plan), *d = static_cast<const char *>(d_plan);
-    return check(spx_launch::sensitivity_ragged(P, reinterpret_cast<const RaggedLp *>(h + P->lp_offset),
-                                                reinterpret_cast<const int32_t *>(h + P->order_offset), d_T,
-                                                reinterpret_cast<const RaggedLp *>(d + P->lp_offset),
-                                                reinterpret_cast<const int32_t *>(d + P->order_offset), d_status,
-                                                d_rowlab, d_collab, d_dual, d_slack, d_redcost, d_rhs_range,
-                                                d_cost_range, as_stream(stream)),
+    return check(spx_launch::sensitivity_ragged(v, d_T, d_status, d_rowlab, d_collab, d_dual, d_slack, d_redcost,
+                                                d_rhs_range, d_cost_range, as_stream(stream)),
                  "ragged sensitivity launch");
 }
 
@@ -1042,17 +940,11 @@ int spx_warm_change_batched(double *d_T, int64_t B, int32_t n, int32_t m, const 
 
 int spx_warm_change_ragged(double *d_T, const void *h_plan, const void *d_plan, const int32_t *d_rowlab,
                            const int32_t *d_collab, const double *d_delta_b, const double *d_delta_c, void *stream) {
-    using namespace spx;
-    const RaggedPlan *P = checked_plan("spx_warm_change_ragged", h_plan);
-    if (!P) return -2;
-    if (P->B == 0 || (!d_delta_b && !d_delta_c)) return 0;
+    spx::PlanView v;
+    if (!checked_plan("spx_warm_change_ragged", h_plan, d_plan, &v)) return -2;
+    if (v.P->B == 0 || (!d_delta_b && !d_delta_c)) return 0;
     SPX_REQUIRE(d_plan && d_T && d_rowlab && d_collab, "spx_warm_change_ragged: null d_plan/T/rowlab/collab");
-    const char *h = static_cast<const char *>(h_plan), *d = static_cast<const char *>(d_plan);
-    return check(spx_launch::warm_change_ragged(P, reinterpret_cast<const RaggedLp *>(h + P->lp_offset),
-                                                reinterpret_cast<const int32_t *>(h + P->order_offset), d_T,
-                                                reinterpret_cast<const RaggedLp *>(d + P->lp_offset),
-                                                reinterpret_cast<const int32_t *>(d + P->order_offset), d_rowlab,
-                                                d_collab, d_delta_b, d_delta_c, as_stream(stream)),
+    return check(spx_launch::warm_change_ragged(v, d_T, d_rowlab, d_collab, d_delta_b, d_delta_c, as_stream(stream)),
                  "ragged warm change launch");
 }
 
@@ -1060,16 +952,18 @@ int spx_warm_solve_batched(int32_t engine, double *d_T, int64_t B, int32_t n, in
                            int32_t max_pivots, const double *d_function, double *d_x, double *d_obj,
                            int32_t *d_status, int32_t *d_npiv, int32_t *d_rowlab, int32_t *d_collab,
                            int32_t *d_trace, double *d_snap, void *stream) {
-    return solve_uniform("spx_warm_solve_batched", engine, true, d_T, B, n, m, rule, max_pivots, d_function, d_x,
-                         d_obj, d_status, d_npiv, d_rowlab, d_collab, d_trace, d_snap, stream);
+    return solve_uniform("spx_warm_solve_batched", engine, B, n, m, max_pivots,
+                         {d_T, d_function, d_x, d_obj, d_status, d_npiv, d_rowlab, d_collab, d_trace, d_snap, rule, true},
+                         stream);
 }
 
 int spx_warm_solve_ragged(double *d_T, const void *h_plan, const void *d_plan, int32_t rule,
                           const double *d_function, double *d_x, double *d_obj, int32_t *d_status,
                           int32_t *d_npiv, int32_t *d_rowlab, int32_t *d_collab, int32_t *d_trace,
                           double *d_snap, void *stream) {
-    return solve_ragged("spx_warm_solve_ragged", true, d_T, h_plan, d_plan, rule, d_function, d_x, d_obj, d_status,
-                        d_npiv, d_rowlab, d_collab, d_trace, d_snap, stream);
+    return solve_ragged("spx_warm_solve_ragged", h_plan, d_plan,
+                        {d_T, d_function, d_x, d_obj, d_status, d_npiv, d_rowlab, d_collab, d_trace, d_snap, rule, true},
+                        stream);
 }
 
 // ---- column-sharded flow ----------------------------------------------------------

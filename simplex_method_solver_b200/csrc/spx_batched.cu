@@ -12,7 +12,7 @@
 //       barriers per pivot.
 // The four cell kinds of the pivot differ only in the numerator, so one division by the pivot
 // (pivot_div, reciprocal hoisted) serves them all without divergence.
-#include "spx_common.cuh"
+#include "spx_launch.cuh"
 
 namespace {
 
@@ -455,23 +455,29 @@ size_t lut_bytes(int n, int m) {
     return (cells * 4 + 15) / 16 * 16;
 }
 
-// Sets the dynamic shared-memory limit of a K4 kernel to K4_DYN_LIMIT once per device, after checking that its static
-// bytes are the K4_STATIC the capacity rule reserves.  A failure is returned once: the runtime's last error is cleared,
-// so that the next launch's cudaGetLastError() does not report it again.
-template <class K>
-cudaError_t configure_k4(K kernel, size_t &configured) {
-    if (configured) return cudaSuccess;
-    cudaFuncAttributes fa;
-    cudaError_t e = cudaFuncGetAttributes(&fa, kernel);
-    if (e == cudaSuccess && fa.sharedSizeBytes > K4_STATIC) return cudaErrorInvalidValue;
-    if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K4_DYN_LIMIT);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        return e;
+// Kernel<<<grid, threads, smem, stream>>>(args...), counted.  Above 48 KB of dynamic shared memory the kernel's limit
+// is first set to K4_DYN_LIMIT, once per device, after checking that its static bytes are the K4_STATIC the capacity
+// rule reserves.  A failure of that set-up is returned once: the runtime's last error is cleared, so that the next
+// launch's cudaGetLastError() does not report it again.
+template <auto Kernel, typename... Args>
+cudaError_t launch_k4(int64_t grid, int threads, size_t smem, cudaStream_t stream, Args... args) {
+    static bool configured_dev[64] = {};
+    bool &configured = configured_dev[spx_host::device_slot()];
+    if (smem > 48 * 1024 && !configured) {
+        cudaFuncAttributes fa;
+        cudaError_t e = cudaFuncGetAttributes(&fa, Kernel);
+        if (e == cudaSuccess && fa.sharedSizeBytes > K4_STATIC) return cudaErrorInvalidValue;
+        if (e == cudaSuccess)
+            e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K4_DYN_LIMIT);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            return e;
+        }
+        configured = true;
     }
-    configured = K4_DYN_LIMIT;
-    return cudaSuccess;
+    Kernel<<<(unsigned)grid, threads, smem, stream>>>(args...);
+    spx_host::count_launch();
+    return cudaGetLastError();
 }
 
 } // namespace
@@ -489,35 +495,22 @@ bool batched_fits(int n, int m) {
     return cells <= CTA_MODE_MIN_CELLS || lut_bytes(n, m) + warp_bytes(n, m) <= K4_DYN_LIMIT;
 }
 
-// returns cudaErrorInvalidValue when one LP does not fit shared memory; warm: the resume (batched_warm_kernel)
-cudaError_t solve_batched(double *T, int64_t B, int n, int m, int rule, int max_pivots, double *x,
-                          double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab,
-                          int32_t *collab, int32_t *trace, double *snap, bool warm, const double *function,
-                          cudaStream_t stream) {
+// returns cudaErrorInvalidValue when one LP does not fit shared memory; io.warm: the resume (batched_warm_kernel)
+cudaError_t solve_batched(int64_t B, int n, int m, int max_pivots, const BatchIO &io, cudaStream_t stream) {
     if (B <= 0) return cudaSuccess;
     if (!batched_fits(n, m)) return cudaErrorInvalidValue;
     const size_t wb = warp_bytes(n, m), lb = lut_bytes(n, m);
+    const int wd = (int)(wb / sizeof(double));
     const int64_t cells = (int64_t)n * (m + 1) + m;
-    BatchedArgs a{T, B, n, m, rule, max_pivots, x, obj, status, npiv, rowlab, collab, trace, snap};
-    static size_t configured_dev[64][4] = {};
-    size_t *configured = configured_dev[spx_host::device_slot()];
+    const BatchedArgs a{io.T, B, n, m, io.rule, max_pivots, io.x, io.obj, io.status, io.npiv, io.rowlab, io.collab,
+                        io.trace, io.snap};
     if (cells > CTA_MODE_MIN_CELLS) {
         // one CTA per LP: one cell per thread where possible (measured on Klee-Minty n=20: 32 cells per warp
         // 891 k pivots/s, 64: 730 k, 128: 623 k), 2..16 warps
         int warps = (int)((cells + CTA_CELLS_PER_WARP - 1) / CTA_CELLS_PER_WARP);
         warps = warps < 2 ? 2 : (warps > 16 ? 16 : warps);
-        const size_t smem = lb + wb;
-        if (smem > 48 * 1024) {
-            const cudaError_t e = warm ? configure_k4(batched_warm_kernel<true>, configured[3])
-                                       : configure_k4(batched_kernel<true>, configured[1]);
-            if (e != cudaSuccess) return e;
-        }
-        if (warm)
-            batched_warm_kernel<true><<<(unsigned)B, warps * 32, smem, stream>>>(a, function, 1, (int)(wb / sizeof(double)));
-        else
-            batched_kernel<true><<<(unsigned)B, warps * 32, smem, stream>>>(a, 1, (int)(wb / sizeof(double)));
-        spx_host::count_launch();
-        return cudaGetLastError();
+        if (io.warm) return launch_k4<batched_warm_kernel<true>>(B, warps * 32, lb + wb, stream, a, io.function, 1, wd);
+        return launch_k4<batched_kernel<true>>(B, warps * 32, lb + wb, stream, a, 1, wd);
     }
     // warps per CTA: as many as fit ~48 KB (several CTAs per SM), at most 8, at least 1
     int wpc = (int)((48 * 1024 - lb) / wb);
@@ -526,18 +519,9 @@ cudaError_t solve_batched(double *T, int64_t B, int n, int m, int rule, int max_
     if (wpc < 1) wpc = 1;
     if ((int64_t)wpc > B) wpc = (int)B;
     const size_t smem = lb + (size_t)wpc * wb;
-    if (smem > 48 * 1024) {
-        const cudaError_t e = warm ? configure_k4(batched_warm_kernel<false>, configured[2])
-                                   : configure_k4(batched_kernel<false>, configured[0]);
-        if (e != cudaSuccess) return e;
-    }
     const int64_t ctas = (B + wpc - 1) / wpc;
-    if (warm)
-        batched_warm_kernel<false><<<(unsigned)ctas, wpc * 32, smem, stream>>>(a, function, wpc, (int)(wb / sizeof(double)));
-    else
-        batched_kernel<false><<<(unsigned)ctas, wpc * 32, smem, stream>>>(a, wpc, (int)(wb / sizeof(double)));
-    spx_host::count_launch();
-    return cudaGetLastError();
+    if (io.warm) return launch_k4<batched_warm_kernel<false>>(ctas, wpc * 32, smem, stream, a, io.function, wpc, wd);
+    return launch_k4<batched_kernel<false>>(ctas, wpc * 32, smem, stream, a, wpc, wd);
 }
 
 // ---- ragged batches: the plan's numbers for K4 ----
@@ -562,37 +546,22 @@ int ragged_warps_per_cta(int64_t slot, int64_t count) {
     return (int)(wpc > count ? count : wpc);
 }
 
-cudaError_t solve_ragged_batched(const RaggedLaunch &l, const RaggedLp *lps, const int32_t *order, double *T, int rule,
-                                 double *x, double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab,
-                                 int32_t *collab, int32_t *trace, double *snap, bool warm, const double *function,
-                                 cudaStream_t stream) {
+cudaError_t solve_ragged_batched(const PlanView &v, const RaggedLaunch &l, const BatchIO &io, cudaStream_t stream) {
     if (l.count <= 0) return cudaSuccess;
-    BatchedArgs a{T, l.count, 0, 0, rule, 0, x, obj, status, npiv, rowlab, collab, trace, snap};
-    static size_t configured_dev[64][4] = {};
-    size_t *configured = configured_dev[spx_host::device_slot()];
-    const bool cta = (l.kernel == RAGGED_CTA);
-    if (l.smem > 48 * 1024) {
-        const cudaError_t e = warm ? (cta ? configure_k4(ragged_batched_warm_kernel<true>, configured[3])
-                                          : configure_k4(ragged_batched_warm_kernel<false>, configured[2]))
-                                   : (cta ? configure_k4(ragged_batched_kernel<true>, configured[1])
-                                          : configure_k4(ragged_batched_kernel<false>, configured[0]));
-        if (e != cudaSuccess) return e;
-    }
+    const BatchedArgs a{io.T, l.count, 0, 0, io.rule, 0, io.x, io.obj, io.status, io.npiv, io.rowlab, io.collab,
+                        io.trace, io.snap};
     const int64_t ctas = (l.count + l.per_cta - 1) / l.per_cta;
-    const int per_cta = cta ? 1 : l.per_cta, slot_doubles = cta ? 0 : (int)l.slot_doubles;
-    if (warm && cta)
-        ragged_batched_warm_kernel<true><<<(unsigned)ctas, l.threads, (size_t)l.smem, stream>>>(
-            a, lps, order + l.first, per_cta, slot_doubles, function);
-    else if (warm)
-        ragged_batched_warm_kernel<false><<<(unsigned)ctas, l.threads, (size_t)l.smem, stream>>>(
-            a, lps, order + l.first, per_cta, slot_doubles, function);
-    else if (cta)
-        ragged_batched_kernel<true><<<(unsigned)ctas, l.threads, (size_t)l.smem, stream>>>(a, lps, order + l.first, 1, 0);
-    else
-        ragged_batched_kernel<false><<<(unsigned)ctas, l.threads, (size_t)l.smem, stream>>>(a, lps, order + l.first,
-                                                                                        l.per_cta, (int)l.slot_doubles);
-    spx_host::count_launch();
-    return cudaGetLastError();
+    const size_t smem = (size_t)l.smem;
+    const int32_t *order = v.d_order + l.first;
+    if (l.kernel == RAGGED_CTA)
+        return io.warm ? launch_k4<ragged_batched_warm_kernel<true>>(ctas, l.threads, smem, stream, a, v.d_lps, order,
+                                                                     1, 0, io.function)
+                       : launch_k4<ragged_batched_kernel<true>>(ctas, l.threads, smem, stream, a, v.d_lps, order, 1, 0);
+    const int wd = (int)l.slot_doubles;
+    return io.warm ? launch_k4<ragged_batched_warm_kernel<false>>(ctas, l.threads, smem, stream, a, v.d_lps, order,
+                                                                  l.per_cta, wd, io.function)
+                   : launch_k4<ragged_batched_kernel<false>>(ctas, l.threads, smem, stream, a, v.d_lps, order,
+                                                             l.per_cta, wd);
 }
 
 } // namespace spx_launch

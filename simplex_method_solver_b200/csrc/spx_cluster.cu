@@ -36,21 +36,6 @@ namespace {
 
 using namespace spx;
 
-struct ClusterArgs {
-    double  *T;          // [B][cells] in/out
-    int64_t  B;
-    int      n, m, rule, max_pivots;
-    int      S, R, Q;    // CTAs per LP, body rows per CTA, header labels per CTA
-    double  *x;          // [B][m] or null
-    double  *obj;        // [B] or null
-    int32_t *status;     // [B]
-    int32_t *npiv;       // [B]
-    int32_t *rowlab;     // [B][m] or null
-    int32_t *collab;     // [B][n] or null
-    int32_t *trace;      // [B][max_pivots][2] or null
-    double  *snap;       // [B][max_pivots+1][cells] or null
-};
-
 // The body of both kernels.  RAGGED == false: shape, R, Q and offsets from the arguments (one shape per launch).
 // RAGGED == true: LP order[blockIdx.x / S] of a ragged batch, its shape and offsets from lps[], R and Q from its shape.
 // WARM == true: a resume (spx_warm_solve_*): each CTA reads the labels of its band and of its header slice from
@@ -267,13 +252,10 @@ int cluster_size(int64_t n, int64_t m) {
 
 // S CTAs per LP (validated by the caller); returns cudaErrorInvalidClusterSize when the device cannot co-schedule
 // one cluster of this size and footprint
-cudaError_t solve_batched_cluster(double *T, int64_t B, int n, int m, int S, int rule, int max_pivots, double *x,
-                                  double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab, int32_t *collab,
-                                  int32_t *trace, double *snap, bool warm, const double *function,
+cudaError_t solve_batched_cluster(int64_t B, int n, int m, int S, int max_pivots, const BatchIO &io,
                                   cudaStream_t stream) {
-    ClusterArgs a{T, B, n, m, rule, max_pivots, S, (n + S - 1) / S, (m + S - 1) / S,
-                  x, obj, status, npiv, rowlab, collab, trace, snap};
-    if (warm) return launch_cluster_kernel<cluster_warm_kernel>(S, B, cluster_bytes(n, m, S), stream, a, function);
+    const ClusterArgs a = cluster_args(io, B, n, m, S, max_pivots);
+    if (io.warm) return launch_cluster_kernel<cluster_warm_kernel>(S, B, cluster_bytes(n, m, S), stream, a, io.function);
     return launch_cluster_kernel<cluster_kernel>(S, B, cluster_bytes(n, m, S), stream, a);
 }
 
@@ -281,15 +263,13 @@ int64_t ragged_cluster_bytes(int n, int m, int S) { return cluster_bytes(n, m, S
 
 // one launch of a ragged plan: the l.count LPs order[l.first ..] at cluster size l.S, l.smem = the largest footprint
 // among them; cudaErrorInvalidClusterSize when the device cannot co-schedule one such cluster
-cudaError_t solve_ragged_cluster(const RaggedLaunch &l, const RaggedLp *lps, const int32_t *order, double *T, int rule,
-                                 double *x, double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab,
-                                 int32_t *collab, int32_t *trace, double *snap, bool warm, const double *function,
-                                 cudaStream_t stream) {
-    ClusterArgs a{T, l.count, 0, 0, rule, 0, l.S, 0, 0, x, obj, status, npiv, rowlab, collab, trace, snap};
-    if (warm)
-        return launch_cluster_kernel<ragged_cluster_warm_kernel>(l.S, l.count, l.smem, stream, a, lps, order + l.first,
-                                                                 function);
-    return launch_cluster_kernel<ragged_cluster_kernel>(l.S, l.count, l.smem, stream, a, lps, order + l.first);
+cudaError_t solve_ragged_cluster(const PlanView &v, const RaggedLaunch &l, const BatchIO &io, cudaStream_t stream) {
+    const ClusterArgs a = cluster_args(io, l.count, 0, 0, l.S, 0);
+    const int32_t *order = v.d_order + l.first;
+    if (io.warm)
+        return launch_cluster_kernel<ragged_cluster_warm_kernel>(l.S, l.count, l.smem, stream, a, v.d_lps, order,
+                                                                 io.function);
+    return launch_cluster_kernel<ragged_cluster_kernel>(l.S, l.count, l.smem, stream, a, v.d_lps, order);
 }
 
 } // namespace spx_launch

@@ -5,6 +5,7 @@
 #include <cooperative_groups.h>
 
 #include "spx_block.cuh"
+#include "spx_launch.cuh"
 
 namespace spx {
 
@@ -123,3 +124,29 @@ cudaError_t launch_cluster_kernel(int S, int64_t clusters, int64_t smem, cudaStr
 }
 
 } // namespace spx
+
+// The arguments of the K7 and K8 kernels.  They live in the including file's anonymous namespace, with its kernels.
+namespace {
+
+struct ClusterArgs {
+    double  *T;          // [B][cells] in/out
+    int64_t  B;
+    int      n, m, rule, max_pivots;
+    int      S, R, Q;    // CTAs per LP, body rows per CTA, header labels per CTA
+    double  *x;          // [B][m] or null
+    double  *obj;        // [B] or null
+    int32_t *status;     // [B]
+    int32_t *npiv;       // [B]
+    int32_t *rowlab;     // [B][m] or null
+    int32_t *collab;     // [B][n] or null
+    int32_t *trace;      // [B][max_pivots][2] or null
+    double  *snap;       // [B][max_pivots+1][cells] or null
+};
+
+// B LPs of n x m at S CTAs each; a ragged launch passes n = m = max_pivots = 0 (its kernels read each LP's own)
+inline ClusterArgs cluster_args(const spx::BatchIO &io, int64_t B, int n, int m, int S, int max_pivots) {
+    return {io.T, B, n, m, io.rule, max_pivots, S, (n + S - 1) / S, (m + S - 1) / S,
+            io.x, io.obj, io.status, io.npiv, io.rowlab, io.collab, io.trace, io.snap};
+}
+
+} // namespace

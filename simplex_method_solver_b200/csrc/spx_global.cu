@@ -30,8 +30,6 @@
 // in one place, the pivot row (owned by one CTA, read by all); the owner wrote it in the update of the previous
 // pivot, before its arrival at barrier A, whose release/acquire at cluster scope orders it before the read.  Every
 // other read of d_T is of the CTA's own band, ordered by __syncthreads().
-#include <algorithm>
-
 #include "spx_cluster.cuh"
 
 namespace cg = cooperative_groups;
@@ -44,21 +42,6 @@ using namespace spx;
 // leave (spills); six 16-byte loads in flight per thread keep 48 KB per SM in flight for the update
 constexpr int    GLOBAL_MIN_CTAS  = 1;
 constexpr int    GLOBAL_UNROLL    = 6;
-
-struct GlobalArgs {
-    double  *T;          // [B][cells] in/out
-    int64_t  B;
-    int      n, m, rule, max_pivots;
-    int      S, R, Q;    // CTAs per LP, body rows per CTA, header labels per CTA
-    double  *x;          // [B][m] or null
-    double  *obj;        // [B] or null
-    int32_t *status;     // [B]
-    int32_t *npiv;       // [B]
-    int32_t *rowlab;     // [B][m] or null
-    int32_t *collab;     // [B][n] or null
-    int32_t *trace;      // [B][max_pivots][2] or null
-    double  *snap;       // [B][max_pivots+1][cells] or null
-};
 
 __device__ __forceinline__ double ld_l2(const double *p) {
     double v;
@@ -75,7 +58,7 @@ __device__ __forceinline__ double2 ld_l2_v2(const double *p) {
 // RAGGED == true: LP order[blockIdx.x / S] of a ragged batch, its shape and offsets from lps[], R and Q from its shape
 // (as cluster_body in spx_cluster.cu).  WARM == true: a resume, as cluster_body's.
 template <bool RAGGED, bool WARM>
-__device__ __forceinline__ void global_body(const GlobalArgs &a, const RaggedLp *__restrict__ lps,
+__device__ __forceinline__ void global_body(const ClusterArgs &a, const RaggedLp *__restrict__ lps,
                                             const int32_t *__restrict__ order, const double *function) {
     cg::cluster_group cluster = cg::this_cluster();
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -283,24 +266,24 @@ __device__ __forceinline__ void global_body(const GlobalArgs &a, const RaggedLp 
     }
 }
 
-__global__ void __launch_bounds__(CLUSTER_THREADS, GLOBAL_MIN_CTAS) global_kernel(GlobalArgs a) {
+__global__ void __launch_bounds__(CLUSTER_THREADS, GLOBAL_MIN_CTAS) global_kernel(ClusterArgs a) {
     global_body<false, false>(a, nullptr, nullptr, nullptr);
 }
 
 // a ragged batch: the LPs order[0 .. a.B) at one cluster size a.S, each cluster its own shape (a.n, a.m, a.R, a.Q,
 // a.max_pivots unused)
 __global__ void __launch_bounds__(CLUSTER_THREADS, GLOBAL_MIN_CTAS)
-ragged_global_kernel(GlobalArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order) {
+ragged_global_kernel(ClusterArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order) {
     global_body<true, false>(a, lps, order, nullptr);
 }
 
 // the resumes of the two kernels above (spx_warm_solve_*): function [B][m] or packed as x, null without obj
-__global__ void __launch_bounds__(CLUSTER_THREADS, GLOBAL_MIN_CTAS) global_warm_kernel(GlobalArgs a, const double *function) {
+__global__ void __launch_bounds__(CLUSTER_THREADS, GLOBAL_MIN_CTAS) global_warm_kernel(ClusterArgs a, const double *function) {
     global_body<false, true>(a, nullptr, nullptr, function);
 }
 
 __global__ void __launch_bounds__(CLUSTER_THREADS, GLOBAL_MIN_CTAS)
-ragged_global_warm_kernel(GlobalArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
+ragged_global_warm_kernel(ClusterArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
                           const double *function) {
     global_body<true, true>(a, lps, order, function);
 }
@@ -333,21 +316,9 @@ cudaError_t busiest_cluster_size(int s_lo, int64_t count, Bytes bytes, int *S_ou
     return cudaSuccess;
 }
 
-// the largest footprint at S over the LPs of one ragged launch (host copies of the plan's descriptors)
-int64_t launch_bytes(const RaggedLaunch &l, const RaggedLp *lps, const int32_t *order, int S) {
-    int64_t big = 0;
-    for (int64_t q = l.first; q < l.first + l.count; ++q) {
-        const RaggedLp &d = lps[order[q]];
-        big = std::max(big, global_bytes(d.n, d.m, S));
-    }
-    return big;
-}
-
 } // namespace
 
 namespace spx_launch {
-
-int64_t get_option(int key);
 
 bool global_fits(int64_t n, int64_t m, int S) {
     return n >= 1 && m >= 1 && global_bytes(n, m, S) <= (int64_t)CLUSTER_DYN_BYTES;
@@ -376,44 +347,39 @@ cudaError_t global_cluster_size(int64_t n, int64_t m, int64_t B, int *S_out) {
 
 // S CTAs per LP (validated by the caller); returns cudaErrorInvalidClusterSize when the device cannot co-schedule
 // one cluster of this size and footprint
-cudaError_t solve_batched_global(double *T, int64_t B, int n, int m, int S, int rule, int max_pivots, double *x,
-                                 double *obj, int32_t *status, int32_t *npiv, int32_t *rowlab, int32_t *collab,
-                                 int32_t *trace, double *snap, bool warm, const double *function,
+cudaError_t solve_batched_global(int64_t B, int n, int m, int S, int max_pivots, const BatchIO &io,
                                  cudaStream_t stream) {
-    GlobalArgs a{T, B, n, m, rule, max_pivots, S, (n + S - 1) / S, (m + S - 1) / S,
-                 x, obj, status, npiv, rowlab, collab, trace, snap};
-    if (warm) return launch_cluster_kernel<global_warm_kernel>(S, B, global_bytes(n, m, S), stream, a, function);
+    const ClusterArgs a = cluster_args(io, B, n, m, S, max_pivots);
+    if (io.warm) return launch_cluster_kernel<global_warm_kernel>(S, B, global_bytes(n, m, S), stream, a, io.function);
     return launch_cluster_kernel<global_kernel>(S, B, global_bytes(n, m, S), stream, a);
 }
 
 int64_t ragged_global_bytes(int n, int m, int S) { return global_bytes(n, m, S); }
 
 // The S and footprint one K8 launch of a ragged plan runs at on the current device: as planned when l.pick_S == 0
-// (no device needed), else busiest_cluster_size() from the planned S over the launch's largest footprint at each S.
-// h_lps / h_order: the host plan's descriptors.
-cudaError_t ragged_global_size(const RaggedLaunch &l, const RaggedLp *h_lps, const int32_t *h_order, int *S_out,
-                               int64_t *smem_out) {
+// (no device needed), else busiest_cluster_size() from the planned S over the launch's largest footprint at each S
+cudaError_t ragged_global_size(const PlanView &v, const RaggedLaunch &l, int *S_out, int64_t *smem_out) {
+    // the largest footprint at S among the launch's LPs
+    auto bytes = [&](int S) { return launch_max(v, l, [S](const RaggedLp &d) { return global_bytes(d.n, d.m, S); }); };
     *S_out = l.S;
     *smem_out = l.smem;
     if (!l.pick_S) return cudaSuccess;
-    const cudaError_t e = busiest_cluster_size<ragged_global_kernel>(
-        l.S, l.count, [&](int S) { return launch_bytes(l, h_lps, h_order, S); }, S_out);
+    const cudaError_t e = busiest_cluster_size<ragged_global_kernel>(l.S, l.count, bytes, S_out);
     if (e != cudaSuccess) return e;
-    *smem_out = launch_bytes(l, h_lps, h_order, *S_out);
+    *smem_out = bytes(*S_out);
     return cudaSuccess;
 }
 
 // one K8 launch of a ragged plan: the l.count LPs order[l.first ..] at S CTAs each with smem bytes per CTA (from
 // ragged_global_size); cudaErrorInvalidClusterSize when the device cannot co-schedule one such cluster
-cudaError_t solve_ragged_global(const RaggedLaunch &l, int S, int64_t smem, const RaggedLp *lps, const int32_t *order,
-                                double *T, int rule, double *x, double *obj, int32_t *status, int32_t *npiv,
-                                int32_t *rowlab, int32_t *collab, int32_t *trace, double *snap, bool warm,
-                                const double *function, cudaStream_t stream) {
-    GlobalArgs a{T, l.count, 0, 0, rule, 0, S, 0, 0, x, obj, status, npiv, rowlab, collab, trace, snap};
-    if (warm)
-        return launch_cluster_kernel<ragged_global_warm_kernel>(S, l.count, smem, stream, a, lps, order + l.first,
-                                                                function);
-    return launch_cluster_kernel<ragged_global_kernel>(S, l.count, smem, stream, a, lps, order + l.first);
+cudaError_t solve_ragged_global(const PlanView &v, const RaggedLaunch &l, int S, int64_t smem, const BatchIO &io,
+                                cudaStream_t stream) {
+    const ClusterArgs a = cluster_args(io, l.count, 0, 0, S, 0);
+    const int32_t *order = v.d_order + l.first;
+    if (io.warm)
+        return launch_cluster_kernel<ragged_global_warm_kernel>(S, l.count, smem, stream, a, v.d_lps, order,
+                                                                io.function);
+    return launch_cluster_kernel<ragged_global_kernel>(S, l.count, smem, stream, a, v.d_lps, order);
 }
 
 } // namespace spx_launch

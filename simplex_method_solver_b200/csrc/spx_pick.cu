@@ -11,6 +11,7 @@
 // local half of K1 (+ column gather into the all-gather message), `select` is
 // the global half of K1 (min key over ranks) + K2 on the winning column.
 #include "spx_block.cuh"
+#include "spx_launch.cuh"
 
 namespace {
 

@@ -22,6 +22,7 @@
 #include <cstdlib>
 
 #include "spx_block.cuh"
+#include "spx_launch.cuh"
 
 namespace cg = cooperative_groups;
 
@@ -247,8 +248,6 @@ int g_res_grid = -1;     // co-resident CTAs on this device (0: cooperative laun
 } // namespace
 
 namespace spx_launch {
-
-int sm_count();
 
 size_t resident_smem(int n) { return (size_t)(((n + 2) & ~1) + n + 2) * sizeof(double); }
 

@@ -15,7 +15,7 @@
 //                     and both meet the other tiles' in global memory through atomicMin.
 #include <cstdint>
 
-#include "spx_common.cuh"
+#include "spx_launch.cuh"
 
 namespace {
 
@@ -253,22 +253,15 @@ cudaError_t sensitivity_uniform(const double *d_T, int64_t B, int n, int m, cons
 }
 
 // one pair of launches per launch of the plan, so LPs of like size share a grid
-cudaError_t sensitivity_ragged(const spx::RaggedPlan *P, const spx::RaggedLp *h_lps, const int32_t *h_order,
-                               const double *d_T, const spx::RaggedLp *d_lps, const int32_t *d_order,
-                               const int32_t *d_status, const int32_t *d_rowlab, const int32_t *d_collab,
-                               double *dual, double *slack, double *redcost, double *rhs, double *cost,
-                               cudaStream_t s) {
-    for (int q = 0; q < P->nlaunch; ++q) {
-        const spx::RaggedLaunch &l = P->launch[q];
+cudaError_t sensitivity_ragged(const spx::PlanView &v, const double *d_T, const int32_t *d_status,
+                               const int32_t *d_rowlab, const int32_t *d_collab, double *dual, double *slack,
+                               double *redcost, double *rhs, double *cost, cudaStream_t s) {
+    for (int q = 0; q < v.P->nlaunch; ++q) {
+        const spx::RaggedLaunch &l = v.P->launch[q];
         SensJob J = sens_job(SENS_RAGGED, d_status, d_rowlab, d_collab, dual, slack, redcost, rhs, cost);
-        J.T = d_T; J.lps = d_lps; J.order = d_order; J.first = l.first; J.count = l.count;
-        int64_t max_n = 0, max_m = 0;
-        for (int64_t u = l.first; u < l.first + l.count; ++u) {
-            const spx::RaggedLp &d = h_lps[h_order[u]];
-            max_n = d.n > max_n ? d.n : max_n;
-            max_m = d.m > max_m ? d.m : max_m;
-        }
-        const cudaError_t e = sens_launch(J, max_n, max_m, s);
+        J.T = d_T; J.lps = v.d_lps; J.order = v.d_order; J.first = l.first; J.count = l.count;
+        const cudaError_t e = sens_launch(J, spx::launch_max(v, l, [](const spx::RaggedLp &d) { return d.n; }),
+                                          spx::launch_max(v, l, [](const spx::RaggedLp &d) { return d.m; }), s);
         if (e != cudaSuccess) return e;
     }
     return cudaSuccess;

@@ -18,22 +18,7 @@
 #include <cstring>
 #include <new>
 
-#include "spx_common.cuh"
-
-namespace spx_launch {
-int64_t colbuf_doubles(int n);
-int64_t shard_msg_doubles(int n);
-cudaError_t shard_candidate(const double *, const double *, int, int, int64_t, int64_t, int, int,
-                            const spx_state *, double *, cudaStream_t);
-cudaError_t shard_select(const double *, int, const double *, int, int, spx_state *, double *,
-                         const unsigned long long *, unsigned long long, cudaStream_t);
-cudaError_t update(const double *, double *, const double *, double *, int, int, int64_t, int64_t,
-                   spx_state *, const double *, int32_t *, int32_t *, int32_t *, int, cudaStream_t);
-cudaError_t ahead_candidate(const double *, const double *, double *, int, int, int64_t, int64_t, int,
-                            const spx_state *, const double *, double *, cudaStream_t);
-cudaError_t ahead_select(const double *, int, const double *, int, const spx_state *, spx_state *,
-                         double *, const unsigned long long *, unsigned long long, cudaStream_t);
-} // namespace spx_launch
+#include "spx_launch.cuh"
 
 namespace {
 

@@ -19,7 +19,7 @@
 // (:152), the pivot trace, and the pricing of the NEXT pivot (first negative
 // new f / new b index, min-reduced into the state) so the next pick starts
 // without scanning.
-#include "spx_common.cuh"
+#include "spx_launch.cuh"
 
 namespace {
 

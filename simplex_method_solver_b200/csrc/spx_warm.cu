@@ -19,7 +19,7 @@
 // compacts the chunk's active columns (headers y_k with db_k != 0) or rows (labels x_k with dc_k != 0) into shared
 // memory in ascending order, and every thread folds them into its own row or column.  The f update's reads are
 // coalesced across threads; the b update's are strided by a row.  No workspace.
-#include "spx_common.cuh"
+#include "spx_launch.cuh"
 
 namespace {
 
@@ -163,19 +163,13 @@ cudaError_t warm_change_uniform(double *T, int64_t B, int n, int m, const int32_
 }
 
 // one launch per launch of the plan, so LPs of like size share a grid (as the sensitivity report)
-cudaError_t warm_change_ragged(const RaggedPlan *P, const RaggedLp *h_lps, const int32_t *h_order, double *T,
-                               const RaggedLp *d_lps, const int32_t *d_order, const int32_t *rowlab,
-                               const int32_t *collab, const double *db, const double *dc, cudaStream_t s) {
-    for (int q = 0; q < P->nlaunch; ++q) {
-        const RaggedLaunch &l = P->launch[q];
-        WarmJob J{T, rowlab, collab, db, dc, 0, 0, d_lps, d_order + l.first, l.count, 0};
-        int64_t max_n = 0, max_m = 0;
-        for (int64_t u = l.first; u < l.first + l.count; ++u) {
-            const RaggedLp &d = h_lps[h_order[u]];
-            max_n = d.n > max_n ? d.n : max_n;
-            max_m = d.m > max_m ? d.m : max_m;
-        }
-        const cudaError_t e = warm_launch(J, max_n, max_m, s);
+cudaError_t warm_change_ragged(const PlanView &v, double *T, const int32_t *rowlab, const int32_t *collab,
+                               const double *db, const double *dc, cudaStream_t s) {
+    for (int q = 0; q < v.P->nlaunch; ++q) {
+        const RaggedLaunch &l = v.P->launch[q];
+        WarmJob J{T, rowlab, collab, db, dc, 0, 0, v.d_lps, v.d_order + l.first, l.count, 0};
+        const cudaError_t e = warm_launch(J, launch_max(v, l, [](const RaggedLp &d) { return d.n; }),
+                                          launch_max(v, l, [](const RaggedLp &d) { return d.m; }), s);
         if (e != cudaSuccess) return e;
     }
     return cudaSuccess;

@@ -155,6 +155,16 @@ def test_cluster_size_query_without_a_device_for_planned_sizes(lib):
     assert lib.spx_ragged_cluster_size(None, 0) == -1
 
 
+def test_cluster_size_query_refuses_an_inconsistent_plan_header(lib):
+    from simplex_method_solver_b200.batched import _HEADER, _LAUNCH
+    rc, _, plan = _plan_raw(lib, [(8, 2, 5), (400, 800, 5)], engine=5)
+    assert rc == 0 and lib.spx_ragged_cluster_size(plan.ctypes.data, 0) == 1
+    count = _HEADER.fields["launch"][1] + _LAUNCH.fields["count"][1]       # launch[0].count
+    plan[count: count + 8].view("<i8")[0] += 1                             # the launches no longer cover B LPs
+    assert lib.spx_ragged_cluster_size(plan.ctypes.data, 0) == -1
+    assert b"inconsistent plan" in lib.spx_last_error()
+
+
 def test_plan_validation(lib):
     rc, err, _ = _plan_raw(lib, [(8, 2, 5), (600, 800, 5), (263857, 2000, 5)], engine=5)
     assert rc < 0 and b"LP 2: a 263857 x 2000 LP exceeds the shared memory of one cluster" in err, err
