@@ -96,7 +96,9 @@ int64_t     spx_launch_count(int reset);
  * were removed.  spx_set_option rejects them with any value and spx_get_option reads 0; the numbers are never reused. */
 #define SPX_OPT_TILED_MIN_BLOCKS 2  /* tiled kernel: resident CTAs per SM the register budget targets (1..4) */
 #define SPX_OPT_TILED_ROWS       5  /* tiled kernel rows per tile (0 = auto; else a multiple of 8 <= 64) */
-#define SPX_OPT_FUSE_DEPTH       6  /* fused loop: pivots applied per pass over the body (0 = default 8, max 8) */
+#define SPX_OPT_FUSE_DEPTH       6  /* one-GPU fused loop: pivots per pass over the body: 1-8 or 16 (0 = default 16;
+                                         spx_get_option reads the depth in use).  The column-sharded loop and
+                                         look-ahead pricing apply at most 8 */
 #define SPX_OPT_FUSE_MIN_BLOCKS  7  /* fused update kernel: resident CTAs per SM its register budget targets (2..4, 0 = default 3) */
 #define SPX_OPT_FUSE_PRICING     8  /* fused loop pricing kernel: 0 auto, 1 one CTA, 2 whole-GPU cooperative */
 #define SPX_OPT_FUSE_LOOKAHEAD   9  /* fused loop in spx_solve: 1 = price pass q+1 on a side stream during update q, 2 = the same with the persistent pricing engine (see spx_fshard_set_lookahead); default 0: off on one GPU */

@@ -487,13 +487,9 @@ int spx_solve(double *d_A0, double *d_A1, double *d_b0, double *d_b1, int32_t n,
         w = carve(d_work, n);
     }
     int64_t done = 0;
-    if (mode == SPX_LOOP_FUSED) {
-        // the fused passes flip the ping-pong buffers once per PASS, not per pivot: the index of the
-        // current buffer travels in the device state while this call runs
-        const int64_t curbuf = hs.npiv & 1;
-        if (check(cudaMemcpyAsync(&d_state->reserved[0], &curbuf, sizeof(curbuf), cudaMemcpyHostToDevice, s), "cur")) return -1;
-        hs.reserved[0] = curbuf;
-    }
+    // the fused passes flip the ping-pong buffers once per PASS, not per pivot: the index of the
+    // current buffer travels in the device state while this call runs
+    if (mode == SPX_LOOP_FUSED) hs.reserved[0] = hs.npiv & 1;
     bool priced = false;      // look-ahead: d_state/d_colbuf already hold the pick of the current table
     while (hs.status == SPX_PIVOT) {
         int64_t k = chunk;
@@ -501,15 +497,22 @@ int spx_solve(double *d_A0, double *d_A1, double *d_b0, double *d_b1, int32_t n,
         if (k <= 0) break;
         const int64_t base = hs.npiv;
         if (mode == SPX_LOOP_FUSED) {
-            // passes of F pivots: price F levels from the stored table (one CTA, O((n+m)F^2) work), then
-            // ONE stream over the body applies them all — 16 B of HBM traffic per cell per F pivots
-            int F = (int)spx_launch::get_option(SPX_OPT_FUSE_DEPTH);
-            if (F <= 0) F = 8;
-            if (F > spx_launch::fuse_max()) F = spx_launch::fuse_max();
+            // passes of F pivots: price F levels from the stored table, then ONE stream over the body applies
+            // them all — 16 B of HBM traffic per cell per F pivots
+            const int F = (int)spx_launch::get_option(SPX_OPT_FUSE_DEPTH);
+            const int64_t cur = hs.reserved[0] & 1;
             // look-ahead (option): the pricing of pass q+1 runs on a side stream during the update of pass q.
             // Off by default on ONE GPU: pricing is 4 % of a pass there and the overlap costs as much as it
             // hides (measured 3.14 k vs 3.21 k pivots/s); on by default in the column-sharded loop.
             const int la = (int)spx_launch::get_option(SPX_OPT_FUSE_LOOKAHEAD);      // 1 per-pass kernels, 2 persistent engine
+            // Without look-ahead, a chunk whose pass count and pivot count differ in parity runs its first pass IN
+            // PLACE, so that it leaves table k in buffer k & 1 without a copy of the body.  Only a pass deeper than
+            // 8 runs in place: its update kernel reads its own cells coherently (ld_own).  Nothing else reads the
+            // body during a pass of this loop.
+            const int64_t npass = (k + F - 1) / F;
+            const bool inplace = la != 1 && la != 2 && ((cur ^ npass ^ (base + k)) & 1) && (k < F ? k : F) > 8;
+            const int64_t reserved = cur | (inplace ? 2 : 0);
+            if (check(cudaMemcpyAsync(&d_state->reserved[0], &reserved, sizeof(reserved), cudaMemcpyHostToDevice, s), "cur")) return -1;
             if (la == 1 || la == 2) {
                 if (check(spx_launch::fused_solve_passes(d_A0, d_A1, d_b0, d_b1, n, m, ld, rule, d_state, d_work, d_rowlab,
                                                          d_collab, d_trace, k, F,
@@ -517,9 +520,11 @@ int spx_solve(double *d_A0, double *d_A1, double *d_b0, double *d_b1, int32_t n,
                           "fused pass launch")) return -1;
             } else {
                 int64_t left = k;
-                while (left > 0) {
+                for (int64_t q = 0; left > 0; ++q) {
                     const int Fp = (int)(left < F ? left : F);
-                    if (check(spx_launch::fused_pass(d_A0, d_A1, d_b0, d_b1, n, m, ld, rule, Fp,
+                    const bool same = inplace && q == 0;                 // both tables of the pass are buffer `cur`
+                    if (check(spx_launch::fused_pass(same ? A[cur] : d_A0, same ? A[cur] : d_A1, same ? b[cur] : d_b0,
+                                                     same ? b[cur] : d_b1, n, m, ld, rule, Fp,
                                                      (int)spx_launch::get_option(SPX_OPT_FUSE_MIN_BLOCKS),
                                                      (int)spx_launch::get_option(SPX_OPT_FUSE_PRICING), 0, d_state, d_work,
                                                      d_rowlab, d_collab, d_trace, s), "fused pass launch")) return -1;
@@ -584,7 +589,8 @@ int spx_solve(double *d_A0, double *d_A1, double *d_b0, double *d_b1, int32_t n,
         done += k;
     }
     if (mode == SPX_LOOP_FUSED) {
-        // restore the library-wide invariant "the current table is in buffer npiv & 1"
+        // restore the library-wide invariant "the current table is in buffer npiv & 1" (after an in-place first
+        // pass, only a call that stopped early or passes of at most 8 levels still need the copy)
         const int cur = (int)(hs.reserved[0] & 1), want = (int)(hs.npiv & 1);
         if (cur != want) {
             if (check(cudaMemcpyAsync(A[want], A[cur], (size_t)(n + 1) * ld * sizeof(double), cudaMemcpyDeviceToDevice, s), "table copy")) return -1;

@@ -40,7 +40,7 @@ bool resident_fits(int n, int m, int64_t ld);
 cudaError_t resident_loop(double *A0, double *A1, double *b0, double *b1, int n, int m, int64_t ld, int rule,
                           int64_t max_steps, spx_state *st, double *colbuf, int32_t *rowlab, int32_t *collab,
                           int32_t *trace, cudaStream_t stream);
-int fuse_max();
+int fuse_max();                 // levels per pass at most of the one-GPU fused loop
 int64_t fused_workspace_bytes(int n, int64_t ld);
 cudaError_t fused_pass(double *A0, double *A1, double *b0, double *b1, int n, int m, int64_t ld, int rule, int F,
                        int minb, int pricing, int phase, spx_state *st, void *work, int32_t *rowlab, int32_t *collab,

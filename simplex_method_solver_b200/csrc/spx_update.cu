@@ -254,12 +254,16 @@ static int pick_tr(int n, int m_loc) {
 
 // process-wide tuning knobs (spx_set_option); every setting computes the same bits
 
-int64_t get_option(int key) { return (key >= 0 && key < 17) ? g_opt[key] : -1; }
+// SPX_OPT_FUSE_DEPTH reads the depth the one-GPU fused loop uses, the default included
+int64_t get_option(int key) {
+    if (key == SPX_OPT_FUSE_DEPTH && g_opt[key] == 0) return fuse_max();
+    return (key >= 0 && key < 17) ? g_opt[key] : -1;
+}
 int set_option(int key, int64_t value) {
     switch (key) {
     case SPX_OPT_TILED_MIN_BLOCKS: if (value < 1 || value > 4) return -1; break;
     case SPX_OPT_TILED_ROWS:       if (value < 0 || value > UPD_TR_MAX || value % 8) return -1; break;
-    case SPX_OPT_FUSE_DEPTH:       if (value < 0 || value > 8) return -1; break;
+    case SPX_OPT_FUSE_DEPTH:       if (value < 0 || (value > 8 && value != fuse_max())) return -1; break;   // whole groups above 8
     case SPX_OPT_FUSE_MIN_BLOCKS:  if (value < 0 || value > 4) return -1; break;
     case SPX_OPT_FUSE_PRICING:     if (value < 0 || value > 2) return -1; break;
     case SPX_OPT_FUSE_LOOKAHEAD:   if (value < 0 || value > 2) return -1; break;
