@@ -390,6 +390,48 @@ int spx_sensitivity_split(const double *d_A, const double *d_b, int32_t n, int32
                           double *d_redcost, double *d_rhs_range, double *d_cost_range, int32_t *h_optimal,
                           void *stream);
 
+/* ---- certificates of infeasible and unbounded LPs (csrc/spx_certificate.cu) ------- */
+/* Conventions of the sensitivity report above: label codes x_k -> k, y_k -> m + k, rowlab [m] over the columns,
+ * collab [n] over the rows, w1 = m + 1, b_i = T[i*w1 + m], d_j = T[n*w1 + j].  Computed for every LP from its final
+ * table, whatever its status, in this sequential statement:
+ *   Farkas row:  farkas_row = the lowest i with b_i finite and < 0 and every T[i][j] (j < m) finite and <= 0, else -1.
+ *                Found: farkas [n] = +0.0 everywhere; then farkas[L-m] = 1.0 when L = collab[r] is a y label; then,
+ *                for j ascending, farkas[H-m] = 0.0 - T[r][j] when H = rowlab[j] is a y label (+0.0 for either zero);
+ *                farkas_bound = b_r.  Not found: farkas all NaN, farkas_bound NaN.
+ *   Ray column:  only when every b_i is finite and >= 0 (-0.0 counts): ray_col = the lowest j with d_j finite and < 0
+ *                and every T[i][j] (i < n) finite and >= 0, else -1.
+ *                Found: ray [m] = +0.0 everywhere; then ray[H] = 1.0 when H = rowlab[c] is an x label; then, for i
+ *                ascending, ray[L] = T[i][c] + 0.0 when L = collab[i] is an x label; ray_slope = d_c.  Not found:
+ *                ray all NaN, ray_slope NaN.
+ * A label outside its range is skipped.  Why they are certificates, for "minimise c.x subject to b + A x >= 0,
+ * x >= 0": row r says a non-negative variable equals b_r < 0 plus a non-positive combination of non-negative ones,
+ * so u = farkas >= 0 has A^T u <= 0 and b.u = b_r < 0 (the LP is infeasible); in a table with b >= 0, raising x_N_c
+ * from the vertex keeps every constraint and lowers f by |d_c| per unit, so d = ray >= 0 has A d >= 0 and
+ * c.d = d_c < 0 (the LP is unbounded).  An SPX_INCORRECT table gets the row the solver stopped on; an SPX_NOCONV
+ * table of the reference rule gets the solver's entering column; an optimal table gets neither.  Every step is a
+ * minimum of indices, a logical OR or a copy, so the results equal the statement bit for bit.
+ *
+ * Outputs: d_row [B] int32, d_farkas, d_bound [B], d_col [B] int32, d_ray, d_slope [B].  Each may be NULL, with one
+ * rule: d_farkas and d_ray are the kernels' only workspace (no memory is allocated), so d_row and d_bound need
+ * d_farkas, and d_col and d_slope need d_ray.  Labels are required.  Arguments, shapes and the plan header are
+ * checked before the device is touched; B = 0 returns 0.  At most three launches per group, no synchronisation.
+ *
+ * Uniform batches: d_T [B][cells] final reference-flat tables (DeviceBatch after K4, K7 or K8), d_rowlab [B][m],
+ * d_collab [B][n]; d_farkas [B][n], d_ray [B][m]. */
+int spx_certificate_batched(const double *d_T, int64_t B, int32_t n, int32_t m, const int32_t *d_rowlab,
+                            const int32_t *d_collab, int32_t *d_row, double *d_farkas, double *d_bound,
+                            int32_t *d_col, double *d_ray, double *d_slope, void *stream);
+/* Ragged batches packed as spx_solve_batched_ragged packs them, one group of launches per launch of the plan:
+ * d_farkas at the prefix sums of n (as d_collab), d_ray at those of m (as d_x); the per-LP outputs [B]. */
+int spx_certificate_ragged(const double *d_T, const void *h_plan, const void *d_plan, const int32_t *d_rowlab,
+                           const int32_t *d_collab, int32_t *d_row, double *d_farkas, double *d_bound,
+                           int32_t *d_col, double *d_ray, double *d_slope, void *stream);
+/* One split table (d_A [(n+1)][ld], d_b [n]; d_rowlab [m], d_collab [n]), e.g. the current table of a streaming
+ * solve; the per-LP outputs have one element. */
+int spx_certificate_split(const double *d_A, const double *d_b, int32_t n, int32_t m, int64_t ld,
+                          const int32_t *d_rowlab, const int32_t *d_collab, int32_t *d_row, double *d_farkas,
+                          double *d_bound, int32_t *d_col, double *d_ray, double *d_slope, void *stream);
+
 /* ---- warm start: change and resume final tables (csrc/spx_warm.cu) ---------------- */
 /* The final table of a batched solve is a dictionary (conventions of the sensitivity report above;
  * label codes x_k -> k, y_k -> m + k, w1 = m + 1, b_i = T[i*w1 + m], d_j = T[n*w1 + j]).  The change

@@ -86,6 +86,49 @@ def _sens_uniform(T, status, rowlab, collab, B: int, n: int, m: int, device) -> 
                        cr.reshape(B, m, 2), status[:B].cpu().numpy() == N.OPTIMAL)
 
 
+class Certificate(NamedTuple):
+    """Certificates of failure read off final tables (spx_certificate_*, include/spx_b200.h), for "minimise c.x
+    subject to b + A x >= 0 and x >= 0".  A Farkas vector u >= 0 has A^T u <= 0 and b.u = farkas_bound < 0: the LP is
+    infeasible.  A ray d >= 0 of a table with b >= 0 has A d >= 0 and c.d = ray_slope < 0: the LP is unbounded.
+    Computed for every LP whatever its status; without a certificate the index is -1 and the arrays are NaN."""
+    infeasible: np.ndarray        # [B] bool: farkas_row >= 0
+    farkas_row: np.ndarray        # [B] int32: the table row that proves infeasibility, or -1
+    farkas: np.ndarray            # [B, n] u, one entry per constraint
+    farkas_bound: np.ndarray      # [B] b.u = b of that row
+    unbounded: np.ndarray         # [B] bool: ray_col >= 0
+    ray_col: np.ndarray           # [B] int32: the table column that proves unboundedness, or -1
+    ray: np.ndarray               # [B, m] d, one entry per variable
+    ray_slope: np.ndarray         # [B] c.d = d of that column
+
+
+class _CertOut:
+    """Device outputs of one certificate call: B LPs, nc per-constraint and nv per-variable entries."""
+
+    def __init__(self, B: int, nc: int, nv: int, device):
+        f64, i32, q = torch.float64, torch.int32, (lambda k: max(k, 1))  # noqa: E731
+        self.B, self.nc, self.nv = B, nc, nv
+        self.t = [torch.empty(q(B), dtype=i32, device=device), torch.empty(q(nc), dtype=f64, device=device),
+                  torch.empty(q(B), dtype=f64, device=device), torch.empty(q(B), dtype=i32, device=device),
+                  torch.empty(q(nv), dtype=f64, device=device), torch.empty(q(B), dtype=f64, device=device)]
+
+    def ptrs(self):
+        return [t.data_ptr() for t in self.t]
+
+    def host(self):
+        """(farkas_row, farkas, farkas_bound, ray_col, ray, ray_slope), flat"""
+        B = self.B
+        return [t[:k].cpu().numpy() for t, k in zip(self.t, (B, self.nc, B, B, self.nv, B))]
+
+
+def _cert_uniform(T, rowlab, collab, B: int, n: int, m: int, device) -> Certificate:
+    out = _CertOut(B, B * n, B * m, device)
+    with torch.cuda.device(device):
+        N.call("spx_certificate_batched", T.data_ptr(), B, n, m, rowlab.data_ptr(), collab.data_ptr(), *out.ptrs(),
+               torch.cuda.current_stream(device).cuda_stream)
+    r, u, ub, c, d, ds = out.host()
+    return Certificate(r >= 0, r, u.reshape(B, n), ub, c >= 0, c, d.reshape(B, m), ds)
+
+
 ENGINES = ("auto", "smem", "cluster", "global", "auto_global")
 ENGINE_CODES = {"auto": N.ENGINE_AUTO, "smem": N.ENGINE_SMEM, "cluster": N.ENGINE_CLUSTER, "global": N.ENGINE_GLOBAL,
                 "auto_global": N.ENGINE_AUTO_GLOBAL}
@@ -256,6 +299,11 @@ class DeviceBatch:
         """Sensitivity report of the final tables the last ``run`` left (K4, K7 and K8 alike); synchronises."""
         return _sens_uniform(self.T, self.status, self.rowlab, self.collab, self.B, self.n, self.m, self.device)
 
+    def certificate(self) -> Certificate:
+        """Farkas vectors and unbounded rays of the final tables the last ``run`` or ``resume`` left (K4, K7 and K8
+        alike); synchronises."""
+        return _cert_uniform(self.T, self.rowlab, self.collab, self.B, self.n, self.m, self.device)
+
     def result(self) -> BatchResult:
         B = self.B
         g = lambda t: None if t is None else t[:B].cpu().numpy()  # noqa: E731
@@ -394,6 +442,39 @@ def _sens_ragged(T, h_plan: np.ndarray, d_plan, status, rowlab, collab, B: int, 
                              status[:B].cpu().numpy() == N.OPTIMAL, shapes.copy(), offsets.copy())
 
 
+class RaggedCertificate(NamedTuple):
+    """Certificates of a ragged batch: per-LP arrays [B], ``farkas`` packed at the prefix sums of n (as ``collab``),
+    ``ray`` at the prefix sums of m (as ``x``)."""
+    infeasible: np.ndarray        # [B] bool
+    farkas_row: np.ndarray        # [B] int32
+    farkas: np.ndarray            # [sum n]
+    farkas_bound: np.ndarray      # [B]
+    unbounded: np.ndarray         # [B] bool
+    ray_col: np.ndarray           # [B] int32
+    ray: np.ndarray               # [sum m]
+    ray_slope: np.ndarray         # [B]
+    shapes: np.ndarray            # [B, 3] int64: n, m, max_pivots
+    offsets: np.ndarray           # [B, 5] int64, as RaggedResult.offsets
+
+    def lp(self, k: int) -> Certificate:
+        """LP k alone, with the shapes ``DeviceBatch.certificate()`` gives for a batch of that one LP."""
+        n, m = int(self.shapes[k, 0]), int(self.shapes[k, 1])
+        xm, xn = int(self.offsets[k, 1]), int(self.offsets[k, 2])
+        s = slice(k, k + 1)
+        return Certificate(self.infeasible[s], self.farkas_row[s], self.farkas[xn: xn + n][None], self.farkas_bound[s],
+                           self.unbounded[s], self.ray_col[s], self.ray[xm: xm + m][None], self.ray_slope[s])
+
+
+def _cert_ragged(T, h_plan: np.ndarray, d_plan, rowlab, collab, B: int, totals, shapes, offsets,
+                 device) -> RaggedCertificate:
+    out = _CertOut(B, int(totals[2]), int(totals[1]), device)
+    with torch.cuda.device(device):
+        N.call("spx_certificate_ragged", T.data_ptr(), h_plan.ctypes.data, d_plan.data_ptr(), rowlab.data_ptr(),
+               collab.data_ptr(), *out.ptrs(), torch.cuda.current_stream(device).cuda_stream)
+    r, u, ub, c, d, ds = out.host()
+    return RaggedCertificate(r >= 0, r, u, ub, c >= 0, c, d, ds, shapes.copy(), offsets.copy())
+
+
 def _caps(max_pivots: Union[int, Sequence[int]], B: int) -> np.ndarray:
     caps = np.asarray(max_pivots, dtype=np.int64)
     if caps.ndim == 0:
@@ -530,6 +611,11 @@ class DeviceRaggedBatch:
         return _sens_ragged(self.T, self.plan.plan, self.d_plan, self.status, self.rowlab, self.collab, self.B,
                             self.totals, self.shapes, self.offsets, self.device)
 
+    def certificate(self) -> RaggedCertificate:
+        """Farkas vectors and unbounded rays of the final tables the last ``run`` or ``resume`` left; synchronises."""
+        return _cert_ragged(self.T, self.plan.plan, self.d_plan, self.rowlab, self.collab, self.B, self.totals,
+                            self.shapes, self.offsets, self.device)
+
     def result(self) -> RaggedResult:
         B, tot = self.B, self.totals
         g = lambda t, k: None if t is None else t[:k].cpu().numpy()  # noqa: E731
@@ -620,6 +706,35 @@ def sensitivity(result: Union[BatchResult, RaggedResult], device=None) -> Union[
     N.lib()
     return _sens_uniform(up(result.tables, np.float64), up(result.status, np.int32), up(rowlab, np.int32),
                          up(collab, np.int32), B, n, m, dev)
+
+
+def certificate(result: Union[BatchResult, RaggedResult], device=None) -> Union[Certificate, RaggedCertificate]:
+    """Farkas vectors and unbounded rays of the final tables of a host ``BatchResult`` (``solve_batched``) or
+    ``RaggedResult`` (``solve_ragged``): uploads the tables and labels and runs the report's kernels on ``device``."""
+    dev = torch.device(device if device is not None else "cuda")
+    up = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dtype=dt).reshape(-1)).to(dev)  # noqa: E731
+    z = np.zeros
+    if isinstance(result, RaggedResult):
+        shapes = np.asarray(result.shapes, dtype=np.int64).reshape(-1, 3)
+        B = shapes.shape[0]
+        plan = ragged_plan(shapes[:, :2], shapes[:, 2], "auto_global")
+        if not np.array_equal(plan.offsets, np.asarray(result.offsets, dtype=np.int64).reshape(-1, 5)):
+            raise ValueError("result.offsets are not the packing of result.shapes")
+        _check_packing(result, plan)
+        if B == 0:
+            return RaggedCertificate(z(0, bool), z(0, np.int32), z(0), z(0), z(0, bool), z(0, np.int32), z(0), z(0),
+                                     shapes.copy(), plan.offsets)
+        N.lib()
+        return _cert_ragged(up(result.tables, np.float64), plan.plan, torch.from_numpy(plan.plan).to(dev),
+                            up(result.rowlab, np.int32), up(result.collab, np.int32), B, plan.totals, shapes,
+                            plan.offsets, dev)
+    rowlab, collab, B, n, m = _uniform_labels(result, "certificate")
+    if np.shape(result.tables) != (B, n * (m + 1) + m):
+        raise ValueError(f"result.tables must be [B, n*(m+1)+m] = [{B}, {n * (m + 1) + m}]")
+    if B == 0:
+        return Certificate(z(0, bool), z(0, np.int32), z((0, n)), z(0), z(0, bool), z(0, np.int32), z((0, m)), z(0))
+    N.lib()
+    return _cert_uniform(up(result.tables, np.float64), up(rowlab, np.int32), up(collab, np.int32), B, n, m, dev)
 
 
 def _new_values(new, old: np.ndarray, name: str):

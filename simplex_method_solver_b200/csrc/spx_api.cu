@@ -932,6 +932,59 @@ int spx_sensitivity_split(const double *d_A, const double *d_b, int32_t n, int32
                  "split sensitivity launch");
 }
 
+// ---- certificates of infeasible and unbounded LPs (csrc/spx_certificate.cu) ----------
+// d_farkas and d_ray are the workspace of their halves: the index and bound of a half need its vector
+static bool cert_outputs_ok(const char *who, const int32_t *row, const double *farkas, const double *bound,
+                            const int32_t *col, const double *ray, const double *slope) {
+    if ((row || bound) && !farkas) {
+        set_error("%s: d_row and d_bound need d_farkas (the workspace of the Farkas half)", who);
+        return false;
+    }
+    if ((col || slope) && !ray) {
+        set_error("%s: d_col and d_slope need d_ray (the workspace of the ray half)", who);
+        return false;
+    }
+    return true;
+}
+
+int spx_certificate_batched(const double *d_T, int64_t B, int32_t n, int32_t m, const int32_t *d_rowlab,
+                            const int32_t *d_collab, int32_t *d_row, double *d_farkas, double *d_bound,
+                            int32_t *d_col, double *d_ray, double *d_slope, void *stream) {
+    SPX_REQUIRE(B >= 0 && n >= 1 && m >= 1, "spx_certificate_batched: bad arguments (B = %lld, n = %d, m = %d)",
+                (long long)B, n, m);
+    if (!cert_outputs_ok("spx_certificate_batched", d_row, d_farkas, d_bound, d_col, d_ray, d_slope)) return -2;
+    if (B == 0) return 0;
+    SPX_REQUIRE(d_T && d_rowlab && d_collab, "spx_certificate_batched: null T/rowlab/collab");
+    return check(spx_launch::certificate_uniform(d_T, B, n, m, d_rowlab, d_collab, d_row, d_farkas, d_bound, d_col,
+                                                 d_ray, d_slope, as_stream(stream)),
+                 "certificate launch");
+}
+
+int spx_certificate_ragged(const double *d_T, const void *h_plan, const void *d_plan, const int32_t *d_rowlab,
+                           const int32_t *d_collab, int32_t *d_row, double *d_farkas, double *d_bound,
+                           int32_t *d_col, double *d_ray, double *d_slope, void *stream) {
+    spx::PlanView v;
+    if (!checked_plan("spx_certificate_ragged", h_plan, d_plan, &v)) return -2;
+    if (!cert_outputs_ok("spx_certificate_ragged", d_row, d_farkas, d_bound, d_col, d_ray, d_slope)) return -2;
+    if (v.P->B == 0) return 0;
+    SPX_REQUIRE(d_plan && d_T && d_rowlab && d_collab, "spx_certificate_ragged: null d_plan/T/rowlab/collab");
+    return check(spx_launch::certificate_ragged(v, d_T, d_rowlab, d_collab, d_row, d_farkas, d_bound, d_col, d_ray,
+                                                d_slope, as_stream(stream)),
+                 "ragged certificate launch");
+}
+
+int spx_certificate_split(const double *d_A, const double *d_b, int32_t n, int32_t m, int64_t ld,
+                          const int32_t *d_rowlab, const int32_t *d_collab, int32_t *d_row, double *d_farkas,
+                          double *d_bound, int32_t *d_col, double *d_ray, double *d_slope, void *stream) {
+    SPX_REQUIRE(n >= 1 && m >= 1 && ld >= m, "spx_certificate_split: bad arguments (n = %d, m = %d, ld = %lld)", n, m,
+                (long long)ld);
+    SPX_REQUIRE(d_A && d_b && d_rowlab && d_collab, "spx_certificate_split: null A/b/rowlab/collab");
+    if (!cert_outputs_ok("spx_certificate_split", d_row, d_farkas, d_bound, d_col, d_ray, d_slope)) return -2;
+    return check(spx_launch::certificate_split(d_A, d_b, n, m, ld, d_rowlab, d_collab, d_row, d_farkas, d_bound, d_col,
+                                               d_ray, d_slope, as_stream(stream)),
+                 "split certificate launch");
+}
+
 // ---- warm start: change and resume final tables (csrc/spx_warm.cu) ------------------
 int spx_warm_change_batched(double *d_T, int64_t B, int32_t n, int32_t m, const int32_t *d_rowlab,
                             const int32_t *d_collab, const double *d_delta_b, const double *d_delta_c, void *stream) {

@@ -93,6 +93,16 @@ cudaError_t sensitivity_ragged(const spx::PlanView &v, const double *d_T, const 
 cudaError_t sensitivity_split(const double *d_A, const double *d_b, int n, int m, int64_t ld, int optimal,
                               const int32_t *d_rowlab, const int32_t *d_collab, double *dual, double *slack,
                               double *redcost, double *rhs, double *cost, cudaStream_t s);
+// ---- certificates of infeasible and unbounded LPs (spx_certificate.cu) ----
+cudaError_t certificate_uniform(const double *d_T, int64_t B, int n, int m, const int32_t *d_rowlab,
+                                const int32_t *d_collab, int32_t *row, double *farkas, double *bound, int32_t *col,
+                                double *ray, double *slope, cudaStream_t s);
+cudaError_t certificate_ragged(const spx::PlanView &v, const double *d_T, const int32_t *d_rowlab,
+                               const int32_t *d_collab, int32_t *row, double *farkas, double *bound, int32_t *col,
+                               double *ray, double *slope, cudaStream_t s);
+cudaError_t certificate_split(const double *d_A, const double *d_b, int n, int m, int64_t ld,
+                              const int32_t *d_rowlab, const int32_t *d_collab, int32_t *row, double *farkas,
+                              double *bound, int32_t *col, double *ray, double *slope, cudaStream_t s);
 cudaError_t warm_change_uniform(double *T, int64_t B, int n, int m, const int32_t *rowlab, const int32_t *collab,
                                 const double *db, const double *dc, cudaStream_t s);
 cudaError_t warm_change_ragged(const spx::PlanView &v, double *T, const int32_t *rowlab, const int32_t *collab,

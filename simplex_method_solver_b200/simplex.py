@@ -46,7 +46,7 @@ import numpy as np
 import torch
 
 from . import _native as N
-from .batched import DeviceBatch, Sensitivity, _SensOut, kernel_for
+from .batched import Certificate, DeviceBatch, Sensitivity, _CertOut, _SensOut, kernel_for
 from .engine import DeviceTableau, Solution, as_rows_function
 
 CAP_TEXT = "pivot limit reached"
@@ -405,6 +405,20 @@ class SimplexMethod:
                              "(solve the LP to optimality first)")
         dual, slack, rc, rr, cr = out.host()
         return Sensitivity(dual, slack, rc, rr.reshape(n, 2), cr.reshape(m, 2), True)
+
+    def certificate(self) -> Certificate:
+        """Farkas vector and unbounded ray of the current table, whatever its state (after ``solve()``,
+        ``get_solution()`` or step-API pivots); no host synchronisation before the launches.  Per-LP fields are
+        scalars and the arrays have no batch axis: farkas [n], ray [m]."""
+        self._not_sharded("certificate()")
+        dev, n, m = self._dev, self.n, self.m
+        c = dev.cur(self._npiv)
+        out = _CertOut(1, n, m, dev.device)
+        dev._call("spx_certificate_split", dev.A[c].data_ptr(), dev.b[c].data_ptr(), n, m, dev.ld,
+                  dev.rowlab.data_ptr(), dev.collab.data_ptr(), *out.ptrs())
+        r, u, ub, col, d, ds = out.host()
+        return Certificate(bool(r[0] >= 0), int(r[0]), u, float(ub[0]), bool(col[0] >= 0), int(col[0]), d,
+                           float(ds[0]))
 
     def _labels_from_codes(self, rowlab, collab):
         name = lambda v: f"x{v + 1}" if v < self.m else f"y{v - self.m + 1}"  # noqa: E731
