@@ -119,10 +119,18 @@ int         spx_selftest_division(const double *d_a, const double *d_p, int64_t 
  * d_rj[count][levels], pivot-column values d_ci[count][levels], i.e. `levels` applications of
  * recalculate_matrix()'s cell formula (simplex.py:173-175) — once the kernel's way (unguarded fast divisions, ONE
  * range test on the result, guarded re-do when it fails) into d_out_lazy, once with every division guarded into
- * d_out_ref.  The caller compares the bits.  *h_redo = how many chains took the re-do. */
+ * d_out_ref.  Chains deeper than 8 levels take the depth-16 kernel's way: a range test after each group of 8, and the
+ * two-operation quotient on the levels whose divisor it flags (spx_selftest_two_op).  The caller compares the bits.
+ * *h_redo = how many chains took the re-do. */
 int         spx_selftest_lazy_guard(const double *d_t0, const double *d_p, const double *d_rj, const double *d_ci,
                                     int32_t levels, int64_t count, double *d_out_lazy, double *d_out_ref,
                                     uint64_t *h_redo, void *stream);
+/* Device self-test of the one-GPU fused update's two-operation quotient (csrc/spx_fused.cu, two_op_flag): for each
+ * divisor d_p[k < np], d_flags[k] = 1 when the update kernel would divide by it with fma(a, yh, RN(a * yl)), else 0.
+ * For every flagged divisor the quotient is compared bit for bit with div.rn.f64 on every candidate numerator at
+ * K = 64 and on per_p pseudo-random numerators; *h_mismatches = the number of differences (0 expected). */
+int         spx_selftest_two_op(const double *d_p, int64_t np, int64_t per_p, int32_t *d_flags,
+                                uint64_t *h_mismatches, void *stream);
 
 /* ---- layout conversion (SimplexMethod.__init__, simplex.py:25-39) -------- */
 /* src_rows is the reference's `constraints` as a dense row-major [n][m+1] fp64

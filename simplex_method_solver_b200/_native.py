@@ -70,6 +70,7 @@ SIGNATURES = {
                                              ctypes.POINTER(ctypes.c_double), _vp]),
     "spx_selftest_lazy_guard": (ctypes.c_int, [_vp, _vp, _vp, _vp, _i32, _i64, _vp, _vp,
                                                ctypes.POINTER(ctypes.c_uint64), _vp]),
+    "spx_selftest_two_op": (ctypes.c_int, [_vp, _i64, _i64, _vp, ctypes.POINTER(ctypes.c_uint64), _vp]),
     "spx_import_table": (ctypes.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i64, _vp]),
     "spx_import_shard": (ctypes.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i64, _i32, _i64, _vp]),
     "spx_export_table": (ctypes.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i64, _vp]),

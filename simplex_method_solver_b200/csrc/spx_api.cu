@@ -287,6 +287,23 @@ int spx_selftest_lazy_guard(const double *d_t0, const double *d_p, const double 
     return rc;
 }
 
+int spx_selftest_two_op(const double *d_p, int64_t np, int64_t per_p, int32_t *d_flags, uint64_t *h_mismatches,
+                        void *stream) {
+    SPX_REQUIRE(d_p && d_flags && h_mismatches && np >= 0 && per_p >= 0, "spx_selftest_two_op: bad arguments");
+    cudaStream_t s = as_stream(stream);
+    unsigned long long *d_cnt = nullptr, cnt = 0;
+    if (check(cudaMalloc(&d_cnt, sizeof(*d_cnt)), "cudaMalloc")) return -1;
+    int rc = 0;
+    if (check(cudaMemsetAsync(d_cnt, 0, sizeof(*d_cnt), s), "memset") ||
+        check(spx_launch::two_op_selftest(d_p, np, per_p, d_flags, d_cnt, s), "selftest launch") ||
+        check(cudaMemcpyAsync(&cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost, s), "read") ||
+        check(cudaStreamSynchronize(s), "sync"))
+        rc = -1;
+    cudaFree(d_cnt);
+    *h_mismatches = cnt;
+    return rc;
+}
+
 // ---- layout conversion ---------------------------------------------------------
 int spx_import_shard(const double *src_rows, const double *src_function, double *d_A, double *d_b,
                      int32_t n, int32_t m, int64_t col0, int32_t m_loc, int64_t ld_loc, void *stream) {

@@ -52,6 +52,8 @@ cudaError_t fused_solo_sync();
 cudaError_t lazy_guard_selftest(const double *t0, const double *p, const double *rj, const double *ci, int F,
                                 int64_t count, double *out_lazy, double *out_ref, unsigned long long *n_redo,
                                 cudaStream_t stream);
+cudaError_t two_op_selftest(const double *p, int64_t np, int64_t per_p, int32_t *flags, unsigned long long *mismatches,
+                            cudaStream_t stream);
 
 // ---- batched engines: K4 (spx_batched.cu), K7 (spx_cluster.cu), K8 (spx_global.cu) ----
 // The uniform launchers solve B LPs of one n x m shape; the ragged launchers run launch l of plan v.  Each returns
