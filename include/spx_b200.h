@@ -57,6 +57,14 @@ extern "C" {
 /* pivoting rules */
 #define SPX_RULE_REFERENCE 0  /* first-negative entering, max-negative-ratio leaving (the reference) */
 #define SPX_RULE_DANTZIG   1  /* most-negative entering (lowest index on ties); leaving as reference */
+/* Devex reference weights (Forrest-Goldfarb): the candidate f_j < 0 with the largest f_j^2 / w_j enters (NaN scores
+ * below every number, lowest j on ties); after every pivot (r, c), phase-1 pivots included, w_j = max(w_j,
+ * u_j^2 * w_c) and w_c = max(1, u_c^2 * w_c), u = the new pivot row; every solve and every resume starts from w = 1.
+ * Phase 1, the leaving row and the pivot arithmetic are the reference's.  Batched entries only
+ * (spx_solve_batched, spx_solve_batched_cluster, spx_solve_batched_global, spx_solve_batched_ragged,
+ * spx_warm_solve_batched, spx_warm_solve_ragged): there d_x is required, it is the weights' workspace until the
+ * epilogue writes x.  Every single-LP and sharded entry rejects it. */
+#define SPX_RULE_DEVEX     2
 
 /* Device-resident solver state, 128 bytes.  Written by the pick kernels, read
  * by the update kernels, so a whole chunk of pivots can be enqueued with no host

@@ -244,7 +244,8 @@ class DeviceBatch:
         self.T[: self.B].copy_(src, non_blocking=non_blocking)
 
     def run(self, rule: int = N.RULE_REFERENCE):
-        """Launch the solver on the resident batch (asynchronous on the current stream)."""
+        """Launch the solver on the resident batch (asynchronous on the current stream).  Under ``N.RULE_DEVEX`` the
+        x buffer holds the weights until the kernel writes x."""
         with torch.cuda.device(self.device):
             entry = _ENTRIES[self.kernel]
             N.call(entry, self.T.data_ptr(), self.B, self.n, self.m, rule, self.max_pivots, self.x.data_ptr(), self.obj.data_ptr(), self.status.data_ptr(),
@@ -286,7 +287,9 @@ class DeviceBatch:
     def resume(self, function, rule: int = N.RULE_REFERENCE):
         """Continue every LP from its resident table and labels for up to ``max_pivots`` more pivots, on this
         batch's engine (``spx_warm_solve_batched``).  function: [B, m] or [m], the LPs' current costs, used only
-        for ``obj``.  Trace and snapshots count from 0 again.  Asynchronous on the current stream."""
+        for ``obj``.  Trace and snapshots count from 0 again.  Under ``N.RULE_DEVEX`` the weights restart at 1, so
+        a capped devex solve and its resume do not pivot as one uncapped solve (they do under the other rules).
+        Asynchronous on the current stream."""
         fn = _per_lp(function, self.B, self.m, "function")
         self._function = torch.from_numpy(fn).to(self.device) if self.B else None    # alive until the kernel ran
         with torch.cuda.device(self.device):
@@ -319,6 +322,9 @@ def solve_batched(tables, n: int, m: int, max_pivots: int = 64, rule: str = "ref
     function coefficients) — the flattened arguments of
     ``SimplexMethod(constraints, function)`` for each LP.
     engine: "auto" (K4 when the LP fits one CTA, else K7), "smem" (K4), "cluster" (K7) or "global" (K8).
+    rule: "reference" (first negative f cell enters), "dantzig" (most negative) or "devex" (largest f_j^2 / w_j
+    under Forrest-Goldfarb reference weights w, include/spx_b200.h: far fewer pivots on badly scaled LPs).  Phase 1
+    and the leaving row are the reference's under every rule.
     """
     tables = np.ascontiguousarray(np.asarray(tables, dtype=np.float64))
     if tables.ndim != 2 or tables.shape[1] != n * (m + 1) + m:
@@ -594,8 +600,8 @@ class DeviceRaggedBatch:
                    torch.cuda.current_stream(self.device).cuda_stream)
 
     def resume(self, function, rule: int = N.RULE_REFERENCE):
-        """As ``DeviceBatch.resume``, each LP for up to its own cap; function packed [sum m] (as ``x``)
-        (``spx_warm_solve_ragged``)."""
+        """As ``DeviceBatch.resume`` (devex weights restart at 1 there too), each LP for up to its own cap; function
+        packed [sum m] (as ``x``) (``spx_warm_solve_ragged``)."""
         fn = np.ascontiguousarray(np.asarray(function, dtype=np.float64).reshape(-1))
         if fn.shape != (self.totals[1],):
             raise ValueError(f"function must be packed [{self.totals[1]}], got {fn.shape[0]} entries")
@@ -772,7 +778,8 @@ def resolve(result: Union[BatchResult, RaggedResult], data, rhs=None, cost=None,
     rhs / cost: the new b ([B, n] or [n]) and c ([B, m] or [m]); for a ragged result packed ([sum n],
     [sum m]) or one array per LP.  None keeps the old values; with neither, the LPs simply continue.
     The final tables and labels are uploaded, changed by delta = new - old (``change``) and resumed for up
-    to max_pivots more pivots with function = the new costs (``resume``).  Returns the result type given.
+    to max_pivots more pivots with function = the new costs (``resume``); under rule="devex" from unit weights.
+    Returns the result type given.
     Non-finite deltas, labels that are not a permutation of 0..n+m-1 and shapes that do not match are
     ValueErrors naming the LP.
     """

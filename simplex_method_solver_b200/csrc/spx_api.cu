@@ -152,6 +152,19 @@ bool route_lp(int n, int m, int engine, int forced, Route *r) {
 
 int forced_cluster_size() { return (int)spx_launch::get_option(SPX_OPT_CLUSTER_SIZE); }
 
+// The rule of a batched entry: reference, Dantzig or devex; devex keeps its weights in d_x, so d_x is required
+bool batched_rule_ok(const char *who, const spx::BatchIO &io, bool empty) {
+    if (io.rule != SPX_RULE_REFERENCE && io.rule != SPX_RULE_DANTZIG && io.rule != SPX_RULE_DEVEX) {
+        set_error("%s: unknown rule %d", who, io.rule);
+        return false;
+    }
+    if (io.rule == SPX_RULE_DEVEX && !empty && !io.x) {
+        set_error("%s: rule SPX_RULE_DEVEX needs d_x (the devex weights' workspace)", who);
+        return false;
+    }
+    return true;
+}
+
 // the result of a K7 or K8 launch, with the refusal of a device that cannot co-schedule one cluster spelled out
 int check_cluster_launch(cudaError_t e, const char *who, int S, int64_t smem) {
     if (e != cudaErrorInvalidClusterSize) return check(e, who);
@@ -171,7 +184,7 @@ int solve_uniform(const char *who, int engine, int64_t B, int32_t n, int32_t m, 
     SPX_REQUIRE(!io.warm || B == 0 || (io.rowlab && io.collab), "%s: null rowlab/collab (the labels to resume from)",
                 who);
     SPX_REQUIRE(!io.warm || B == 0 || !io.obj || io.function, "%s: null function with obj", who);
-    SPX_REQUIRE(io.rule == SPX_RULE_REFERENCE || io.rule == SPX_RULE_DANTZIG, "%s: unknown rule %d", who, io.rule);
+    if (!batched_rule_ok(who, io, B == 0)) return -2;
     Route r;
     if (!route_lp(n, m, engine, forced_cluster_size(), &r)) {
         prefix_error("%s: ", who);
@@ -364,6 +377,21 @@ int spx_init_state(spx_state *d_state, int32_t *d_rowlab, int32_t *d_collab, int
 }
 
 // ---- K1 + K2 ------------------------------------------------------------------
+// The single-LP and sharded loops price with the reference and Dantzig rules; devex is a rule of the batched entries
+static bool single_lp_rule_ok(const char *who, int rule, bool reject_unknown = true) {
+    if (rule == SPX_RULE_DEVEX) {
+        set_error("%s: rule SPX_RULE_DEVEX is a rule of the batched entries only (spx_solve_batched, "
+                  "spx_solve_batched_cluster, spx_solve_batched_global, spx_solve_batched_ragged, "
+                  "spx_warm_solve_batched, spx_warm_solve_ragged)", who);
+        return false;
+    }
+    if (reject_unknown && rule != SPX_RULE_REFERENCE && rule != SPX_RULE_DANTZIG) {
+        set_error("%s: unknown rule %d", who, rule);
+        return false;
+    }
+    return true;
+}
+
 static int validate_split(const char *who, const void *A, const void *b, int n, int m, int64_t ld) {
     SPX_REQUIRE(A && b, "%s: null tableau pointer", who);
     SPX_REQUIRE(n >= 1 && m >= 0, "%s: bad shape n=%d m=%d", who, n, m);
@@ -376,7 +404,7 @@ int spx_pick(const double *d_A, const double *d_b, int32_t n, int32_t m, int64_t
              int32_t sticky, spx_state *d_state, double *d_colbuf, void *stream) {
     if (validate_split("spx_pick", d_A, d_b, n, m, ld)) return -2;
     SPX_REQUIRE(d_state && d_colbuf, "spx_pick: null state/colbuf");
-    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_pick: unknown rule %d", rule);
+    if (!single_lp_rule_ok("spx_pick", rule)) return -2;
     return check(spx_launch::pick(d_A, d_b, n, m, ld, rule, sticky, d_state, d_colbuf, as_stream(stream)),
                  "pick launch");
 }
@@ -462,7 +490,7 @@ int spx_solve(double *d_A0, double *d_A1, double *d_b0, double *d_b1, int32_t n,
     if (validate_split("spx_solve", d_A1, d_b1, n, m, ld)) return -2;
     SPX_REQUIRE(d_state && d_colbuf && d_rowlab && d_collab, "spx_solve: null state/colbuf/labels");
     SPX_REQUIRE(chunk >= 1, "spx_solve: chunk must be >= 1");
-    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_solve: unknown rule %d", rule);
+    if (!single_lp_rule_ok("spx_solve", rule)) return -2;
     SPX_REQUIRE(mode >= SPX_LOOP_AUTO && mode <= SPX_LOOP_FUSED, "spx_solve: unknown mode %d", mode);
     if (mode == SPX_LOOP_AUTO) {
         // L2-resident tableaus: one persistent kernel; big ones: look-ahead streaming; else classic
@@ -631,6 +659,7 @@ int spx_fused_pass(double *d_A0, double *d_A1, double *d_b0, double *d_b1, int32
     SPX_REQUIRE(d_state && d_work && d_rowlab && d_collab && ((uintptr_t)d_work & 127) == 0 &&
                 work_bytes >= spx_launch::fused_workspace_bytes(n, ld) && depth >= 1 && depth <= spx_launch::fuse_max() &&
                 phase >= 0 && phase <= 2, "spx_fused_pass: bad arguments");
+    if (!single_lp_rule_ok("spx_fused_pass", rule, false)) return -2;
     return check(spx_launch::fused_pass(d_A0, d_A1, d_b0, d_b1, n, m, ld, rule, depth,
                                         (int)spx_launch::get_option(SPX_OPT_FUSE_MIN_BLOCKS),
                                         (int)spx_launch::get_option(SPX_OPT_FUSE_PRICING), phase, d_state, d_work,
@@ -851,7 +880,7 @@ static int solve_ragged(const char *who, const void *h_plan, const void *d_plan,
     SPX_REQUIRE(d_plan && io.T && io.status && io.npiv, "%s: null d_plan/T/status/npiv", who);
     SPX_REQUIRE(!io.warm || (io.rowlab && io.collab), "%s: null rowlab/collab (the labels to resume from)", who);
     SPX_REQUIRE(!io.warm || !io.obj || io.function, "%s: null function with obj", who);
-    SPX_REQUIRE(io.rule == SPX_RULE_REFERENCE || io.rule == SPX_RULE_DANTZIG, "%s: unknown rule %d", who, io.rule);
+    if (!batched_rule_ok(who, io, false)) return -2;
     cudaStream_t s = as_stream(stream);
     char what[96];
     for (int i = 0; i < v.P->nlaunch; ++i) {
@@ -1050,7 +1079,7 @@ int spx_shard_candidate(const double *d_A, const double *d_b, int32_t n, int32_t
                         void *stream) {
     if (validate_split("spx_shard_candidate", d_A, d_b, n, m_loc, ld_loc)) return -2;
     SPX_REQUIRE(d_state && d_send && col0 >= 0, "spx_shard_candidate: bad arguments");
-    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_shard_candidate: unknown rule %d", rule);
+    if (!single_lp_rule_ok("spx_shard_candidate", rule)) return -2;
     return check(spx_launch::shard_candidate(d_A, d_b, n, m_loc, ld_loc, col0, rule, sticky, d_state, d_send,
                                              as_stream(stream)), "candidate launch");
 }
@@ -1058,7 +1087,7 @@ int spx_shard_candidate(const double *d_A, const double *d_b, int32_t n, int32_t
 int spx_shard_select(const double *d_gathered, int32_t nranks, const double *d_b, int32_t n, int32_t rule,
                      int32_t sticky, spx_state *d_state, double *d_colbuf, const uint64_t *d_flags,
                      uint64_t seq, void *stream) {
-    (void)rule;
+    if (!single_lp_rule_ok("spx_shard_select", rule, false)) return -2;
     SPX_REQUIRE(d_gathered && d_b && d_state && d_colbuf && nranks >= 1 && n >= 1,
                 "spx_shard_select: bad arguments");
     return check(spx_launch::shard_select(d_gathered, nranks, d_b, n, sticky, d_state, d_colbuf,
@@ -1072,7 +1101,7 @@ int spx_ahead_candidate(const double *d_A, const double *d_bin, double *d_bout, 
     if (validate_split("spx_ahead_candidate", d_A, d_bin, n, m_loc, ld_loc)) return -2;
     SPX_REQUIRE(d_bout && d_bout != d_bin && d_state && d_colbuf && d_send && col0 >= 0,
                 "spx_ahead_candidate: bad arguments");
-    SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_ahead_candidate: unknown rule %d", rule);
+    if (!single_lp_rule_ok("spx_ahead_candidate", rule)) return -2;
     return check(spx_launch::ahead_candidate(d_A, d_bin, d_bout, n, m_loc, ld_loc, col0, rule, d_state, d_colbuf,
                                              d_send, as_stream(stream)), "candidate launch");
 }

@@ -73,9 +73,43 @@ __device__ __forceinline__ int warp_ratio_decide(const Ratio &q, bool my_elig_na
     return (zero != SPX_NONE) ? zero : -1;                                 // first zero ratio, else min_val > 0
 }
 
+// Devex entering column of the f row f[0..m) under the weights w (devex_key: the minimum of (key, j)); warp-uniform
+__device__ __forceinline__ int warp_devex_entering(const double *f, const double *w, int m, int lane) {
+    unsigned long long best = ~0ull;
+    int bj = SPX_NONE;
+    for (int j = lane; j < m; j += 32) {
+        const double v = f[j];
+        if (v < 0.0) {
+            const unsigned long long k = devex_key(v, w[j]);
+            if (k < best) { best = k; bj = j; }
+        }
+    }
+    unsigned long long g = best;
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1) {
+        const unsigned long long o = __shfl_xor_sync(0xffffffffu, g, s);
+        g = o < g ? o : g;
+    }
+    return __reduce_min_sync(0xffffffffu, best == g ? bj : SPX_NONE);
+}
+
+// The devex weights w[0..m) after pivot (r, c) of the table `cur`, by one warp in place.  u_j is the cell the update
+// writes into the new pivot row; every lane reads w_c before any lane overwrites it.
+__device__ __forceinline__ void warp_devex_update(const double *cur, double *w, int m, int r, int c, int lane) {
+    const double *prow = cur + r * (m + 1);
+    const PivotDiv d = pivot_div_prepare(prow[c]);
+    const double wc = w[c];
+    __syncwarp();
+    for (int j = lane; j < m; j += 32)
+        w[j] = devex_weight(w[j], pivot_div(j == c ? 1.0 : -prow[j], d), wc, j == c);
+}
+
 // K1 + K2 by ONE warp on the shared-memory table `cur`: returns SPX_PIVOT with (r, c) or the
-// terminal status.  All 32 lanes take the same branches (ballots / redux only).
-__device__ __forceinline__ int warp_pick(const double *cur, int n, int m, int rule, int lane, int &r, int &c) {
+// terminal status.  All 32 lanes take the same branches (ballots / redux only).  DEVEX: the entering column of
+// phase 2 by the devex weights w (global memory) instead of `rule`.
+template <bool DEVEX = false>
+__device__ __forceinline__ int warp_pick(const double *cur, int n, int m, int rule, int lane, int &r, int &c,
+                                         const double *w = nullptr) {
     const int w1 = m + 1, fo = n * w1;
     // ---- K1: phase-1 row (:72-76), its first positive cell (:81-85) ...
     const int r1 = warp_first_index(n, lane, [&](int i) { return cur[i * w1 + m] < 0.0; });
@@ -86,7 +120,9 @@ __device__ __forceinline__ int warp_pick(const double *cur, int n, int m, int ru
         return SPX_PIVOT;
     }
     // ---- ... or the entering column from the f row (:94-98)
-    if (rule == SPX_RULE_REFERENCE) {
+    if constexpr (DEVEX) {
+        c = warp_devex_entering(cur + fo, w, m, lane);
+    } else if (rule == SPX_RULE_REFERENCE) {
         c = warp_first_index(m, lane, [&](int j) { return cur[fo + j] < 0.0; });
     } else {   // Dantzig: most negative, lowest index on ties
         unsigned long long best = ~0ull;
@@ -135,7 +171,9 @@ __device__ __forceinline__ bool x_label(int lab, int m) {
 // WARM == true:  a resume (spx_warm_solve_batched): labels read from a.rowlab / a.collab, f0 and f1 for obj from
 //                `function` [B][m], and no label outside [0, m) indexes xs.
 
-template <bool CTA, bool WARM>
+// DEVEX: the devex rule (SPX_RULE_DEVEX) with the weights in the LP's x slice, a.x[lp][0..m): set to 1 here, updated
+// by the warp that prices, after each pick, and overwritten by x in the epilogue.
+template <bool CTA, bool WARM, bool DEVEX = false>
 __device__ __forceinline__ void batched_solve(const BatchedArgs &a, const double *function, int warps_per_cta,
                                               int warp_doubles) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -174,6 +212,8 @@ __device__ __forceinline__ void batched_solve(const BatchedArgs &a, const double
 
     double *Tg = a.T + lp * (int64_t)cells;
     for (int k = tl; k < cells; k += nl) cur[k] = Tg[k];
+    double *w = DEVEX ? a.x + lp * m : nullptr;
+    if constexpr (DEVEX) for (int j = tl; j < m; j += nl) w[j] = 1.0;
     if constexpr (WARM) {
         for (int j = tl; j < m; j += nl) rl[j] = a.rowlab[lp * m + j];
         for (int i = tl; i < n; i += nl) cl[i] = a.collab[lp * n + i];
@@ -197,10 +237,12 @@ __device__ __forceinline__ void batched_solve(const BatchedArgs &a, const double
         }
         int r = -1, c = -1;
         if (!CTA) {
-            status = warp_pick(cur, n, m, a.rule, lane, r, c);
+            status = warp_pick<DEVEX>(cur, n, m, a.rule, lane, r, c, w);
+            if (DEVEX && status == SPX_PIVOT) warp_devex_update(cur, w, m, r, c, lane);
         } else {
             if (warp == 0) {
-                const int st = warp_pick(cur, n, m, a.rule, lane, r, c);
+                const int st = warp_pick<DEVEX>(cur, n, m, a.rule, lane, r, c, w);
+                if (DEVEX && st == SPX_PIVOT) warp_devex_update(cur, w, m, r, c, lane);
                 if (lane == 0) { s_ctl[0] = st; s_ctl[1] = r; s_ctl[2] = c; }
             }
             __syncthreads();
@@ -265,6 +307,13 @@ batched_warm_kernel(BatchedArgs a, const double *function, int warps_per_cta, in
     batched_solve<CTA, true>(a, function, warps_per_cta, warp_doubles);
 }
 
+// batched_kernel (WARM == false, function null) and batched_warm_kernel (WARM == true) under the devex rule
+template <bool CTA, bool WARM>
+__global__ void __launch_bounds__(CTA ? 512 : 256, CTA ? 1 : 6)
+batched_devex_kernel(BatchedArgs a, const double *function, int warps_per_cta, int warp_doubles) {
+    batched_solve<CTA, WARM, true>(a, function, warps_per_cta, warp_doubles);
+}
+
 // One LP of a ragged batch, start to finish: batched_kernel's loop with the shape and the offsets taken from the LP's
 // descriptor `d`, by its group of nl threads (tl = index in the group): one warp (CTA == false) or the first nl
 // threads of the CTA (CTA == true).  base: its two tables, x, labels in shared memory.  In warp mode the warps of one
@@ -273,7 +322,7 @@ batched_warm_kernel(BatchedArgs a, const double *function, int warps_per_cta, in
 // (batched_kernel keeps its own copy of the loop: it runs at the 40-register cap of its launch bounds in warp mode,
 // and any restructuring of its code moves its spills.)  WARM: the resume, as batched_solve's; gd: LP lp's descriptor
 // in global memory (d is its copy).
-template <bool CTA, bool WARM>
+template <bool CTA, bool WARM, bool DEVEX>
 __device__ __forceinline__ void ragged_body(const BatchedArgs &a, const RaggedLp &d, int64_t lp, const uint16_t *cell_i,
                                              const uint16_t *cell_j, double *base, int *s_ctl, int tl, int nl,
                                              const double *function, const RaggedLp *gd) {
@@ -294,6 +343,8 @@ __device__ __forceinline__ void ragged_body(const BatchedArgs &a, const RaggedLp
 
     double *Tg = a.T + d.t;
     for (int k = tl; k < cells; k += nl) cur[k] = Tg[k];
+    double *w = DEVEX ? a.x + d.xm : nullptr;            // batched_solve's devex weights, in the LP's x slice
+    if constexpr (DEVEX) for (int j = tl; j < m; j += nl) w[j] = 1.0;
     double c0 = 0.0, c1 = 0.0;                            // a resume: the current costs for obj
     if constexpr (WARM) {
         // The offsets come from the descriptor in global memory (gd, read once each), not from d: warp mode runs at
@@ -323,10 +374,12 @@ __device__ __forceinline__ void ragged_body(const BatchedArgs &a, const RaggedLp
         }
         int r = -1, c = -1;
         if (!CTA) {
-            status = warp_pick(cur, n, m, a.rule, lane, r, c);
+            status = warp_pick<DEVEX>(cur, n, m, a.rule, lane, r, c, w);
+            if (DEVEX && status == SPX_PIVOT) warp_devex_update(cur, w, m, r, c, lane);
         } else {
             if (warp == 0) {
-                const int st = warp_pick(cur, n, m, a.rule, lane, r, c);
+                const int st = warp_pick<DEVEX>(cur, n, m, a.rule, lane, r, c, w);
+                if (DEVEX && st == SPX_PIVOT) warp_devex_update(cur, w, m, r, c, lane);
                 if (lane == 0) { s_ctl[0] = st; s_ctl[1] = r; s_ctl[2] = c; }
             }
             group_sync();
@@ -383,7 +436,7 @@ __device__ __forceinline__ void ragged_body(const BatchedArgs &a, const RaggedLp
 // bounds as batched_kernel<false>.  CTA mode: slot = CTA; the CTA is launched at the warp count of
 // the largest LP of the launch, builds the lookup table of its own LP, and only the warps its LP needs stay (the
 // warp count the uniform entry gives that shape: 32 cells per warp, 2..16 warps).
-template <bool CTA, bool WARM>
+template <bool CTA, bool WARM, bool DEVEX = false>
 __device__ __forceinline__ void ragged_batched(const BatchedArgs &a, const RaggedLp *__restrict__ lps,
                                                const int32_t *__restrict__ order, int warps_per_cta, int warp_doubles,
                                                const double *function) {
@@ -407,7 +460,7 @@ __device__ __forceinline__ void ragged_batched(const BatchedArgs &a, const Ragge
         }
         __syncwarp();
         double *base = reinterpret_cast<double *>(slot_raw + WARP_LUT_BYTES);
-        ragged_body<false, WARM>(a, d, lp, cell_i, cell_j, base, s_ctl, lane, 32, function, lps + lp);
+        ragged_body<false, WARM, DEVEX>(a, d, lp, cell_i, cell_j, base, s_ctl, lane, 32, function, lps + lp);
         return;
     }
     const int64_t lp = order[slot];
@@ -427,7 +480,7 @@ __device__ __forceinline__ void ragged_batched(const BatchedArgs &a, const Ragge
     if ((int)threadIdx.x >= nl) return;
     const size_t lut_bytes = ((size_t)cells * 4 + 15) / 16 * 16;
     double *base = reinterpret_cast<double *>(smem_raw + lut_bytes);
-    ragged_body<true, WARM>(a, d, lp, cell_i, cell_j, base, s_ctl, (int)threadIdx.x, nl, function, lps + lp);
+    ragged_body<true, WARM, DEVEX>(a, d, lp, cell_i, cell_j, base, s_ctl, (int)threadIdx.x, nl, function, lps + lp);
 }
 
 template <bool CTA>
@@ -443,6 +496,14 @@ __global__ void __launch_bounds__(CTA ? 512 : 256, CTA ? 1 : 6)
 ragged_batched_warm_kernel(BatchedArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
                            int warps_per_cta, int warp_doubles, const double *function) {
     ragged_batched<CTA, true>(a, lps, order, warps_per_cta, warp_doubles, function);
+}
+
+// ragged_batched_kernel (WARM == false, function null) and ragged_batched_warm_kernel (WARM == true) under the devex rule
+template <bool CTA, bool WARM>
+__global__ void __launch_bounds__(CTA ? 512 : 256, CTA ? 1 : 6)
+ragged_batched_devex_kernel(BatchedArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
+                            int warps_per_cta, int warp_doubles, const double *function) {
+    ragged_batched<CTA, WARM, true>(a, lps, order, warps_per_cta, warp_doubles, function);
 }
 
 size_t warp_bytes(int n, int m) {
@@ -509,6 +570,9 @@ cudaError_t solve_batched(int64_t B, int n, int m, int max_pivots, const BatchIO
         // 891 k pivots/s, 64: 730 k, 128: 623 k), 2..16 warps
         int warps = (int)((cells + CTA_CELLS_PER_WARP - 1) / CTA_CELLS_PER_WARP);
         warps = warps < 2 ? 2 : (warps > 16 ? 16 : warps);
+        if (io.rule == SPX_RULE_DEVEX)
+            return io.warm ? launch_k4<batched_devex_kernel<true, true>>(B, warps * 32, lb + wb, stream, a, io.function, 1, wd)
+                           : launch_k4<batched_devex_kernel<true, false>>(B, warps * 32, lb + wb, stream, a, nullptr, 1, wd);
         if (io.warm) return launch_k4<batched_warm_kernel<true>>(B, warps * 32, lb + wb, stream, a, io.function, 1, wd);
         return launch_k4<batched_kernel<true>>(B, warps * 32, lb + wb, stream, a, 1, wd);
     }
@@ -520,6 +584,9 @@ cudaError_t solve_batched(int64_t B, int n, int m, int max_pivots, const BatchIO
     if ((int64_t)wpc > B) wpc = (int)B;
     const size_t smem = lb + (size_t)wpc * wb;
     const int64_t ctas = (B + wpc - 1) / wpc;
+    if (io.rule == SPX_RULE_DEVEX)
+        return io.warm ? launch_k4<batched_devex_kernel<false, true>>(ctas, wpc * 32, smem, stream, a, io.function, wpc, wd)
+                       : launch_k4<batched_devex_kernel<false, false>>(ctas, wpc * 32, smem, stream, a, nullptr, wpc, wd);
     if (io.warm) return launch_k4<batched_warm_kernel<false>>(ctas, wpc * 32, smem, stream, a, io.function, wpc, wd);
     return launch_k4<batched_kernel<false>>(ctas, wpc * 32, smem, stream, a, wpc, wd);
 }
@@ -553,6 +620,18 @@ cudaError_t solve_ragged_batched(const PlanView &v, const RaggedLaunch &l, const
     const int64_t ctas = (l.count + l.per_cta - 1) / l.per_cta;
     const size_t smem = (size_t)l.smem;
     const int32_t *order = v.d_order + l.first;
+    const double *fn = io.warm ? io.function : nullptr;
+    if (io.rule == SPX_RULE_DEVEX) {
+        if (l.kernel == RAGGED_CTA)
+            return io.warm ? launch_k4<ragged_batched_devex_kernel<true, true>>(ctas, l.threads, smem, stream, a, v.d_lps,
+                                                                               order, 1, 0, fn)
+                           : launch_k4<ragged_batched_devex_kernel<true, false>>(ctas, l.threads, smem, stream, a, v.d_lps,
+                                                                                order, 1, 0, fn);
+        return io.warm ? launch_k4<ragged_batched_devex_kernel<false, true>>(ctas, l.threads, smem, stream, a, v.d_lps,
+                                                                            order, l.per_cta, (int)l.slot_doubles, fn)
+                       : launch_k4<ragged_batched_devex_kernel<false, false>>(ctas, l.threads, smem, stream, a, v.d_lps,
+                                                                             order, l.per_cta, (int)l.slot_doubles, fn);
+    }
     if (l.kernel == RAGGED_CTA)
         return io.warm ? launch_k4<ragged_batched_warm_kernel<true>>(ctas, l.threads, smem, stream, a, v.d_lps, order,
                                                                      1, 0, io.function)

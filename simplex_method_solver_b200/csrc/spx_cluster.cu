@@ -41,7 +41,7 @@ using namespace spx;
 // WARM == true: a resume (spx_warm_solve_*): each CTA reads the labels of its band and of its header slice from
 // a.rowlab / a.collab, f0 and f1 for obj come from `function` (packed as x) in the epilogue, and no label outside
 // [0, m) indexes x or s_x01.
-template <bool RAGGED, bool WARM>
+template <bool RAGGED, bool WARM, bool DEVEX = false>
 __device__ __forceinline__ void cluster_body(const ClusterArgs &a, const RaggedLp *__restrict__ lps,
                                              const int32_t *__restrict__ order, const double *function) {
     cg::cluster_group cluster = cg::this_cluster();
@@ -84,6 +84,11 @@ __device__ __forceinline__ void cluster_body(const ClusterArgs &a, const RaggedL
         for (int j = tid; j < cols; j += nt) rl[j] = j0 + j;
     }
     if (tid < 2) s_x01[tid] = 0.0;
+    // devex: the weights in the LP's x slice (DevexPrev, spx_cluster.cuh), w(0) = 1 stored by each slice's owner
+    double *wg = DEVEX ? a.x + (RAGGED ? d.xm : lp * m) : nullptr;
+    if constexpr (DEVEX) for (int j = tid; j < cols; j += nt) wg[j0 + j] = 1.0;
+    DevexPrev dv;
+    dv.c = -1;
     cluster.sync();                                        // every CTA runs and is loaded before any DSMEM access
     const double f0 = (m >= 1) ? f[0] : 0.0;               // self.function is never mutated (:29,:49)
     const double f1 = (m >= 2) ? f[1] : 0.0;
@@ -100,7 +105,13 @@ __device__ __forceinline__ void cluster_body(const ClusterArgs &a, const RaggedL
             if (rank == 0) for (int j = tid; j < m; j += nt) sg[fo + j] = f[j];
         }
         // ---- K1: entering column of the f row (:94-98), the same in every CTA
-        const int cf = f_row_entering(f, m, a.rule, sc);
+        int cf;
+        if constexpr (DEVEX) {
+            if (dv.c >= 0) dv.wc = ld_l2(wg + dv.c);
+            cf = devex_entering(f, m, [&](int j) { return devex_weight_now(wg, prow, dv, j); }, sc);
+        } else {
+            cf = f_row_entering(f, m, a.rule, sc);
+        }
         // ---- one pass over the band: phase-1 row (:72-76) and the ratio scan of column cf (:107-136)
         Ratio q = ratio_identity();
         int key = SPX_NONE, bneg = SPX_NONE;
@@ -136,7 +147,10 @@ __device__ __forceinline__ void cluster_body(const ClusterArgs &a, const RaggedL
         // ---- stash the old pivot row (from its owner) and the band's old pivot-column entries
         const int owner = r / R, holder = c / Q;           // owners of row r and of the header label of column c
         const double *orow = cluster.map_shared_rank(band, owner) + (size_t)(r - owner * R) * w1;
-        for (int j = tid; j < w1; j += nt) prow[j] = orow[j];
+        for (int j = tid; j < w1; j += nt) {
+            if (DEVEX && dv.c >= 0 && j >= j0 && j < j0 + cols) wg[j] = devex_weight_now(wg, prow, dv, j);   // w(k)
+            prow[j] = orow[j];
+        }
         for (int i = tid; i < rows; i += nt) pcol[i] = band[i * w1 + c];
         const double fc = f[c];
         int32_t lab_r = 0, lab_c = 0;                      // :152, old labels read before B, written after B
@@ -151,6 +165,7 @@ __device__ __forceinline__ void cluster_body(const ClusterArgs &a, const RaggedL
         // :173-175 the rest) differ only in the numerator, so one division by the pivot serves them all
         const double p = prow[c];
         const PivotDiv d = pivot_div_prepare(p);
+        if constexpr (DEVEX) { dv.c = c; dv.d = d; }
         for (int k = tid; k < bandcells; k += nt) {
             int i = __float2int_rz((float)k * inv_w1), j = k - i * w1;     // k < 2^24: off by at most one row
             if (j < 0) { --i; j += w1; } else if (j >= w1) { ++i; j -= w1; }
@@ -229,6 +244,15 @@ ragged_cluster_warm_kernel(ClusterArgs a, const RaggedLp *__restrict__ lps, cons
     cluster_body<true, true>(a, lps, order, function);
 }
 
+// the four kernels above under the devex rule (SPX_RULE_DEVEX): RAGGED as the ragged_ ones, WARM as the _warm_ ones
+// (function null for a fresh solve)
+template <bool RAGGED, bool WARM>
+__global__ void __launch_bounds__(CLUSTER_THREADS, 1)
+cluster_devex_kernel(ClusterArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
+                     const double *function) {
+    cluster_body<RAGGED, WARM, true>(a, lps, order, function);
+}
+
 // the per-CTA footprint of the header comment, for S CTAs per LP
 int64_t cluster_bytes(int64_t n, int64_t m, int S) {
     const int64_t R = (n + S - 1) / S, Q = (m + S - 1) / S;
@@ -255,6 +279,11 @@ int cluster_size(int64_t n, int64_t m) {
 cudaError_t solve_batched_cluster(int64_t B, int n, int m, int S, int max_pivots, const BatchIO &io,
                                   cudaStream_t stream) {
     const ClusterArgs a = cluster_args(io, B, n, m, S, max_pivots);
+    if (io.rule == SPX_RULE_DEVEX)
+        return io.warm ? launch_cluster_kernel<cluster_devex_kernel<false, true>>(S, B, cluster_bytes(n, m, S), stream, a,
+                                                                                 nullptr, nullptr, io.function)
+                       : launch_cluster_kernel<cluster_devex_kernel<false, false>>(S, B, cluster_bytes(n, m, S), stream,
+                                                                                  a, nullptr, nullptr, nullptr);
     if (io.warm) return launch_cluster_kernel<cluster_warm_kernel>(S, B, cluster_bytes(n, m, S), stream, a, io.function);
     return launch_cluster_kernel<cluster_kernel>(S, B, cluster_bytes(n, m, S), stream, a);
 }
@@ -266,6 +295,11 @@ int64_t ragged_cluster_bytes(int n, int m, int S) { return cluster_bytes(n, m, S
 cudaError_t solve_ragged_cluster(const PlanView &v, const RaggedLaunch &l, const BatchIO &io, cudaStream_t stream) {
     const ClusterArgs a = cluster_args(io, l.count, 0, 0, l.S, 0);
     const int32_t *order = v.d_order + l.first;
+    if (io.rule == SPX_RULE_DEVEX)
+        return io.warm ? launch_cluster_kernel<cluster_devex_kernel<true, true>>(l.S, l.count, l.smem, stream, a, v.d_lps,
+                                                                                order, io.function)
+                       : launch_cluster_kernel<cluster_devex_kernel<true, false>>(l.S, l.count, l.smem, stream, a, v.d_lps,
+                                                                                 order, nullptr);
     if (io.warm)
         return launch_cluster_kernel<ragged_cluster_warm_kernel>(l.S, l.count, l.smem, stream, a, v.d_lps, order,
                                                                  io.function);

@@ -28,6 +28,48 @@ struct EqKey {          // Dantzig: the f cell whose orderable image is the mini
     __device__ bool operator()(double v) const { return v < 0.0 && orderable(v) == key; }
 };
 
+// a read of global memory another CTA of the cluster writes: from L2 (ld.global.cg), never a stale L1 line
+__device__ __forceinline__ double ld_l2(const double *p) {
+    double v;
+    asm volatile("ld.global.cg.f64 %0, [%1];" : "=d"(v) : "l"(p));
+    return v;
+}
+
+// ---- devex (SPX_RULE_DEVEX) in a cluster: one copy of the weights per LP in its x slice wg[0..m), ONE PIVOT BEHIND.
+// During the pricing of pivot k, wg holds w(k-1) (w(0) = 1 at pivot 0); every CTA prices with w(k) = w(k-1) updated by
+// pivot k-1 on the fly, from its pivot-row stash (still pivot k-1's row) and w(k-1)[c(k-1)].  Between barriers A(k)
+// and B(k), the owner of the header slice [j0, j0+Q) stores w(k) over w(k-1) there: every CTA has read w(k-1) before A
+// (pricing), nobody reads wg again before B, and the store reads the stash before the CTA overwrites it with pivot
+// k's row.  No barrier and no shared memory is added, and every CTA computes the same bits.
+struct DevexPrev {
+    int      c;     // column of the previous pivot, -1 before the first
+    PivotDiv d;     // its pivot
+    double   wc;    // w(k-1)[c], read in pricing k
+};
+
+// w(k)[j] from wg (= w(k-1)) and the previous pivot's row stash prow
+__device__ __forceinline__ double devex_weight_now(const double *wg, const double *prow, const DevexPrev &pv, int j) {
+    const double wj = ld_l2(wg + j);
+    if (pv.c < 0) return wj;
+    return devex_weight(wj, pivot_div(j == pv.c ? 1.0 : -prow[j], pv.d), pv.wc, j == pv.c);
+}
+
+// K1 under devex: the minimum of (devex_key, j) over the candidates f_j < 0, weight(j) = w_j; the whole CTA calls it
+template <class Weight>
+__device__ __forceinline__ int devex_entering(const double *f, int m, Weight weight, Scratch &sc) {
+    unsigned long long best = ~0ull;
+    int bj = SPX_NONE;
+    for (int j = (int)threadIdx.x; j < m; j += (int)blockDim.x) {
+        const double v = f[j];
+        if (v < 0.0) {
+            const unsigned long long k = devex_key(v, weight(j));
+            if (k < best) { best = k; bj = j; }
+        }
+    }
+    const unsigned long long g = block_min_u64(best, sc);
+    return block_min_int(best == g ? bj : SPX_NONE, sc);
+}
+
 // K1: the entering column of the f row (:94-98), SPX_NONE when there is none; the whole CTA calls it
 __device__ __forceinline__ int f_row_entering(const double *f, int m, int rule, Scratch &sc) {
     if (rule == SPX_RULE_REFERENCE) return block_first_index(f, m, IsNeg(), sc);

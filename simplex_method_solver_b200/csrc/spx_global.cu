@@ -43,11 +43,6 @@ using namespace spx;
 constexpr int    GLOBAL_MIN_CTAS  = 1;
 constexpr int    GLOBAL_UNROLL    = 6;
 
-__device__ __forceinline__ double ld_l2(const double *p) {
-    double v;
-    asm volatile("ld.global.cg.f64 %0, [%1];" : "=d"(v) : "l"(p));
-    return v;
-}
 __device__ __forceinline__ double2 ld_l2_v2(const double *p) {
     double2 v;
     asm volatile("ld.global.cg.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "l"(p));
@@ -57,7 +52,7 @@ __device__ __forceinline__ double2 ld_l2_v2(const double *p) {
 // The body of both kernels.  RAGGED == false: shape, R, Q and offsets from the arguments (one shape per launch).
 // RAGGED == true: LP order[blockIdx.x / S] of a ragged batch, its shape and offsets from lps[], R and Q from its shape
 // (as cluster_body in spx_cluster.cu).  WARM == true: a resume, as cluster_body's.
-template <bool RAGGED, bool WARM>
+template <bool RAGGED, bool WARM, bool DEVEX = false>
 __device__ __forceinline__ void global_body(const ClusterArgs &a, const RaggedLp *__restrict__ lps,
                                             const int32_t *__restrict__ order, const double *function) {
     cg::cluster_group cluster = cg::this_cluster();
@@ -106,6 +101,11 @@ __device__ __forceinline__ void global_body(const ClusterArgs &a, const RaggedLp
         for (int j = tid; j < cols; j += nt) rl[j] = j0 + j;
     }
     if (tid < 2) s_x01[tid] = 0.0;
+    // devex: the weights in the LP's x slice (DevexPrev, spx_cluster.cuh), w(0) = 1 stored by each slice's owner
+    double *wg = DEVEX ? a.x + (RAGGED ? lpd.xm : lp * m) : nullptr;
+    if constexpr (DEVEX) for (int j = tid; j < cols; j += nt) wg[j0 + j] = 1.0;
+    DevexPrev dv;
+    dv.c = -1;
     cluster.sync();                                        // every CTA runs and is loaded before any DSMEM access
     const double f0 = (m >= 1) ? f[0] : 0.0;               // self.function is never mutated (:29,:49)
     const double f1 = (m >= 2) ? f[1] : 0.0;
@@ -121,7 +121,13 @@ __device__ __forceinline__ void global_body(const ClusterArgs &a, const RaggedLp
             if (rank == 0) for (int j = tid; j < m; j += nt) sg[fo + j] = f[j];
         }
         // ---- K1: entering column of the f row (:94-98), the same in every CTA
-        const int cf = f_row_entering(f, m, a.rule, sc);
+        int cf;
+        if constexpr (DEVEX) {
+            if (dv.c >= 0) dv.wc = ld_l2(wg + dv.c);
+            cf = devex_entering(f, m, [&](int j) { return devex_weight_now(wg, prow, dv, j); }, sc);
+        } else {
+            cf = f_row_entering(f, m, a.rule, sc);
+        }
         // ---- one pass over the band's rows: phase-1 row (:72-76) and the ratio scan of column cf (:107-136)
         Ratio q = ratio_identity();
         int key = SPX_NONE, bneg = SPX_NONE;
@@ -162,7 +168,10 @@ __device__ __forceinline__ void global_body(const ClusterArgs &a, const RaggedLp
         const int owner = r / R, holder = c / Q;           // owners of row r and of the header label of column c
         // row r was written by its owner before barrier A (the update of the previous pivot): read from L2
         const double *orow = Tg + (int64_t)r * w1;
-        for (int j = tid; j < w1; j += nt) prow[j] = ld_l2(orow + j);
+        for (int j = tid; j < w1; j += nt) {
+            if (DEVEX && dv.c >= 0 && j >= j0 && j < j0 + cols) wg[j] = devex_weight_now(wg, prow, dv, j);   // w(k)
+            prow[j] = ld_l2(orow + j);
+        }
         for (int i = tid; i < rows; i += nt) pcol[i] = ld_l2(band + (int64_t)i * w1 + c);
         const double fc = f[c];
         int32_t lab_r = 0, lab_c = 0;                      // :152, old labels read before B, written after B
@@ -177,6 +186,7 @@ __device__ __forceinline__ void global_body(const ClusterArgs &a, const RaggedLp
         // :173-175 the rest) differ only in the numerator, so one division by the pivot serves them all
         const double p = prow[c];
         const PivotDiv d = pivot_div_prepare(p);
+        if constexpr (DEVEX) { dv.c = c; dv.d = d; }
         const int rloc = r - r0;                           // the pivot row in band coordinates (may be outside)
         auto cell = [&](double t, int i, int j) {
             const double ci = pcol[i];
@@ -288,6 +298,15 @@ ragged_global_warm_kernel(ClusterArgs a, const RaggedLp *__restrict__ lps, const
     global_body<true, true>(a, lps, order, function);
 }
 
+// the four kernels above under the devex rule (SPX_RULE_DEVEX): RAGGED as the ragged_ ones, WARM as the _warm_ ones
+// (function null for a fresh solve)
+template <bool RAGGED, bool WARM>
+__global__ void __launch_bounds__(CLUSTER_THREADS, GLOBAL_MIN_CTAS)
+global_devex_kernel(ClusterArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
+                    const double *function) {
+    global_body<RAGGED, WARM, true>(a, lps, order, function);
+}
+
 // the per-CTA footprint of the header comment, for S CTAs per LP
 int64_t global_bytes(int64_t n, int64_t m, int S) {
     const int64_t R = (n + S - 1) / S, Q = (m + S - 1) / S;
@@ -350,6 +369,11 @@ cudaError_t global_cluster_size(int64_t n, int64_t m, int64_t B, int *S_out) {
 cudaError_t solve_batched_global(int64_t B, int n, int m, int S, int max_pivots, const BatchIO &io,
                                  cudaStream_t stream) {
     const ClusterArgs a = cluster_args(io, B, n, m, S, max_pivots);
+    if (io.rule == SPX_RULE_DEVEX)
+        return io.warm ? launch_cluster_kernel<global_devex_kernel<false, true>>(S, B, global_bytes(n, m, S), stream, a,
+                                                                                nullptr, nullptr, io.function)
+                       : launch_cluster_kernel<global_devex_kernel<false, false>>(S, B, global_bytes(n, m, S), stream, a,
+                                                                                 nullptr, nullptr, nullptr);
     if (io.warm) return launch_cluster_kernel<global_warm_kernel>(S, B, global_bytes(n, m, S), stream, a, io.function);
     return launch_cluster_kernel<global_kernel>(S, B, global_bytes(n, m, S), stream, a);
 }
@@ -376,6 +400,11 @@ cudaError_t solve_ragged_global(const PlanView &v, const RaggedLaunch &l, int S,
                                 cudaStream_t stream) {
     const ClusterArgs a = cluster_args(io, l.count, 0, 0, S, 0);
     const int32_t *order = v.d_order + l.first;
+    if (io.rule == SPX_RULE_DEVEX)
+        return io.warm ? launch_cluster_kernel<global_devex_kernel<true, true>>(S, l.count, smem, stream, a, v.d_lps, order,
+                                                                               io.function)
+                       : launch_cluster_kernel<global_devex_kernel<true, false>>(S, l.count, smem, stream, a, v.d_lps,
+                                                                                order, nullptr);
     if (io.warm)
         return launch_cluster_kernel<ragged_global_warm_kernel>(S, l.count, smem, stream, a, v.d_lps, order,
                                                                 io.function);

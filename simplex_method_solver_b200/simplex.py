@@ -95,6 +95,11 @@ class SimplexMethod:
         self.function = function                             # :29 (same object, never mutated)
         self.row = ['x' + str(k) for k in range(1, self.m + 1)] + ['-b']      # :30,:32
         self.column = ['y' + str(k) for k in range(1, self.n + 1)] + ['f']    # :31,:33
+        if rule == "devex":
+            # get_solution() runs the batched kernels in rounds of growing caps, each a fresh solve from unit weights,
+            # so the pivots would depend on the round sizes
+            raise ValueError("rule='devex' is a rule of the batched API only: batched.solve_batched, "
+                             "batched.solve_ragged, batched.resolve, DeviceBatch and DeviceRaggedBatch")
         if rule not in N.RULES:
             raise ValueError(f"unknown rule {rule!r}")
         if engine not in ("auto", "warp", "stream", "sharded", "cluster", "global"):

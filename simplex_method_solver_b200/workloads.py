@@ -101,6 +101,20 @@ def mixed_lps(B: int, seed: int = 0):
     return out
 
 
+def scaled_lps(B: int, seed: int = 0):
+    """mixed_lps(B, seed) with the units of every x_j changed: column j of the constraints and c_j multiplied by
+    10^U(-2, 2) (draws from seed + 7, one per column of each LP in turn).  The same LPs up to scale, so the pivot counts
+    of the scale-dependent entering rules (reference, Dantzig) and of devex can be compared on badly scaled inputs.
+    Returns a list of B (rows [n, m+1], c [m]) pairs."""
+    g = np.random.default_rng(seed + 7)
+    out = []
+    for rows, c in mixed_lps(B, seed):
+        s = 10.0 ** g.uniform(-2.0, 2.0, c.shape[0])
+        rows[:, : c.shape[0]] *= s
+        out.append((rows, c * s))
+    return out
+
+
 def mixed_large_lps(B: int = 1024, seed: int = 0):
     """mixed_lps(B, seed) with cap 20,000 each, then 32 LPs above K7's capacity with cap 4,000 each: 8 each of
     D(600, 800), phase-1 1000 x 1000, D(2000, 300) and D(64, 12000), in that order (seeds seed * 1_000_003 + B + q
