@@ -65,6 +65,17 @@ extern "C" {
  * spx_warm_solve_batched, spx_warm_solve_ragged): there d_x is required, it is the weights' workspace until the
  * epilogue writes x.  Every single-LP and sharded entry rejects it. */
 #define SPX_RULE_DEVEX     2
+/* Dantzig with Bland's rule on degenerate pivots, and a ratio-tested phase 1.  t = the lowest row with b < 0.  Phase 1
+ * (t exists): the candidates are the j with T[t][j] > 0 (none: SPX_INCORRECT); phase 2: the j with f_j < 0 (none:
+ * SPX_OPTIMAL).  c_D = the candidate with the largest T[t][j] (phase 1) or -f_j (phase 2), lowest j on ties; c_B = the
+ * candidate with the lowest header label.  The leaving row of column c is the least (ratio, not target, row label, i)
+ * over row t (ratio (0 - b_t) / T[t][c]) and the rows i != t with T[i][c] < 0 and !(b_i < 0) (ratio
+ * b_i / (0 - T[i][c])); ratios compare by value, -0 = +0, NaN after every number; no row: SPX_NOCONV.  The pivot is
+ * (leave(c_D), c_D) unless that ratio is +-0, then (leave(c_B), c_B).  A feasible row stays feasible, and the rule
+ * ends in exact arithmetic (DESIGN.md, "Dantzig with Bland's rule on degenerate pivots").  Stateless: a capped solve
+ * and its resume pivot as one uncapped solve.  Batched entries only, as SPX_RULE_DEVEX, without its need of d_x. */
+#define SPX_RULE_DANTZIG_BLAND 4
+/* 3 is not a rule: every entry refuses it as unknown */
 
 /* Device-resident solver state, 128 bytes.  Written by the pick kernels, read
  * by the update kernels, so a whole chunk of pivots can be enqueued with no host

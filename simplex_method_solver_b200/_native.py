@@ -19,13 +19,16 @@ LOOP_MODES = {None: LOOP_AUTO, "auto": LOOP_AUTO, False: LOOP_CLASSIC, "classic"
               True: LOOP_LOOKAHEAD, "lookahead": LOOP_LOOKAHEAD, "resident": LOOP_RESIDENT,
               "fused": LOOP_FUSED}
 PIVOT, OPTIMAL, INCORRECT, NOCONV, CAP, PEER_TIMEOUT = 1, 0, -1, -2, -3, -4
-RULE_REFERENCE, RULE_DANTZIG, RULE_DEVEX = 0, 1, 2
+RULE_REFERENCE, RULE_DANTZIG, RULE_DEVEX, RULE_DANTZIG_BLAND = 0, 1, 2, 4
 # keys 1, 3, 4, 10 and 15 are retired (include/spx_b200.h)
 OPT_TILED_MIN_BLOCKS, OPT_TILED_ROWS, OPT_FUSE_DEPTH = 2, 5, 6
 OPT_FUSE_MIN_BLOCKS, OPT_FUSE_PRICING, OPT_FUSE_LOOKAHEAD, OPT_FUSE_TILE_ROWS, OPT_FUSE_PAIRS = 7, 8, 9, 11, 12
 OPT_SHARD_THREADS, OPT_SHARD_CTAS, OPT_CLUSTER_SIZE = 13, 14, 16
-# "devex" (reference weights, include/spx_b200.h) is a rule of the batched engines only (batched.py)
-RULES = {"reference": RULE_REFERENCE, "bland": RULE_REFERENCE, "dantzig": RULE_DANTZIG, "devex": RULE_DEVEX}
+# "devex" (reference weights) and "dantzig_bland" (Dantzig with Bland's rule on degenerate pivots and a ratio-tested
+# phase 1), include/spx_b200.h, are rules of the batched engines only (batched.py).  "bland" is the reference's
+# first-negative entering, not "dantzig_bland".
+RULES = {"reference": RULE_REFERENCE, "bland": RULE_REFERENCE, "dantzig": RULE_DANTZIG, "devex": RULE_DEVEX,
+         "dantzig_bland": RULE_DANTZIG_BLAND}
 ENGINE_AUTO, ENGINE_SMEM, ENGINE_CLUSTER, ENGINE_GLOBAL, ENGINE_AUTO_GLOBAL = 0, 1, 2, 4, 5
 
 # the two ValueError texts of pick_element(), /root/reference/src/simplex.py:89,139

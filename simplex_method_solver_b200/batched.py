@@ -245,7 +245,7 @@ class DeviceBatch:
 
     def run(self, rule: int = N.RULE_REFERENCE):
         """Launch the solver on the resident batch (asynchronous on the current stream).  Under ``N.RULE_DEVEX`` the
-        x buffer holds the weights until the kernel writes x."""
+        x buffer holds the weights until the kernel writes x.  ``N.RULE_DANTZIG_BLAND`` is a rule of this call too."""
         with torch.cuda.device(self.device):
             entry = _ENTRIES[self.kernel]
             N.call(entry, self.T.data_ptr(), self.B, self.n, self.m, rule, self.max_pivots, self.x.data_ptr(), self.obj.data_ptr(), self.status.data_ptr(),
@@ -288,7 +288,8 @@ class DeviceBatch:
         """Continue every LP from its resident table and labels for up to ``max_pivots`` more pivots, on this
         batch's engine (``spx_warm_solve_batched``).  function: [B, m] or [m], the LPs' current costs, used only
         for ``obj``.  Trace and snapshots count from 0 again.  Under ``N.RULE_DEVEX`` the weights restart at 1, so
-        a capped devex solve and its resume do not pivot as one uncapped solve (they do under the other rules).
+        a capped devex solve and its resume do not pivot as one uncapped solve (they do under the other rules,
+        ``N.RULE_DANTZIG_BLAND`` included: it reads only the table and the labels).
         Asynchronous on the current stream."""
         fn = _per_lp(function, self.B, self.m, "function")
         self._function = torch.from_numpy(fn).to(self.device) if self.B else None    # alive until the kernel ran
@@ -323,8 +324,9 @@ def solve_batched(tables, n: int, m: int, max_pivots: int = 64, rule: str = "ref
     ``SimplexMethod(constraints, function)`` for each LP.
     engine: "auto" (K4 when the LP fits one CTA, else K7), "smem" (K4), "cluster" (K7) or "global" (K8).
     rule: "reference" (first negative f cell enters), "dantzig" (most negative) or "devex" (largest f_j^2 / w_j
-    under Forrest-Goldfarb reference weights w, include/spx_b200.h: far fewer pivots on badly scaled LPs).  Phase 1
-    and the leaving row are the reference's under every rule.
+    under Forrest-Goldfarb reference weights w, include/spx_b200.h: far fewer pivots on badly scaled LPs); under
+    these three, phase 1 and the leaving row are the reference's.  "dantzig_bland" (include/spx_b200.h) is Dantzig
+    with a ratio-tested phase 1 and Bland's rule on degenerate pivots: it ends LPs on which the others cycle.
     """
     tables = np.ascontiguousarray(np.asarray(tables, dtype=np.float64))
     if tables.ndim != 2 or tables.shape[1] != n * (m + 1) + m:
@@ -558,7 +560,7 @@ class DeviceRaggedBatch:
         self.T[: self.totals[0]].copy_(src, non_blocking=non_blocking)
 
     def run(self, rule: int = N.RULE_REFERENCE):
-        """Launch the plan on the resident batch (asynchronous on the current stream)."""
+        """Launch the plan on the resident batch (asynchronous on the current stream); rule as ``DeviceBatch.run``."""
         with torch.cuda.device(self.device):
             N.call("spx_solve_batched_ragged", self.T.data_ptr(), self.plan.plan.ctypes.data, self.d_plan.data_ptr(),
                    rule, self.x.data_ptr(), self.obj.data_ptr(), self.status.data_ptr(), self.npiv.data_ptr(),
@@ -651,7 +653,7 @@ def solve_ragged(lps, max_pivots: Union[int, Sequence[int]] = 64, rule: str = "r
     Each LP's results are, bit for bit, those ``solve_batched`` returns for that LP alone
     (``RaggedResult.lp(k)``).  engine: "auto" (per LP, K4 when it fits one CTA, else K7),
     "auto_global" (as "auto", and K8 above K7's capacity), or "smem", "cluster" or "global"
-    for every LP.
+    for every LP.  rule: as ``solve_batched``'s ("reference", "dantzig", "devex" or "dantzig_bland").
     """
     shapes, packed = pack_ragged(lps)
     db = DeviceRaggedBatch(shapes, max_pivots, trace, snapshots, device, engine)
@@ -779,6 +781,7 @@ def resolve(result: Union[BatchResult, RaggedResult], data, rhs=None, cost=None,
     [sum m]) or one array per LP.  None keeps the old values; with neither, the LPs simply continue.
     The final tables and labels are uploaded, changed by delta = new - old (``change``) and resumed for up
     to max_pivots more pivots with function = the new costs (``resume``); under rule="devex" from unit weights.
+    rule="dantzig_bland" keeps no state, so a resume without changes pivots on as one longer solve would.
     Returns the result type given.
     Non-finite deltas, labels that are not a permutation of 0..n+m-1 and shapes that do not match are
     ValueErrors naming the LP.

@@ -152,9 +152,11 @@ bool route_lp(int n, int m, int engine, int forced, Route *r) {
 
 int forced_cluster_size() { return (int)spx_launch::get_option(SPX_OPT_CLUSTER_SIZE); }
 
-// The rule of a batched entry: reference, Dantzig or devex; devex keeps its weights in d_x, so d_x is required
+// The rule of a batched entry: reference, Dantzig, devex or Dantzig-Bland; devex keeps its weights in d_x, so d_x is
+// required
 bool batched_rule_ok(const char *who, const spx::BatchIO &io, bool empty) {
-    if (io.rule != SPX_RULE_REFERENCE && io.rule != SPX_RULE_DANTZIG && io.rule != SPX_RULE_DEVEX) {
+    if (io.rule != SPX_RULE_REFERENCE && io.rule != SPX_RULE_DANTZIG && io.rule != SPX_RULE_DEVEX &&
+        io.rule != SPX_RULE_DANTZIG_BLAND) {
         set_error("%s: unknown rule %d", who, io.rule);
         return false;
     }
@@ -377,12 +379,14 @@ int spx_init_state(spx_state *d_state, int32_t *d_rowlab, int32_t *d_collab, int
 }
 
 // ---- K1 + K2 ------------------------------------------------------------------
-// The single-LP and sharded loops price with the reference and Dantzig rules; devex is a rule of the batched entries
+// The single-LP and sharded loops price with the reference and Dantzig rules; devex and Dantzig-Bland are rules of the
+// batched entries
 static bool single_lp_rule_ok(const char *who, int rule, bool reject_unknown = true) {
-    if (rule == SPX_RULE_DEVEX) {
-        set_error("%s: rule SPX_RULE_DEVEX is a rule of the batched entries only (spx_solve_batched, "
+    if (rule == SPX_RULE_DEVEX || rule == SPX_RULE_DANTZIG_BLAND) {
+        set_error("%s: rule %s is a rule of the batched entries only (spx_solve_batched, "
                   "spx_solve_batched_cluster, spx_solve_batched_global, spx_solve_batched_ragged, "
-                  "spx_warm_solve_batched, spx_warm_solve_ragged)", who);
+                  "spx_warm_solve_batched, spx_warm_solve_ragged)", who,
+                  rule == SPX_RULE_DEVEX ? "SPX_RULE_DEVEX" : "SPX_RULE_DANTZIG_BLAND");
         return false;
     }
     if (reject_unknown && rule != SPX_RULE_REFERENCE && rule != SPX_RULE_DANTZIG) {

@@ -154,6 +154,66 @@ __device__ __forceinline__ int warp_pick(const double *cur, int n, int m, int ru
     return (r < 0) ? SPX_NOCONV : SPX_PIVOT;                                      // :138-139
 }
 
+__device__ __forceinline__ unsigned long long warp_min_key(unsigned long long v) {
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1) {
+        const unsigned long long o = __shfl_xor_sync(0xffffffffu, v, s);
+        v = o < v ? o : v;
+    }
+    return v;
+}
+
+// SPX_RULE_DANTZIG_BLAND's leaving row of column c by one warp (t: the target row, SPX_NONE in phase 2; cl: the row
+// labels); -1 when no row is a candidate, rk = its ratio key; warp-uniform
+__device__ __forceinline__ int warp_db_leave(const double *cur, int n, int m, int c, int t, const int32_t *cl, int lane,
+                                             unsigned long long &rk) {
+    const int w1 = m + 1;
+    unsigned long long k = ~0ull, s = ~0ull;
+    for (int i = lane; i < n; i += 32) db_leave_fold(k, s, i, cur[i * w1 + c], cur[i * w1 + m], t, cl[i]);
+    rk = warp_min_key(k);
+    s = warp_min_key(k == rk ? s : ~0ull);
+    return rk == ~0ull ? -1 : (int)(s & 0x7fffffffu);
+}
+
+// K1 + K2 under SPX_RULE_DANTZIG_BLAND by ONE warp on `cur` with its header labels rl and row labels cl: returns
+// SPX_PIVOT with (r, c) or the terminal status; warp-uniform
+__device__ __forceinline__ int warp_pick_db(const double *cur, int n, int m, const int32_t *rl, const int32_t *cl,
+                                            int lane, int &r, int &c) {
+    const int w1 = m + 1;
+    const int t = warp_first_index(n, lane, [&](int i) { return cur[i * w1 + m] < 0.0; });
+    const bool ph1 = t != SPX_NONE;
+    const double *e = cur + (ph1 ? t : n) * w1;           // phase 1: row t; phase 2: the f row
+    unsigned long long dk = ~0ull, bk = ~0ull;            // Dantzig's key and Bland's key of this lane's candidates
+    int dj = SPX_NONE;
+    for (int j = lane; j < m; j += 32) {
+        const double v = e[j];
+        if (ph1 ? v > 0.0 : v < 0.0) {
+            const unsigned long long k = ph1 ? db_pos_key(v) : orderable(v);
+            if (k < dk) { dk = k; dj = j; }
+            const unsigned long long b = db_label_key(rl[j], j);
+            bk = b < bk ? b : bk;
+        }
+    }
+    const unsigned long long g = warp_min_key(dk);
+    if (g == ~0ull) return ph1 ? SPX_INCORRECT : SPX_OPTIMAL;
+    c = __reduce_min_sync(0xffffffffu, dk == g ? dj : SPX_NONE);
+    unsigned long long rk;
+    r = warp_db_leave(cur, n, m, c, t, cl, lane, rk);
+    if (r >= 0 && rk == DB_ZERO_RATIO) {                   // a degenerate step: Bland's column and its leaving row
+        c = (int)(warp_min_key(bk) & 0xffffffffu);
+        r = warp_db_leave(cur, n, m, c, t, cl, lane, rk);
+    }
+    return r < 0 ? SPX_NOCONV : SPX_PIVOT;
+}
+
+// K1 + K2 of batched_solve / ragged_body: DB selects SPX_RULE_DANTZIG_BLAND, else warp_pick<DEVEX>
+template <bool DEVEX, bool DB>
+__device__ __forceinline__ int warp_pick_any(const double *cur, int n, int m, int rule, int lane, int &r, int &c,
+                                             const double *w, const int32_t *rl, const int32_t *cl) {
+    if constexpr (DB) return warp_pick_db(cur, n, m, rl, cl, lane, r, c);
+    else return warp_pick<DEVEX>(cur, n, m, rule, lane, r, c, w);
+}
+
 // CTA == false: one warp per LP, warps_per_cta LPs per CTA, __syncwarp between the phases
 //               (cfg1: 14 cells, cfg3: 26 cells — one cell per lane).
 // CTA == true : one CTA per LP for tables of hundreds of cells (Klee-Minty n=20: 440 cells, 2^20-1
@@ -173,7 +233,7 @@ __device__ __forceinline__ bool x_label(int lab, int m) {
 
 // DEVEX: the devex rule (SPX_RULE_DEVEX) with the weights in the LP's x slice, a.x[lp][0..m): set to 1 here, updated
 // by the warp that prices, after each pick, and overwritten by x in the epilogue.
-template <bool CTA, bool WARM, bool DEVEX = false>
+template <bool CTA, bool WARM, bool DEVEX = false, bool DB = false>
 __device__ __forceinline__ void batched_solve(const BatchedArgs &a, const double *function, int warps_per_cta,
                                               int warp_doubles) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -237,11 +297,11 @@ __device__ __forceinline__ void batched_solve(const BatchedArgs &a, const double
         }
         int r = -1, c = -1;
         if (!CTA) {
-            status = warp_pick<DEVEX>(cur, n, m, a.rule, lane, r, c, w);
+            status = warp_pick_any<DEVEX, DB>(cur, n, m, a.rule, lane, r, c, w, rl, cl);
             if (DEVEX && status == SPX_PIVOT) warp_devex_update(cur, w, m, r, c, lane);
         } else {
             if (warp == 0) {
-                const int st = warp_pick<DEVEX>(cur, n, m, a.rule, lane, r, c, w);
+                const int st = warp_pick_any<DEVEX, DB>(cur, n, m, a.rule, lane, r, c, w, rl, cl);
                 if (DEVEX && st == SPX_PIVOT) warp_devex_update(cur, w, m, r, c, lane);
                 if (lane == 0) { s_ctl[0] = st; s_ctl[1] = r; s_ctl[2] = c; }
             }
@@ -314,6 +374,13 @@ batched_devex_kernel(BatchedArgs a, const double *function, int warps_per_cta, i
     batched_solve<CTA, WARM, true>(a, function, warps_per_cta, warp_doubles);
 }
 
+// batched_kernel (WARM == false, function null) and batched_warm_kernel (WARM == true) under SPX_RULE_DANTZIG_BLAND
+template <bool CTA, bool WARM>
+__global__ void __launch_bounds__(CTA ? 512 : 256, CTA ? 1 : 6)
+batched_db_kernel(BatchedArgs a, const double *function, int warps_per_cta, int warp_doubles) {
+    batched_solve<CTA, WARM, false, true>(a, function, warps_per_cta, warp_doubles);
+}
+
 // One LP of a ragged batch, start to finish: batched_kernel's loop with the shape and the offsets taken from the LP's
 // descriptor `d`, by its group of nl threads (tl = index in the group): one warp (CTA == false) or the first nl
 // threads of the CTA (CTA == true).  base: its two tables, x, labels in shared memory.  In warp mode the warps of one
@@ -322,7 +389,7 @@ batched_devex_kernel(BatchedArgs a, const double *function, int warps_per_cta, i
 // (batched_kernel keeps its own copy of the loop: it runs at the 40-register cap of its launch bounds in warp mode,
 // and any restructuring of its code moves its spills.)  WARM: the resume, as batched_solve's; gd: LP lp's descriptor
 // in global memory (d is its copy).
-template <bool CTA, bool WARM, bool DEVEX>
+template <bool CTA, bool WARM, bool DEVEX, bool DB = false>
 __device__ __forceinline__ void ragged_body(const BatchedArgs &a, const RaggedLp &d, int64_t lp, const uint16_t *cell_i,
                                              const uint16_t *cell_j, double *base, int *s_ctl, int tl, int nl,
                                              const double *function, const RaggedLp *gd) {
@@ -374,11 +441,11 @@ __device__ __forceinline__ void ragged_body(const BatchedArgs &a, const RaggedLp
         }
         int r = -1, c = -1;
         if (!CTA) {
-            status = warp_pick<DEVEX>(cur, n, m, a.rule, lane, r, c, w);
+            status = warp_pick_any<DEVEX, DB>(cur, n, m, a.rule, lane, r, c, w, rl, cl);
             if (DEVEX && status == SPX_PIVOT) warp_devex_update(cur, w, m, r, c, lane);
         } else {
             if (warp == 0) {
-                const int st = warp_pick<DEVEX>(cur, n, m, a.rule, lane, r, c, w);
+                const int st = warp_pick_any<DEVEX, DB>(cur, n, m, a.rule, lane, r, c, w, rl, cl);
                 if (DEVEX && st == SPX_PIVOT) warp_devex_update(cur, w, m, r, c, lane);
                 if (lane == 0) { s_ctl[0] = st; s_ctl[1] = r; s_ctl[2] = c; }
             }
@@ -436,7 +503,7 @@ __device__ __forceinline__ void ragged_body(const BatchedArgs &a, const RaggedLp
 // bounds as batched_kernel<false>.  CTA mode: slot = CTA; the CTA is launched at the warp count of
 // the largest LP of the launch, builds the lookup table of its own LP, and only the warps its LP needs stay (the
 // warp count the uniform entry gives that shape: 32 cells per warp, 2..16 warps).
-template <bool CTA, bool WARM, bool DEVEX = false>
+template <bool CTA, bool WARM, bool DEVEX = false, bool DB = false>
 __device__ __forceinline__ void ragged_batched(const BatchedArgs &a, const RaggedLp *__restrict__ lps,
                                                const int32_t *__restrict__ order, int warps_per_cta, int warp_doubles,
                                                const double *function) {
@@ -460,7 +527,7 @@ __device__ __forceinline__ void ragged_batched(const BatchedArgs &a, const Ragge
         }
         __syncwarp();
         double *base = reinterpret_cast<double *>(slot_raw + WARP_LUT_BYTES);
-        ragged_body<false, WARM, DEVEX>(a, d, lp, cell_i, cell_j, base, s_ctl, lane, 32, function, lps + lp);
+        ragged_body<false, WARM, DEVEX, DB>(a, d, lp, cell_i, cell_j, base, s_ctl, lane, 32, function, lps + lp);
         return;
     }
     const int64_t lp = order[slot];
@@ -480,7 +547,7 @@ __device__ __forceinline__ void ragged_batched(const BatchedArgs &a, const Ragge
     if ((int)threadIdx.x >= nl) return;
     const size_t lut_bytes = ((size_t)cells * 4 + 15) / 16 * 16;
     double *base = reinterpret_cast<double *>(smem_raw + lut_bytes);
-    ragged_body<true, WARM, DEVEX>(a, d, lp, cell_i, cell_j, base, s_ctl, (int)threadIdx.x, nl, function, lps + lp);
+    ragged_body<true, WARM, DEVEX, DB>(a, d, lp, cell_i, cell_j, base, s_ctl, (int)threadIdx.x, nl, function, lps + lp);
 }
 
 template <bool CTA>
@@ -504,6 +571,15 @@ __global__ void __launch_bounds__(CTA ? 512 : 256, CTA ? 1 : 6)
 ragged_batched_devex_kernel(BatchedArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
                             int warps_per_cta, int warp_doubles, const double *function) {
     ragged_batched<CTA, WARM, true>(a, lps, order, warps_per_cta, warp_doubles, function);
+}
+
+// ragged_batched_kernel (WARM == false, function null) and ragged_batched_warm_kernel (WARM == true) under
+// SPX_RULE_DANTZIG_BLAND
+template <bool CTA, bool WARM>
+__global__ void __launch_bounds__(CTA ? 512 : 256, CTA ? 1 : 6)
+ragged_batched_db_kernel(BatchedArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
+                         int warps_per_cta, int warp_doubles, const double *function) {
+    ragged_batched<CTA, WARM, false, true>(a, lps, order, warps_per_cta, warp_doubles, function);
 }
 
 size_t warp_bytes(int n, int m) {
@@ -573,6 +649,9 @@ cudaError_t solve_batched(int64_t B, int n, int m, int max_pivots, const BatchIO
         if (io.rule == SPX_RULE_DEVEX)
             return io.warm ? launch_k4<batched_devex_kernel<true, true>>(B, warps * 32, lb + wb, stream, a, io.function, 1, wd)
                            : launch_k4<batched_devex_kernel<true, false>>(B, warps * 32, lb + wb, stream, a, nullptr, 1, wd);
+        if (io.rule == SPX_RULE_DANTZIG_BLAND)
+            return io.warm ? launch_k4<batched_db_kernel<true, true>>(B, warps * 32, lb + wb, stream, a, io.function, 1, wd)
+                           : launch_k4<batched_db_kernel<true, false>>(B, warps * 32, lb + wb, stream, a, nullptr, 1, wd);
         if (io.warm) return launch_k4<batched_warm_kernel<true>>(B, warps * 32, lb + wb, stream, a, io.function, 1, wd);
         return launch_k4<batched_kernel<true>>(B, warps * 32, lb + wb, stream, a, 1, wd);
     }
@@ -587,6 +666,9 @@ cudaError_t solve_batched(int64_t B, int n, int m, int max_pivots, const BatchIO
     if (io.rule == SPX_RULE_DEVEX)
         return io.warm ? launch_k4<batched_devex_kernel<false, true>>(ctas, wpc * 32, smem, stream, a, io.function, wpc, wd)
                        : launch_k4<batched_devex_kernel<false, false>>(ctas, wpc * 32, smem, stream, a, nullptr, wpc, wd);
+    if (io.rule == SPX_RULE_DANTZIG_BLAND)
+        return io.warm ? launch_k4<batched_db_kernel<false, true>>(ctas, wpc * 32, smem, stream, a, io.function, wpc, wd)
+                       : launch_k4<batched_db_kernel<false, false>>(ctas, wpc * 32, smem, stream, a, nullptr, wpc, wd);
     if (io.warm) return launch_k4<batched_warm_kernel<false>>(ctas, wpc * 32, smem, stream, a, io.function, wpc, wd);
     return launch_k4<batched_kernel<false>>(ctas, wpc * 32, smem, stream, a, wpc, wd);
 }
@@ -631,6 +713,17 @@ cudaError_t solve_ragged_batched(const PlanView &v, const RaggedLaunch &l, const
                                                                             order, l.per_cta, (int)l.slot_doubles, fn)
                        : launch_k4<ragged_batched_devex_kernel<false, false>>(ctas, l.threads, smem, stream, a, v.d_lps,
                                                                              order, l.per_cta, (int)l.slot_doubles, fn);
+    }
+    if (io.rule == SPX_RULE_DANTZIG_BLAND) {
+        if (l.kernel == RAGGED_CTA)
+            return io.warm ? launch_k4<ragged_batched_db_kernel<true, true>>(ctas, l.threads, smem, stream, a, v.d_lps,
+                                                                            order, 1, 0, fn)
+                           : launch_k4<ragged_batched_db_kernel<true, false>>(ctas, l.threads, smem, stream, a, v.d_lps,
+                                                                             order, 1, 0, fn);
+        return io.warm ? launch_k4<ragged_batched_db_kernel<false, true>>(ctas, l.threads, smem, stream, a, v.d_lps,
+                                                                         order, l.per_cta, (int)l.slot_doubles, fn)
+                       : launch_k4<ragged_batched_db_kernel<false, false>>(ctas, l.threads, smem, stream, a, v.d_lps,
+                                                                          order, l.per_cta, (int)l.slot_doubles, fn);
     }
     if (l.kernel == RAGGED_CTA)
         return io.warm ? launch_k4<ragged_batched_warm_kernel<true>>(ctas, l.threads, smem, stream, a, v.d_lps, order,

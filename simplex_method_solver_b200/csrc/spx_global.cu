@@ -52,7 +52,7 @@ __device__ __forceinline__ double2 ld_l2_v2(const double *p) {
 // The body of both kernels.  RAGGED == false: shape, R, Q and offsets from the arguments (one shape per launch).
 // RAGGED == true: LP order[blockIdx.x / S] of a ragged batch, its shape and offsets from lps[], R and Q from its shape
 // (as cluster_body in spx_cluster.cu).  WARM == true: a resume, as cluster_body's.
-template <bool RAGGED, bool WARM, bool DEVEX = false>
+template <bool RAGGED, bool WARM, bool DEVEX = false, bool DB = false>
 __device__ __forceinline__ void global_body(const ClusterArgs &a, const RaggedLp *__restrict__ lps,
                                             const int32_t *__restrict__ order, const double *function) {
     cg::cluster_group cluster = cg::this_cluster();
@@ -120,47 +120,54 @@ __device__ __forceinline__ void global_body(const ClusterArgs &a, const RaggedLp
             for (int64_t k = tid; k < bandcells; k += nt) sg[(int64_t)r0 * w1 + k] = ld_l2(band + k);
             if (rank == 0) for (int j = tid; j < m; j += nt) sg[fo + j] = f[j];
         }
-        // ---- K1: entering column of the f row (:94-98), the same in every CTA
-        int cf;
-        if constexpr (DEVEX) {
-            if (dv.c >= 0) dv.wc = ld_l2(wg + dv.c);
-            cf = devex_entering(f, m, [&](int j) { return devex_weight_now(wg, prow, dv, j); }, sc);
+        int r, c;
+        if constexpr (DB) {                                // the rounds of cluster_db_pick (spx_cluster.cuh)
+            status = cluster_db_pick(cluster, f, m, S, r0, rows, j0, cols, rl, cl, sc,
+                                     [&](int i, int j) { return ld_l2(band + (int64_t)i * w1 + j); },
+                                     [&](int t, int j) { return ld_l2(Tg + (int64_t)t * w1 + j); }, r, c);
         } else {
-            cf = f_row_entering(f, m, a.rule, sc);
-        }
-        // ---- one pass over the band's rows: phase-1 row (:72-76) and the ratio scan of column cf (:107-136)
-        Ratio q = ratio_identity();
-        int key = SPX_NONE, bneg = SPX_NONE;
-        for (int i = tid; i < rows; i += nt) {
-            const double *row = band + (int64_t)i * w1;
-            const double b_i = ld_l2(row + m);
-            if (b_i < 0.0) bneg = min(bneg, i);
-            if (cf != SPX_NONE) {
-                const bool first = (q.elig_row == SPX_NONE);
-                const bool is_nan = ratio_accumulate(q, r0 + i, ld_l2(row + cf), b_i);
-                if (first && q.elig_row != SPX_NONE) key = 2 * (r0 + i) + (is_nan ? 1 : 0);
+            // ---- K1: entering column of the f row (:94-98), the same in every CTA
+            int cf;
+            if constexpr (DEVEX) {
+                if (dv.c >= 0) dv.wc = ld_l2(wg + dv.c);
+                cf = devex_entering(f, m, [&](int j) { return devex_weight_now(wg, prow, dv, j); }, sc);
+            } else {
+                cf = f_row_entering(f, m, a.rule, sc);
             }
-        }
-        block_min_int2(bneg, key, sc);
-        if (cf != SPX_NONE) q = block_ratio_reduce(q, sc);
-        int bcol = SPX_NONE;                               // first positive cell of the phase-1 row (:81-85)
-        if (bneg != SPX_NONE) {
-            const double *row = band + (int64_t)bneg * w1;
-            bcol = block_first_index_fn(m, [row](int j) { return ld_l2(row + j); }, IsPos(), sc);
-        }
-        if (tid == 0) {
-            s_part.q = q;
-            s_part.elig_key = key;
-            s_part.bneg_row = (bneg == SPX_NONE) ? SPX_NONE : r0 + bneg;
-            s_part.bneg_col = bcol;
-        }
-        cluster.sync();                                    // A: every partial is published; the pivot row is final
+            // ---- one pass over the band's rows: phase-1 row (:72-76) and the ratio scan of column cf (:107-136)
+            Ratio q = ratio_identity();
+            int key = SPX_NONE, bneg = SPX_NONE;
+            for (int i = tid; i < rows; i += nt) {
+                const double *row = band + (int64_t)i * w1;
+                const double b_i = ld_l2(row + m);
+                if (b_i < 0.0) bneg = min(bneg, i);
+                if (cf != SPX_NONE) {
+                    const bool first = (q.elig_row == SPX_NONE);
+                    const bool is_nan = ratio_accumulate(q, r0 + i, ld_l2(row + cf), b_i);
+                    if (first && q.elig_row != SPX_NONE) key = 2 * (r0 + i) + (is_nan ? 1 : 0);
+                }
+            }
+            block_min_int2(bneg, key, sc);
+            if (cf != SPX_NONE) q = block_ratio_reduce(q, sc);
+            int bcol = SPX_NONE;                               // first positive cell of the phase-1 row (:81-85)
+            if (bneg != SPX_NONE) {
+                const double *row = band + (int64_t)bneg * w1;
+                bcol = block_first_index_fn(m, [row](int j) { return ld_l2(row + j); }, IsPos(), sc);
+            }
+            if (tid == 0) {
+                s_part.q = q;
+                s_part.elig_key = key;
+                s_part.bneg_row = (bneg == SPX_NONE) ? SPX_NONE : r0 + bneg;
+                s_part.bneg_col = bcol;
+            }
+            cluster.sync();                                    // A: every partial is published; the pivot row is final
 
-        // ---- decision: each CTA merges the S partials itself
-        if (tid < 32) cluster_decide(cluster, &s_part, S, cf, s_ctl);
-        __syncthreads();
-        status = s_ctl[0];
-        const int r = s_ctl[1], c = s_ctl[2];
+            // ---- decision: each CTA merges the S partials itself
+            if (tid < 32) cluster_decide(cluster, &s_part, S, cf, s_ctl);
+            __syncthreads();
+            status = s_ctl[0];
+            r = s_ctl[1]; c = s_ctl[2];
+        }
         if (status != SPX_PIVOT) break;
         if (npiv >= (RAGGED ? lpd.max_pivots : a.max_pivots)) { status = SPX_CAP; break; }
 
@@ -307,6 +314,15 @@ global_devex_kernel(ClusterArgs a, const RaggedLp *__restrict__ lps, const int32
     global_body<RAGGED, WARM, true>(a, lps, order, function);
 }
 
+// the four kernels above under SPX_RULE_DANTZIG_BLAND: RAGGED as the ragged_ ones, WARM as the _warm_ ones (function
+// null for a fresh solve)
+template <bool RAGGED, bool WARM>
+__global__ void __launch_bounds__(CLUSTER_THREADS, GLOBAL_MIN_CTAS)
+global_db_kernel(ClusterArgs a, const RaggedLp *__restrict__ lps, const int32_t *__restrict__ order,
+                 const double *function) {
+    global_body<RAGGED, WARM, false, true>(a, lps, order, function);
+}
+
 // the per-CTA footprint of the header comment, for S CTAs per LP
 int64_t global_bytes(int64_t n, int64_t m, int S) {
     const int64_t R = (n + S - 1) / S, Q = (m + S - 1) / S;
@@ -374,6 +390,11 @@ cudaError_t solve_batched_global(int64_t B, int n, int m, int S, int max_pivots,
                                                                                 nullptr, nullptr, io.function)
                        : launch_cluster_kernel<global_devex_kernel<false, false>>(S, B, global_bytes(n, m, S), stream, a,
                                                                                  nullptr, nullptr, nullptr);
+    if (io.rule == SPX_RULE_DANTZIG_BLAND)
+        return io.warm ? launch_cluster_kernel<global_db_kernel<false, true>>(S, B, global_bytes(n, m, S), stream, a,
+                                                                             nullptr, nullptr, io.function)
+                       : launch_cluster_kernel<global_db_kernel<false, false>>(S, B, global_bytes(n, m, S), stream, a,
+                                                                              nullptr, nullptr, nullptr);
     if (io.warm) return launch_cluster_kernel<global_warm_kernel>(S, B, global_bytes(n, m, S), stream, a, io.function);
     return launch_cluster_kernel<global_kernel>(S, B, global_bytes(n, m, S), stream, a);
 }
@@ -405,6 +426,11 @@ cudaError_t solve_ragged_global(const PlanView &v, const RaggedLaunch &l, int S,
                                                                                io.function)
                        : launch_cluster_kernel<global_devex_kernel<true, false>>(S, l.count, smem, stream, a, v.d_lps,
                                                                                 order, nullptr);
+    if (io.rule == SPX_RULE_DANTZIG_BLAND)
+        return io.warm ? launch_cluster_kernel<global_db_kernel<true, true>>(S, l.count, smem, stream, a, v.d_lps, order,
+                                                                            io.function)
+                       : launch_cluster_kernel<global_db_kernel<true, false>>(S, l.count, smem, stream, a, v.d_lps,
+                                                                             order, nullptr);
     if (io.warm)
         return launch_cluster_kernel<ragged_global_warm_kernel>(S, l.count, smem, stream, a, v.d_lps, order,
                                                                 io.function);

@@ -175,9 +175,10 @@ int spx_shard_open(spx_shard **out, int32_t rank, int32_t nranks, int32_t n, int
                 rank, nranks);
     SPX_REQUIRE(n >= 1 && m_loc >= 0 && ld_loc >= 16 && ld_loc % 16 == 0 && ld_loc >= m_loc && col0 >= 0,
                 "spx_shard_open: bad shape");
-    SPX_REQUIRE(rule != SPX_RULE_DEVEX, "spx_shard_open: rule SPX_RULE_DEVEX is a rule of the batched entries only "
-                "(spx_solve_batched, spx_solve_batched_cluster, spx_solve_batched_global, spx_solve_batched_ragged, "
-                "spx_warm_solve_batched, spx_warm_solve_ragged)");
+    SPX_REQUIRE(rule != SPX_RULE_DEVEX && rule != SPX_RULE_DANTZIG_BLAND, "spx_shard_open: rule %s is a rule of the "
+                "batched entries only (spx_solve_batched, spx_solve_batched_cluster, spx_solve_batched_global, "
+                "spx_solve_batched_ragged, spx_warm_solve_batched, spx_warm_solve_ragged)",
+                rule == SPX_RULE_DEVEX ? "SPX_RULE_DEVEX" : "SPX_RULE_DANTZIG_BLAND");
     SPX_REQUIRE(rule == SPX_RULE_REFERENCE || rule == SPX_RULE_DANTZIG, "spx_shard_open: unknown rule %d", rule);
     spx_shard *h = new (std::nothrow) spx_shard();
     SPX_REQUIRE(h, "spx_shard_open: out of host memory");

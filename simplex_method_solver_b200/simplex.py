@@ -100,6 +100,12 @@ class SimplexMethod:
             # so the pivots would depend on the round sizes
             raise ValueError("rule='devex' is a rule of the batched API only: batched.solve_batched, "
                              "batched.solve_ragged, batched.resolve, DeviceBatch and DeviceRaggedBatch")
+        if rule == "dantzig_bland":
+            # Bland's column is the lowest label, and get_solution()'s rounds restart the labels at x1.. / y1..
+            raise ValueError("rule='dantzig_bland' is a rule of the batched API only (batched.solve_batched, "
+                             "batched.solve_ragged, batched.resolve, DeviceBatch and DeviceRaggedBatch): it chooses "
+                             "by label, and SimplexMethod.get_solution() runs fresh batched rounds that restart the "
+                             "labels at x1.. / y1..")
         if rule not in N.RULES:
             raise ValueError(f"unknown rule {rule!r}")
         if engine not in ("auto", "warp", "stream", "sharded", "cluster", "global"):
